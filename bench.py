@@ -2,7 +2,8 @@
 """Benchmark of the embedding-vs-gallery matching path (BASELINE.json metric: face queries/s at a
 1 M x 512 gallery, top-5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch F] ...
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch F]
+                    [--dump-outputs DIR] ...
 
 One "step" = one batch of F query embeddings matched against the whole resident gallery
 (normalise -> scan -> top-k -> threshold).  Prints ONE JSON line (see DESIGN.md "Measurement").
@@ -284,7 +285,7 @@ def ours_arm(args, rank, world):
                  torch.empty((F,), dtype=torch.uint8, device=dev)) for _ in range(nb)]
         return Qh, Qd, outs
 
-    def time_device(F, steps, warmup, Qd, outs, clocks=False, preload_s=None):
+    def time_device(F, steps, warmup, Qd, outs, clocks=False, preload_s=None, keep_last=False):
         preload_s = args.clock_preload_s if preload_s is None else preload_s
         def step(i):
             if sharded:
@@ -341,6 +342,8 @@ def ours_arm(args, rank, world):
         total_ms = ev0.elapsed_time(ev1)
         dom_ms, dom_launches = N.profile_collect()
         ck = sampler.stop() if sampler else None
+        # the passes below reuse the output buffers: copy the last timed step's results out first
+        last = [x.cpu().numpy() for x in outs[(steps - 1) % nb]] if keep_last else None
         # per-stage split (untimed for `value`): every stage bracketed, a few steps
         N.check(N.lib.frg_profile_enable(1))
         nsplit = max(5, min(steps, 30))
@@ -370,12 +373,14 @@ def ours_arm(args, rank, world):
         return {"batch": F, "value": F * scale / (ms * 1e-3), "ms_per_step": ms, "variant": variant,
                 "launches_per_step": launches_per_step, "dom_ms": dom_ms, "dom_launches": dom_launches,
                 "dom_steps": (steps + 3) // 4,          # steps whose dominant kernel was bracketed
-                "total_ms": total_ms, "clocks": ck, "stage_ms": stages, "step_ms_spread": spread}
+                "total_ms": total_ms, "clocks": ck, "stage_ms": stages, "step_ms_spread": spread, "last": last}
 
     # ---- headline batch: device-timed region
     F = args.batch
     Qh, Qd, outs = make_batches(F)
-    main = time_device(F, args.steps, args.warmup, Qd, outs, clocks=True)
+    main = time_device(F, args.steps, args.warmup, Qd, outs, clocks=True, keep_last=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *main["last"])
     variant = main["variant"]
     clocks = main["clocks"]
     peaks["use_sustained"] = power_capped(clocks)
@@ -875,6 +880,31 @@ def emit_json(obj):
         os.write(_REAL_STDOUT, data)
 
 
+DUMP_LIMIT_BYTES = 60 << 20          # data bytes: the files stay under 64 MB (10^6 or 2^20) with their headers
+
+
+def dump_outputs(path, rows, scores, accept):
+    """--dump-outputs: what the last timed step handed its caller, one DIR/<name>.npy per array, so that two
+    builds run with the same arguments (hence the same inputs) can be compared output for output.
+
+      rows.npy         float64 [F, k]  gallery rows, best first (-1: no row)
+      scores.npy       float32 [F, k]
+      accept.npy       float32 [F]     1 = the best score reaches the threshold
+      query_index.npy  float64 [F]     position of each written query in the batch
+
+    Where the whole batch would pass DUMP_LIMIT_BYTES, a fixed seeded sample of the queries is written, in batch
+    order."""
+    F = len(rows)
+    per_query = rows.shape[1] * (8 + 4) + 4 + 8
+    keep = np.arange(F)
+    if F * per_query > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(F, DUMP_LIMIT_BYTES // per_query, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("rows", rows[keep].astype(np.float64)), ("scores", scores[keep].astype(np.float32)),
+                    ("accept", accept[keep].astype(np.float32)), ("query_index", keep.astype(np.float64))):
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def ncu_traffic(variant, n, dim, F, world):
     """dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernel, from the ncu --set full
     capture committed under profiles/ (only when it was taken on this very workload), else None."""
@@ -966,7 +996,14 @@ def main():
     ap.add_argument("--no-check", action="store_true")
     ap.add_argument("--cpu-procs", type=int, default=0)
     ap.add_argument("--cpu-queries", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rows, scores and accept decisions of the last timed step as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
