@@ -10,13 +10,13 @@ from . import _native
 from ._native import NativeError
 from .gallery import GalleryStore, StaleRows
 from .matcher import (CAMPUS_THRESHOLD, CAMPUS_UNKNOWN, LIVE_THRESHOLD, CameraProcessor,
-                      FaceRecognitionProcessor, Matcher, MatchResult)
+                      FaceRecognitionProcessor, Matcher, MatchResult, RangeResult)
 from .manager import BroadcastSource, EmbeddingManager, GalleryView, ListSource
-from .enrol import EnrolmentChecker, EnrolmentGallery
+from .enrol import EnrolmentChecker, EnrolmentGallery, find_duplicate_pairs
 from .clustering import UnknownClusterer
 from .aggregator import BatchAggregator
 
-__all__ = ["GalleryStore", "Matcher", "MatchResult", "FaceRecognitionProcessor", "CameraProcessor",
+__all__ = ["GalleryStore", "Matcher", "MatchResult", "RangeResult", "find_duplicate_pairs", "FaceRecognitionProcessor", "CameraProcessor",
            "EmbeddingManager", "GalleryView", "ListSource", "BroadcastSource", "EnrolmentChecker", "EnrolmentGallery", "StaleRows", "UnknownClusterer",
            "BatchAggregator", "NativeError", "LIVE_THRESHOLD",
            "CAMPUS_THRESHOLD", "CAMPUS_UNKNOWN"]

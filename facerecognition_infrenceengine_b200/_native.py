@@ -76,6 +76,8 @@ SIGNATURES = {
     "frg_match_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
     "frg_first_match": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
     "frg_first_match_host": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), _P, _P]),
+    "frg_match_range": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
+    "frg_match_range_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
     "frg_merge_topk": (C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                  C.c_float, _P, _P, _P, _P]),
     "frg_merge_topk_strided": (C.c_int, [C.c_int32, _P, C.c_int64, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32,

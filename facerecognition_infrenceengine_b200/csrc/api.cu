@@ -1105,6 +1105,143 @@ int frg_first_match_host(frg_store* s, const float* q, int32_t nq, const frg_mat
   return rc;
 }
 
+// --------------------------------------------------------------------------------------------- range search
+// Tensor-core path (unit cosine stores with a plane and a covered dim): query prep (fp32 unit queries, bf16 image,
+// eps[q]) -> filter with the fixed floor threshold - eps[q] -> range_select_kernel -> exact range scan of the
+// queries whose candidates overflowed.  Everything else: the exact range scan over all queries.
+static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
+                      int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  reset_launches();
+  if (!s || !p || nq < 0 || (nq > 0 && (!q || !out_counts || !out_rows || !out_scores))) {
+    set_error("match_range: bad argument");
+    return FRG_ERR_INVALID;
+  }
+  if (max_hits < 1) { set_error("match_range: max_hits=%d must be >= 1", max_hits); return FRG_ERR_INVALID; }
+  if (p->metric != FRG_METRIC_COSINE && p->metric != FRG_METRIC_EUCLIDEAN) { set_error("match_range: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
+  if (p->variant < FRG_VARIANT_AUTO || p->variant > FRG_VARIANT_TC_BF16) { set_error("match_range: unknown variant %d", p->variant); return FRG_ERR_INVALID; }
+  if (p->variant == FRG_VARIANT_TC_BF16) {
+    set_error("match_range: FRG_VARIANT_TC_BF16 has no exact scores to hold against the threshold (use AUTO, TC_EXACT or SCAN_F32)");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  if (!s->master) { set_error("match_range: a bf16-only store has no fp32 master for the exact scores"); return FRG_ERR_UNSUPPORTED; }
+  if (p->variant == FRG_VARIANT_TC_EXACT && p->metric == FRG_METRIC_EUCLIDEAN) {
+    set_error("match_range: the Euclidean range search runs on the exact scan only (FRG_VARIANT_SCAN_F32 / AUTO)");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  const char* why = "";
+  if (!range_scan_supported(s->dim, &why)) { set_error("match_range: %s", why); return FRG_ERR_UNSUPPORTED; }
+  const bool unit = !(s->flags & FRG_STORE_RAW) && !(p->flags & FRG_QUERY_PRENORMALISED);
+  const bool tc_ok = s->plane != nullptr && unit && p->metric == FRG_METRIC_COSINE && tc_supported(s->dim, p->metric, &why);
+  const bool use_tc = p->variant == FRG_VARIANT_TC_EXACT || (p->variant == FRG_VARIANT_AUTO && tc_ok);
+  if (use_tc && !tc_ok) {
+    set_error("match_range: FRG_VARIANT_TC_EXACT needs a unit-row store with a scan plane, normalised queries and "
+              "dim 128 / 256 / 512");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  if (nq == 0) return FRG_OK;
+  DeviceGuard g(s->device);
+  if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
+  DeviceInfo di;
+  FRG_CHECK(device_info(s->device, &di));
+  std::lock_guard<std::mutex> lk(s->mu);
+  FRG_CHECK(store_begin_read(s, st));
+  const GalleryWindow w = window_of(s, p->tenant, use_tc);
+  if (w.rows > 0x7fffffff) { set_error("match_range: more than 2^31-1 rows in one shard"); return FRG_ERR_UNSUPPORTED; }
+  const int64_t row_offset = p->row_offset + w.row0;
+  const bool strict = (p->flags & FRG_FIRST_STRICT) != 0;
+  ScanArgs a;
+  a.master = w.master; a.plane = w.plane; a.tags = w.tags; a.rows = w.rows; a.dim = w.dim;
+  a.nq = nq; a.k = 1; a.metric = p->metric; a.tenant = p->tenant; a.sm_count = di.sm_count;
+  const size_t qn_bytes = (size_t(nq) * w.dim * sizeof(float) + 255) & ~size_t(255);
+  unsigned char* ws = nullptr;
+  int rc = FRG_OK;
+  if (use_tc && w.rows > 0) {
+    const size_t qb_bytes = (size_t(nq) * w.dim * sizeof(__nv_bfloat16) + 255) & ~size_t(255);
+    const size_t eps_bytes = (size_t(nq) * sizeof(float) + 255) & ~size_t(255);
+    const int32_t* tile_list = nullptr;
+    int n_list = 0;
+    const int64_t plan_rows = tc_effective_rows(&w, nq, st, &tile_list, &n_list);
+    if (plan_rows < 0) return FRG_ERR_CUDA;
+    const size_t tc_bytes = tc_workspace_bytes(plan_rows, w.dim, nq, 1, di.sm_count, true);
+    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + qb_bytes + eps_bytes + tc_bytes, st));
+    float* qn = reinterpret_cast<float*>(ws);
+    __nv_bfloat16* qb = reinterpret_cast<__nv_bfloat16*>(ws + qn_bytes);
+    float* eps = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes);
+    unsigned char* tc_ws = ws + qn_bytes + qb_bytes + eps_bytes;
+    uint32_t* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
+    tc_workspace_init_targets(plan_rows, w.dim, nq, 1, di.sm_count, tc_ws, &keys, &ct0, &nf0, true);
+    int* flagged = nullptr; int* n_flagged = nullptr;
+    profile_begin(st, kStagePrep);
+    rc = launch_normalise_queries(q, nq, w.dim, true, qn, qb, keys, ct0, nf0, st, eps, s->gmax_bits);
+    profile_end(st, 1);
+    if (rc == FRG_OK)
+      rc = launch_tc_range(&w, qn, qb, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, tc_ws,
+                           di.sm_count, out_counts, out_rows, out_scores, &flagged, &n_flagged, st, plan_rows,
+                           tile_list, n_list);
+    if (rc == FRG_OK) {
+      a.qn = qn;
+      profile_begin(st, kStageFallback);
+      rc = launch_range_scan(a, flagged, n_flagged, max_hits, p->threshold, strict, row_offset, out_counts,
+                             out_rows, out_scores, st);
+      profile_end(st, 1);
+    }
+    g_variant = "range_tc";
+  } else {
+    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes, st));
+    float* qn = reinterpret_cast<float*>(ws);
+    a.qn = qn;
+    rc = launch_normalise_queries(q, nq, w.dim, p->metric == FRG_METRIC_COSINE && !(p->flags & FRG_QUERY_PRENORMALISED),
+                                  qn, nullptr, nullptr, nullptr, nullptr, st);
+    profile_begin(st, kStageDominant);
+    if (rc == FRG_OK)
+      rc = launch_range_scan(a, nullptr, nullptr, max_hits, p->threshold, strict, row_offset, out_counts, out_rows,
+                             out_scores, st);
+    profile_end(st, 3);
+    g_variant = "range_scan";
+  }
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
+int frg_match_range(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
+                    int64_t* out_counts, int64_t* out_rows, float* out_scores, void* stream) {
+  return range_impl(s, q, nq, max_hits, p, out_counts, out_rows, out_scores, static_cast<cudaStream_t>(stream));
+}
+
+int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
+                         int64_t* out_counts, int64_t* out_rows, float* out_scores) {
+  if (!s || !p || nq < 0 || (nq > 0 && (!q || !out_counts || !out_rows || !out_scores)) || max_hits < 1) {
+    // the device entry point names the argument
+    return range_impl(s, q, nq, max_hits, p, out_counts, out_rows, out_scores, nullptr);
+  }
+  if (nq == 0) return range_impl(s, q, nq, max_hits, p, out_counts, out_rows, out_scores, nullptr);
+  DeviceGuard g(s->device);
+  cudaStream_t st = cudaStreamPerThread;
+  const size_t slots = size_t(nq) * size_t(max_hits);
+  const size_t qb = size_t(nq) * s->dim * sizeof(float), cb = size_t(nq) * sizeof(int64_t);
+  const size_t o_c = (qb + 255) & ~size_t(255), o_r = (o_c + cb + 255) & ~size_t(255),
+               o_s = (o_r + slots * sizeof(int64_t) + 255) & ~size_t(255);
+  unsigned char* d = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), o_s + slots * sizeof(float), st));
+  int rc = FRG_OK;
+  cudaError_t e = cudaMemcpyAsync(d, q, qb, cudaMemcpyHostToDevice, st);
+  if (e != cudaSuccess) rc = cuda_fail(e, "H2D queries", __FILE__, __LINE__);
+  if (rc == FRG_OK)
+    rc = range_impl(s, reinterpret_cast<float*>(d), nq, max_hits, p, reinterpret_cast<int64_t*>(d + o_c),
+                    reinterpret_cast<int64_t*>(d + o_r), reinterpret_cast<float*>(d + o_s), st);
+  if (rc == FRG_OK) {
+    e = cudaMemcpyAsync(out_counts, d + o_c, cb, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_rows, d + o_r, slots * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_scores, d + o_s, slots * sizeof(float), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) rc = cuda_fail(e, "D2H results", __FILE__, __LINE__);
+    else rc = store_fault(s);
+  }
+  cudaFreeAsync(d, st);
+  return rc;
+}
+
 int frg_merge_topk(int32_t device, const float* scores, const int64_t* rows, int32_t parts,
                    int32_t nq, int32_t k, int32_t metric, float threshold,
                    int64_t* out_rows, float* out_scores, uint8_t* out_accept, void* stream) {

@@ -323,9 +323,10 @@ constexpr int kEuclidPad = 16;      // plane: one more 32-byte group of k (one U
 constexpr int kEuclidQPad = 64;     // query image: padded to a whole 128-byte swizzle row (the tile's k-block)
 constexpr float kEuclidNone = -3.0e38f;   // "no score yet" of the Euclidean filter (scores are unbounded below)
 int tc_supported(int dim, int metric, const char** why);
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count);
+// range: the plan of launch_tc_range (k is ignored there)
+size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range = false);
 void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               uint32_t** keys, int** cand_total, int** n_flagged);
+                               uint32_t** keys, int** cand_total, int** n_flagged, bool range = false);
 // metric cosine: qb = [nq][dim] bf16 unit queries, eps == nullptr (constant bound).
 // metric euclidean: qb = [nq][dim + kEuclidQPad] augmented image, eps[nq] per-query bounds.
 // push: the select stage sends every query's final top-k straight to all ranks (XPush::peer_bufs != null)
@@ -335,6 +336,24 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
                     uint8_t* out_accept, int** flagged_out, int** n_flagged_out, cudaStream_t st,
                     int64_t plan_rows, const int32_t* tile_list, int n_list,
                     const __nv_bfloat16* qb_prepass = nullptr, const float* coef = nullptr);
+
+// tc_match.cu: range search over a unit cosine store (frg_match_range).  The filter keeps every row with
+// S >= threshold - eps[q] (no pre-pass); range_select_kernel rescores each candidate exactly, keeps those that pass
+// (score >= threshold, '>' when strict), writes the first max_hits in gallery order and the count.  Queries whose
+// candidates overflowed the plan are left in (flagged, n_flagged) for launch_range_scan's flagged mode.
+int launch_tc_range(const GalleryWindow* s, const float* qn, const __nv_bfloat16* qb, const float* eps, int nq,
+                    int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned char* ws,
+                    int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores, int** flagged_out,
+                    int** n_flagged_out, cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list);
+
+// scan_f32.cu: exact, counting range scan.  Pass 1: every warp owns a contiguous row range and counts its hits per
+// query; a per-query exclusive scan over the warp counts gives the total and each warp's output offset; pass 2: the
+// warps whose offset is below max_hits recompute and write their hits in row order.  flagged == nullptr: all nq
+// queries; else only the n_flagged[0] listed ones (device-side count, the tensor-core path's overflow fallback).
+int range_scan_supported(int dim, const char** why);
+int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagged, int max_hits, float threshold,
+                      bool strict, int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                      cudaStream_t st);
 
 // first_match.cu
 int launch_first_match(const float* master, const int32_t* tags, int64_t rows, int dim, const float* qn, int nq,

@@ -526,4 +526,212 @@ int launch_scan_f32_flagged(const ScanArgs& a, const int* flagged, int* ctl, int
   return rc;
 }
 
+
+// ------------------------------------------------------------------------------------------ range search
+// Exact, counting range scan (frg_match_range: the SCAN_F32 variant over all queries, and the tensor-core path's
+// fallback over the flagged ones).  Deterministic and sort-free: warp gw of W owns the contiguous rows
+// [gw * rows / W, (gw + 1) * rows / W), so the concatenation of the warps' hits in warp order IS gallery order.
+//   pass 1 (range_count_kernel):  per (query, warp) hit count -> cnt[slot][W]
+//   range_offsets_kernel:         per query, exclusive scan over the W counts -> off[slot][W], total -> out_counts;
+//                                 the slots past min(total, max_hits) get the "none" marker
+//   pass 2 (range_write_kernel):  a warp with hits whose offset is below max_hits recomputes its rows and writes
+//                                 its hits at off, off + 1, ... (row order) while they are below max_hits
+// Scores come from row_dots + butterfly, the arithmetic of scan_pass: bit-identical to the other exact paths.
+// Queries are taken QB at a time (slot = position in `flagged`, or the query itself); the number of slots is read
+// on the device, so with nothing flagged every launch exits at once.
+__device__ __forceinline__ int64_t range_warp_row(int64_t rows, int64_t w, int64_t nw) { return rows * w / nw; }
+
+template <int METRIC>
+__device__ __forceinline__ bool range_pass(float sdot, float threshold, int strict) {
+  if (METRIC == FRG_METRIC_COSINE) return strict ? (sdot > threshold) : (sdot >= threshold);   // false for NaN
+  const float d = __fsqrt_rn(sdot);                                                            // sdot = d^2 >= 0
+  return strict ? (d < threshold) : (d <= threshold);
+}
+
+template <int NJ, int QB, int METRIC, bool WRITE>
+__global__ void __launch_bounds__(kScanWarps * 32, 2)
+range_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ tags, int64_t rows,
+                  const float* __restrict__ qn, int nq, const int* __restrict__ flagged,
+                  const int* __restrict__ n_flagged, int32_t tenant, float threshold, int strict, int max_hits,
+                  int64_t row_offset, int* __restrict__ cnt, const int* __restrict__ off,
+                  int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
+  constexpr int DIM = NJ * 128;
+  pdl_wait();
+  pdl_trigger();
+  const int n_slots = flagged ? *n_flagged : nq;
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = int64_t(gridDim.x) * kScanWarps;
+  const int64_t gw = int64_t(blockIdx.x) * kScanWarps + (threadIdx.x >> 5);
+  const int64_t r0 = range_warp_row(rows, gw, nw), r1 = range_warp_row(rows, gw + 1, nw);
+  const int my_b = lane_query<QB>(lane);
+  const bool rep = lane_is_rep<QB>(lane);
+  for (int s0 = 0; s0 < n_slots; s0 += QB) {
+    const int nb = n_slots - s0 < QB ? n_slots - s0 : QB;
+    const int slot = s0 + (my_b < nb ? my_b : 0);
+    const int q = flagged ? flagged[slot] : slot;
+    // pass 2: this lane's query needs this warp iff the warp has hits that land below max_hits
+    int pos = 0, room = 0;
+    if (WRITE) {
+      if (my_b < nb && cnt[size_t(slot) * nw + gw] > 0) {
+        pos = off[size_t(slot) * nw + gw];
+        room = max_hits;
+      }
+      if (!__any_sync(0xffffffffu, pos < room)) continue;
+    }
+    float4 qv[QB][NJ];
+#pragma unroll
+    for (int b = 0; b < QB; ++b) {
+      const int qb_ = flagged ? flagged[s0 + (b < nb ? b : 0)] : s0 + (b < nb ? b : 0);
+#pragma unroll
+      for (int j = 0; j < NJ; ++j) qv[b][j] = __ldg(reinterpret_cast<const float4*>(qn + size_t(qb_) * DIM) + j * 32 + lane);
+    }
+    int count = 0;
+    for (int64_t r = r0; r < r1; ++r) {
+      const int32_t tg = __ldg(tags + r);
+      float4 g[NJ];                                                     // issued together with the tag load
+      const float4* pr = reinterpret_cast<const float4*>(master + r * DIM) + lane;
+#pragma unroll
+      for (int j = 0; j < NJ; ++j) g[j] = ldg_stream(pr + j * 32);
+      if (tg < 0 || (tenant >= 0 && tg != tenant)) continue;           // warp-uniform
+      float a[QB];
+      row_dots<NJ, QB, METRIC>(g, qv, a);
+      const float sdot = butterfly<QB>(a, lane);
+      const bool hit = my_b < nb && range_pass<METRIC>(sdot, threshold, strict);
+      if (WRITE) {
+        if (hit && pos < room) {
+          if (rep) {
+            out_rows[size_t(q) * max_hits + pos] = r + row_offset;
+            out_scores[size_t(q) * max_hits + pos] = METRIC == FRG_METRIC_COSINE ? sdot : __fsqrt_rn(sdot);
+          }
+          ++pos;
+        }
+        if (!__any_sync(0xffffffffu, pos < room)) break;
+      } else {
+        count += hit ? 1 : 0;
+      }
+    }
+    if (!WRITE && rep && my_b < nb) cnt[size_t(slot) * nw + gw] = count;
+  }
+}
+
+// one CTA per slot: exclusive scan of the slot's nw warp counts (each thread a contiguous strip, then a block scan
+// of the strip sums), the total, and the "none" marker in the unused output slots
+__global__ void __launch_bounds__(256)
+range_offsets_kernel(int nq, const int* __restrict__ flagged, const int* __restrict__ n_flagged, int nw,
+                     const int* __restrict__ cnt, int* __restrict__ off, int max_hits, float none_score,
+                     int64_t* __restrict__ out_counts, int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
+  __shared__ long long part[256];
+  pdl_wait();
+  pdl_trigger();
+  const int slot = blockIdx.x;
+  if (slot >= (flagged ? *n_flagged : nq)) return;
+  const int q = flagged ? flagged[slot] : slot;
+  const int t = threadIdx.x;
+  const int per = (nw + blockDim.x - 1) / blockDim.x;
+  const int a = t * per < nw ? t * per : nw, b = a + per < nw ? a + per : nw;
+  const int* c = cnt + size_t(slot) * nw;
+  long long sum = 0;
+  for (int i = a; i < b; ++i) sum += c[i];
+  part[t] = sum;
+  __syncthreads();
+  for (int o = 1; o < int(blockDim.x); o <<= 1) {          // Hillis-Steele inclusive scan
+    const long long v = t >= o ? part[t - o] : 0;
+    __syncthreads();
+    part[t] += v;
+    __syncthreads();
+  }
+  long long run = part[t] - sum;
+  int* o_ = off + size_t(slot) * nw;
+  for (int i = a; i < b; ++i) {
+    o_[i] = run < max_hits ? int(run) : max_hits;
+    run += c[i];
+  }
+  const long long total = part[blockDim.x - 1];
+  if (t == 0) out_counts[q] = total;
+  for (long long i = (total < max_hits ? total : max_hits) + t; i < max_hits; i += blockDim.x) {
+    out_rows[size_t(q) * max_hits + i] = kNoRow;
+    out_scores[size_t(q) * max_hits + i] = none_score;
+  }
+}
+
+int range_scan_supported(int dim, const char** why) {
+  if (dim != 128 && dim != 256 && dim != 512 && dim != 1024) { *why = "the range scan is built for dim 128, 256, 512 and 1024"; return 0; }
+  return 1;
+}
+
+template <int NJ, int QB, int METRIC>
+static int launch_range_passes(const ScanArgs& a, int grid, const int* flagged, const int* n_flagged, int max_hits,
+                               float threshold, bool strict, int64_t row_offset, int* cnt, int* off,
+                               int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  const int nw = grid * kScanWarps;
+  const int s = strict ? 1 : 0;
+  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, false>, dim3(grid), dim3(kScanWarps * 32), 0, st, true,
+                         a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged, a.tenant, threshold, s, max_hits,
+                         row_offset, cnt, off, out_rows, out_scores));
+  note_launch(nullptr);
+  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(a.nq), dim3(256), 0, st, true, a.nq, flagged, n_flagged, nw, cnt,
+                         off, max_hits, METRIC == FRG_METRIC_COSINE ? kNoScore : INFINITY, out_counts, out_rows,
+                         out_scores));
+  note_launch(nullptr);
+  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, true>, dim3(grid), dim3(kScanWarps * 32), 0, st, true,
+                         a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged, a.tenant, threshold, s, max_hits,
+                         row_offset, cnt, off, out_rows, out_scores));
+  note_launch(nullptr);
+  FRG_CUDA(cudaGetLastError());
+  return FRG_OK;
+}
+
+template <int NJ, int QB>
+static int launch_range_m(const ScanArgs& a, int grid, const int* flagged, const int* n_flagged, int max_hits,
+                          float threshold, bool strict, int64_t row_offset, int* cnt, int* off, int64_t* out_counts,
+                          int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  if (a.metric == FRG_METRIC_COSINE)
+    return launch_range_passes<NJ, QB, FRG_METRIC_COSINE>(a, grid, flagged, n_flagged, max_hits, threshold, strict,
+                                                          row_offset, cnt, off, out_counts, out_rows, out_scores, st);
+  return launch_range_passes<NJ, QB, FRG_METRIC_EUCLIDEAN>(a, grid, flagged, n_flagged, max_hits, threshold, strict,
+                                                           row_offset, cnt, off, out_counts, out_rows, out_scores, st);
+}
+
+template <int NJ>
+static int launch_range_qb(const ScanArgs& a, int qb, int grid, const int* flagged, const int* n_flagged,
+                           int max_hits, float threshold, bool strict, int64_t row_offset, int* cnt, int* off,
+                           int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+#define FRG_RANGE_QB(QB) return launch_range_m<NJ, QB>(a, grid, flagged, n_flagged, max_hits, threshold, strict, \
+                                                      row_offset, cnt, off, out_counts, out_rows, out_scores, st)
+  if (qb == 1) { FRG_RANGE_QB(1); }
+  if (qb == 2) { FRG_RANGE_QB(2); }
+  if constexpr (NJ <= 4) { if (qb == 4) { FRG_RANGE_QB(4); } }
+  if constexpr (NJ <= 2) { if (qb == 8) { FRG_RANGE_QB(8); } }
+#undef FRG_RANGE_QB
+  set_error("range scan: unsupported queries-per-pass %d for dim %d", qb, NJ * 128);
+  return FRG_ERR_UNSUPPORTED;
+}
+
+int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagged, int max_hits, float threshold,
+                      bool strict, int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                      cudaStream_t st) {
+  const char* why = "";
+  if (!range_scan_supported(a.dim, &why)) { set_error("range scan: %s", why); return FRG_ERR_UNSUPPORTED; }
+  if (a.nq <= 0) return FRG_OK;
+  if (flagged && a.rows <= 0) return FRG_OK;
+  // the same rows-in-flight sizing as the top-k scan; at least one warp, so an empty gallery still gets its counts
+  const int grid = scan_grid(a);
+  const size_t n_cnt = size_t(grid) * kScanWarps * a.nq;
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_cnt * 2 * sizeof(int), st));
+  int* cnt = reinterpret_cast<int*>(ws);
+  int* off = cnt + n_cnt;
+  const int qb = scan_qb(a.dim, a.nq);
+  int rc;
+  switch (a.dim) {
+    case 128: rc = launch_range_qb<1>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
+    case 256: rc = launch_range_qb<2>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
+    case 512: rc = launch_range_qb<4>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
+    default:  rc = launch_range_qb<8>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
+  }
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
 }  // namespace frg

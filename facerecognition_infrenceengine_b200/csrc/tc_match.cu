@@ -996,7 +996,10 @@ static int reg_k(int k) { return k == 1 ? 1 : (k <= 4 ? 4 : (k <= 8 ? 8 : 16)); 
 
 // dim < 0: Euclidean plane (|dim| columns).  Its probe and filter phases need DIFFERENT query images (lower / upper
 // bounds of the exact score), so the pre-pass is never folded into the filter kernel there.
-static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl) {
+// Range search (range = true): no pre-pass, and a fixed dense list of kRangeBudget entries per query instead of one
+// sized from k (DESIGN.md section 7.3).
+constexpr int kRangeBudget = 4096;
+static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range = false) {
   const bool euclid_plane = dim < 0;
   pl->qtiles = (nq + kTileQ - 1) / kTileQ;
   pl->pair = tc_uses_pairs(nq);
@@ -1006,7 +1009,7 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   // wins for a handful of queries (F = 1: 198 vs 208 us) and loses from F = 64 on (F = 1024: 814 vs
   // 735 us).  FRG_TC_FUSED=0/1 forces either path.
   static const int fused_env = []() { const char* e = getenv("FRG_TC_FUSED"); return e ? atoi(e) : -1; }();
-  pl->fused = !euclid_plane && (fused_env >= 0 ? fused_env != 0 : nq <= 8);
+  pl->fused = !euclid_plane && !range && (fused_env >= 0 ? fused_env != 0 : nq <= 8);
   const int tile_rows = pl->pair ? 2 * kTileR : kTileR;
   // pre-pass sample: every stride-th 128-row tile, stride the largest power of two <= 64 that still
   // leaves >= 16 K sampled rows
@@ -1053,6 +1056,7 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   int stage_entries = int(3.0 * eff_stride * (k + 10.0 * sqrt(double(k)) + 10.0));
   if (stage_entries < 256) stage_entries = 256;
   if (stage_entries > 8192) stage_entries = 8192;
+  if (range) stage_entries = kRangeBudget;
   pl->stage_entries = stage_entries;
   // private segments: one per (query, chunk, column half); x2 headroom for imbalance across them
   const int nseg = pl->chunks_main * (kEpiWarps / 4);
@@ -1132,17 +1136,17 @@ int64_t tc_effective_rows(const GalleryWindow* s, int nq, cudaStream_t st, const
   return int64_t(n) * gran;
 }
 
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count) {
+size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range) {
   TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl);
+  tc_plan(rows, dim, nq, k, sm_count, &pl, range);
   return pl.total;
 }
 
 // the pieces of the workspace the query-prep kernel initialises (group keys := key(-1), counters := 0)
 void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               uint32_t** keys, int** cand_total, int** n_flagged) {
+                               uint32_t** keys, int** cand_total, int** n_flagged, bool range) {
   TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl);
+  tc_plan(rows, dim, nq, k, sm_count, &pl, range);
   *keys = reinterpret_cast<uint32_t*>(ws + pl.off_keys);
   *cand_total = reinterpret_cast<int*>(ws + pl.off_cnt);
   *n_flagged = reinterpret_cast<int*>(ws + pl.off_flag) + nq;
@@ -1240,6 +1244,142 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   }
 #undef FRG_SELECT
 #undef FRG_SELECT_M
+  note_launch(nullptr);
+  FRG_CUDA(cudaGetLastError());
+  profile_end(st, 1);
+  return FRG_OK;
+}
+
+
+// ------------------------------------------------------------------------------------------ range search
+// The filter's floor for a range search is the fixed threshold - eps[q] (rigorous: |S - s| <= eps[q], so every row
+// with exact s >= threshold has S >= the floor), not a group-maximum floor: no pre-pass runs.  The filter kernel is
+// the top-k one, untouched - its prologue derives floor = (k-th largest group key) - 2 eps[q]; with k = 1 and every
+// group key of query q set to threshold + eps[q] - 1e-6 that is threshold - eps[q] - 1e-6 (the 1e-6 covers the
+// rounding of the two fp32 operations).  Thresholds at or below -1 - eps[q] leave the key at "nothing seen": no
+// floor, every valid row is a candidate.
+__global__ void __launch_bounds__(256)
+range_floor_kernel(const float* __restrict__ eps, float threshold, uint32_t* __restrict__ keys, int nq) {
+  pdl_wait();             // the query prep's eps[] and its reset of the keys
+  pdl_trigger();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nq * kGroups) return;
+  const float f = threshold + __ldg(eps + i / kGroups) - 1e-6f;
+  if (f > kNoScore) keys[i] = float_key(f);
+}
+
+// ONE CTA (4 warps) per query over the dense candidate list of a range-mode filter: every candidate is rescored
+// exactly in fp32 from the master (same element -> lane mapping and xor 16..1 reduction as the streaming scan, so
+// the scores are bit-identical to launch_range_scan's), the survivors of the threshold rule are packed as
+// (row << 32 | score bits) in shared memory, sorted by row (bitonic) and the first max_hits written in gallery order.
+__global__ void __launch_bounds__(kSelectWarps * 32)
+range_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand_total, int dense_cap, int dim,
+                    const float* __restrict__ qn, const float* __restrict__ master, float threshold, int strict,
+                    int max_hits, int64_t row_offset, int64_t* __restrict__ out_counts,
+                    int64_t* __restrict__ out_rows, float* __restrict__ out_scores, int* __restrict__ flagged,
+                    int* __restrict__ n_flagged) {
+  extern __shared__ unsigned long long hits[];        // [pow2 >= dense_cap]
+  __shared__ int s_m;
+  const int lane = threadIdx.x & 31;
+  const int w = threadIdx.x >> 5;
+  const int q = blockIdx.x;
+  pdl_wait();             // the filter kernel's candidate lists
+  pdl_trigger();
+  const int total = cand_total[q];
+  if (total > dense_cap) {                           // also set by a poisoned total (segment overflow)
+    if (threadIdx.x == 0) flagged[atomicAdd(n_flagged, 1)] = q;
+    return;
+  }
+  if (threadIdx.x == 0) s_m = 0;
+  __syncthreads();
+  const int2* mine = dense + size_t(q) * dense_cap;
+  const int nvec = dim >> 2;
+  const float4* qq = reinterpret_cast<const float4*>(qn + size_t(q) * dim);
+  for (int c = w; c < total; c += kSelectWarps) {
+    const int row = mine[c].x;
+    const float4* g = reinterpret_cast<const float4*>(master + size_t(row) * dim);
+    float a = 0.f;
+#pragma unroll 4
+    for (int v = lane; v < nvec; v += 32) {
+      const float4 x = __ldg(g + v), y = __ldg(qq + v);
+      a = fmaf(x.x, y.x, a); a = fmaf(x.y, y.y, a); a = fmaf(x.z, y.z, a); a = fmaf(x.w, y.w, a);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    const bool pass = strict ? (a > threshold) : (a >= threshold);      // false for NaN
+    if (lane == 0 && pass) hits[atomicAdd(&s_m, 1)] = (uint64_t(uint32_t(row)) << 32) | __float_as_uint(a);
+  }
+  __syncthreads();
+  const int m = s_m;
+  int n2 = 1;
+  while (n2 < m) n2 <<= 1;
+  for (int i = m + threadIdx.x; i < n2; i += blockDim.x) hits[i] = ~0ull;
+  __syncthreads();
+  // rows are distinct: ascending keys = gallery order
+  for (int kk = 2; kk <= n2; kk <<= 1) {
+    for (int j = kk >> 1; j > 0; j >>= 1) {
+      for (int i = threadIdx.x; i < n2; i += blockDim.x) {
+        const int ij = i ^ j;
+        if (ij > i) {
+          const unsigned long long x = hits[i], y = hits[ij];
+          if ((x > y) == ((i & kk) == 0)) { hits[i] = y; hits[ij] = x; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  for (int i = threadIdx.x; i < max_hits; i += blockDim.x) {
+    const bool filled = i < m;
+    out_rows[size_t(q) * max_hits + i] = filled ? int64_t(hits[i] >> 32) + row_offset : int64_t(kNoRow);
+    out_scores[size_t(q) * max_hits + i] = filled ? __uint_as_float(uint32_t(hits[i])) : kNoScore;
+  }
+  if (threadIdx.x == 0) out_counts[q] = m;
+}
+
+int launch_tc_range(const GalleryWindow* s, const float* qn, const __nv_bfloat16* qb, const float* eps, int nq,
+                    int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned char* ws,
+                    int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores, int** flagged_out,
+                    int** n_flagged_out, cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list) {
+  TcPlan pl;
+  tc_plan(plan_rows, s->dim, nq, 1, sm_count, &pl, true);
+  int* cnt = reinterpret_cast<int*>(ws + pl.off_cnt);
+  int2* cand = reinterpret_cast<int2*>(ws + pl.off_cand);
+  int2* dense = reinterpret_cast<int2*>(ws + pl.off_dense);
+  int* flagged = reinterpret_cast<int*>(ws + pl.off_flag);
+  int* n_flagged = flagged + nq;
+  *flagged_out = flagged;
+  *n_flagged_out = n_flagged;
+  const bool masked = tenant >= 0 || s->maybe_dead;
+
+  CUtensorMap qm, gm;
+  FRG_CHECK(make_map(&qm, qb, s->dim, nq, size_t(s->dim) * 2, kTileQ));
+  FRG_CHECK(make_map(&gm, s->plane, s->dim, s->rows, size_t(s->plane_dim) * 2, kTileR));
+
+  TcScanParams p{};
+  p.fault = s->fault;
+  p.tile_list = tile_list; p.n_list = n_list;
+  p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = tc_stages(s->dim);
+  p.dim = s->dim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
+  p.n_rows = int(s->rows); p.group_key = reinterpret_cast<uint32_t*>(ws + pl.off_keys); p.k = 1;
+  p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
+  p.tile_scale = 1;
+  profile_begin(st, kStageFloor);
+  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq * kGroups + 255) / 256), dim3(256), 0, st, true, eps, threshold,
+                         p.group_key, nq));
+  note_launch(nullptr);
+  profile_end(st, 1);
+  profile_begin(st, kStageDominant);
+  FRG_CHECK(launch_tc_scan_m<kModeFilter>(masked, pl.pair, qm, gm, gm, p, pl.qtiles, pl.chunks_main, st));
+  profile_end(st, 1);
+
+  profile_begin(st, kStageSelect);
+  int n2 = 1;
+  while (n2 < pl.stage_entries) n2 <<= 1;
+  const size_t smem = size_t(n2) * sizeof(unsigned long long);
+  FRG_CUDA(func_attr_once(range_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  FRG_CUDA(launch_kernel(range_select_kernel, dim3(nq), dim3(kSelectWarps * 32), smem, st, true, dense, cnt,
+                         pl.stage_entries, s->dim, qn, s->master, threshold, strict ? 1 : 0, max_hits, row_offset,
+                         out_counts, out_rows, out_scores, flagged, n_flagged));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   profile_end(st, 1);

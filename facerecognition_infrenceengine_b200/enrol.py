@@ -118,7 +118,54 @@ class EnrolmentChecker:
                     return False, (i, j)
         return True, None
 
+    def audit_duplicates(self, company_id: Optional[str] = None, kind: Optional[str] = None,
+                         batch: int = 1024) -> List[Tuple[str, str, float]]:
+        """:func:`find_duplicate_pairs` over this checker's gallery at its duplicate threshold (one company's
+        collection with `company_id` / `kind`, as ``check_duplicate_face`` scans it)."""
+        tenant = None if company_id is None and kind is None else enrolment_tenant(company_id, kind)
+        return find_duplicate_pairs(self.store, self.duplicate_threshold, tenant, batch, self.matcher)
+
     @staticmethod
     def template_from_poses(pose_embeddings: Sequence[np.ndarray]) -> np.ndarray:
         """trainingServer.py:355."""
         return np.mean(pose_embeddings, axis=0)
+
+
+def find_duplicate_pairs(store, threshold: float = DUPLICATE_THRESHOLD, company_id: Optional[str] = None,
+                         batch: int = 1024, matcher=None) -> List[Tuple[str, str, float]]:
+    """Whole-gallery duplicate audit: every pair of live rows a < b (gallery order) with cos > threshold - the rule
+    of the enrol-time check (trainingServer.py:170-200), applied to what is already enrolled.  company_id: only
+    that tenant's rows (an :class:`EnrolmentGallery` takes the key of ``enrolment_tenant``).  Each pair is
+    reported once, from the lower row's query, as (id_a, id_b, score); pairs whose ids are equal are skipped (an
+    enrolment gallery holds several templates per person: the id is the template's `ref_id` when it has one).
+    Mechanism: the stored rows are read back in batches and sent as queries through ``Matcher.match_range``, so
+    the whole audit is one N x N contraction - on the tensor cores when the store keeps a scan plane."""
+    base = store.store if isinstance(store, EnrolmentGallery) else store
+    matcher = matcher if matcher is not None else Matcher(base)
+    code = None if company_id is None else base.tenant_code(company_id, create=False)
+
+    def ident(row: int) -> Optional[str]:
+        pid = base.id_of(row)
+        ref = (base.metadata(pid) or {}).get("ref_id") if pid is not None else None
+        return ref if ref is not None else pid
+
+    pairs: List[Tuple[str, str, float]] = []
+    with _reading(base):
+        n = base.rows
+        for r0 in range(0, n, batch):
+            vecs, tags = base.read_rows(r0, min(batch, n - r0))
+            live = np.nonzero((tags >= 0) if code is None else (tags == code))[0]
+            if not len(live):
+                continue
+            res = matcher.match_range(vecs[live], threshold, company_id=company_id, max_hits=16, strict=True,
+                                      with_ids=False)
+            for a, rows, scores in zip((r0 + live).tolist(), res.rows, res.scores):
+                later = rows > a
+                if not later.any():
+                    continue
+                ia = ident(a)
+                for b, sc in zip(rows[later].tolist(), scores[later].tolist()):
+                    ib = ident(b)
+                    if ia != ib:
+                        pairs.append((ia, ib, sc))
+    return pairs

@@ -34,6 +34,32 @@ class MatchResult:
     layout_version: int = 0      # GalleryStore.layout_version the rows belong to (compact() renumbers rows)
 
 
+@dataclass
+class RangeResult:
+    counts: np.ndarray            # int64 [F]   rows at or above the threshold (Euclidean: at or below)
+    rows: List[np.ndarray]        # per query: int64, COMPLETE, best first (score desc / distance asc, then row asc)
+    scores: List[np.ndarray]      # per query: fp32, exact, in the same order
+    ids: Optional[List[List[Optional[str]]]] = None
+    variant: str = ""
+    layout_version: int = 0
+
+
+def best_first(rows: np.ndarray, scores: np.ndarray, metric: str = "cosine"):
+    """The project's result order over a complete hit list: score desc (distance asc), then row asc."""
+    order = np.lexsort((rows, scores if metric == "euclidean" else -scores))
+    return rows[order], scores[order]
+
+
+def range_lists(counts: np.ndarray, rows: np.ndarray, scores: np.ndarray, metric: str = "cosine"):
+    """[F, max_hits] gallery-order blocks whose counts all fit -> per-query best-first arrays."""
+    out_r, out_s = [], []
+    for f, c in enumerate(counts.tolist()):
+        r, sc = best_first(rows[f, :c], scores[f, :c], metric)
+        out_r.append(r)
+        out_s.append(sc)
+    return out_r, out_s
+
+
 def _params(metric: str, variant: str, threshold: float, tenant: int, row_offset: int) -> N.MatchParams:
     return N.MatchParams(N.METRICS[metric], N.VARIANTS[variant], float(np.float32(threshold)),
                          int(tenant), int(row_offset), 0, 0)
@@ -100,6 +126,44 @@ class Matcher:
                                 C.c_void_p(rows.data_ptr()), C.c_void_p(scores.data_ptr()),
                                 C.c_void_p(accept.data_ptr()), C.c_void_p(stream)))
         return rows, scores, accept
+
+    # ---- every row whose score reaches the threshold (exact fp32)
+    def range_host(self, Q: np.ndarray, threshold: float, tenant: int = -1, max_hits: int = 64, strict: bool = False,
+                   variant: str = "auto", row_offset: int = 0):
+        """One frg_match_range_host call: (counts int64 [F], rows int64 [F, max_hits], scores fp32 [F, max_hits]),
+        the FIRST max_hits hits of every query in gallery order (+ row_offset); counts[f] > max_hits = truncated."""
+        Q = np.ascontiguousarray(Q, dtype=np.float32).reshape(-1, self.store.dim)
+        F = len(Q)
+        counts = np.zeros(F, np.int64)
+        rows, scores = np.empty((F, max_hits), np.int64), np.empty((F, max_hits), np.float32)
+        p = _params(self.metric, variant, threshold, tenant, row_offset)
+        p.flags = N.FIRST_STRICT if strict else 0
+        N.check(N.lib.frg_match_range_host(self.store.handle, Q.ctypes.data, F, int(max_hits), C.byref(p),
+                                           counts.ctypes.data, rows.ctypes.data, scores.ctypes.data))
+        return counts, rows, scores
+
+    def match_range(self, Q: np.ndarray, threshold: float, company_id: Optional[str] = None, max_hits: int = 64,
+                    strict: bool = False, variant: str = "auto", with_ids: bool = True) -> RangeResult:
+        """Every live row with score >= threshold ('>' when strict; Euclidean: distance <= threshold), as COMPLETE
+        best-first lists.  max_hits only sizes the first call: the queries whose count exceeded it are re-run once,
+        those queries only, with room for their largest count."""
+        Q = np.ascontiguousarray(Q, dtype=np.float32).reshape(-1, self.store.dim)
+        tenant = -1 if company_id is None else self.store.tenant_code(company_id, create=False)
+        with _reading(self.store):
+            layout = getattr(self.store, "layout_version", 0)
+            counts, rows, scores = self.range_host(Q, threshold, tenant, max_hits, strict, variant)
+            variant_ran = N.last_variant()
+            over = np.nonzero(counts > max_hits)[0]
+            if len(over):
+                c2, r2, s2 = self.range_host(Q[over], threshold, tenant, int(counts[over].max()), strict, variant)
+                counts[over] = c2
+            lists_r, lists_s = range_lists(np.minimum(counts, max_hits), rows, scores, self.metric)
+            for j, f in enumerate(over.tolist()):
+                lists_r[f], lists_s[f] = best_first(r2[j, :c2[j]], s2[j, :c2[j]], self.metric)
+            out = RangeResult(counts, lists_r, lists_s, variant=variant_ran, layout_version=layout)
+            if with_ids:
+                out.ids = [self.store.ids_of(r[None, :])[0] if len(r) else [] for r in lists_r]
+        return out
 
     # ---- first row, in gallery order, whose score reaches the threshold (exact fp32)
     def first_above(self, Q: np.ndarray, threshold: float, strict: bool = False, company_id: Optional[str] = None,

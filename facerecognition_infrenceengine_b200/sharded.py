@@ -29,7 +29,7 @@ import numpy as np
 
 from . import _native as N
 from .gallery import GalleryStore
-from .matcher import LIVE_THRESHOLD, Matcher, MatchResult
+from .matcher import LIVE_THRESHOLD, Matcher, MatchResult, RangeResult, best_first
 
 
 def block_layout(F: int, k: int) -> Tuple[int, int]:
@@ -496,6 +496,64 @@ class ShardedMatcher:
         best, sc = best.cpu().numpy(), sc.cpu().numpy()
         hit = best != none
         return np.where(hit, best, -1), np.where(hit, sc, np.float32(-1.0)).astype(np.float32)
+
+    def match_range(self, Q: np.ndarray, threshold: float, company_id: Optional[str] = None, max_hits: int = 64,
+                    strict: bool = False, variant: str = "auto", with_ids: bool = True,
+                    local_range: Optional[Callable] = None) -> RangeResult:
+        """``Matcher.match_range`` over the row-sharded gallery.  Collective: every rank passes the same batch.
+        Each rank runs the range search on its block (global rows: its row offset); ONE all-gather brings every
+        rank's counts and first max_hits hits to every rank.  Ranks hold contiguous blocks, so concatenating the
+        hit lists in rank order is global gallery order; the counts add up.  Queries whose total count exceeded
+        max_hits are re-run once, on every rank alike (the decision is taken from the gathered counts).
+        local_range(Q, threshold, strict, tenant, max_hits, row_offset) -> (counts [F], rows [F, max_hits],
+        scores [F, max_hits]) replaces the device call (host-logic tests)."""
+        Q = np.ascontiguousarray(Q, dtype=np.float32).reshape(-1, self.g.dim)
+        tenant = -1 if company_id is None else self.g.tenant_code(company_id, create=False)
+        local = local_range or (lambda Qx, thr, st, tn, mh, off: self._matcher.range_host(
+            Qx, thr, tn, mh, st, variant, off))
+        counts, rows, scores = self._range_gathered(Q, threshold, strict, tenant, max_hits, local)
+        over = np.nonzero(counts.sum(axis=0) > max_hits)[0]
+        if len(over):
+            mh2 = int(counts.sum(axis=0)[over].max())
+            c2, r2, s2 = self._range_gathered(Q[over], threshold, strict, tenant, mh2, local)
+        lists_r, lists_s = [], []
+        for f in range(len(Q)):
+            j = np.searchsorted(over, f)
+            if j < len(over) and over[j] == f:
+                c, r, s = c2[:, j], r2[:, j], s2[:, j]
+            else:
+                c, r, s = counts[:, f], rows[:, f], scores[:, f]
+            rr = np.concatenate([r[p, :c[p]] for p in range(len(c))])
+            ss = np.concatenate([s[p, :c[p]] for p in range(len(c))])
+            rr, ss = best_first(rr, ss, self.metric)
+            lists_r.append(rr)
+            lists_s.append(ss)
+        total = np.array([len(r) for r in lists_r], np.int64)
+        out = RangeResult(total, lists_r, lists_s, variant="sharded")
+        if with_ids:
+            out.ids = [[self.g.id_of(x) for x in r.tolist()] for r in lists_r]
+        return out
+
+    def _range_gathered(self, Q, threshold, strict, tenant, max_hits, local):
+        """Every rank's (counts [world, F], rows [world, F, max_hits], scores [world, F, max_hits])."""
+        F = len(Q)
+        counts, rows, scores = local(Q, threshold, strict, tenant, max_hits, self.g.offset)
+        if self.g.world == 1:
+            return counts[None], rows[None], scores[None]
+        import torch
+        import torch.distributed as dist
+        # one int64 block per rank: [counts F | rows F*max_hits | score bits F*max_hits]
+        block = np.concatenate([np.asarray(counts, np.int64), np.asarray(rows, np.int64).ravel(),
+                                np.asarray(scores, np.float32).view(np.int32).astype(np.int64).ravel()])
+        on_gpu = dist.get_backend(self.g.group) == "nccl"
+        dev = torch.device("cuda", self.g.store.device if self.g.device is None else self.g.device) if on_gpu else "cpu"
+        mine = torch.from_numpy(block).to(dev)
+        gathered = torch.empty((self.g.world * len(block),), dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(gathered, mine, group=self.g.group)
+        g = gathered.cpu().numpy().reshape(self.g.world, -1)
+        n = F * max_hits
+        return (g[:, :F], g[:, F:F + n].reshape(-1, F, max_hits),
+                g[:, F + n:].astype(np.int32).view(np.float32).reshape(-1, F, max_hits))
 
     def ids_of(self, rows) -> List[List[Optional[str]]]:
         """Global rows of a match result -> id strings (None for unfilled slots)."""

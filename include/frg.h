@@ -171,6 +171,24 @@ FRG_API int frg_first_match(frg_store* s, const float* q, int32_t nq, const frg_
 FRG_API int frg_first_match_host(frg_store* s, const float* q, int32_t nq, const frg_match_params_t* p,
                          int64_t* out_rows, float* out_scores);
 
+/* ---- every row whose score reaches the threshold ("range search"; NOT in the reference: parity unpinned, the
+ *      generalisation of trainingServer.py:170-200 from "first hit" to "all hits": watchlists, template clean-up,
+ *      duplicate audits of a whole gallery).
+ * out_counts [nq] int64: the exact number of live rows (tenant-filtered) with score >= p->threshold (cosine; '>'
+ *   with FRG_FIRST_STRICT) or dist <= p->threshold (euclidean; '<' with FRG_FIRST_STRICT).
+ * out_rows [nq*max_hits] int64, out_scores [nq*max_hits] fp32: the FIRST min(count, max_hits) of those rows IN
+ *   GALLERY ORDER (row ascending, + p->row_offset) with their exact fp32 scores (euclidean: distances); unused slots
+ *   row -1 / score -1.0f (euclidean +inf).  count > max_hits tells the caller the list is truncated.
+ * p->flags: FRG_FIRST_STRICT, FRG_QUERY_PRENORMALISED.  p->variant: AUTO (the tensor-core filter for unit cosine
+ *   stores with a scan plane and dim 128 / 256 / 512, else the exact scan), TC_EXACT (cosine only) or SCAN_F32;
+ *   TC_BF16 and bf16-only stores: FRG_ERR_UNSUPPORTED.  max_hits >= 1.  An empty gallery gives counts 0.
+ * The scores are bit-identical on both paths; frg_last_variant() names the one that ran (range_tc / range_scan). */
+FRG_API int frg_match_range(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
+                            int64_t* out_counts, int64_t* out_rows, float* out_scores, void* stream);
+FRG_API int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32_t max_hits,
+                                 const frg_match_params_t* p, int64_t* out_counts, int64_t* out_rows,
+                                 float* out_scores);
+
 /* ---- k-way merge of per-shard results (multi-GPU tail, SURVEY.md section 8e).
  * scores/rows: [parts][nq][k] (each list best-first, unfilled slots row -1), e.g. the output of an
  * all-gather of every rank's frg_match result.  Order: score desc (euclidean: asc), then row asc. */
