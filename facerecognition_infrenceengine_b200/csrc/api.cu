@@ -121,19 +121,27 @@ static int store_fault(const frg_store* s) {
 
 static bool has_master(const frg_store* s) { return !(s->flags & FRG_STORE_BF16_ONLY); }
 static bool has_plane(const frg_store* s) { return (s->flags & (FRG_STORE_BF16_PLANE | FRG_STORE_BF16_ONLY)) != 0; }
-
-static size_t row_bytes(const frg_store* s) {
-  return size_t(s->dim) * (has_master(s) ? sizeof(float) : 0) +
-         size_t(s->plane_dim) * (has_plane(s) ? sizeof(__nv_bfloat16) : 0) + sizeof(int32_t);
+// a unit store with a full master scans an int8 plane (tc_match.cu); raw and bf16-only stores keep a bf16 one
+static bool has_plane8(const frg_store* s) {
+  return (s->flags & FRG_STORE_BF16_PLANE) && !(s->flags & (FRG_STORE_RAW | FRG_STORE_BF16_ONLY));
+}
+// bytes of one scan-plane row
+static size_t plane_row_bytes(const frg_store* s) {
+  if (!has_plane(s)) return 0;
+  return has_plane8(s) ? size_t(s->dim) : size_t(s->plane_dim) * sizeof(__nv_bfloat16);
 }
 
-static int alloc_arrays(frg_store* s, int64_t cap, float** m, __nv_bfloat16** p, int32_t** t) {
+static size_t row_bytes(const frg_store* s) {
+  return size_t(s->dim) * (has_master(s) ? sizeof(float) : 0) + plane_row_bytes(s) + sizeof(int32_t);
+}
+
+// p: the scan plane, bf16 or int8 (has_plane8) - its element type is the caller's to know
+static int alloc_arrays(frg_store* s, int64_t cap, float** m, void** p, int32_t** t) {
   *m = nullptr; *p = nullptr; *t = nullptr;
   const int64_t c = cap > 0 ? cap : 1;
   cudaError_t e = cudaSuccess;
   if (has_master(s)) e = cudaMalloc(reinterpret_cast<void**>(m), size_t(c) * s->dim * sizeof(float));
-  if (e == cudaSuccess && has_plane(s))
-    e = cudaMalloc(reinterpret_cast<void**>(p), size_t(c) * s->plane_dim * sizeof(__nv_bfloat16));
+  if (e == cudaSuccess && has_plane(s)) e = cudaMalloc(p, size_t(c) * plane_row_bytes(s));
   if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(t), size_t(c) * sizeof(int32_t));
   if (e != cudaSuccess) {
     cudaFree(*m); cudaFree(*p); cudaFree(*t);
@@ -142,20 +150,25 @@ static int alloc_arrays(frg_store* s, int64_t cap, float** m, __nv_bfloat16** p,
   }
   return FRG_OK;
 }
+static void* plane_ptr(const frg_store* s) { return s->plane8 ? static_cast<void*>(s->plane8) : static_cast<void*>(s->plane); }
+static void set_plane(frg_store* s, void* p) {
+  if (has_plane8(s)) s->plane8 = static_cast<int8_t*>(p);
+  else s->plane = static_cast<__nv_bfloat16*>(p);
+}
 
 // grow to at least `cap` rows; s->mu held.  Synchronous (rare, off the hot path).
 static int grow_locked(frg_store* s, int64_t cap) {
   if (cap <= s->capacity) return FRG_OK;
   FRG_CUDA(cudaDeviceSynchronize());
-  float* m; __nv_bfloat16* p; int32_t* t;
+  float* m; void* p; int32_t* t;
   FRG_CHECK(alloc_arrays(s, cap, &m, &p, &t));
   if (s->rows > 0) {
     if (m) FRG_CUDA(cudaMemcpy(m, s->master, size_t(s->rows) * s->dim * sizeof(float), cudaMemcpyDeviceToDevice));
-    if (p) FRG_CUDA(cudaMemcpy(p, s->plane, size_t(s->rows) * s->plane_dim * sizeof(__nv_bfloat16), cudaMemcpyDeviceToDevice));
+    if (p) FRG_CUDA(cudaMemcpy(p, plane_ptr(s), size_t(s->rows) * plane_row_bytes(s), cudaMemcpyDeviceToDevice));
     FRG_CUDA(cudaMemcpy(t, s->tags, size_t(s->rows) * sizeof(int32_t), cudaMemcpyDeviceToDevice));
   }
-  cudaFree(s->master); cudaFree(s->plane); cudaFree(s->tags);
-  s->master = m; s->plane = p; s->tags = t;
+  cudaFree(s->master); cudaFree(plane_ptr(s)); cudaFree(s->tags);
+  s->master = m; set_plane(s, p); s->tags = t;
   s->capacity = cap;
   s->readers.clear();
   s->has_write = false;
@@ -245,7 +258,7 @@ static void extents_note_upsert(frg_store* s, const int64_t* hrows, const int32_
 // tenant's rows can sit in (FRG_TENANT_WINDOW=0 turns the window off)
 static GalleryWindow window_of(const frg_store* s, int32_t tenant, bool for_tc = false) {
   GalleryWindow w;
-  w.master = s->master; w.plane = s->plane; w.tags = s->tags; w.gmax_bits = s->gmax_bits; w.fault = s->fault_dev;
+  w.master = s->master; w.plane = s->plane; w.plane8 = s->plane8; w.tags = s->tags; w.gmax_bits = s->gmax_bits; w.fault = s->fault_dev;
   w.rows = s->rows; w.row0 = 0; w.dim = s->dim; w.plane_dim = s->plane_dim; w.flags = s->flags;
   w.maybe_dead = s->maybe_dead;
   static const bool on = []() { const char* e = getenv("FRG_TENANT_WINDOW"); return !e || atoi(e) != 0; }();
@@ -269,6 +282,7 @@ static GalleryWindow window_of(const frg_store* s, int32_t tenant, bool for_tc =
     w.row0 = lo; w.rows = hi - lo;
     if (w.master) w.master += lo * s->dim;
     if (w.plane) w.plane += lo * s->plane_dim;
+    if (w.plane8) w.plane8 += lo * s->dim;
     w.tags += lo;
   }
   return w;
@@ -392,12 +406,14 @@ int frg_store_create(int32_t device, int32_t dim, int64_t capacity, uint32_t fla
   const char* why = "";
   s->plane_dim = ((flags & FRG_STORE_RAW) && (flags & FRG_STORE_BF16_PLANE) && tc_supported(dim, FRG_METRIC_EUCLIDEAN, &why))
                      ? dim + kEuclidPad : dim;
-  int rc = alloc_arrays(s, capacity, &s->master, &s->plane, &s->tags);
+  void* plane = nullptr;
+  int rc = alloc_arrays(s, capacity, &s->master, &plane, &s->tags);
+  set_plane(s, plane);
   if (rc == FRG_OK) {
     cudaError_t eg = cudaMalloc(reinterpret_cast<void**>(&s->gmax_bits), 2 * sizeof(uint32_t));
     if (eg == cudaSuccess) eg = cudaMemset(s->gmax_bits, 0, 2 * sizeof(uint32_t));
     if (eg != cudaSuccess) {
-      cudaFree(s->master); cudaFree(s->plane); cudaFree(s->tags); cudaFree(s->gmax_bits);
+      cudaFree(s->master); cudaFree(plane_ptr(s)); cudaFree(s->tags); cudaFree(s->gmax_bits);
       rc = cuda_fail(eg, "cudaMalloc(gmax)", __FILE__, __LINE__);
     }
   }
@@ -408,7 +424,7 @@ int frg_store_create(int32_t device, int32_t dim, int64_t capacity, uint32_t fla
       ef = cudaHostGetDevicePointer(reinterpret_cast<void**>(&s->fault_dev), s->fault_host, 0);
     }
     if (ef != cudaSuccess) {
-      cudaFree(s->master); cudaFree(s->plane); cudaFree(s->tags); cudaFree(s->gmax_bits);
+      cudaFree(s->master); cudaFree(plane_ptr(s)); cudaFree(s->tags); cudaFree(s->gmax_bits);
       if (s->fault_host) cudaFreeHost(s->fault_host);
       rc = cuda_fail(ef, "cudaHostAlloc(fault word)", __FILE__, __LINE__);
     }
@@ -432,7 +448,7 @@ int frg_store_destroy(frg_store* s) {
   {
     DeviceGuard g(s->device);
     cudaDeviceSynchronize();
-    cudaFree(s->master); cudaFree(s->plane); cudaFree(s->tags); cudaFree(s->gmax_bits);
+    cudaFree(s->master); cudaFree(plane_ptr(s)); cudaFree(s->tags); cudaFree(s->gmax_bits);
     if (s->fault_host) cudaFreeHost(s->fault_host);
     for (auto& kv : s->tile_lists) { cudaFree(kv.second.dev); if (kv.second.ready) cudaEventDestroy(kv.second.ready); }
     for (void* p : s->retired) cudaFree(p);
@@ -474,8 +490,8 @@ static int upsert_impl(frg_store* s, const int64_t* rows, const float* vecs, con
   if (!rows && s->rows + n > s->capacity) FRG_CHECK(grow_locked(s, next_capacity(s->capacity, s->rows + n)));
   FRG_CHECK(store_begin_write(s, st));
   const bool normalise = !(flags & FRG_ROWS_PRENORMALISED) && !(s->flags & FRG_STORE_RAW);
-  FRG_CHECK(launch_ingest(vecs, rows, tags, n, s->rows, s->dim, normalise, s->master, s->plane, s->plane_dim,
-                          s->gmax_bits, s->tags, st));
+  FRG_CHECK(launch_ingest(vecs, rows, tags, n, s->rows, s->dim, normalise, s->master, s->plane, s->plane8,
+                          s->plane_dim, s->gmax_bits, s->tags, st));
   if (host_known) extents_note_upsert(s, hrows, htags, n, s->rows);
   else s->extents_known = false;             // positions / tags live in device memory only
   if (!rows) s->rows += n;
@@ -672,7 +688,7 @@ int frg_store_compact(frg_store* s, int64_t* old_to_new) {
   if (first < m) {
     static const int64_t chunk_rows = []() { const char* e = getenv("FRG_COMPACT_CHUNK_ROWS"); const long v = e ? atol(e) : 65536; return int64_t(v < 1 ? 65536 : v); }();
     const int64_t chunk = m - first < chunk_rows ? m - first : chunk_rows;
-    float* bm; __nv_bfloat16* bp; int32_t* bt;
+    float* bm; void* bp; int32_t* bt;
     int64_t* dsrc = nullptr;
     FRG_CHECK(alloc_arrays(s, chunk, &bm, &bp, &bt));            // nothing has changed yet if this fails
     cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&dsrc), size_t(chunk) * sizeof(int64_t));
@@ -682,10 +698,13 @@ int frg_store_compact(frg_store* s, int64_t* old_to_new) {
       const int64_t cnt = m - a < chunk ? m - a : chunk;
       e = cudaMemcpy(dsrc, src.data() + a, size_t(cnt) * sizeof(int64_t), cudaMemcpyHostToDevice);
       if (e != cudaSuccess) { rc = cuda_fail(e, "compact staging", __FILE__, __LINE__); break; }
-      rc = launch_gather_rows(dsrc, cnt, s->dim, s->plane_dim, s->master, s->plane, s->tags, bm, bp, bt, nullptr);
+      rc = launch_gather_rows(dsrc, cnt, s->dim, int(plane_row_bytes(s)), s->master, plane_ptr(s), s->tags, bm, bp, bt,
+                              nullptr);
       if (rc != FRG_OK) break;
       if (bm) e = cudaMemcpyAsync(s->master + a * s->dim, bm, size_t(cnt) * s->dim * sizeof(float), cudaMemcpyDeviceToDevice, nullptr);
-      if (e == cudaSuccess && bp) e = cudaMemcpyAsync(s->plane + a * s->plane_dim, bp, size_t(cnt) * s->plane_dim * sizeof(__nv_bfloat16), cudaMemcpyDeviceToDevice, nullptr);
+      if (e == cudaSuccess && bp)
+        e = cudaMemcpyAsync(static_cast<unsigned char*>(plane_ptr(s)) + a * plane_row_bytes(s), bp,
+                            size_t(cnt) * plane_row_bytes(s), cudaMemcpyDeviceToDevice, nullptr);
       if (e == cudaSuccess) e = cudaMemcpyAsync(s->tags + a, bt, size_t(cnt) * sizeof(int32_t), cudaMemcpyDeviceToDevice, nullptr);
       if (e != cudaSuccess) rc = cuda_fail(e, "compact move", __FILE__, __LINE__);
     }
@@ -748,7 +767,7 @@ int frg_store_fill_synthetic(frg_store* s, int64_t n, int64_t global_row0, uint6
   std::lock_guard<std::mutex> lk(s->mu);
   if (s->rows + n > s->capacity) FRG_CHECK(grow_locked(s, s->rows + n));
   FRG_CHECK(store_begin_write(s, st));
-  FRG_CHECK(launch_synth(n, s->rows, global_row0, seed, tag, s->dim, s->master, s->plane, s->plane_dim,
+  FRG_CHECK(launch_synth(n, s->rows, global_row0, seed, tag, s->dim, s->master, s->plane, s->plane8, s->plane_dim,
                          s->gmax_bits, s->tags, st));
   extent_add(s, tag, s->rows, s->rows + n);
   span_add(s, tag, s->rows, s->rows + n);
@@ -767,10 +786,11 @@ static int pick_variant(const frg_store* s, const frg_match_params_t* p, int nq)
   // store's augmented plane (norm terms), its bound scales with the norms (queries.cu).
   const bool unit = !(s->flags & FRG_STORE_RAW) && !(p->flags & FRG_QUERY_PRENORMALISED);
   const bool fits = p->metric == FRG_METRIC_EUCLIDEAN ? s->plane_dim == s->dim + kEuclidPad : unit;
-  const bool tc_ok = s->plane != nullptr && fits && tc_supported(s->dim, p->metric, &why);
+  const bool tc_ok = (p->metric == FRG_METRIC_EUCLIDEAN ? s->plane != nullptr : (s->plane || s->plane8)) && fits &&
+                     tc_supported(s->dim, p->metric, &why);
   if (p->variant != FRG_VARIANT_AUTO) return p->variant;
   if (!s->master) return FRG_VARIANT_TC_BF16;          // bf16-only store: the coarse scores are the scores
-  // dispatch table (DESIGN.md): the tensor-core filter reads 2 B/element instead of 4 and wins from
+  // dispatch table (DESIGN.md): the tensor-core filter reads 1 B/element (int8 plane) instead of 4 and wins from
   // the smallest batches on; the exact scan remains for galleries without a scan plane, for the
   // Euclidean metric and for dims the tile shapes do not cover.
   (void)nq;
@@ -824,10 +844,10 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
                     const ExchangeTail& tail = ExchangeTail()) {
   const char* why = "";
   const bool euclid = p->metric == FRG_METRIC_EUCLIDEAN;
-  if (!s->plane) { set_error("match: the store was created without FRG_STORE_BF16_PLANE"); return FRG_ERR_UNSUPPORTED; }
+  if (!s->plane && !s->plane8) { set_error("match: the store was created without FRG_STORE_BF16_PLANE"); return FRG_ERR_UNSUPPORTED; }
   if (!tc_supported(s->dim, p->metric, &why)) { set_error("match: %s", why); return FRG_ERR_UNSUPPORTED; }
   if (euclid) {
-    if (s->plane_dim != s->dim + kEuclidPad) {
+    if (!s->plane || s->plane_dim != s->dim + kEuclidPad) {
       set_error("match: the Euclidean tensor-core filter needs a FRG_STORE_RAW store with a scan plane");
       return FRG_ERR_UNSUPPORTED;
     }
@@ -845,37 +865,48 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
     set_error("match: FRG_VARIANT_TC_EXACT needs the fp32 master; this store is bf16-only");
     return FRG_ERR_UNSUPPORTED;
   }
+  const char* variant_name = rescore ? "tc_exact" : "tc_bf16";
+  // int8 plane (unit store with a master): there are no bf16 scores to return - FRG_VARIANT_TC_BF16 is served
+  // with exact scores, which meet its tolerance a fortiori
+  const bool i8 = !euclid && s->plane8 != nullptr;
+  if (i8) rescore = true;
   const size_t qn_bytes = (size_t(nq) * s->dim * sizeof(float) + 255) & ~size_t(255);
-  const size_t qb_bytes = (size_t(nq) * (s->dim + (euclid ? kEuclidQPad : 0)) * sizeof(__nv_bfloat16) + 255) & ~size_t(255);
+  const size_t qb_bytes = (size_t(nq) * (s->dim + (euclid ? kEuclidQPad : 0)) * (i8 ? 1 : sizeof(__nv_bfloat16)) + 255) & ~size_t(255);
   const size_t eps_bytes = (size_t(nq) * sizeof(float) + 255) & ~size_t(255);     // per-query filter error bound
   const size_t qb2_bytes = euclid ? qb_bytes : 0;                                 // the pre-pass (lower-bound) image
-  const size_t coef_bytes = euclid ? ((size_t(nq) * 4 * sizeof(float) + 255) & ~size_t(255)) : 0;
+  // Euclidean: the bound coefficients [nq][4]; int8: the per-query step of the integer scores [nq]
+  const size_t coef_bytes = euclid ? ((size_t(nq) * 4 * sizeof(float) + 255) & ~size_t(255)) : i8 ? eps_bytes : 0;
   const int32_t* tile_list = nullptr;
   int n_list = 0;
   const int64_t plan_rows = tc_effective_rows(s, nq, st, &tile_list, &n_list);
   if (plan_rows < 0) return FRG_ERR_CUDA;
   const int plan_dim = euclid ? -s->dim : s->dim;          // (negative: Euclidean plane, tc_plan)
-  const size_t tc_bytes = tc_workspace_bytes(plan_rows, plan_dim, nq, k, sm_count);
+  const size_t tc_bytes = tc_workspace_bytes(plan_rows, plan_dim, nq, k, sm_count, false, i8);
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + qb_bytes + eps_bytes + qb2_bytes + coef_bytes + tc_bytes, st));
   float* qn = reinterpret_cast<float*>(ws);
   __nv_bfloat16* qb = reinterpret_cast<__nv_bfloat16*>(ws + qn_bytes);
   float* eps = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes);
   __nv_bfloat16* qb2 = euclid ? reinterpret_cast<__nv_bfloat16*>(ws + qn_bytes + qb_bytes + eps_bytes) : nullptr;
-  float* coef = euclid ? reinterpret_cast<float*>(ws + qn_bytes + qb_bytes + eps_bytes + qb2_bytes) : nullptr;
+  float* coef = (euclid || i8) ? reinterpret_cast<float*>(ws + qn_bytes + qb_bytes + eps_bytes + qb2_bytes) : nullptr;
   unsigned char* tc_ws = ws + qn_bytes + qb_bytes + eps_bytes + qb2_bytes + coef_bytes;
   int* flagged = nullptr; int* n_flagged = nullptr;
-  uint32_t* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
-  tc_workspace_init_targets(plan_rows, plan_dim, nq, k, sm_count, tc_ws, &keys, &ct0, &nf0);
+  void* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
+  tc_workspace_init_targets(plan_rows, plan_dim, nq, k, sm_count, tc_ws, &keys, &ct0, &nf0, false, i8);
+  int8_t* qi8 = i8 ? reinterpret_cast<int8_t*>(qb) : nullptr;
   profile_begin(st, kStagePrep);
-  int rc = euclid ? launch_prepare_queries_euclid(q, nq, s->dim, s->gmax_bits, qn, qb, qb2, coef, eps, keys, ct0, nf0, st)
-                  : launch_normalise_queries(q, nq, s->dim, !(p->flags & FRG_QUERY_PRENORMALISED), qn, qb, keys, ct0,
-                                             nf0, st, eps, s->gmax_bits);
+  int rc = euclid ? launch_prepare_queries_euclid(q, nq, s->dim, s->gmax_bits, qn, qb, qb2, coef, eps,
+                                                  static_cast<uint32_t*>(keys), ct0, nf0, st)
+           : i8   ? launch_prepare_queries_i8(q, nq, s->dim, qn, qi8, coef, eps, s->gmax_bits,
+                                              static_cast<unsigned long long*>(keys), ct0, nf0, st)
+                  : launch_normalise_queries(q, nq, s->dim, !(p->flags & FRG_QUERY_PRENORMALISED), qn, qb,
+                                             static_cast<uint32_t*>(keys), ct0, nf0, st, eps, s->gmax_bits);
   profile_end(st, 1);
   if (rc == FRG_OK)
-    rc = launch_tc_match(s, p->metric, qn, qb, eps, nq, k, p->tenant, rescore, p->threshold, p->row_offset, tc_ws,
-                         sm_count, tail.active ? tail.x : XPush(), out_rows, out_scores, out_accept, &flagged,
-                         &n_flagged, st, plan_rows, tile_list, n_list, qb2, coef);
+    rc = launch_tc_match(s, p->metric, qn, i8 ? nullptr : qb, eps, nq, k, p->tenant, rescore, p->threshold,
+                         p->row_offset, tc_ws, sm_count, tail.active ? tail.x : XPush(), out_rows, out_scores,
+                         out_accept, &flagged, &n_flagged, st, plan_rows, tile_list, n_list, qb2,
+                         euclid ? coef : nullptr, qi8, i8 ? coef : nullptr);
   if (rc == FRG_OK) {
     // queries whose candidate lists overflowed are redone exactly, inside the same enqueue
     ScanArgs a;
@@ -891,7 +922,7 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
     // to wait for every rank's packets and merge each query's `world` lists as they arrive
     rc = launch_exchange_merge(tail.x, nq, k, p->metric, p->threshold, sm_count, tail.fin_rows, tail.fin_scores,
                                tail.fin_accept, st);
-  g_variant = rescore ? "tc_exact" : "tc_bf16";
+  g_variant = variant_name;
   cudaError_t e = cudaFreeAsync(ws, st);
   if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
   return rc;
@@ -1106,7 +1137,7 @@ int frg_first_match_host(frg_store* s, const float* q, int32_t nq, const frg_mat
 }
 
 // --------------------------------------------------------------------------------------------- range search
-// Tensor-core path (unit cosine stores with a plane and a covered dim): query prep (fp32 unit queries, bf16 image,
+// Tensor-core path (unit cosine stores with a plane and a covered dim): query prep (fp32 unit queries, int8 image,
 // eps[q]) -> filter with the fixed floor threshold - eps[q] -> range_select_kernel -> exact range scan of the
 // queries whose candidates overflowed.  Everything else: the exact range scan over all queries.
 static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
@@ -1131,7 +1162,7 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
   const char* why = "";
   if (!range_scan_supported(s->dim, &why)) { set_error("match_range: %s", why); return FRG_ERR_UNSUPPORTED; }
   const bool unit = !(s->flags & FRG_STORE_RAW) && !(p->flags & FRG_QUERY_PRENORMALISED);
-  const bool tc_ok = s->plane != nullptr && unit && p->metric == FRG_METRIC_COSINE && tc_supported(s->dim, p->metric, &why);
+  const bool tc_ok = s->plane8 != nullptr && unit && p->metric == FRG_METRIC_COSINE && tc_supported(s->dim, p->metric, &why);
   const bool use_tc = p->variant == FRG_VARIANT_TC_EXACT || (p->variant == FRG_VARIANT_AUTO && tc_ok);
   if (use_tc && !tc_ok) {
     set_error("match_range: FRG_VARIANT_TC_EXACT needs a unit-row store with a scan plane, normalised queries and "
@@ -1156,26 +1187,28 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
   unsigned char* ws = nullptr;
   int rc = FRG_OK;
   if (use_tc && w.rows > 0) {
-    const size_t qb_bytes = (size_t(nq) * w.dim * sizeof(__nv_bfloat16) + 255) & ~size_t(255);
+    const size_t qb_bytes = (size_t(nq) * w.dim + 255) & ~size_t(255);              // int8 image
     const size_t eps_bytes = (size_t(nq) * sizeof(float) + 255) & ~size_t(255);
     const int32_t* tile_list = nullptr;
     int n_list = 0;
     const int64_t plan_rows = tc_effective_rows(&w, nq, st, &tile_list, &n_list);
     if (plan_rows < 0) return FRG_ERR_CUDA;
-    const size_t tc_bytes = tc_workspace_bytes(plan_rows, w.dim, nq, 1, di.sm_count, true);
-    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + qb_bytes + eps_bytes + tc_bytes, st));
+    const size_t tc_bytes = tc_workspace_bytes(plan_rows, w.dim, nq, 1, di.sm_count, true, true);
+    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + qb_bytes + 2 * eps_bytes + tc_bytes, st));
     float* qn = reinterpret_cast<float*>(ws);
-    __nv_bfloat16* qb = reinterpret_cast<__nv_bfloat16*>(ws + qn_bytes);
+    int8_t* qi8 = reinterpret_cast<int8_t*>(ws + qn_bytes);
     float* eps = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes);
-    unsigned char* tc_ws = ws + qn_bytes + qb_bytes + eps_bytes;
-    uint32_t* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
-    tc_workspace_init_targets(plan_rows, w.dim, nq, 1, di.sm_count, tc_ws, &keys, &ct0, &nf0, true);
+    float* qstep = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes + eps_bytes);
+    unsigned char* tc_ws = ws + qn_bytes + qb_bytes + 2 * eps_bytes;
+    void* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
+    tc_workspace_init_targets(plan_rows, w.dim, nq, 1, di.sm_count, tc_ws, &keys, &ct0, &nf0, true, true);
     int* flagged = nullptr; int* n_flagged = nullptr;
     profile_begin(st, kStagePrep);
-    rc = launch_normalise_queries(q, nq, w.dim, true, qn, qb, keys, ct0, nf0, st, eps, s->gmax_bits);
+    rc = launch_prepare_queries_i8(q, nq, w.dim, qn, qi8, qstep, eps, s->gmax_bits,
+                                   static_cast<unsigned long long*>(keys), ct0, nf0, st);
     profile_end(st, 1);
     if (rc == FRG_OK)
-      rc = launch_tc_range(&w, qn, qb, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, tc_ws,
+      rc = launch_tc_range(&w, qn, qi8, qstep, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, tc_ws,
                            di.sm_count, out_counts, out_rows, out_scores, &flagged, &n_flagged, st, plan_rows,
                            tile_list, n_list);
     if (rc == FRG_OK) {

@@ -5,6 +5,8 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 
+#include <cmath>
+
 #include <map>
 #include <mutex>
 #include <string>
@@ -149,14 +151,18 @@ struct frg_store {
   int64_t version = 0;
   bool maybe_dead = false;            // a row was tombstoned since the last compaction (or tag -1 was upserted)
   float* master = nullptr;            // [capacity][dim] fp32, unit rows
-  __nv_bfloat16* plane = nullptr;     // [capacity][plane_dim] bf16 image (scan plane) or null
+  __nv_bfloat16* plane = nullptr;     // [capacity][plane_dim] bf16 image (scan plane of raw and bf16-only stores) or null
+  // Unit-row store with FRG_STORE_BF16_PLANE: the scan plane is int8 instead, [capacity][dim], element =
+  // clamp(rint(g / i8_gallery_step(dim)), -127, 127) (plane stays null).  gmax_bits[1] holds its largest residual.
+  int8_t* plane8 = nullptr;
   // plane_dim == dim for unit-row stores.  A FRG_STORE_RAW store's plane is the EUCLIDEAN scan plane:
   // plane_dim = dim + kEuclidPad (16): columns dim..dim+2 hold -0.5*||g||^2 split exactly into three bf16 terms,
   // columns dim+3..dim+5 the row's error-bound terms ||g - bf16(g)||, ||g||, ||g||^2 rounded up (the rest 0), so that
   // Qaug . Gaug = q.g - 0.5*||g||^2 +- bound with Qaug = [q, 1, 1, 1, +-A, +-B, +-C, 0...] (queries.cu, tc_match.cu)
   int plane_dim = 0;
   uint32_t* gmax_bits = nullptr;      // device uint32[2], float bits: [0] max ||g||^2 ever ingested (raw stores with a
-                                      // Euclidean plane), [1] max ||g - bf16(g)||^2 (any store with a plane)
+                                      // Euclidean plane), [1] max ||g - g^||^2 (any store with a plane; g^ = the
+                                      // row's bf16 image, or its int8 image times the store's step)
   int32_t* tags = nullptr;            // [capacity]
   // Fault word in pinned, device-mapped host memory: a kernel whose TMA / MMA pipeline barrier timed out sets it
   // instead of trapping (a trap would kill the CUDA context of the whole service).  Sticky; reported by
@@ -189,10 +195,17 @@ struct frg_store {
 };
 
 namespace frg {
+// Dequantisation step of a unit store's int8 scan plane, fixed per dim: alpha / 127 with alpha = 0.165 * sqrt(512 /
+// dim), i.e. 3.73 standard deviations of an element of a random unit vector.  At dim 512 alpha = 0.165 sits just above
+// the largest element of the synthetic gallery (0.161; its row maxima: median 0.125, 99.9th percentile 0.149), so
+// ordinary rows never saturate; a row that does is clamped to +-127 and its larger residual is measured like any
+// other (gmax_bits[1]), so the filter's bound stays rigorous.
+inline float i8_gallery_step(int dim) { return float(0.165 * std::sqrt(512.0 / double(dim)) / 127.0); }
 // What the match kernels see of a store: the whole gallery, or the row window of one tenant.
 struct GalleryWindow {
   const float* master = nullptr;
   const __nv_bfloat16* plane = nullptr;
+  const int8_t* plane8 = nullptr;
   const int32_t* tags = nullptr;
   uint32_t* gmax_bits = nullptr;
   uint32_t* fault = nullptr;          // frg_store::fault_dev
@@ -232,6 +245,13 @@ int64_t tc_effective_rows(const GalleryWindow* s, int nq, cudaStream_t st, const
 int launch_normalise_queries(const float* q, int nq, int dim, bool normalise, float* qn,
                              __nv_bfloat16* qn_bf16, uint32_t* group_keys, int* cand_total, int* n_flagged,
                              cudaStream_t st, float* eps = nullptr, const uint32_t* bounds = nullptr);
+// queries.cu: the int8 filter's prep (unit store with an int8 plane): qn = unit fp32 queries, qi8 = int8 image
+// rint(qn / c_q) with c_q = max|qn| / 127, qstep[f] = c_q * i8_gallery_step(dim) (S = integer product * qstep),
+// eps[f] = rigorous bound of |S - fp32 score| against any row of the store (bounds[1]: the rows' largest residual).
+// Resets the 64-bit group keys of the pre-pass (group_keys: [nq][32] uint64) and the counters.
+int launch_prepare_queries_i8(const float* q, int nq, int dim, float* qn, int8_t* qi8, float* qstep, float* eps,
+                              const uint32_t* bounds, unsigned long long* group_keys, int* cand_total, int* n_flagged,
+                              cudaStream_t st);
 // queries.cu: Euclidean tensor-core prep: qn = q as given, bf16 image [nq][dim + kEuclidQPad] = [q, 1, 1, 1, 0...],
 // eps[f] = filter error bound of query f from ||q|| and the store's max row norm
 // q_aug: the filter's image [q, 1, 1, 1, +A, +B, +C, 0...], q_aug_lo: the pre-pass image (-A, -B, -C); coef[f][4] = the
@@ -324,10 +344,13 @@ constexpr int kEuclidQPad = 64;     // query image: padded to a whole 128-byte s
 constexpr float kEuclidNone = -3.0e38f;   // "no score yet" of the Euclidean filter (scores are unbounded below)
 int tc_supported(int dim, int metric, const char** why);
 // range: the plan of launch_tc_range (k is ignored there)
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range = false);
+// i8: the int8 filter of a unit store (64-bit group keys, per-query floor)
+size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range = false, bool i8 = false);
+// keys: [nq][32] group keys, uint32 (bf16 filter) or uint64 (int8 filter)
 void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               uint32_t** keys, int** cand_total, int** n_flagged, bool range = false);
-// metric cosine: qb = [nq][dim] bf16 unit queries, eps == nullptr (constant bound).
+                               void** keys, int** cand_total, int** n_flagged, bool range = false, bool i8 = false);
+// metric cosine, int8 plane (s->plane8): qi8 / qstep / eps from launch_prepare_queries_i8, qb unused.
+// metric cosine, bf16 plane (bf16-only store): qb = [nq][dim] bf16 unit queries, eps[nq] per-query bounds.
 // metric euclidean: qb = [nq][dim + kEuclidQPad] augmented image, eps[nq] per-query bounds.
 // push: the select stage sends every query's final top-k straight to all ranks (XPush::peer_bufs != null)
 int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const __nv_bfloat16* qb, const float* eps,
@@ -335,13 +358,14 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
                     unsigned char* ws, int sm_count, const XPush& push, int64_t* out_rows, float* out_scores,
                     uint8_t* out_accept, int** flagged_out, int** n_flagged_out, cudaStream_t st,
                     int64_t plan_rows, const int32_t* tile_list, int n_list,
-                    const __nv_bfloat16* qb_prepass = nullptr, const float* coef = nullptr);
+                    const __nv_bfloat16* qb_prepass = nullptr, const float* coef = nullptr,
+                    const int8_t* qi8 = nullptr, const float* qstep = nullptr);
 
 // tc_match.cu: range search over a unit cosine store (frg_match_range).  The filter keeps every row with
 // S >= threshold - eps[q] (no pre-pass); range_select_kernel rescores each candidate exactly, keeps those that pass
 // (score >= threshold, '>' when strict), writes the first max_hits in gallery order and the count.  Queries whose
 // candidates overflowed the plan are left in (flagged, n_flagged) for launch_range_scan's flagged mode.
-int launch_tc_range(const GalleryWindow* s, const float* qn, const __nv_bfloat16* qb, const float* eps, int nq,
+int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps, int nq,
                     int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned char* ws,
                     int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores, int** flagged_out,
                     int** n_flagged_out, cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list);
@@ -362,15 +386,17 @@ int launch_first_match(const float* master, const int32_t* tags, int64_t rows, i
 
 // store_kernels.cu
 // plane_dim > dim: Euclidean scan plane (bias columns written, gmax_bits folded); else plane_dim == dim
+// plane8: the int8 scan plane of a unit store (written instead of plane, residual folded into gmax_bits[1])
 int launch_ingest(const float* vecs, const int64_t* rows, const int32_t* tags, int64_t n, int64_t append_at,
-                  int dim, bool normalise, float* master, __nv_bfloat16* plane, int plane_dim, uint32_t* gmax_bits,
-                  int32_t* tag_out, cudaStream_t st);
+                  int dim, bool normalise, float* master, __nv_bfloat16* plane, int8_t* plane8, int plane_dim,
+                  uint32_t* gmax_bits, int32_t* tag_out, cudaStream_t st);
 int launch_tombstone(const int64_t* rows, int64_t n, int64_t limit, int32_t* tags, cudaStream_t st);
 int launch_synth(int64_t n, int64_t append_at, int64_t global_row0, uint64_t seed, int32_t tag, int dim,
-                 float* master, __nv_bfloat16* plane, int plane_dim, uint32_t* gmax_bits, int32_t* tag_out,
-                 cudaStream_t st);
-int launch_gather_rows(const int64_t* src_rows, int64_t n, int dim, int plane_dim, const float* master_in,
-                       const __nv_bfloat16* plane_in, const int32_t* tags_in, float* master_out,
-                       __nv_bfloat16* plane_out, int32_t* tags_out, cudaStream_t st);
+                 float* master, __nv_bfloat16* plane, int8_t* plane8, int plane_dim, uint32_t* gmax_bits,
+                 int32_t* tag_out, cudaStream_t st);
+// plane_row_bytes: bytes of a scan-plane row (multiple of 8), 0 = no plane
+int launch_gather_rows(const int64_t* src_rows, int64_t n, int dim, int plane_row_bytes, const float* master_in,
+                       const void* plane_in, const int32_t* tags_in, float* master_out, void* plane_out,
+                       int32_t* tags_out, cudaStream_t st);
 
 }  // namespace frg

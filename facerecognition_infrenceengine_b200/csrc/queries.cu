@@ -1,7 +1,7 @@
 // Query preparation: the reference re-normalises every face embedding before the scan
 // (`face.normed_embedding / np.linalg.norm(face.normed_embedding)`, infrenceServer.py:532,
 // peopleCount.py:863).  One warp per query; writes the fp32 unit query and, for the tensor-core
-// variants, its bf16 image.
+// variants, its bf16 or int8 image.
 #include <cstring>
 
 #include "frg_internal.cuh"
@@ -70,6 +70,89 @@ normalise_queries_kernel(const float* __restrict__ q, int nq, int dim, int norma
       eps[w] = 1.01f * (1.00390625f * __fsqrt_rn(rg) + __fsqrt_rn(rq)) + 1e-4f;
     }
   }
+}
+
+// Int8 filter prep (unit store with an int8 plane, tc_match.cu).  Per query: the unit fp32 query, its int8 image
+// qi = rint(q / c_q) with c_q = max|q| / 127 (no element saturates), the integer product's step
+// qstep = c_q * c_g (S = sum qi * gi * qstep, exact up to that one fp32 product: the tensor core accumulates in s32),
+// and eps = a rigorous bound of |S - s| for every row of the store:
+//   |q^.g^ - q.g| <= ||q^|| ||g^ - g|| + ||q^ - q|| ||g||,   ||q^|| <= 1 + ||q^ - q||,  ||g|| = 1
+// with q^ = c_q qi, g^ = c_g gi, ||g^ - g|| <= sqrt(bounds[1]) (the largest residual of any stored row) and ||q^ - q||
+// measured here.  + 1 % for the fp32 evaluation of the residual norms; + 4e-5 for the fp32 accumulation of the exact
+// scan whose scores are the results (<= dim 2^-24 ||q|| ||g|| = 3.1e-5 at dim 512) and the fp32 conversions of the
+// floor.  ~1.9e-2 for ordinary 512-d data.
+__global__ void __launch_bounds__(128)
+prepare_queries_i8_kernel(const float* __restrict__ q, int nq, int dim, float step_g, float* __restrict__ qn,
+                          int8_t* __restrict__ qi8, float* __restrict__ qstep, float* __restrict__ eps,
+                          const uint32_t* __restrict__ bounds, unsigned long long* __restrict__ group_keys,
+                          int* __restrict__ cand_total, int* __restrict__ n_flagged) {
+  pdl_wait();
+  pdl_trigger();
+  const int lane = threadIdx.x & 31;
+  const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= nq) return;
+  // the pre-pass folds (score, row) keys with a 64-bit atomicMax: 0 = nothing seen
+  group_keys[size_t(w) * 32 + lane] = 0ull;
+  if (lane == 0) cand_total[w] = 0;
+  if (w == 0 && lane < 3) n_flagged[lane] = 0;      // count, ticket, probe arrivals
+  const float4* src = reinterpret_cast<const float4*>(q + size_t(w) * dim);
+  float4* dst = reinterpret_cast<float4*>(qn + size_t(w) * dim);
+  const int nvec = dim >> 2;
+  float ss = 0.f;
+  for (int v = lane; v < nvec; v += 32) {
+    const float4 x = __ldg(src + v);
+    ss = fmaf(x.x, x.x, ss); ss = fmaf(x.y, x.y, ss); ss = fmaf(x.z, x.z, ss); ss = fmaf(x.w, x.w, ss);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+  const float norm = __fsqrt_rn(ss);
+  float amax = 0.f;
+  for (int v = lane; v < nvec; v += 32) {
+    float4 x = __ldg(src + v);
+    x.x = __fdiv_rn(x.x, norm); x.y = __fdiv_rn(x.y, norm);
+    x.z = __fdiv_rn(x.z, norm); x.w = __fdiv_rn(x.w, norm);
+    dst[v] = x;
+    amax = fmaxf(amax, fmaxf(fmaxf(fabsf(x.x), fabsf(x.y)), fmaxf(fabsf(x.z), fabsf(x.w))));
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, o));
+  // a zero / non-finite query (NaN elements: no row can match it) keeps step 1 and an all-zero image; its eps is NaN
+  const float c_q = amax > 0.f && amax < INFINITY ? amax / 127.f : 1.f;
+  float rq = ss == ss && norm > 0.f ? 0.f : NAN;
+  for (int v = lane; v < nvec; v += 32) {
+    const float4 x4 = dst[v];                  // this lane's own writes
+    const float x[4] = {x4.x, x4.y, x4.z, x4.w};
+    uint32_t packed = 0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      float t = rintf(__fdiv_rn(x[e], c_q));
+      t = t == t ? fminf(fmaxf(t, -127.f), 127.f) : 0.f;
+      const float d = fmaf(-t, c_q, x[e]);
+      rq = fmaf(d, d, rq);
+      packed |= (uint32_t(int(t)) & 0xFFu) << (8 * e);
+    }
+    reinterpret_cast<uint32_t*>(qi8 + size_t(w) * dim)[v] = packed;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) rq += __shfl_xor_sync(0xffffffffu, rq, o);
+  if (lane == 0) {
+    const float rq_n = __fsqrt_rn(rq);
+    const float rg_n = __fsqrt_rn(__uint_as_float(bounds[1]));
+    qstep[w] = c_q * step_g;
+    eps[w] = 1.01f * ((1.0f + rq_n) * rg_n + rq_n) + 4e-5f;
+  }
+}
+
+int launch_prepare_queries_i8(const float* q, int nq, int dim, float* qn, int8_t* qi8, float* qstep, float* eps,
+                              const uint32_t* bounds, unsigned long long* group_keys, int* cand_total, int* n_flagged,
+                              cudaStream_t st) {
+  if (nq <= 0) return FRG_OK;
+  FRG_CUDA(func_attr_once(prepare_queries_i8_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+  FRG_CUDA(launch_kernel(prepare_queries_i8_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, true, q, nq, dim,
+                         i8_gallery_step(dim), qn, qi8, qstep, eps, bounds, group_keys, cand_total, n_flagged));
+  note_launch(nullptr);
+  FRG_CUDA(cudaGetLastError());
+  return FRG_OK;
 }
 
 __device__ __forceinline__ uint32_t bf16_up_bits(float x) {      // smallest bf16 >= x, x >= 0

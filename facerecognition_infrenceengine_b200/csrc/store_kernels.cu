@@ -1,4 +1,4 @@
-// Gallery-store kernels: ingest (normalise + write master / bf16 plane / tag), tombstone, stable
+// Gallery-store kernels: ingest (normalise + write master / scan plane (bf16 or int8) / tag), tombstone, stable
 // gather (compaction) and the synthetic generator.  All are HBM-bound row movers: one warp per
 // row, 16-byte accesses, no shared memory.
 #include "frg_internal.cuh"
@@ -24,8 +24,26 @@ __device__ __forceinline__ float store_bf16x4(__nv_bfloat16* dst, float4 v) {
   return fmaf(a, a, fmaf(b, b, fmaf(c, c, d * d)));
 }
 
+// writes the int8 image of v (step c: element = clamp(rint(x / c), -127, 127), NaN -> 0) and returns ||v - c * i8(v)||^2
+// of the four elements.  Saturated elements are clamped, not wrapped: their larger residual is part of the sum.
+__device__ __forceinline__ float store_i8x4(int8_t* dst, float4 v, float c) {
+  const float x[4] = {v.x, v.y, v.z, v.w};
+  uint32_t packed = 0;
+  float rr = 0.f;
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    float t = rintf(__fdiv_rn(x[e], c));
+    t = t == t ? fminf(fmaxf(t, -127.f), 127.f) : 0.f;
+    const float d = fmaf(-t, c, x[e]);
+    rr = fmaf(d, d, rr);
+    packed |= (uint32_t(int(t)) & 0xFFu) << (8 * e);
+  }
+  *reinterpret_cast<uint32_t*>(dst) = packed;
+  return rr;
+}
+
 // The tensor-core filter's error bound is DATA-DEPENDENT and rigorous: |q^.g^ - q.g| <= ||q^|| ||g^ - g|| +
-// ||q^ - q|| ||g|| (q^, g^ the bf16 images).  bounds[1] keeps the largest ||g^ - g||^2 of any row ever stored
+// ||q^ - q|| ||g|| (q^, g^ the bf16 images, or the int8 images times their steps).  bounds[1] keeps the largest ||g^ - g||^2 of any row ever stored
 // (non-negative floats order like their bit patterns); the query side is measured per query (queries.cu).
 // A NaN row (zero vector) is left out: it can never match either way.
 __device__ __forceinline__ float fold_residual(uint32_t* bounds, float rr, int lane) {
@@ -75,8 +93,9 @@ __device__ __forceinline__ void store_bias_columns(__nv_bfloat16* row_aug, float
 __global__ void __launch_bounds__(256)
 ingest_kernel(const float* __restrict__ vecs, const int64_t* __restrict__ rows,
               const int32_t* __restrict__ tags, int64_t n, int64_t append_at, int64_t limit, int dim,
-              int normalise, float* __restrict__ master, __nv_bfloat16* __restrict__ plane, int plane_dim,
-              uint32_t* __restrict__ gmax_bits, int32_t* __restrict__ tag_out) {
+              int normalise, float* __restrict__ master, __nv_bfloat16* __restrict__ plane,
+              int8_t* __restrict__ plane8, float step8, int plane_dim, uint32_t* __restrict__ gmax_bits,
+              int32_t* __restrict__ tag_out) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = (int64_t(gridDim.x) * blockDim.x) >> 5;
@@ -107,8 +126,9 @@ ingest_kernel(const float* __restrict__ vecs, const int64_t* __restrict__ rows,
       ss_stored = fmaf(x.z, x.z, ss_stored); ss_stored = fmaf(x.w, x.w, ss_stored);
       if (m) m[v] = x;
       if (plane) rr += store_bf16x4(plane + dst * plane_dim + v * 4, x);
+      if (plane8) rr += store_i8x4(plane8 + dst * dim + v * 4, x, step8);
     }
-    if (plane) rr = fold_residual(gmax_bits, rr, lane);
+    if (plane || plane8) rr = fold_residual(gmax_bits, rr, lane);
     if (plane && plane_dim > dim) store_bias_columns(plane + dst * plane_dim + dim, warp_sum(ss_stored), rr, gmax_bits, lane);
     if (lane == 0) tag_out[dst] = tags ? tags[i] : 0;
   }
@@ -124,10 +144,10 @@ __global__ void tombstone_kernel(const int64_t* __restrict__ rows, int64_t n, in
 }
 
 __global__ void __launch_bounds__(256)
-gather_rows_kernel(const int64_t* __restrict__ src_rows, int64_t n, int dim, int plane_dim,
-                   const float* __restrict__ master_in, const __nv_bfloat16* __restrict__ plane_in,
+gather_rows_kernel(const int64_t* __restrict__ src_rows, int64_t n, int dim, int plane_row_bytes,
+                   const float* __restrict__ master_in, const unsigned char* __restrict__ plane_in,
                    const int32_t* __restrict__ tags_in, float* __restrict__ master_out,
-                   __nv_bfloat16* __restrict__ plane_out, int32_t* __restrict__ tags_out) {
+                   unsigned char* __restrict__ plane_out, int32_t* __restrict__ tags_out) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = (int64_t(gridDim.x) * blockDim.x) >> 5;
@@ -140,9 +160,9 @@ gather_rows_kernel(const int64_t* __restrict__ src_rows, int64_t n, int dim, int
       for (int v = lane; v < nvec; v += 32) mo[v] = mi[v];
     }
     if (plane_in) {
-      const uint2* pi = reinterpret_cast<const uint2*>(plane_in + s * plane_dim);
-      uint2* po = reinterpret_cast<uint2*>(plane_out + i * plane_dim);
-      for (int v = lane; v < (plane_dim >> 2); v += 32) po[v] = pi[v];
+      const uint2* pi = reinterpret_cast<const uint2*>(plane_in + s * plane_row_bytes);
+      uint2* po = reinterpret_cast<uint2*>(plane_out + i * plane_row_bytes);
+      for (int v = lane; v < (plane_row_bytes >> 3); v += 32) po[v] = pi[v];
     }
     if (lane == 0) tags_out[i] = tags_in[s];
   }
@@ -170,8 +190,8 @@ __device__ __forceinline__ int nibble_sum(uint32_t h) {
 // for dim <= 1024).  sum(x^2) is an exact integer, so norm and quotients are bit-identical to numpy.
 __global__ void __launch_bounds__(256)
 synth_kernel(int64_t n, int64_t append_at, int64_t global_row0, uint32_t k0, uint32_t k1, int32_t tag,
-             int dim, float* __restrict__ master, __nv_bfloat16* __restrict__ plane, int plane_dim,
-             uint32_t* __restrict__ gmax_bits, int32_t* __restrict__ tag_out) {
+             int dim, float* __restrict__ master, __nv_bfloat16* __restrict__ plane, int8_t* __restrict__ plane8,
+             float step8, int plane_dim, uint32_t* __restrict__ gmax_bits, int32_t* __restrict__ tag_out) {
   const int lane = threadIdx.x & 31;
   const int64_t warp = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int64_t nwarps = (int64_t(gridDim.x) * blockDim.x) >> 5;
@@ -217,13 +237,17 @@ synth_kernel(int64_t n, int64_t append_at, int64_t global_row0, uint32_t k0, uin
           rr += store_bf16x4(plane + dst * plane_dim + b * 8, lo);
           rr += store_bf16x4(plane + dst * plane_dim + b * 8 + 4, hi);
         }
+        if (plane8) {
+          rr += store_i8x4(plane8 + dst * dim + b * 8, lo, step8);
+          rr += store_i8x4(plane8 + dst * dim + b * 8 + 4, hi, step8);
+        }
         ss_stored = fmaf(lo.x, lo.x, ss_stored); ss_stored = fmaf(lo.y, lo.y, ss_stored);
         ss_stored = fmaf(lo.z, lo.z, ss_stored); ss_stored = fmaf(lo.w, lo.w, ss_stored);
         ss_stored = fmaf(hi.x, hi.x, ss_stored); ss_stored = fmaf(hi.y, hi.y, ss_stored);
         ss_stored = fmaf(hi.z, hi.z, ss_stored); ss_stored = fmaf(hi.w, hi.w, ss_stored);
       }
     }
-    if (plane) rr = fold_residual(gmax_bits, rr, lane);
+    if (plane || plane8) rr = fold_residual(gmax_bits, rr, lane);
     if (plane && plane_dim > dim) store_bias_columns(plane + dst * plane_dim + dim, warp_sum(ss_stored), rr, gmax_bits, lane);
     if (lane == 0) tag_out[dst] = tag;
   }
@@ -237,14 +261,14 @@ static int grid_for_rows(int64_t n, int warps_per_block) {
 }
 
 int launch_ingest(const float* vecs, const int64_t* rows, const int32_t* tags, int64_t n, int64_t append_at,
-                  int dim, bool normalise, float* master, __nv_bfloat16* plane, int plane_dim, uint32_t* gmax_bits,
-                  int32_t* tag_out, cudaStream_t st) {
+                  int dim, bool normalise, float* master, __nv_bfloat16* plane, int8_t* plane8, int plane_dim,
+                  uint32_t* gmax_bits, int32_t* tag_out, cudaStream_t st) {
   if (n <= 0) return FRG_OK;
   // limit: appended rows land below append_at + n, in-place rows below append_at
   const int64_t limit = rows ? append_at : append_at + n;
   ingest_kernel<<<grid_for_rows(n, 8), 256, 0, st>>>(vecs, rows, tags, n, append_at, limit, dim,
-                                                     normalise ? 1 : 0, master, plane, plane_dim, gmax_bits,
-                                                     tag_out);
+                                                     normalise ? 1 : 0, master, plane, plane8, i8_gallery_step(dim),
+                                                     plane_dim, gmax_bits, tag_out);
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   return FRG_OK;
@@ -259,23 +283,24 @@ int launch_tombstone(const int64_t* rows, int64_t n, int64_t limit, int32_t* tag
 }
 
 int launch_synth(int64_t n, int64_t append_at, int64_t global_row0, uint64_t seed, int32_t tag, int dim,
-                 float* master, __nv_bfloat16* plane, int plane_dim, uint32_t* gmax_bits, int32_t* tag_out,
-                 cudaStream_t st) {
+                 float* master, __nv_bfloat16* plane, int8_t* plane8, int plane_dim, uint32_t* gmax_bits,
+                 int32_t* tag_out, cudaStream_t st) {
   if (n <= 0) return FRG_OK;
   synth_kernel<<<grid_for_rows(n, 8), 256, 0, st>>>(n, append_at, global_row0, uint32_t(seed),
-                                                    uint32_t(seed >> 32), tag, dim, master, plane, plane_dim,
-                                                    gmax_bits, tag_out);
+                                                    uint32_t(seed >> 32), tag, dim, master, plane, plane8,
+                                                    i8_gallery_step(dim), plane_dim, gmax_bits, tag_out);
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   return FRG_OK;
 }
 
-int launch_gather_rows(const int64_t* src_rows, int64_t n, int dim, int plane_dim, const float* master_in,
-                       const __nv_bfloat16* plane_in, const int32_t* tags_in, float* master_out,
-                       __nv_bfloat16* plane_out, int32_t* tags_out, cudaStream_t st) {
+int launch_gather_rows(const int64_t* src_rows, int64_t n, int dim, int plane_row_bytes, const float* master_in,
+                       const void* plane_in, const int32_t* tags_in, float* master_out, void* plane_out,
+                       int32_t* tags_out, cudaStream_t st) {
   if (n <= 0) return FRG_OK;
-  gather_rows_kernel<<<grid_for_rows(n, 8), 256, 0, st>>>(src_rows, n, dim, plane_dim, master_in, plane_in, tags_in,
-                                                          master_out, plane_out, tags_out);
+  gather_rows_kernel<<<grid_for_rows(n, 8), 256, 0, st>>>(src_rows, n, dim, plane_in ? plane_row_bytes : 0, master_in,
+                                                          static_cast<const unsigned char*>(plane_in), tags_in,
+                                                          master_out, static_cast<unsigned char*>(plane_out), tags_out);
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   return FRG_OK;

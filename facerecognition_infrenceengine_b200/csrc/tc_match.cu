@@ -148,6 +148,15 @@ __device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, 
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                             uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // arrives on the same-offset mbarrier of BOTH CTAs of the pair once the issued MMAs have retired
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
   asm volatile(
@@ -178,12 +187,23 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
+                                        uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // arrives on the mbarrier once every previously issued tcgen05.mma of this thread has completed
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
+template <typename T>     // float (kind::f16 accumulators) or int (kind::i8)
+__device__ __forceinline__ void tmem_ld32(uint32_t taddr, T (&v)[32]) {
+  static_assert(sizeof(T) == 4, "32-bit accumulators");
   uint32_t* r = reinterpret_cast<uint32_t*>(v);
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32"
@@ -198,7 +218,7 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-// K-major, 128B-swizzled operand tile: rows of 64 bf16 (128 B), 8-row groups 1024 B apart.
+// K-major, 128B-swizzled operand tile: rows of 64 bf16 or 128 int8 (128 B), 8-row groups 1024 B apart.
 // Field layout: start>>4 [0,14) | LBO>>4 [16,30) | SBO>>4 [32,46) | version=1 [46,48) | swizzle [61,64).
 __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
   return uint64_t((smem_addr & 0x3FFFFu) >> 4) | (uint64_t(1) << 16) | (uint64_t(1024 >> 4) << 32) |
@@ -216,6 +236,7 @@ __device__ __forceinline__ uint64_t umma_desc_sw32(uint32_t smem_addr) {
 constexpr int kTileQ = 128;          // queries per CTA tile (TMEM lanes); UMMA M = 128, or 256 across a CTA pair
 constexpr int kTileR = 128;          // gallery rows staged per CTA and k-block (TMA box rows)
 constexpr int kBlockK = 64;          // one 128-byte swizzle row of bf16
+constexpr int kBlockKI8 = 128;       // ... of int8
 constexpr int kMaxStages = 8;        // ring depth: 6 by default (all a 512-column query tile leaves room for)
 constexpr int kMaxKBlocks = 8;       // 512 columns / 64
 constexpr int kStageBytes = kTileR * kBlockK * 2;          // 16 KB
@@ -229,6 +250,26 @@ constexpr float kCoarseEps = 7.9e-3f;                      // a-priori |bf16 fil
 constexpr uint32_t make_idesc(int m, int n) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(n >> 3) << 17) | (uint32_t(m >> 4) << 24);
 }
+// kind::i8: D=s32 [4,6)=2, A=signed int8 [7,10)=1, B=signed int8 [10,13)=1, K-major both, same N / M fields
+constexpr uint32_t make_idesc_i8(int m, int n) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | (uint32_t(n >> 3) << 17) | (uint32_t(m >> 4) << 24);
+}
+
+// The epilogue's element: fp32 scores of the bf16 filter, raw s32 products of the int8 filter (compared with an
+// integer floor: one IMNMX per score, no conversion)
+template <bool I8> struct Acc;
+template <> struct Acc<false> {
+  using T = float;
+  static __device__ __forceinline__ T none() { return -INFINITY; }
+  static __device__ __forceinline__ T mx(T a, T b) { return fmaxf(a, b); }
+  static __device__ __forceinline__ int bits(T a) { return __float_as_int(a); }
+};
+template <> struct Acc<true> {
+  using T = int;
+  static __device__ __forceinline__ T none() { return INT_MIN; }
+  static __device__ __forceinline__ T mx(T a, T b) { return max(a, b); }
+  static __device__ __forceinline__ int bits(T a) { return a; }
+};
 
 enum TcMode { kModeGroupMax = 0, kModeFilter = 1, kModeFused = 2 };
 constexpr int kGroups = 32;
@@ -237,7 +278,7 @@ constexpr int kGroups = 32;
 // (query, group) on order-preserving keys)
 
 struct TcScanParams {
-  int dim;                 // 512 etc. (multiple of 64)
+  int dim;                 // 512 etc. (multiple of 64; of 128 for the int8 filter)
   int n_rows;              // gallery rows
   int tile_scale;          // pre-pass: only every tile_scale-th 128-row tile is visited (1 = all)
   int nq;                  // real queries
@@ -245,6 +286,12 @@ struct TcScanParams {
   const int32_t* tags;     // per REAL row
   // GROUPMAX output: [nq][32] maxima of the row groups (row mod 32) as ordered keys, atomicMax-folded
   uint32_t* group_key;
+  // int8 filter: GROUPMAX folds [nq][32] 64-bit keys (s32 product biased by 2^31 << 32 | row): each group's winning
+  // row is known, i8_floor_kernel rescores the k best of them exactly.  FILTER reads floor[q] (a floor of the exact
+  // score, float) and qstep[q] (S = s32 product * qstep) and compares with the integer floor derived from them.
+  unsigned long long* group_key64;
+  const float* floor;
+  const float* qstep;
   // FILTER inputs / outputs
   int k;                   // L[q] = k-th largest of the 32 group maxima (computed in the prologue)
   int* arrive;             // FUSED: CTAs that have published their probe-tile maxima
@@ -280,13 +327,20 @@ struct TcScanParams {
 // owns the full/tmem_empty barriers and issues the MMAs; commits are multicast to both CTAs.
 // GROUPED (FILTER mode): the block maximum is built from four 8-column group maxima, and a thread that holds a
 // candidate visits only the group(s) that contain one - the rare path costs a quarter of the 32-column walk.
-template <int MODE, bool MASKED, bool PAIR, bool GROUPED = false>
+// I8: int8 operands (unit cosine store's int8 plane): tcgen05.mma kind::i8, K = 32 per MMA, 128 int8 per k-block,
+// exact s32 accumulators; half the MMA time and half the plane bytes of bf16 per score.  Not FUSED.
+template <int MODE, bool MASKED, bool PAIR, bool GROUPED = false, bool I8 = false>
 __global__ void __launch_bounds__(kTcThreads, 1)
 tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant__ CUtensorMap g_map,
                const __grid_constant__ CUtensorMap pad_map, const TcScanParams p) {
+  static_assert(!(I8 && MODE == kModeFused), "the int8 filter takes its floor from i8_floor_kernel");
+  using A = Acc<I8>;
+  using AccT = typename A::T;
   constexpr int kAccN = PAIR ? 2 * kTileR : kTileR;        // accumulator columns = gallery rows per tile
   constexpr int kTmemCols = 2 * kAccN;
-  constexpr uint32_t kIdesc = make_idesc(PAIR ? 2 * kTileQ : kTileQ, kAccN);
+  constexpr int kBlk = I8 ? kBlockKI8 : kBlockK;             // elements per 128-byte k-block
+  constexpr uint32_t kIdesc = I8 ? make_idesc_i8(PAIR ? 2 * kTileQ : kTileQ, kAccN)
+                                 : make_idesc(PAIR ? 2 * kTileQ : kTileQ, kAccN);
   const uint32_t cta_rank = PAIR ? cluster_ctarank() : 0u;
   const bool leader = cta_rank == 0;
   extern __shared__ unsigned char smem_raw[];
@@ -294,8 +348,8 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
   unsigned char* sm = smem_raw + (base - raw);
-  const int kblocks = p.dim / kBlockK;
-  const uint32_t q_bytes = uint32_t(kTileQ) * p.dim * 2;            // resident query tile
+  const int kblocks = p.dim / kBlk;
+  const uint32_t q_bytes = uint32_t(kTileQ) * p.dim * (I8 ? 1 : 2);   // resident query tile
   const uint32_t q_smem = base;
   const uint32_t stage_smem = base + q_bytes;
   const int nstages = p.stages;
@@ -359,7 +413,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
       tma_prefetch_desc(&g_map);
       if (p.pad) tma_prefetch_desc(&pad_map);
       const uint64_t g_hint = gridDim.x > (PAIR ? 2 : 1) ? kEvictLast : kEvictFirst;
-      constexpr uint32_t kQBlockBytes = kTileQ * kBlockK * 2;
+      constexpr uint32_t kQBlockBytes = kTileQ * 128;
       int stage = 0; uint32_t phase = 0;
       for (int it = 0; it < n_iter && !*abort_flag; ++it) {
         const int t = tile_of(it);
@@ -369,17 +423,17 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
             // the query tile's k-block kb, issued just ahead of the first gallery block that meets it
             if (PAIR) {
               if (leader) mbar_expect_tx(bar_q(kb), 2 * kQBlockBytes);
-              tma_load_2d_pair(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlockK, qtile * kTileQ, kEvictLast);
+              tma_load_2d_pair(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlk, qtile * kTileQ, kEvictLast);
             } else {
               mbar_expect_tx(bar_q(kb), kQBlockBytes);
-              tma_load_2d(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlockK, qtile * kTileQ, kEvictLast);
+              tma_load_2d(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlk, qtile * kTileQ, kEvictLast);
             }
           }
           mbar_wait(bar_empty(stage), phase ^ 1, abort_flag);
           const bool padkb = p.pad && kb == kblocks - 1;
           const CUtensorMap* map = padkb ? &pad_map : &g_map;
           const uint32_t bytes = padkb ? kPadStageBytes : kStageBytes;
-          const int c0 = padkb ? 0 : kb * kBlockK;
+          const int c0 = padkb ? 0 : kb * kBlk;
           if (PAIR) {
             if (leader) mbar_expect_tx(bar_full(stage), 2 * bytes);
             tma_load_2d_pair(stage_smem + stage * kStageBytes, map, bar_full(stage), c0, row0, g_hint);
@@ -412,7 +466,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
           mbar_wait(bar_full(stage), phase, abort_flag);
           tc_fence_after();
           // descriptor start-address field is (addr >> 4): a k-block of A is 16 KB, a stage of B 16 KB
-          const uint64_t a0 = a_base + uint64_t(kb * ((kTileQ * kBlockK * 2) >> 4));
+          const uint64_t a0 = a_base + uint64_t(kb * ((kTileQ * 128) >> 4));
           const uint64_t b0 = b_base + uint64_t(stage * (kStageBytes >> 4));
           const bool padkb = p.pad && kb == kblocks - 1;
           if (elect_one()) {
@@ -423,11 +477,16 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
               else umma_bf16(d_tmem, a0, bp, kIdesc, 1u);
             } else {
 #pragma unroll
-              for (int kk = 0; kk < kBlockK / 16; ++kk) {
-                // advance 16 bf16 = 32 bytes along K inside the swizzle row: +2 in the (addr >> 4) field
+              for (int kk = 0; kk < 4; ++kk) {
+                // advance one MMA's K (16 bf16 / 32 int8) = 32 bytes inside the swizzle row: +2 in the (addr >> 4) field
                 const uint32_t acc = (kb | kk) != 0 ? 1u : 0u;
-                if (PAIR) umma_bf16_pair(d_tmem, a0 + uint64_t(kk * 2), b0 + uint64_t(kk * 2), kIdesc, acc);
-                else umma_bf16(d_tmem, a0 + uint64_t(kk * 2), b0 + uint64_t(kk * 2), kIdesc, acc);
+                if (I8) {
+                  if (PAIR) umma_i8_pair(d_tmem, a0 + uint64_t(kk * 2), b0 + uint64_t(kk * 2), kIdesc, acc);
+                  else umma_i8(d_tmem, a0 + uint64_t(kk * 2), b0 + uint64_t(kk * 2), kIdesc, acc);
+                } else {
+                  if (PAIR) umma_bf16_pair(d_tmem, a0 + uint64_t(kk * 2), b0 + uint64_t(kk * 2), kIdesc, acc);
+                  else umma_bf16(d_tmem, a0 + uint64_t(kk * 2), b0 + uint64_t(kk * 2), kIdesc, acc);
+                }
               }
             }
             // smem slot reusable / accumulator readable once these MMAs retire (both CTAs in pair mode)
@@ -459,8 +518,11 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     const int q = qtile * kTileQ + q_local;
     const bool q_real = q < p.nq;
 
-    float gmax[kGroups];                                 // GROUPMAX / FUSED probe: running maximum per row group
-    float thr = INFINITY;
+    AccT gmax[kGroups];                                  // GROUPMAX / FUSED probe: running maximum per row group
+    int gblk[kGroups];                                   // I8 GROUPMAX: 32-row block of each group's maximum
+    AccT thr;
+    if constexpr (I8) thr = INT_MAX;
+    else thr = INFINITY;
     int emitted = 0;
     int2* my_seg = nullptr;
     // L[q] = k-th largest of the 32 group maxima published so far.  The groups are disjoint row sets,
@@ -498,12 +560,25 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
       const float eps_q = p.eps ? __ldg(p.eps + q) : kCoarseEps;
       return (floor_v <= p.none_score) ? -3.0e38f : floor_v - 2.0f * eps_q;
     };
+    // int8 filter: the integer floor of the s32 products, from the float floor (i8_floor_kernel, or threshold - eps
+    // for a range search) and the query's step, rounded down with a margin of 3 (|floor / qstep| < 2^23: the fp32
+    // quotient is within 1 of the real one).  NaN floor (a NaN query, which no row can match): no candidates.
+    auto derive_thr_i8 = [&]() {
+      const float f = __ldg(p.floor + q);
+      if (!(f == f)) return INT_MAX;
+      const float t = fminf(fmaxf(__fdiv_rn(f, __ldg(p.qstep + q)), -1.0e9f), 1.0e9f);
+      return __float2int_rd(t) - 3;
+    };
     if (MODE != kModeFilter) {
 #pragma unroll
-      for (int j = 0; j < kGroups; ++j) gmax[j] = p.none_score;
+      for (int j = 0; j < kGroups; ++j) {
+        if constexpr (I8) { gmax[j] = A::none(); gblk[j] = 0; }
+        else gmax[j] = p.none_score;
+      }
     }
     if (MODE != kModeGroupMax && q_real) {
-      if (MODE == kModeFilter) thr = derive_thr();
+      if constexpr (I8) thr = derive_thr_i8();
+      else if (MODE == kModeFilter) thr = derive_thr();
       my_seg = p.cand + ((size_t(q) * chunks + chunk) * (kEpiWarps / 4) + half) * p.seg;
     }
 
@@ -538,37 +613,45 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
       const uint32_t taddr = tmem_base + (uint32_t(quarter * 32) << 16) +
                              uint32_t(buf * kAccN + half * kBlocksPerWarp * 32);
       // software-pipelined TMEM reads: the load of block b+1 is in flight while block b is processed
-      float va[32], vb[32];
-      auto process = [&](float (&v)[32], int b) {
+      AccT va[32], vb[32];
+      auto process = [&](AccT (&v)[32], int b) {
         const uint32_t vm = vmask[b];
         if (vm != 0xffffffffu) {           // warp-uniform: tombstones / other tenants / rows past the end
 #pragma unroll
-          for (int j = 0; j < 32; ++j) v[j] = (vm >> j) & 1u ? v[j] : -INFINITY;
+          for (int j = 0; j < 32; ++j) v[j] = (vm >> j) & 1u ? v[j] : A::none();
         }
         if (MODE == kModeGroupMax) {
           // column j of every 32-row block belongs to group j (tiles start at multiples of 32)
+          if constexpr (I8) {
+            const int blk = (tile_row0 >> 5) + b;
 #pragma unroll
-          for (int j = 0; j < 32; ++j) gmax[j] = fmaxf(gmax[j], v[j]);
+            for (int j = 0; j < 32; ++j) {
+              if (v[j] > gmax[j]) { gmax[j] = v[j]; gblk[j] = blk; }
+            }
+          } else {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) gmax[j] = fmaxf(gmax[j], v[j]);
+          }
         } else if (MODE == kModeFused && probe) {
           // this warp sees half of the tile's rows: it owns 16 of the 32 groups, (column mod 16)
 #pragma unroll
-          for (int j = 0; j < 32; ++j) gmax[j & 15] = fmaxf(gmax[j & 15], v[j]);
+          for (int j = 0; j < 32; ++j) gmax[j & 15] = A::mx(gmax[j & 15], v[j]);
         } else if (GROUPED) {
-          float g0 = v[0], g1 = v[8], g2 = v[16], g3 = v[24];
+          AccT g0 = v[0], g1 = v[8], g2 = v[16], g3 = v[24];
 #pragma unroll
           for (int j = 1; j < 8; ++j) {
-            g0 = fmaxf(g0, v[j]); g1 = fmaxf(g1, v[8 + j]); g2 = fmaxf(g2, v[16 + j]); g3 = fmaxf(g3, v[24 + j]);
+            g0 = A::mx(g0, v[j]); g1 = A::mx(g1, v[8 + j]); g2 = A::mx(g2, v[16 + j]); g3 = A::mx(g3, v[24 + j]);
           }
-          if (fmaxf(fmaxf(g0, g1), fmaxf(g2, g3)) >= thr) {
+          if (A::mx(A::mx(g0, g1), A::mx(g2, g3)) >= thr) {
             const int row0 = tile_row0 + (half * kBlocksPerWarp + b) * 32;
-            const float gm[4] = {g0, g1, g2, g3};
+            const AccT gm[4] = {g0, g1, g2, g3};
 #pragma unroll
             for (int g = 0; g < 4; ++g) {
               if (gm[g] >= thr) {
 #pragma unroll
                 for (int j = 8 * g; j < 8 * g + 8; ++j) {
                   if (v[j] >= thr) {
-                    if (emitted < p.seg) my_seg[emitted] = make_int2(row0 + j, __float_as_int(v[j]));
+                    if (emitted < p.seg) my_seg[emitted] = make_int2(row0 + j, A::bits(v[j]));
                     ++emitted;
                   }
                 }
@@ -576,15 +659,15 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
             }
           }
         } else {
-          float m = v[0];
+          AccT m = v[0];
 #pragma unroll
-          for (int j = 1; j < 32; ++j) m = fmaxf(m, v[j]);
+          for (int j = 1; j < 32; ++j) m = A::mx(m, v[j]);
           if (m >= thr) {
             const int row0 = tile_row0 + (half * kBlocksPerWarp + b) * 32;
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               if (v[j] >= thr) {
-                if (emitted < p.seg) my_seg[emitted] = make_int2(row0 + j, __float_as_int(v[j]));
+                if (emitted < p.seg) my_seg[emitted] = make_int2(row0 + j, A::bits(v[j]));
                 ++emitted;
               }
             }
@@ -612,7 +695,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
       }
       if (++buf == 2) { buf = 0; tphase ^= 1; }
 
-      if (MODE == kModeFused) {
+      if constexpr (MODE == kModeFused && !I8) {
         const int since = it - (n_probe - 1);           // 0 at the last probe tile
         if (since == 0) {
           // publish the probe tile's maxima (groups half*16 .. +15), tell the grid, derive the floor
@@ -641,10 +724,18 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     }
     if (q_real && !idle) {
       if (MODE == kModeGroupMax) {
-        uint32_t* o = p.group_key + size_t(q) * kGroups;
+        if constexpr (I8) {
+          unsigned long long* o = p.group_key64 + size_t(q) * kGroups;
 #pragma unroll
-        for (int j = 0; j < kGroups; ++j)
-          if (gmax[j] > p.none_score) atomicMax(o + j, float_key(gmax[j]));
+          for (int j = 0; j < kGroups; ++j)
+            if (gmax[j] != A::none())
+              atomicMax(o + j, (uint64_t(uint32_t(gmax[j]) ^ 0x80000000u) << 32) | uint32_t(gblk[j] * 32 + j));
+        } else {
+          uint32_t* o = p.group_key + size_t(q) * kGroups;
+#pragma unroll
+          for (int j = 0; j < kGroups; ++j)
+            if (gmax[j] > p.none_score) atomicMax(o + j, float_key(gmax[j]));
+        }
       } else {
         // pack this thread's few candidates into the query's dense list: one atomicAdd per (query, CTA),
         // outside the scan loop.  A private-segment overflow poisons the total so that select flags it
@@ -669,9 +760,53 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
   }
 }
 
+// ------------------------------------------------------------------------------------------ int8 floor
+// One warp per query, between the int8 pre-pass and the filter: the pre-pass left, per row group, the (s32 product,
+// row) of the group's best sampled row.  The k best of those are k DISTINCT valid rows (the groups are disjoint);
+// they are rescored exactly, with the streaming scan's arithmetic, so e_k = the smallest of those k exact scores is
+// <= tau, the k-th best exact score.  Every row of the true top-k has S >= s - eps >= tau - eps >= e_k - eps:
+// floor[q] = e_k - eps[q] is rigorous, without the coarse error of a sampled floor or a second eps.  Fewer than k
+// groups seen: no floor.  NaN eps (a NaN query, which no row matches): NaN floor, no candidates.
+__global__ void __launch_bounds__(128)
+i8_floor_kernel(const unsigned long long* __restrict__ keys, int nq, int k, int dim, const float* __restrict__ qn,
+                const float* __restrict__ master, const float* __restrict__ eps, float* __restrict__ floor_out) {
+  pdl_wait();             // the pre-pass's group keys
+  pdl_trigger();
+  const int lane = threadIdx.x & 31;
+  const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= nq) return;
+  unsigned long long key = keys[size_t(w) * kGroups + lane];
+  const float4* qq = reinterpret_cast<const float4*>(qn + size_t(w) * dim);
+  const int nvec = dim >> 2;
+  float e_k = INFINITY;
+  int got = 0;
+  for (int r = 0; r < k; ++r) {
+    const uint32_t hi = uint32_t(key >> 32), lo = uint32_t(key);
+    const uint32_t mh = __reduce_max_sync(0xffffffffu, hi);
+    if (mh == 0u) break;                               // warp-uniform: no group left
+    const uint32_t ml = __reduce_max_sync(0xffffffffu, hi == mh ? lo : 0u);
+    if (hi == mh && lo == ml) key = 0ull;              // rows are distinct across groups: exactly one lane
+    const float4* g = reinterpret_cast<const float4*>(master + size_t(ml) * dim);
+    float a = 0.f;
+#pragma unroll 4
+    for (int v = lane; v < nvec; v += 32) {
+      const float4 x = __ldg(g + v), y = __ldg(qq + v);
+      a = fmaf(x.x, y.x, a); a = fmaf(x.y, y.y, a); a = fmaf(x.z, y.z, a); a = fmaf(x.w, y.w, a);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    e_k = fminf(e_k, a == a ? a : -INFINITY);
+    ++got;
+  }
+  if (lane == 0) {
+    const float e = __ldg(eps + w);
+    floor_out[w] = !(e == e) ? NAN : (got < k ? -3.0e38f : e_k - e);
+  }
+}
+
 // ------------------------------------------------------------------------------------------ stage 3
-// One warp per query: tau from the candidate segments, keep S >= tau - 2*eps, rescore in fp32, top-k.
-constexpr int kMaxKeep = 128;      // rescored rows per query before the query is handed to the fallback
+// One CTA per query: tau from the candidate list, keep the rows that can still be in the top-k, rescore in fp32, top-k.
+constexpr int kMaxKeep = 256;      // rescored rows per query before the query is handed to the fallback
 
 template <int K>
 __device__ __forceinline__ void lane_insert(float (&sc)[K], int32_t (&ix)[K], float s, int32_t r) {
@@ -713,12 +848,17 @@ constexpr int kSelectWarps = 4;
 // EUCLID: the coarse scores are S = q.g - 0.5*||g||^2 (larger = nearer); the kept rows are rescored as the
 // exact direct-difference d^2 = sum (g - q)^2 (the streaming scan's arithmetic and order), ranked by
 // (-d^2 desc, row asc) and reported as distances; accept iff d <= threshold.
+// Cosine with rescoring: two steps.  The k best coarse rows are rescored first; the smallest of their exact scores,
+// tau_e, is <= the true k-th best tau (k distinct rows reach it), so every row of the true top-k has
+// S >= tau - eps >= tau_e - eps: only those are rescored next (about 30 rows at dim 512 with the int8 filter's eps,
+// instead of ~140 above tau_c - 2 eps).
+// qstep != nullptr: the candidates carry the int8 filter's s32 products, S = product * qstep[q].
 template <int K, bool EUCLID>
 __global__ void __launch_bounds__(kSelectWarps * 32)
 select_rescore_kernel(const int2* __restrict__ dense, const int* __restrict__ cand_total,
                       int dense_cap, int nq, int k, int dim, const float* __restrict__ qn,
                       const float* __restrict__ eps, const __nv_bfloat16* __restrict__ plane, int plane_dim,
-                      const float* __restrict__ coef,
+                      const float* __restrict__ coef, const float* __restrict__ qstep,
                       const float* __restrict__ master, int rescore, float threshold, int64_t row_offset,
                       int64_t* __restrict__ out_rows, float* __restrict__ out_scores,
                       uint8_t* __restrict__ out_accept, int* __restrict__ flagged, int* __restrict__ n_flagged,
@@ -749,11 +889,13 @@ select_rescore_kernel(const int2* __restrict__ dense, const int* __restrict__ ca
   // EUCLID: an entry's coarse score is an UPPER bound U of the row's exact score (the filter's query image adds the
   // row's own error bound, queries.cu); tau must be a floor of the true k-th best, so entries are ranked by their
   // LOWER bounds L = U - 2 err, err recomputed from the row's bound columns (the same bf16 numbers the tensor core
-  // multiplied) - and every entry with U >= tau survives.  Cosine: ranked by the score itself, margin 2 eps below.
+  // multiplied) - and every entry with U >= tau survives.  Cosine: ranked by the score itself (below: tau_e - eps).
   const float ca = EUCLID ? coef[size_t(q) * 4] : 0.f, cb = EUCLID ? coef[size_t(q) * 4 + 1] : 0.f,
               cc = EUCLID ? coef[size_t(q) * 4 + 2] : 0.f;
+  const float step = qstep ? __ldg(qstep + q) : 0.f;
+  auto coarse = [&](int y) { return qstep ? float(y) * step : __int_as_float(y); };
   auto rank_key = [&](const int2& e) {
-    const float u_ = __int_as_float(e.y);
+    const float u_ = coarse(e.y);
     if (!EUCLID) return u_;
     const __nv_bfloat16* pr = plane + size_t(e.x) * plane_dim + dim + 3;
     const float err = fmaf(ca, __bfloat162float(pr[0]), fmaf(cb, __bfloat162float(pr[1]), cc * __bfloat162float(pr[2])));
@@ -813,74 +955,95 @@ select_rescore_kernel(const int2* __restrict__ dense, const int* __restrict__ ca
     return;
   }
 
-  // (b) compact the rows that can still be in the true top-k (their order is irrelevant: the final
-  //     order below is total)
-  const float keep_thr = EUCLID ? tau : tau - 2.0f * (eps ? __ldg(eps + q) : kCoarseEps);
+  const int nvec = dim >> 2;
+  const float4* qq = reinterpret_cast<const float4*>(qn + size_t(q) * dim);
+  // exact fp32 rescoring of keep_row[i0 .. m) into keep_sc, 2 rows per warp and round - the typical k + 3 survivors
+  // occupy all four warps - with the row's 16-byte loads unrolled four deep (a 512-d row = 4 loads per lane: one DRAM
+  // round trip, not four); same element -> lane mapping and summation order as the streaming scan
+  auto rescore_rows = [&](int i_begin, int m_end) {
+    constexpr int kRescoreRows = 2;
+    for (int i0 = i_begin + w * kRescoreRows; i0 < m_end; i0 += kSelectWarps * kRescoreRows) {
+      float a[kRescoreRows];
+      const float4* g[kRescoreRows];
+#pragma unroll
+      for (int u = 0; u < kRescoreRows; ++u) {
+        a[u] = 0.f;
+        const int i = i0 + u < m_end ? i0 + u : i0;
+        g[u] = reinterpret_cast<const float4*>(master + size_t(keep_row[i]) * dim);
+      }
+#pragma unroll 4
+      for (int v = lane; v < nvec; v += 32) {
+        const float4 y = __ldg(qq + v);
+        float4 x[kRescoreRows];
+#pragma unroll
+        for (int u = 0; u < kRescoreRows; ++u) x[u] = __ldg(g[u] + v);
+#pragma unroll
+        for (int u = 0; u < kRescoreRows; ++u) {
+          if (EUCLID) {
+            float d;
+            d = x[u].x - y.x; a[u] = fmaf(d, d, a[u]); d = x[u].y - y.y; a[u] = fmaf(d, d, a[u]);
+            d = x[u].z - y.z; a[u] = fmaf(d, d, a[u]); d = x[u].w - y.w; a[u] = fmaf(d, d, a[u]);
+          } else {
+            a[u] = fmaf(x[u].x, y.x, a[u]); a[u] = fmaf(x[u].y, y.y, a[u]);
+            a[u] = fmaf(x[u].z, y.z, a[u]); a[u] = fmaf(x[u].w, y.w, a[u]);
+          }
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < kRescoreRows; ++u) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) a[u] += __shfl_xor_sync(0xffffffffu, a[u], o);
+        if (lane == 0 && i0 + u < m_end) keep_sc[i0 + u] = EUCLID ? -a[u] : a[u];
+      }
+    }
+  };
+
+  // (b) cosine: rescore the m0 <= k coarse winners first (every warp holds them in lanes 0..k-1); keep threshold
+  //     tau_e - eps.  Euclidean: keep U >= tau (the lower-bound ranking above).
+  int m0 = 0;
+  float keep_thr = tau;
+  if (!EUCLID) {
+    m0 = __popc(__ballot_sync(0xffffffffu, lane < k && top_ix >= 0));
+    if (w == 0 && lane < m0) keep_row[lane] = top_ix;
+    __syncthreads();
+    rescore_rows(0, m0);
+    __syncthreads();
+    float te = m0 < k ? -INFINITY : INFINITY;
+    for (int i = 0; i < m0; ++i) { const float x = keep_sc[i]; te = fminf(te, x == x ? x : -INFINITY); }
+    keep_thr = te - (eps ? __ldg(eps + q) : kCoarseEps);
+  }
+  // compact the other rows that can still be in the true top-k (their order is irrelevant: the final order below
+  // is total) behind the m0 rescored ones
   for (int c0 = w * 32; c0 < n; c0 += 4 * kSelectWarps * 32) {     // 4 independent loads per lane per round
     int2 e[4];
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
       const int c = c0 + u * kSelectWarps * 32 + lane;
-      e[u] = c < n ? mine[c] : make_int2(-1, __float_as_int(-INFINITY));
+      e[u] = c < n ? mine[c] : make_int2(-1, 0);
     }
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
-      const bool kp = (c0 + u * kSelectWarps * 32 + lane < n) && __int_as_float(e[u].y) >= keep_thr;
+      const float sv = EUCLID ? __int_as_float(e[u].y) : coarse(e[u].y);
+      bool kp = (c0 + u * kSelectWarps * 32 + lane < n) && sv >= keep_thr;
+      if (kp)
+        for (int i = 0; i < m0; ++i) kp &= keep_row[i] != e[u].x;     // already rescored
       const unsigned bal = __ballot_sync(0xffffffffu, kp);
       if (bal) {
         int base = 0;
         if (lane == 0) base = atomicAdd(&s_m, __popc(bal));
         base = __shfl_sync(0xffffffffu, base, 0);
-        const int pos = base + __popc(bal & ((1u << lane) - 1));
+        const int pos = m0 + base + __popc(bal & ((1u << lane) - 1));
         if (kp && pos < kMaxKeep) keep_row[pos] = e[u].x;
       }
     }
   }
   __syncthreads();
-  int m = s_m;
+  int m = m0 + s_m;
   const bool overflow = m > kMaxKeep;            // too many survivors: rescored in part, then redone by the fallback
   if (overflow) m = kMaxKeep;
 
-  // (c) exact fp32 rescoring, 2 rows per warp and round - the typical k + 3 survivors occupy all four
-  //     warps - with the row's 16-byte loads unrolled four deep (a 512-d row = 4 loads per lane: one DRAM
-  //     round trip, not four); same element -> lane mapping and summation order as the streaming scan
-  constexpr int kRescoreRows = 2;
-  const int nvec = dim >> 2;
-  const float4* qq = reinterpret_cast<const float4*>(qn + size_t(q) * dim);
-  for (int i0 = w * kRescoreRows; i0 < m; i0 += kSelectWarps * kRescoreRows) {
-    float a[kRescoreRows];
-    const float4* g[kRescoreRows];
-#pragma unroll
-    for (int u = 0; u < kRescoreRows; ++u) {
-      a[u] = 0.f;
-      const int i = i0 + u < m ? i0 + u : i0;
-      g[u] = reinterpret_cast<const float4*>(master + size_t(keep_row[i]) * dim);
-    }
-#pragma unroll 4
-    for (int v = lane; v < nvec; v += 32) {
-      const float4 y = __ldg(qq + v);
-      float4 x[kRescoreRows];
-#pragma unroll
-      for (int u = 0; u < kRescoreRows; ++u) x[u] = __ldg(g[u] + v);
-#pragma unroll
-      for (int u = 0; u < kRescoreRows; ++u) {
-        if (EUCLID) {
-          float d;
-          d = x[u].x - y.x; a[u] = fmaf(d, d, a[u]); d = x[u].y - y.y; a[u] = fmaf(d, d, a[u]);
-          d = x[u].z - y.z; a[u] = fmaf(d, d, a[u]); d = x[u].w - y.w; a[u] = fmaf(d, d, a[u]);
-        } else {
-          a[u] = fmaf(x[u].x, y.x, a[u]); a[u] = fmaf(x[u].y, y.y, a[u]);
-          a[u] = fmaf(x[u].z, y.z, a[u]); a[u] = fmaf(x[u].w, y.w, a[u]);
-        }
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < kRescoreRows; ++u) {
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) a[u] += __shfl_xor_sync(0xffffffffu, a[u], o);
-      if (lane == 0 && i0 + u < m) keep_sc[i0 + u] = EUCLID ? -a[u] : a[u];
-    }
-  }
+  // (c) exact fp32 rescoring of the rest
+  rescore_rows(m0, m);
   __syncthreads();
   if (w != 0) return;
 
@@ -930,18 +1093,20 @@ static int get_encode(EncodeTiledFn* out) {
 }
 
 // 2-D bf16 row-major [rows][dim] view with a row pitch (bytes), box = box_k x box_rows; box_k = 64 with the
-// 128B swizzle (a k-block) or 16 with the 32B swizzle (the Euclidean pad block)
+// 128B swizzle (a k-block) or 16 with the 32B swizzle (the Euclidean pad block).  i8: an int8 view, box = one
+// 128-byte k-block of 128 elements, 128B swizzle.
 static int make_map(CUtensorMap* map, const void* ptr, int dim, int64_t rows, size_t pitch_bytes, int box_rows,
-                    int box_k = kBlockK) {
+                    int box_k = kBlockK, bool i8 = false) {
   EncodeTiledFn enc = nullptr;
   FRG_CHECK(get_encode(&enc));
+  if (i8) box_k = kBlockKI8;
   cuuint64_t gdim[2] = {cuuint64_t(dim), cuuint64_t(rows)};
   cuuint64_t gstride[1] = {cuuint64_t(pitch_bytes)};
   cuuint32_t box[2] = {cuuint32_t(box_k), cuuint32_t(box_rows)};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), gdim, gstride, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   box_k == kBlockK ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_32B,
+  CUresult r = enc(map, i8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr),
+                   gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   (i8 || box_k == kBlockK) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_32B,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed (%d): rows=%lld pitch=%zu", int(r), (long long)rows, pitch_bytes); return FRG_ERR_CUDA; }
   return FRG_OK;
@@ -954,16 +1119,17 @@ static int gcd_int(int a, int b) { while (b) { int t = a % b; a = b; b = t; } re
 // (FRG_TC_STAGES up to 12) measured no faster at dim 128 / 256 - those shapes are bound by the TMEM read
 // rate of the epilogue (DESIGN.md section 4.2), not by bytes in flight.
 constexpr size_t kSmemLimit = 227 * 1024;
-static int tc_stages(int qdim) {
-  const size_t fixed = size_t(kTileQ) * qdim * 2 + 256 + 1024;
+// q_row_bytes: bytes of one query row of the resident tile (dim x 2 bf16, dim x 1 int8)
+static int tc_stages(int q_row_bytes) {
+  const size_t fixed = size_t(kTileQ) * q_row_bytes + 256 + 1024;
   int st = int((kSmemLimit - fixed) / kStageBytes);
   static const int cap = []() { const char* e = getenv("FRG_TC_STAGES"); return e ? atoi(e) : 6; }();
   if (st > cap) st = cap;
   if (st > kMaxStages) st = kMaxStages;
   return st < 2 ? 2 : st;
 }
-static size_t tc_smem_bytes(int qdim) {
-  return size_t(kTileQ) * qdim * 2 + size_t(tc_stages(qdim)) * kStageBytes + 256 + 1024;
+static size_t tc_smem_bytes(int q_row_bytes) {
+  return size_t(kTileQ) * q_row_bytes + size_t(tc_stages(q_row_bytes)) * kStageBytes + 256 + 1024;
 }
 
 int tc_supported(int dim, int metric, const char** why) {
@@ -981,7 +1147,7 @@ struct TcPlan {
   bool pair;              // CTA-pair kernels (F > 128)
   bool fused;             // pre-pass folded into the filter kernel (probe tile + published group maxima)
   int qtiles, stride, chunks_pre, chunks_main, kreg, seg, stage_entries;
-  size_t off_keys, off_cnt, off_cand, off_dense, off_flag, total;
+  size_t off_keys, off_cnt, off_cand, off_dense, off_flag, off_floor, total;
 };
 
 // FUSED: share of every CTA's chunk probed before the floor is derived (FRG_TC_PROBE_DIV, default 64)
@@ -998,8 +1164,14 @@ static int reg_k(int k) { return k == 1 ? 1 : (k <= 4 ? 4 : (k <= 8 ? 8 : 16)); 
 // bounds of the exact score), so the pre-pass is never folded into the filter kernel there.
 // Range search (range = true): no pre-pass, and a fixed dense list of kRangeBudget entries per query instead of one
 // sized from k (DESIGN.md section 7.3).
+// i8: the int8 filter - pre-pass at most every kI8MaxStride-th tile (FRG_TC_I8_STRIDE), floor from i8_floor_kernel,
+// never fused.
 constexpr int kRangeBudget = 4096;
-static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range = false) {
+static int i8_max_stride() {
+  static const int v = []() { const char* e = getenv("FRG_TC_I8_STRIDE"); const int d = e ? atoi(e) : 16; return d < 1 ? 16 : d; }();
+  return v;
+}
+static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range = false, bool i8 = false) {
   const bool euclid_plane = dim < 0;
   pl->qtiles = (nq + kTileQ - 1) / kTileQ;
   pl->pair = tc_uses_pairs(nq);
@@ -1009,13 +1181,14 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   // wins for a handful of queries (F = 1: 198 vs 208 us) and loses from F = 64 on (F = 1024: 814 vs
   // 735 us).  FRG_TC_FUSED=0/1 forces either path.
   static const int fused_env = []() { const char* e = getenv("FRG_TC_FUSED"); return e ? atoi(e) : -1; }();
-  pl->fused = !euclid_plane && !range && (fused_env >= 0 ? fused_env != 0 : nq <= 8);
+  pl->fused = !euclid_plane && !range && !i8 && (fused_env >= 0 ? fused_env != 0 : nq <= 8);
   const int tile_rows = pl->pair ? 2 * kTileR : kTileR;
   // pre-pass sample: every stride-th 128-row tile, stride the largest power of two <= 64 that still
   // leaves >= 16 K sampled rows
   static const int64_t pre_min_rows = []() { const char* e = getenv("FRG_TC_PRE_MIN_ROWS"); const long v = e ? atol(e) : 16384; return int64_t(v < 1 ? 16384 : v); }();
+  const int max_stride = i8 ? i8_max_stride() : 64;
   int stride = 1;
-  while (stride < 64 && rows / (stride * 2) >= pre_min_rows) stride *= 2;
+  while (stride < max_stride && rows / (stride * 2) >= pre_min_rows) stride *= 2;
   pl->stride = stride;
   const int tiles_all = int((rows + tile_rows - 1) / tile_rows);
   auto chunks_for = [&](int tiles) {
@@ -1045,6 +1218,10 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   // at tail mass Gamma(k)/n_view, and the 2*eps widening about doubles the count at dim 512.  Room for
   // mean + ~10 sigma keeps the overflow probability negligible; the exact fallback covers the rest.
   // (x1.5: the group-max floor is a little looser than an exact k-th best of the sample)
+  // int8 filter: its eps is ~4x bf16's, but its floor e_k - eps drops the second eps and the group-max error; the
+  // CPU rehearsal of the synthetic gallery (tools/int8_band_sim.py, 1 M x 512, k = 5, 128 queries) gives 399 / 791 /
+  // 815 (median / p99 / max) candidates per query at stride 16 and 218 / 468 / 534 at stride 8, against 1793 and 896
+  // entries from the same formula (profiles/r04_int8_band_sim.json).
   // fused: the probe is 1/64 of every chunk, or one tile per CTA if that is more
   int eff_stride = stride;
   if (pl->fused) {
@@ -1065,19 +1242,20 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   pl->seg = seg;
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-  pl->off_keys = take(size_t(nq) * kGroups * 4);
+  pl->off_keys = take(size_t(nq) * kGroups * (i8 ? 8 : 4));
   pl->off_cnt = take(size_t(nq) * 4);
   pl->off_cand = take(size_t(nq) * nseg * seg * 8);
   pl->off_dense = take(size_t(nq) * stage_entries * 8);
   pl->off_flag = take(size_t(nq) * 4 + 12);    // flagged[nq], count, ticket, probe-arrival counter
+  pl->off_floor = take(i8 ? size_t(nq) * 4 : 0);
   pl->total = off;
 }
 
-template <int MODE, bool MASKED, bool PAIR, bool GROUPED = false>
+template <int MODE, bool MASKED, bool PAIR, bool GROUPED = false, bool I8 = false>
 static int launch_tc_scan(const CUtensorMap& qm, const CUtensorMap& gm, const CUtensorMap& pm, const TcScanParams& p,
                           int qtiles, int chunks, cudaStream_t st) {
-  const size_t smem = tc_smem_bytes(p.dim);
-  auto kern = tc_scan_kernel<MODE, MASKED, PAIR, GROUPED>;
+  const size_t smem = tc_smem_bytes(I8 ? p.dim : 2 * p.dim);
+  auto kern = tc_scan_kernel<MODE, MASKED, PAIR, GROUPED, I8>;
   FRG_CUDA(func_attr_once(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kSmemLimit)));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(qtiles, chunks);
@@ -1098,7 +1276,7 @@ static int launch_tc_scan(const CUtensorMap& qm, const CUtensorMap& gm, const CU
   return FRG_OK;
 }
 
-template <int MODE>
+template <int MODE, bool I8 = false>
 static int launch_tc_scan_m(bool masked, bool pair, const CUtensorMap& qm, const CUtensorMap& gm,
                             const CUtensorMap& pm, const TcScanParams& p, int qtiles, int chunks, cudaStream_t st) {
   // measured (profiles/r02_ab_grouped.txt, same box, sustained clocks): 3-7 % off the whole step at batch 256-1024,
@@ -1107,16 +1285,16 @@ static int launch_tc_scan_m(bool masked, bool pair, const CUtensorMap& qm, const
   static const bool grouped = []() { const char* e = getenv("FRG_TC_GROUPED"); return !e || atoi(e) != 0; }();
   if (MODE == kModeFilter && grouped) {
     if (pair)
-      return masked ? launch_tc_scan<kModeFilter, true, true, true>(qm, gm, pm, p, qtiles, chunks, st)
-                    : launch_tc_scan<kModeFilter, false, true, true>(qm, gm, pm, p, qtiles, chunks, st);
-    return masked ? launch_tc_scan<kModeFilter, true, false, true>(qm, gm, pm, p, qtiles, chunks, st)
-                  : launch_tc_scan<kModeFilter, false, false, true>(qm, gm, pm, p, qtiles, chunks, st);
+      return masked ? launch_tc_scan<kModeFilter, true, true, true, I8>(qm, gm, pm, p, qtiles, chunks, st)
+                    : launch_tc_scan<kModeFilter, false, true, true, I8>(qm, gm, pm, p, qtiles, chunks, st);
+    return masked ? launch_tc_scan<kModeFilter, true, false, true, I8>(qm, gm, pm, p, qtiles, chunks, st)
+                  : launch_tc_scan<kModeFilter, false, false, true, I8>(qm, gm, pm, p, qtiles, chunks, st);
   }
   if (pair)
-    return masked ? launch_tc_scan<MODE, true, true>(qm, gm, pm, p, qtiles, chunks, st)
-                  : launch_tc_scan<MODE, false, true>(qm, gm, pm, p, qtiles, chunks, st);
-  return masked ? launch_tc_scan<MODE, true, false>(qm, gm, pm, p, qtiles, chunks, st)
-                : launch_tc_scan<MODE, false, false>(qm, gm, pm, p, qtiles, chunks, st);
+    return masked ? launch_tc_scan<MODE, true, true, false, I8>(qm, gm, pm, p, qtiles, chunks, st)
+                  : launch_tc_scan<MODE, false, true, false, I8>(qm, gm, pm, p, qtiles, chunks, st);
+  return masked ? launch_tc_scan<MODE, true, false, false, I8>(qm, gm, pm, p, qtiles, chunks, st)
+                : launch_tc_scan<MODE, false, false, false, I8>(qm, gm, pm, p, qtiles, chunks, st);
 }
 
 bool tc_uses_pairs(int nq) {
@@ -1136,18 +1314,18 @@ int64_t tc_effective_rows(const GalleryWindow* s, int nq, cudaStream_t st, const
   return int64_t(n) * gran;
 }
 
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range) {
+size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range, bool i8) {
   TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl, range);
+  tc_plan(rows, dim, nq, k, sm_count, &pl, range, i8);
   return pl.total;
 }
 
-// the pieces of the workspace the query-prep kernel initialises (group keys := key(-1), counters := 0)
+// the pieces of the workspace the query-prep kernel initialises (group keys := "nothing seen", counters := 0)
 void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               uint32_t** keys, int** cand_total, int** n_flagged, bool range) {
+                               void** keys, int** cand_total, int** n_flagged, bool range, bool i8) {
   TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl, range);
-  *keys = reinterpret_cast<uint32_t*>(ws + pl.off_keys);
+  tc_plan(rows, dim, nq, k, sm_count, &pl, range, i8);
+  *keys = ws + pl.off_keys;
   *cand_total = reinterpret_cast<int*>(ws + pl.off_cnt);
   *n_flagged = reinterpret_cast<int*>(ws + pl.off_flag) + nq;
 }
@@ -1159,17 +1337,21 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
                     unsigned char* ws, int sm_count, const XPush& push, int64_t* out_rows, float* out_scores,
                     uint8_t* out_accept, int** flagged_out, int** n_flagged_out, cudaStream_t st,
                     int64_t plan_rows, const int32_t* tile_list, int n_list, const __nv_bfloat16* qb_prepass,
-                    const float* coef) {
+                    const float* coef, const int8_t* qi8, const float* qstep) {
   const bool euclid = metric == FRG_METRIC_EUCLIDEAN;
+  const bool i8 = s->plane8 != nullptr;
   if (euclid && (!qb_prepass || !coef)) { set_error("tc_match: the Euclidean filter needs both query images"); return FRG_ERR_INVALID; }
-  if (euclid != (s->plane_dim != s->dim)) { set_error("tc_match: metric does not fit the store's scan plane"); return FRG_ERR_UNSUPPORTED; }
+  if (euclid ? (!s->plane || s->plane_dim == s->dim) : (i8 ? !qi8 || !qstep || !eps || !rescore : !s->plane)) {
+    set_error("tc_match: metric / query image does not fit the store's scan plane");
+    return FRG_ERR_UNSUPPORTED;
+  }
   // columns of the query tile: dim, or dim + kEuclidQPad (its last k-block meets the plane's 16-column pad block)
   const int kdim = euclid ? s->dim + kEuclidQPad : s->dim;
-  const size_t pitch = size_t(s->plane_dim) * 2;
+  const size_t pitch = i8 ? size_t(s->dim) : size_t(s->plane_dim) * 2;
   // (tile_list: a tenant-filtered call whose window is mostly other tenants' rows walks only the tiles that hold
   // rows of the tenant; everything is planned for plan_rows = listed tiles x rows per tile)
   TcPlan pl;
-  tc_plan(plan_rows, euclid ? -s->dim : s->dim, nq, k, sm_count, &pl);
+  tc_plan(plan_rows, euclid ? -s->dim : s->dim, nq, k, sm_count, &pl, false, i8);
   uint32_t* keys = reinterpret_cast<uint32_t*>(ws + pl.off_keys);
   int* cnt = reinterpret_cast<int*>(ws + pl.off_cnt);
   int2* cand = reinterpret_cast<int2*>(ws + pl.off_cand);
@@ -1181,22 +1363,46 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   const bool masked = tenant >= 0 || s->maybe_dead;
 
   CUtensorMap qm, qm_pre, gm_full, pm;
-  FRG_CHECK(make_map(&qm, qb, kdim, nq, size_t(kdim) * 2, kTileQ));
+  if (i8) FRG_CHECK(make_map(&qm, qi8, kdim, nq, size_t(kdim), kTileQ, kBlockK, true));
+  else FRG_CHECK(make_map(&qm, qb, kdim, nq, size_t(kdim) * 2, kTileQ));
   if (euclid) FRG_CHECK(make_map(&qm_pre, qb_prepass, kdim, nq, size_t(kdim) * 2, kTileQ));   // lower-bound image
   else qm_pre = qm;
-  FRG_CHECK(make_map(&gm_full, s->plane, s->dim, s->rows, pitch, kTileR));   // box = one CTA's half
+  if (i8) FRG_CHECK(make_map(&gm_full, s->plane8, s->dim, s->rows, pitch, kTileR, kBlockK, true));
+  else FRG_CHECK(make_map(&gm_full, s->plane, s->dim, s->rows, pitch, kTileR));   // box = one CTA's half
   if (euclid) FRG_CHECK(make_map(&pm, s->plane + s->dim, kEuclidPad, s->rows, pitch, kTileR, kEuclidPad));
   else pm = gm_full;                                                          // never dereferenced (p.pad == 0)
 
   TcScanParams p{};
   p.fault = s->fault;
   p.tile_list = tile_list; p.n_list = n_list;
-  p.eps = eps; p.none_score = euclid ? kEuclidNone : kNoScore; p.pad = euclid ? 1 : 0; p.stages = tc_stages(kdim);
+  p.eps = eps; p.none_score = euclid ? kEuclidNone : kNoScore; p.pad = euclid ? 1 : 0;
+  p.stages = tc_stages(i8 ? kdim : 2 * kdim);
   p.dim = kdim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
   p.n_rows = int(s->rows); p.group_key = keys; p.k = k;
   p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
   int rc;
-  if (pl.fused) {
+  if (i8) {
+    // 1. int8 pre-pass over the sampled tiles: (s32 product, row) of every row group's best sampled row
+    p.group_key64 = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
+    p.floor = reinterpret_cast<float*>(ws + pl.off_floor);
+    p.qstep = qstep;
+    p.tile_scale = pl.stride;
+    profile_begin(st, kStagePrepass);
+    FRG_CHECK((launch_tc_scan_m<kModeGroupMax, true>(masked, pl.pair, qm, gm_full, gm_full, p, pl.qtiles, pl.chunks_pre, st)));
+    profile_end(st, 1);
+    // 2. exact floor e_k - eps from the k best group winners
+    profile_begin(st, kStageFloor);
+    FRG_CUDA(launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, true, p.group_key64, nq, k, s->dim,
+                           qn, s->master, eps, const_cast<float*>(p.floor)));
+    note_launch(nullptr);
+    profile_end(st, 1);
+    // 3. filter over the whole plane against the integer floor
+    p.tile_scale = 1;
+    profile_begin(st, kStageDominant);
+    rc = launch_tc_scan_m<kModeFilter, true>(masked, pl.pair, qm, gm_full, gm_full, p, pl.qtiles, pl.chunks_main, st);
+    FRG_CHECK(rc);
+    profile_end(st, 1);
+  } else if (pl.fused) {
     // 1+2. ONE kernel: every CTA probes its first tile, publishes the group maxima, derives L[q] from
     // what all CTAs published, filters the rest of its chunk and finally the probe tile itself
     p.tile_scale = 1;
@@ -1231,7 +1437,8 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
 #define FRG_SELECT_M(KK, EU)                                                                                    \
   FRG_CUDA(func_attr_once(select_rescore_kernel<KK, EU>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)); \
   FRG_CUDA(launch_kernel(select_rescore_kernel<KK, EU>, dim3(grid), dim3(kSelectWarps * 32), 0, st, true, dense, \
-      cnt, pl.stage_entries, nq, k, s->dim, qn, eps, s->plane, s->plane_dim, coef, s->master, rs, threshold,     \
+      cnt, pl.stage_entries, nq, k, s->dim, qn, eps, s->plane, s->plane_dim, coef, i8 ? qstep : nullptr,         \
+      s->master, rs, threshold,                                                                                    \
       row_offset, out_rows, out_scores,                                                                             \
       out_accept, flagged, n_flagged, push))
 #define FRG_SELECT(KK)                                                                                          \
@@ -1253,19 +1460,14 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
 
 // ------------------------------------------------------------------------------------------ range search
 // The filter's floor for a range search is the fixed threshold - eps[q] (rigorous: |S - s| <= eps[q], so every row
-// with exact s >= threshold has S >= the floor), not a group-maximum floor: no pre-pass runs.  The filter kernel is
-// the top-k one, untouched - its prologue derives floor = (k-th largest group key) - 2 eps[q]; with k = 1 and every
-// group key of query q set to threshold + eps[q] - 1e-6 that is threshold - eps[q] - 1e-6 (the 1e-6 covers the
-// rounding of the two fp32 operations).  Thresholds at or below -1 - eps[q] leave the key at "nothing seen": no
-// floor, every valid row is a candidate.
+// with exact s >= threshold has S >= the floor), not a sampled floor: no pre-pass runs.  It goes into the per-query
+// floor array the int8 filter's prologue reads (eps[q] already covers the fp32 rounding of the subtraction).
 __global__ void __launch_bounds__(256)
-range_floor_kernel(const float* __restrict__ eps, float threshold, uint32_t* __restrict__ keys, int nq) {
-  pdl_wait();             // the query prep's eps[] and its reset of the keys
+range_floor_kernel(const float* __restrict__ eps, float threshold, float* __restrict__ floor_out, int nq) {
+  pdl_wait();             // the query prep's eps[]
   pdl_trigger();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= nq * kGroups) return;
-  const float f = threshold + __ldg(eps + i / kGroups) - 1e-6f;
-  if (f > kNoScore) keys[i] = float_key(f);
+  if (i < nq) floor_out[i] = threshold - __ldg(eps + i);
 }
 
 // ONE CTA (4 warps) per query over the dense candidate list of a range-mode filter: every candidate is rescored
@@ -1336,12 +1538,14 @@ range_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand
   if (threadIdx.x == 0) out_counts[q] = m;
 }
 
-int launch_tc_range(const GalleryWindow* s, const float* qn, const __nv_bfloat16* qb, const float* eps, int nq,
-                    int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned char* ws,
-                    int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores, int** flagged_out,
-                    int** n_flagged_out, cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list) {
+int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
+                    int nq, int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset,
+                    unsigned char* ws, int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                    int** flagged_out, int** n_flagged_out, cudaStream_t st, int64_t plan_rows,
+                    const int32_t* tile_list, int n_list) {
+  if (!s->plane8) { set_error("tc_range: the store has no int8 scan plane"); return FRG_ERR_UNSUPPORTED; }
   TcPlan pl;
-  tc_plan(plan_rows, s->dim, nq, 1, sm_count, &pl, true);
+  tc_plan(plan_rows, s->dim, nq, 1, sm_count, &pl, true, true);
   int* cnt = reinterpret_cast<int*>(ws + pl.off_cnt);
   int2* cand = reinterpret_cast<int2*>(ws + pl.off_cand);
   int2* dense = reinterpret_cast<int2*>(ws + pl.off_dense);
@@ -1352,24 +1556,25 @@ int launch_tc_range(const GalleryWindow* s, const float* qn, const __nv_bfloat16
   const bool masked = tenant >= 0 || s->maybe_dead;
 
   CUtensorMap qm, gm;
-  FRG_CHECK(make_map(&qm, qb, s->dim, nq, size_t(s->dim) * 2, kTileQ));
-  FRG_CHECK(make_map(&gm, s->plane, s->dim, s->rows, size_t(s->plane_dim) * 2, kTileR));
+  FRG_CHECK(make_map(&qm, qi8, s->dim, nq, size_t(s->dim), kTileQ, kBlockK, true));
+  FRG_CHECK(make_map(&gm, s->plane8, s->dim, s->rows, size_t(s->dim), kTileR, kBlockK, true));
 
   TcScanParams p{};
   p.fault = s->fault;
   p.tile_list = tile_list; p.n_list = n_list;
   p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = tc_stages(s->dim);
   p.dim = s->dim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
-  p.n_rows = int(s->rows); p.group_key = reinterpret_cast<uint32_t*>(ws + pl.off_keys); p.k = 1;
+  p.n_rows = int(s->rows); p.k = 1;
+  p.floor = reinterpret_cast<float*>(ws + pl.off_floor); p.qstep = qstep;
   p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
   p.tile_scale = 1;
   profile_begin(st, kStageFloor);
-  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq * kGroups + 255) / 256), dim3(256), 0, st, true, eps, threshold,
-                         p.group_key, nq));
+  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, true, eps, threshold,
+                         const_cast<float*>(p.floor), nq));
   note_launch(nullptr);
   profile_end(st, 1);
   profile_begin(st, kStageDominant);
-  FRG_CHECK(launch_tc_scan_m<kModeFilter>(masked, pl.pair, qm, gm, gm, p, pl.qtiles, pl.chunks_main, st));
+  FRG_CHECK((launch_tc_scan_m<kModeFilter, true>(masked, pl.pair, qm, gm, gm, p, pl.qtiles, pl.chunks_main, st)));
   profile_end(st, 1);
 
   profile_begin(st, kStageSelect);

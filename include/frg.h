@@ -57,7 +57,10 @@ extern "C" {
 #define FRG_VARIANT_TC_BF16   3  /* tcgen05 bf16 scores returned as-is ("bf16 gallery mode", own tolerance) */
 
 /* frg_store_create flags */
-#define FRG_STORE_BF16_PLANE  1u /* keep the bf16 scan plane next to the fp32 master (needed by TC variants) */
+#define FRG_STORE_BF16_PLANE  1u /* keep a scan plane next to the fp32 master (needed by TC variants).  For a unit
+                                   (non-raw) store it is an INT8 plane, dim bytes per row, one store-wide scale fixed
+                                   by dim (0.165 / 127 per step at dim 512; saturating): a 512-d row takes 2.5 KB.
+                                   FRG_VARIANT_TC_BF16 on such a store returns exact scores. */
 #define FRG_STORE_RAW         2u /* never normalise on ingest (Euclidean galleries, cluster means).  Together with
                                    FRG_STORE_BF16_PLANE the plane is the EUCLIDEAN scan plane: each row carries
                                    -0.5*||g||^2 (and its own error-bound terms) in 16 more bf16 columns, so that the
