@@ -25,11 +25,6 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line) {
   return e == cudaErrorMemoryAllocation ? FRG_ERR_NOMEM : FRG_ERR_CUDA;
 }
 
-bool pdl_enabled() {
-  static const bool on = []() { const char* e = getenv("FRG_PDL"); return !e || atoi(e) != 0; }();
-  return on;
-}
-
 void note_launch(const char* variant) {
   ++g_launches;
   if (variant) g_variant = variant;
@@ -255,14 +250,13 @@ static void extents_note_upsert(frg_store* s, const int64_t* hrows, const int32_
 }
 
 // the whole gallery, or - for a tenant-filtered call whose tag extents are known - only the row window that
-// tenant's rows can sit in (FRG_TENANT_WINDOW=0 turns the window off)
+// tenant's rows can sit in
 static GalleryWindow window_of(const frg_store* s, int32_t tenant, bool for_tc = false) {
   GalleryWindow w;
   w.master = s->master; w.plane = s->plane; w.plane8 = s->plane8; w.tags = s->tags; w.gmax_bits = s->gmax_bits; w.fault = s->fault_dev;
   w.rows = s->rows; w.row0 = 0; w.dim = s->dim; w.plane_dim = s->plane_dim; w.flags = s->flags;
   w.maybe_dead = s->maybe_dead;
-  static const bool on = []() { const char* e = getenv("FRG_TENANT_WINDOW"); return !e || atoi(e) != 0; }();
-  if (on && tenant >= 0 && s->extents_known) {
+  if (tenant >= 0 && s->extents_known) {
     int64_t lo = 0, hi = 0;
     auto it = s->extents.find(tenant);
     if (it != s->extents.end()) { lo = it->second.lo; hi = it->second.hi < s->rows ? it->second.hi : s->rows; }
@@ -270,9 +264,8 @@ static GalleryWindow window_of(const frg_store* s, int32_t tenant, bool for_tc =
     // A window that is mostly other tenants' rows (a company's block + one person re-enrolled at the far end):
     // keep the WHOLE store as the window and let the tensor-core kernels walk only the tiles of the tenant's
     // intervals.  (The exact scan and first_match still take the bounding window.)
-    static const bool lists_on = []() { const char* e = getenv("FRG_TILE_LIST"); return !e || atoi(e) != 0; }();
     auto sp = s->spans.find(tenant);
-    if (lists_on && for_tc && sp != s->spans.end() && !sp->second.scattered && hi - lo >= 32768 &&
+    if (for_tc && sp != s->spans.end() && !sp->second.scattered && hi - lo >= 32768 &&
         sp->second.covered * 4 <= hi - lo) {
       w.owner = const_cast<frg_store*>(s);
       w.want_tile_list = true;
@@ -686,7 +679,7 @@ int frg_store_compact(frg_store* s, int64_t* old_to_new) {
   int64_t first = 0;
   while (first < m && src[size_t(first)] == first) ++first;
   if (first < m) {
-    static const int64_t chunk_rows = []() { const char* e = getenv("FRG_COMPACT_CHUNK_ROWS"); const long v = e ? atol(e) : 65536; return int64_t(v < 1 ? 65536 : v); }();
+    constexpr int64_t chunk_rows = 65536;
     const int64_t chunk = m - first < chunk_rows ? m - first : chunk_rows;
     float* bm; void* bp; int32_t* bt;
     int64_t* dsrc = nullptr;

@@ -181,7 +181,7 @@ int launch_exchange_push(const XPush& x, const int64_t* local_rows, const float*
   if (nq <= 0) return FRG_OK;
   int grid = (nq + 3) / 4;
   if (grid > 4 * sm_count) grid = 4 * sm_count;
-  FRG_CUDA(launch_kernel(exchange_push_kernel, dim3(grid), dim3(128), 0, st, true, x, local_rows, local_scores, nq, k));
+  FRG_CUDA(launch_kernel(exchange_push_kernel, dim3(grid), dim3(128), 0, st, x, local_rows, local_scores, nq, k));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   return FRG_OK;
@@ -194,7 +194,7 @@ int launch_exchange_merge(const XPush& x, int nq, int k, int metric, float thres
   if (grid > 4 * sm_count) grid = 4 * sm_count;
   if (grid < 1) grid = 1;
 #define FRG_XM(K)                                                                                              \
-  FRG_CUDA(launch_kernel(exchange_merge_kernel<K>, dim3(grid), dim3(128), 0, st, true, x, nq, k, metric, threshold, \
+  FRG_CUDA(launch_kernel(exchange_merge_kernel<K>, dim3(grid), dim3(128), 0, st, x, nq, k, metric, threshold, \
                          out_rows, out_scores, out_accept))
   if (k == 1) FRG_XM(1);
   else if (k <= 4) FRG_XM(4);

@@ -51,7 +51,7 @@ void profile_end(cudaStream_t st, int launches);
 // predecessor has called pdl_trigger() or exited): its launch latency and prologue (barrier init, TMEM
 // allocation, descriptor prefetch) overlap the predecessor's tail.  pdl_wait() then blocks until the
 // predecessor has completed and its writes are visible - it precedes every read of earlier results.
-// Without the attribute both calls are no-ops.  FRG_PDL=0 turns the attribute off.
+// Without the attribute both calls are no-ops.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -88,18 +88,17 @@ __device__ __forceinline__ int warp_argbest(float s, RowT r, RowT none, int lane
   return bl;
 }
 #endif
-bool pdl_enabled();
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                 bool pdl, Args&&... args) {
+                                 Args&&... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = (pdl && pdl_enabled()) ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

@@ -148,7 +148,7 @@ int launch_prepare_queries_i8(const float* q, int nq, int dim, float* qn, int8_t
                               cudaStream_t st) {
   if (nq <= 0) return FRG_OK;
   FRG_CUDA(func_attr_once(prepare_queries_i8_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-  FRG_CUDA(launch_kernel(prepare_queries_i8_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, true, q, nq, dim,
+  FRG_CUDA(launch_kernel(prepare_queries_i8_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, q, nq, dim,
                          i8_gallery_step(dim), qn, qi8, qstep, eps, bounds, group_keys, cand_total, n_flagged));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
@@ -249,7 +249,7 @@ int launch_prepare_queries_euclid(const float* q, int nq, int dim, const uint32_
   const float none = kEuclidNone;
   memcpy(&none_bits, &none, sizeof(none_bits));
   const uint32_t none_key = ~none_bits;        // float_key() of a negative value: all bits complemented
-  FRG_CUDA(launch_kernel(prepare_queries_euclid_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, true, q, nq, dim, gmax_bits,
+  FRG_CUDA(launch_kernel(prepare_queries_euclid_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, q, nq, dim, gmax_bits,
                          qn, q_aug, q_aug_lo, coef, eps, group_keys, none_key, cand_total, n_flagged));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
@@ -264,7 +264,7 @@ int launch_normalise_queries(const float* q, int nq, int dim, bool normalise, fl
   // same smem/L1 split as the tensor-core kernels that follow: no carve-out switch between launches
   FRG_CUDA(func_attr_once(normalise_queries_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
   FRG_CUDA(launch_kernel(normalise_queries_kernel, dim3((nq + warps_per_block - 1) / warps_per_block), dim3(128), 0, st,
-                         true, q, nq, dim, normalise ? 1 : 0, qn, qn_bf16, group_keys, cand_total, n_flagged, eps, bounds));
+                         q, nq, dim, normalise ? 1 : 0, qn, qn_bf16, group_keys, cand_total, n_flagged, eps, bounds));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   return FRG_OK;

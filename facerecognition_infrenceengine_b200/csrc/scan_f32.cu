@@ -465,26 +465,26 @@ static int launch_flagged_k(const ScanArgs& a, int grid, const int* flagged, int
   if (a.master && a.metric == FRG_METRIC_COSINE && a.tenant >= 0) {
     auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_COSINE, KMAX, float, true>;
     FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, true, a.master, a.tags, a.rows, a.qn,
+    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn,
                            a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
                            out_accept, push));
   } else if (a.master && a.metric == FRG_METRIC_EUCLIDEAN) {
     auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_EUCLIDEAN, KMAX, float, false>;
     FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, true, a.master, a.tags, a.rows, a.qn,
+    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn,
                            a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
                            out_accept, push));
   } else if (a.master) {
     auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_COSINE, KMAX, float, false>;
     FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, true, a.master, a.tags, a.rows, a.qn,
+    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn,
                            a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
                            out_accept, push));
   } else {
     // bf16-only store: the exact re-do reads the scan plane (fp32 query x bf16 row, fp32 accumulation)
     auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_COSINE, KMAX, __nv_bfloat16, false>;
     FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, true, a.plane, a.tags, a.rows, a.qn,
+    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.plane, a.tags, a.rows, a.qn,
                            a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
                            out_accept, push));
   }
@@ -665,15 +665,15 @@ static int launch_range_passes(const ScanArgs& a, int grid, const int* flagged, 
                                int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
   const int nw = grid * kScanWarps;
   const int s = strict ? 1 : 0;
-  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, false>, dim3(grid), dim3(kScanWarps * 32), 0, st, true,
+  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, false>, dim3(grid), dim3(kScanWarps * 32), 0, st,
                          a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged, a.tenant, threshold, s, max_hits,
                          row_offset, cnt, off, out_rows, out_scores));
   note_launch(nullptr);
-  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(a.nq), dim3(256), 0, st, true, a.nq, flagged, n_flagged, nw, cnt,
+  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(a.nq), dim3(256), 0, st, a.nq, flagged, n_flagged, nw, cnt,
                          off, max_hits, METRIC == FRG_METRIC_COSINE ? kNoScore : INFINITY, out_counts, out_rows,
                          out_scores));
   note_launch(nullptr);
-  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, true>, dim3(grid), dim3(kScanWarps * 32), 0, st, true,
+  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, true>, dim3(grid), dim3(kScanWarps * 32), 0, st,
                          a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged, a.tenant, threshold, s, max_hits,
                          row_offset, cnt, off, out_rows, out_scores));
   note_launch(nullptr);

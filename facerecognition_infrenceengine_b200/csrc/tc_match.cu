@@ -1,5 +1,8 @@
 // Tensor-core variants (FRG_VARIANT_TC_EXACT / FRG_VARIANT_TC_BF16): the query x gallery contraction
-// on tcgen05 with the threshold / top-k in the epilogue, so no score matrix reaches HBM.
+// on tcgen05 with the threshold / top-k in the epilogue, so no score matrix reaches HBM.  Which store runs which filter:
+//   - a unit cosine store with an fp32 master: the int8 filter (I8; pre-pass, i8_floor_kernel, filter, select);
+//   - the Euclidean plane of a raw store and a bf16-only store: the bf16 filter described below;
+//   - a bf16-only store matched with nq <= 8 queries: the bf16 filter with the pre-pass folded in (MODE = FUSED).
 //
 //   S[q, r] = sum_k Qb[q, k] * Gb[r, k]        Qb, Gb = bf16 images of the unit fp32 vectors
 //
@@ -20,8 +23,8 @@
 //      streaming scan), order by (score desc, row asc), apply the threshold.
 //   4. queries whose lists overflowed (adversarial duplicates, sparse tenants) are re-done by the
 //      exact streaming scan inside the same enqueue (scan_f32_flagged_kernel) - never by the host.
-//   For a handful of queries (nq <= 8) steps 1 and 2 run as ONE kernel (MODE = FUSED: every CTA probes
-//   its first tile, publishes the group maxima, derives the floor, filters, re-visits the probe tile).
+//   For a handful of queries on a bf16-only store (nq <= 8) steps 1 and 2 run as ONE kernel (MODE = FUSED: every
+//   CTA probes its first tile, publishes the group maxima, derives the floor, filters, re-visits the probe tile).
 //
 // Kernel anatomy (one CTA per SM, 320 threads):
 //   warp 0   TMA producer: gallery tiles [128 rows x 64 k] bf16, 128B-swizzled, 6-stage mbarrier ring
@@ -36,7 +39,6 @@
 #include <cuda.h>
 
 #include <cmath>
-#include <cstdlib>
 
 #include "frg_internal.cuh"
 
@@ -237,7 +239,7 @@ constexpr int kTileQ = 128;          // queries per CTA tile (TMEM lanes); UMMA 
 constexpr int kTileR = 128;          // gallery rows staged per CTA and k-block (TMA box rows)
 constexpr int kBlockK = 64;          // one 128-byte swizzle row of bf16
 constexpr int kBlockKI8 = 128;       // ... of int8
-constexpr int kMaxStages = 8;        // ring depth: 6 by default (all a 512-column query tile leaves room for)
+constexpr int kMaxStages = 8;        // barrier slots of the ring; kStages (6) of them are used
 constexpr int kMaxKBlocks = 8;       // 512 columns / 64
 constexpr int kStageBytes = kTileR * kBlockK * 2;          // 16 KB
 constexpr int kPadStageBytes = kTileR * kEuclidPad * 2;    // 4 KB of a stage: the Euclidean plane's pad block
@@ -309,7 +311,7 @@ struct TcScanParams {
   // Euclidean plane: the LAST k-block of the query tile meets a 16-column pad block of the plane (pad_map:
   // box 16 x 128 rows, 32B swizzle, 4 KB per stage) with ONE K = 16 MMA instead of four
   int pad;
-  int stages;              // depth of the TMA ring (tc_stages)
+  int stages;              // depth of the TMA ring (kStages)
   uint32_t* fault;         // the store's fault word (host-mapped): set when a pipeline barrier timed out
   // Tile list (tenant-filtered calls over a window that is mostly other tenants' rows): the kernel walks
   // n_list listed tiles instead of every tile of the window; entry = absolute tile index (tile = kAccN rows)
@@ -325,11 +327,9 @@ struct TcScanParams {
 // staging only ITS 128-row half of every B tile: half the shared-memory operand traffic per flop of
 // the single-CTA form, which is what lifts the tensor pipe at large batches.  The leader CTA (rank 0)
 // owns the full/tmem_empty barriers and issues the MMAs; commits are multicast to both CTAs.
-// GROUPED (FILTER mode): the block maximum is built from four 8-column group maxima, and a thread that holds a
-// candidate visits only the group(s) that contain one - the rare path costs a quarter of the 32-column walk.
 // I8: int8 operands (unit cosine store's int8 plane): tcgen05.mma kind::i8, K = 32 per MMA, 128 int8 per k-block,
 // exact s32 accumulators; half the MMA time and half the plane bytes of bf16 per score.  Not FUSED.
-template <int MODE, bool MASKED, bool PAIR, bool GROUPED = false, bool I8 = false>
+template <int MODE, bool MASKED, bool PAIR, bool I8 = false>
 __global__ void __launch_bounds__(kTcThreads, 1)
 tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant__ CUtensorMap g_map,
                const __grid_constant__ CUtensorMap pad_map, const TcScanParams p) {
@@ -636,7 +636,13 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
           // this warp sees half of the tile's rows: it owns 16 of the 32 groups, (column mod 16)
 #pragma unroll
           for (int j = 0; j < 32; ++j) gmax[j & 15] = A::mx(gmax[j & 15], v[j]);
-        } else if (GROUPED) {
+        } else {
+          // The block maximum is built from four 8-column group maxima, and a thread that holds a candidate walks
+          // only the group(s) that contain one: ~35 instructions instead of ~110 for all 32 columns.  A warp takes
+          // this path whenever one of its 32 queries has a candidate among the 32 rows (about a quarter of all
+          // blocks), and the slowest epilogue warp decides when the accumulator buffer goes back to the MMA warp.
+          // Measured against the 32-column walk (profiles/r02_ab_grouped.txt, same box, sustained clocks): -3.6 /
+          // -4.8 / -7 % of the step at F = 256 / 512 / 1024, neutral at F <= 128 (HBM-bound, the epilogue has slack).
           AccT g0 = v[0], g1 = v[8], g2 = v[16], g3 = v[24];
 #pragma unroll
           for (int j = 1; j < 8; ++j) {
@@ -655,20 +661,6 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
                     ++emitted;
                   }
                 }
-              }
-            }
-          }
-        } else {
-          AccT m = v[0];
-#pragma unroll
-          for (int j = 1; j < 32; ++j) m = A::mx(m, v[j]);
-          if (m >= thr) {
-            const int row0 = tile_row0 + (half * kBlocksPerWarp + b) * 32;
-#pragma unroll
-            for (int j = 0; j < 32; ++j) {
-              if (v[j] >= thr) {
-                if (emitted < p.seg) my_seg[emitted] = make_int2(row0 + j, A::bits(v[j]));
-                ++emitted;
               }
             }
           }
@@ -1116,21 +1108,16 @@ static int gcd_int(int a, int b) { while (b) { int t = a % b; a = b; b = t; } re
 
 // dynamic shared memory: [alignment slack 1 KB][query tile][ring][barriers 256 B].  Six 16 KB stages
 // (96 KB in flight per SM) already reach the HBM peak; a deeper ring beside shorter query tiles
-// (FRG_TC_STAGES up to 12) measured no faster at dim 128 / 256 - those shapes are bound by the TMEM read
+// (up to 12 stages) measured no faster at dim 128 / 256 - those shapes are bound by the TMEM read
 // rate of the epilogue (DESIGN.md section 4.2), not by bytes in flight.
 constexpr size_t kSmemLimit = 227 * 1024;
+constexpr int kStages = 6;
 // q_row_bytes: bytes of one query row of the resident tile (dim x 2 bf16, dim x 1 int8)
-static int tc_stages(int q_row_bytes) {
-  const size_t fixed = size_t(kTileQ) * q_row_bytes + 256 + 1024;
-  int st = int((kSmemLimit - fixed) / kStageBytes);
-  static const int cap = []() { const char* e = getenv("FRG_TC_STAGES"); return e ? atoi(e) : 6; }();
-  if (st > cap) st = cap;
-  if (st > kMaxStages) st = kMaxStages;
-  return st < 2 ? 2 : st;
-}
 static size_t tc_smem_bytes(int q_row_bytes) {
-  return size_t(kTileQ) * q_row_bytes + size_t(tc_stages(q_row_bytes)) * kStageBytes + 256 + 1024;
+  return size_t(kTileQ) * q_row_bytes + size_t(kStages) * kStageBytes + 256 + 1024;
 }
+static_assert(kStages <= kMaxStages && size_t(kTileQ) * 512 * 2 + size_t(kStages) * kStageBytes + 256 + 1024 <= kSmemLimit,
+              "the ring must fit beside the largest query tile (512 bf16 columns)");
 
 int tc_supported(int dim, int metric, const char** why) {
   // the tiles take any multiple of 64 up to 512 columns; the exact pass behind the filter (rescoring
@@ -1150,11 +1137,9 @@ struct TcPlan {
   size_t off_keys, off_cnt, off_cand, off_dense, off_flag, off_floor, total;
 };
 
-// FUSED: share of every CTA's chunk probed before the floor is derived (FRG_TC_PROBE_DIV, default 64)
-static int probe_div() {
-  static const int v = []() { const char* e = getenv("FRG_TC_PROBE_DIV"); const int d = e ? atoi(e) : 64; return d < 1 ? 64 : d; }();
-  return v;
-}
+// FUSED: share of every CTA's chunk probed before the floor is derived (1/64; larger probes, up to 1/8, measured no
+// faster, DESIGN.md section 4.2)
+constexpr int kProbeDiv = 64;
 
 bool tc_uses_pairs(int nq);
 
@@ -1164,13 +1149,8 @@ static int reg_k(int k) { return k == 1 ? 1 : (k <= 4 ? 4 : (k <= 8 ? 8 : 16)); 
 // bounds of the exact score), so the pre-pass is never folded into the filter kernel there.
 // Range search (range = true): no pre-pass, and a fixed dense list of kRangeBudget entries per query instead of one
 // sized from k (DESIGN.md section 7.3).
-// i8: the int8 filter - pre-pass at most every kI8MaxStride-th tile (FRG_TC_I8_STRIDE), floor from i8_floor_kernel,
-// never fused.
+// i8: the int8 filter - pre-pass at most every 16th tile, floor from i8_floor_kernel, never fused.
 constexpr int kRangeBudget = 4096;
-static int i8_max_stride() {
-  static const int v = []() { const char* e = getenv("FRG_TC_I8_STRIDE"); const int d = e ? atoi(e) : 16; return d < 1 ? 16 : d; }();
-  return v;
-}
 static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range = false, bool i8 = false) {
   const bool euclid_plane = dim < 0;
   pl->qtiles = (nq + kTileQ - 1) / kTileQ;
@@ -1179,16 +1159,14 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   // Fusing the pre-pass into the filter kernel saves a launch and a query-tile reload but probes a
   // smaller sample (one tile per CTA), i.e. a looser floor and more candidates: measured on B200 it
   // wins for a handful of queries (F = 1: 198 vs 208 us) and loses from F = 64 on (F = 1024: 814 vs
-  // 735 us).  FRG_TC_FUSED=0/1 forces either path.
-  static const int fused_env = []() { const char* e = getenv("FRG_TC_FUSED"); return e ? atoi(e) : -1; }();
-  pl->fused = !euclid_plane && !range && !i8 && (fused_env >= 0 ? fused_env != 0 : nq <= 8);
+  // 735 us).
+  pl->fused = !euclid_plane && !range && !i8 && nq <= 8;
   const int tile_rows = pl->pair ? 2 * kTileR : kTileR;
-  // pre-pass sample: every stride-th 128-row tile, stride the largest power of two <= 64 that still
+  // pre-pass sample: every stride-th 128-row tile, stride the largest power of two <= 64 (int8: <= 16) that still
   // leaves >= 16 K sampled rows
-  static const int64_t pre_min_rows = []() { const char* e = getenv("FRG_TC_PRE_MIN_ROWS"); const long v = e ? atol(e) : 16384; return int64_t(v < 1 ? 16384 : v); }();
-  const int max_stride = i8 ? i8_max_stride() : 64;
+  const int max_stride = i8 ? 16 : 64;
   int stride = 1;
-  while (stride < max_stride && rows / (stride * 2) >= pre_min_rows) stride *= 2;
+  while (stride < max_stride && rows / (stride * 2) >= 16384) stride *= 2;
   pl->stride = stride;
   const int tiles_all = int((rows + tile_rows - 1) / tile_rows);
   auto chunks_for = [&](int tiles) {
@@ -1208,8 +1186,6 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
     const int tiles_pre = (tiles_all + stride - 1) / stride;
     int c = cols <= units ? units / cols : 1;
     if (c > tiles_pre) c = tiles_pre;
-    static const int pre_cap = []() { const char* e = getenv("FRG_TC_PRE_CHUNKS"); return e ? atoi(e) : 0; }();
-    if (pre_cap > 0) c = pre_cap < tiles_pre ? pre_cap : tiles_pre;
     pl->chunks_pre = c < 1 ? 1 : c;
   }
   pl->chunks_main = chunks_for(tiles_all);
@@ -1225,8 +1201,7 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   // fused: the probe is 1/64 of every chunk, or one tile per CTA if that is more
   int eff_stride = stride;
   if (pl->fused) {
-    const int pd = probe_div();
-    const int64_t probe_rows = int64_t((tiles_all / pl->chunks_main + pd - 1) / pd) * pl->chunks_main * tile_rows;
+    const int64_t probe_rows = int64_t((tiles_all / pl->chunks_main + kProbeDiv - 1) / kProbeDiv) * pl->chunks_main * tile_rows;
     eff_stride = int(rows / (probe_rows > 0 ? probe_rows : 1)) + 1;
     if (eff_stride > 64) eff_stride = 64;
   }
@@ -1251,11 +1226,11 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   pl->total = off;
 }
 
-template <int MODE, bool MASKED, bool PAIR, bool GROUPED = false, bool I8 = false>
+template <int MODE, bool MASKED, bool PAIR, bool I8>
 static int launch_tc_scan(const CUtensorMap& qm, const CUtensorMap& gm, const CUtensorMap& pm, const TcScanParams& p,
                           int qtiles, int chunks, cudaStream_t st) {
   const size_t smem = tc_smem_bytes(I8 ? p.dim : 2 * p.dim);
-  auto kern = tc_scan_kernel<MODE, MASKED, PAIR, GROUPED, I8>;
+  auto kern = tc_scan_kernel<MODE, MASKED, PAIR, I8>;
   FRG_CUDA(func_attr_once(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kSmemLimit)));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(qtiles, chunks);
@@ -1270,7 +1245,7 @@ static int launch_tc_scan(const CUtensorMap& qm, const CUtensorMap& gm, const CU
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 2;
   FRG_CUDA(cudaLaunchKernelEx(&cfg, kern, qm, gm, pm, p));
   note_launch(nullptr);
   return FRG_OK;
@@ -1279,28 +1254,14 @@ static int launch_tc_scan(const CUtensorMap& qm, const CUtensorMap& gm, const CU
 template <int MODE, bool I8 = false>
 static int launch_tc_scan_m(bool masked, bool pair, const CUtensorMap& qm, const CUtensorMap& gm,
                             const CUtensorMap& pm, const TcScanParams& p, int qtiles, int chunks, cudaStream_t st) {
-  // measured (profiles/r02_ab_grouped.txt, same box, sustained clocks): 3-7 % off the whole step at batch 256-1024,
-  // neutral below - at large batches the epilogue's rare path is not rare enough to be free (a warp enters it
-  // whenever one of its 32 queries has a candidate among 32 rows: ~a quarter of all blocks)
-  static const bool grouped = []() { const char* e = getenv("FRG_TC_GROUPED"); return !e || atoi(e) != 0; }();
-  if (MODE == kModeFilter && grouped) {
-    if (pair)
-      return masked ? launch_tc_scan<kModeFilter, true, true, true, I8>(qm, gm, pm, p, qtiles, chunks, st)
-                    : launch_tc_scan<kModeFilter, false, true, true, I8>(qm, gm, pm, p, qtiles, chunks, st);
-    return masked ? launch_tc_scan<kModeFilter, true, false, true, I8>(qm, gm, pm, p, qtiles, chunks, st)
-                  : launch_tc_scan<kModeFilter, false, false, true, I8>(qm, gm, pm, p, qtiles, chunks, st);
-  }
   if (pair)
-    return masked ? launch_tc_scan<MODE, true, true, false, I8>(qm, gm, pm, p, qtiles, chunks, st)
-                  : launch_tc_scan<MODE, false, true, false, I8>(qm, gm, pm, p, qtiles, chunks, st);
-  return masked ? launch_tc_scan<MODE, true, false, false, I8>(qm, gm, pm, p, qtiles, chunks, st)
-                : launch_tc_scan<MODE, false, false, false, I8>(qm, gm, pm, p, qtiles, chunks, st);
+    return masked ? launch_tc_scan<MODE, true, true, I8>(qm, gm, pm, p, qtiles, chunks, st)
+                  : launch_tc_scan<MODE, false, true, I8>(qm, gm, pm, p, qtiles, chunks, st);
+  return masked ? launch_tc_scan<MODE, true, false, I8>(qm, gm, pm, p, qtiles, chunks, st)
+                : launch_tc_scan<MODE, false, false, I8>(qm, gm, pm, p, qtiles, chunks, st);
 }
 
-bool tc_uses_pairs(int nq) {
-  static const int pair_env = []() { const char* e = getenv("FRG_TC_PAIR"); return e ? atoi(e) : 1; }();
-  return pair_env != 0 && (nq + kTileQ - 1) / kTileQ >= 2;
-}
+bool tc_uses_pairs(int nq) { return (nq + kTileQ - 1) / kTileQ >= 2; }
 
 // rows the plan is made for: the window's, or (tile list in use) listed tiles x rows per tile
 int64_t tc_effective_rows(const GalleryWindow* s, int nq, cudaStream_t st, const int32_t** list, int* n_list) {
@@ -1376,7 +1337,7 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   p.fault = s->fault;
   p.tile_list = tile_list; p.n_list = n_list;
   p.eps = eps; p.none_score = euclid ? kEuclidNone : kNoScore; p.pad = euclid ? 1 : 0;
-  p.stages = tc_stages(i8 ? kdim : 2 * kdim);
+  p.stages = kStages;
   p.dim = kdim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
   p.n_rows = int(s->rows); p.group_key = keys; p.k = k;
   p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
@@ -1392,7 +1353,7 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
     profile_end(st, 1);
     // 2. exact floor e_k - eps from the k best group winners
     profile_begin(st, kStageFloor);
-    FRG_CUDA(launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, true, p.group_key64, nq, k, s->dim,
+    FRG_CUDA(launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, p.group_key64, nq, k, s->dim,
                            qn, s->master, eps, const_cast<float*>(p.floor)));
     note_launch(nullptr);
     profile_end(st, 1);
@@ -1406,7 +1367,7 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
     // 1+2. ONE kernel: every CTA probes its first tile, publishes the group maxima, derives L[q] from
     // what all CTAs published, filters the rest of its chunk and finally the probe tile itself
     p.tile_scale = 1;
-    p.probe_div = probe_div();
+    p.probe_div = kProbeDiv;
     p.arrive = n_flagged + 2;
     {
       // the first wave holds min(all CTAs, one per SM): later waves find the counter already there
@@ -1436,7 +1397,7 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   const int rs = rescore ? 1 : 0;
 #define FRG_SELECT_M(KK, EU)                                                                                    \
   FRG_CUDA(func_attr_once(select_rescore_kernel<KK, EU>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)); \
-  FRG_CUDA(launch_kernel(select_rescore_kernel<KK, EU>, dim3(grid), dim3(kSelectWarps * 32), 0, st, true, dense, \
+  FRG_CUDA(launch_kernel(select_rescore_kernel<KK, EU>, dim3(grid), dim3(kSelectWarps * 32), 0, st, dense, \
       cnt, pl.stage_entries, nq, k, s->dim, qn, eps, s->plane, s->plane_dim, coef, i8 ? qstep : nullptr,         \
       s->master, rs, threshold,                                                                                    \
       row_offset, out_rows, out_scores,                                                                             \
@@ -1562,14 +1523,14 @@ int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, 
   TcScanParams p{};
   p.fault = s->fault;
   p.tile_list = tile_list; p.n_list = n_list;
-  p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = tc_stages(s->dim);
+  p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
   p.dim = s->dim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
   p.n_rows = int(s->rows); p.k = 1;
   p.floor = reinterpret_cast<float*>(ws + pl.off_floor); p.qstep = qstep;
   p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
   p.tile_scale = 1;
   profile_begin(st, kStageFloor);
-  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, true, eps, threshold,
+  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, eps, threshold,
                          const_cast<float*>(p.floor), nq));
   note_launch(nullptr);
   profile_end(st, 1);
@@ -1582,7 +1543,7 @@ int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, 
   while (n2 < pl.stage_entries) n2 <<= 1;
   const size_t smem = size_t(n2) * sizeof(unsigned long long);
   FRG_CUDA(func_attr_once(range_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  FRG_CUDA(launch_kernel(range_select_kernel, dim3(nq), dim3(kSelectWarps * 32), smem, st, true, dense, cnt,
+  FRG_CUDA(launch_kernel(range_select_kernel, dim3(nq), dim3(kSelectWarps * 32), smem, st, dense, cnt,
                          pl.stage_entries, s->dim, qn, s->master, threshold, strict ? 1 : 0, max_hits, row_offset,
                          out_counts, out_rows, out_scores, flagged, n_flagged));
   note_launch(nullptr);

@@ -577,19 +577,21 @@ def test_bf16_only_store(frg, tmp_path):
     Q, target = synth.queries(f, n, d, seed=9, gallery_seed=21)
     Q[3] = G[11]
     m = frg.Matcher(store)
-    r = m.match(Q, k, 0.45)
-    assert r.variant == "tc_bf16"
     S = mo.cosine_scores(Q, G)
     ref_rows, ref_scores = mo.topk_from_scores(S, k)
-    assert np.abs(r.scores - ref_scores).max() <= COARSE_EPS
-    for f_ in range(f):
-        true_of_returned = S[f_, r.rows[f_]]
-        assert (true_of_returned >= ref_scores[f_, k - 1] - 2 * COARSE_EPS).all()
-        must = ref_rows[f_][ref_scores[f_] > ref_scores[f_, k - 1] + 2 * COARSE_EPS]
-        assert set(must) <= set(r.rows[f_])
-    assert list(r.rows[3]) == sorted([11] + list(range(2000, 9000, 2)))[:k]     # exact ties -> lowest rows
     hit = (target >= 0) & ~np.isin(target, np.arange(2000, 9000, 2))
-    assert (r.rows[hit, 0] == target[hit]).all()
+    # all 70 queries run the pre-pass and the filter; the first 4 alone run the fused probe+filter kernel (nq <= 8)
+    for nq in (f, 4):
+        r = m.match(Q[:nq], k, 0.45)
+        assert r.variant == "tc_bf16"
+        assert np.abs(r.scores - ref_scores[:nq]).max() <= COARSE_EPS
+        for f_ in range(nq):
+            true_of_returned = S[f_, r.rows[f_]]
+            assert (true_of_returned >= ref_scores[f_, k - 1] - 2 * COARSE_EPS).all()
+            must = ref_rows[f_][ref_scores[f_] > ref_scores[f_, k - 1] + 2 * COARSE_EPS]
+            assert set(must) <= set(r.rows[f_])
+        assert list(r.rows[3]) == sorted([11] + list(range(2000, 9000, 2)))[:k]     # exact ties -> lowest rows
+        assert (r.rows[hit[:nq], 0] == target[:nq][hit[:nq]]).all()
     for variant in ("scan_f32", "tc_exact"):
         with pytest.raises(frg.NativeError):
             m.match(Q, k, 0.45, variant=variant)

@@ -1,6 +1,6 @@
 """BASELINE config 1 on the GPU (run on the GPU box): 10 000 x 512 gallery, frames of F faces, top-1 + threshold,
 one frg_match_host call per frame (host buffers in and out, result waited for) and device-timed.
-    [FRG_TC_FUSED=0|1] python tools/config1_probe.py [rows] [variant]"""
+    python tools/config1_probe.py [rows] [variant]"""
 import sys
 import time
 

@@ -1,5 +1,5 @@
 """Per-stage device timings of the cosine TC pipeline for other row lengths (run on the GPU box).
-    python tools/dim_probe.py rows dim k batch [batch ...]      (FRG_TC_STAGES=6 pins the old ring depth)
+    python tools/dim_probe.py rows dim k batch [batch ...]
 """
 import json
 import sys

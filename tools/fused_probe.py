@@ -1,5 +1,6 @@
-"""Fused probe+filter kernel vs separate pre-pass, device-timed without stage events (run on the GPU box).
-    FRG_TC_FUSED=0|1 python tools/fused_probe.py [k] [batches...]"""
+"""Top-k step time of a bf16-only store at small batches, device-timed without stage events (run on the GPU box).
+Up to 8 queries run the fused probe+filter kernel, larger batches the separate pre-pass and filter.
+    python tools/fused_probe.py [k] [batches...]"""
 import sys
 
 import torch
@@ -11,7 +12,7 @@ from oracle import synth
 n, d = 1_000_000, 512
 k = int(sys.argv[1]) if len(sys.argv) > 1 else 5
 batches = [int(a) for a in sys.argv[2:]] or [1, 8, 16, 32, 64, 128]
-store = frg.GalleryStore(dim=d, capacity=n)
+store = frg.GalleryStore(dim=d, capacity=n, bf16_only=True)
 store.fill_synthetic(n, 0, 1234)
 m = frg.Matcher(store)
 for F in batches:

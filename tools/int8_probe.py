@@ -34,8 +34,7 @@ def main():
     store.fill_synthetic(a.rows, 0, synth.GALLERY_SEED)
     Q, _ = synth.queries(1024, a.rows, a.dim)
     m = frg.Matcher(store)
-    res = {"gpu": gpu, "rows": a.rows, "dim": a.dim, "k": 5, "stride_env": os.environ.get("FRG_TC_I8_STRIDE", "16"),
-           "batches": {}}
+    res = {"gpu": gpu, "rows": a.rows, "dim": a.dim, "k": 5, "batches": {}}
     for F in [int(x) for x in a.batches.split(",")]:
         q = np.ascontiguousarray(Q[:F])
         for _ in range(3):
