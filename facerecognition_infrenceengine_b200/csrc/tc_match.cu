@@ -508,18 +508,25 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     // ===== epilogue: thread = query (TMEM lane), columns = gallery rows =====
     const int quarter = warp & 3;                        // tcgen05.ld: warp w may touch lanes 32*(w%4)..+31
     // FILTER: the two warps of a quarter split every tile's columns (the epilogue is issue-latency
-    // bound, two warps per scheduler hide it).  GROUPMAX: one warp per quarter does all columns (the
+    // bound, two warps per scheduler hide it).  bf16 GROUPMAX: one warp per quarter does all columns (the
     // other only keeps the barrier protocol), so each (query, group) maximum costs ONE atomic per CTA.
-    constexpr int kSplit = MODE != kModeGroupMax ? kEpiWarps / 4 : 1;
-    const int half = MODE != kModeGroupMax ? (warp - 2) >> 2 : 0;
-    const bool idle = MODE == kModeGroupMax && warp >= 6;
+    // I8 GROUPMAX splits the columns like the filter and folds the two warps' maxima in shared memory at the end.
+    constexpr bool kSplitCols = MODE != kModeGroupMax || I8;
+    constexpr int kSplit = kSplitCols ? kEpiWarps / 4 : 1;
+    const int half = kSplitCols ? (warp - 2) >> 2 : 0;
+    const bool idle = !kSplitCols && warp >= 6;
     constexpr int kBlocksPerWarp = (kAccN / 32) / kSplit;
     const int q_local = quarter * 32 + lane;
     const int q = qtile * kTileQ + q_local;
     const bool q_real = q < p.nq;
 
-    AccT gmax[kGroups];                                  // GROUPMAX / FUSED probe: running maximum per row group
-    int gblk[kGroups];                                   // I8 GROUPMAX: 32-row block of each group's maximum
+    // GROUPMAX / FUSED probe: running maximum per row group.  I8 GROUPMAX keeps ONE packed key per group instead,
+    // acc * 256 + lb (|acc| <= 127^2 * 512 < 2^23, so the key is exact and orders by (acc, lb)), lb = the CTA-local
+    // 32-row block of the maximum within a window of kWinTiles tiles: one IMAD + IMNMX per score carries the winner.
+    // The larger block wins an exact tie; any winner is a valid distinct row of its group.
+    AccT gmax[kGroups];
+    constexpr int kTileBlocks = kAccN / 32;
+    constexpr int kWinTiles = 256 / kTileBlocks;
     AccT thr;
     if constexpr (I8) thr = INT_MAX;
     else thr = INFINITY;
@@ -572,10 +579,25 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     if (MODE != kModeFilter) {
 #pragma unroll
       for (int j = 0; j < kGroups; ++j) {
-        if constexpr (I8) { gmax[j] = A::none(); gblk[j] = 0; }
+        if constexpr (I8) gmax[j] = A::none();
         else gmax[j] = p.none_score;
       }
     }
+    // I8 GROUPMAX: fold the packed keys of the window that began at iteration it0 into the (query, group) 64-bit keys,
+    // (s32 product biased by 2^31) << 32 | row
+    auto publish_i8 = [&](int it0) {
+      if constexpr (I8) {
+        unsigned long long* o = p.group_key64 + size_t(q) * kGroups;
+#pragma unroll
+        for (int j = 0; j < kGroups; ++j) {
+          if (gmax[j] != A::none()) {
+            const int lb = gmax[j] & 255;
+            const int row = gtile(tile_of(it0 + lb / kTileBlocks)) * kAccN + (lb % kTileBlocks) * 32 + j;
+            atomicMax(o + j, (uint64_t(uint32_t(gmax[j] >> 8) ^ 0x80000000u) << 32) | uint32_t(row));
+          }
+        }
+      }
+    };
     if (MODE != kModeGroupMax && q_real) {
       if constexpr (I8) thr = derive_thr_i8();
       else if (MODE == kModeFilter) thr = derive_thr();
@@ -583,6 +605,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     }
 
     int buf = 0; uint32_t tphase = 0;
+    int win0 = 0;                                          // I8 GROUPMAX: first iteration of the current lb window
     for (int it = 0; it < n_iter && !*abort_flag; ++it) {
       const int t = tile_of(it);
       const int tile_row0 = gtile(t) * kAccN;              // first gallery row of this tile
@@ -616,17 +639,20 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
       AccT va[32], vb[32];
       auto process = [&](AccT (&v)[32], int b) {
         const uint32_t vm = vmask[b];
-        if (vm != 0xffffffffu) {           // warp-uniform: tombstones / other tenants / rows past the end
+        if (!(I8 && MODE == kModeGroupMax) && vm != 0xffffffffu) {   // warp-uniform: tombstones / other tenants / rows past the end
 #pragma unroll
           for (int j = 0; j < 32; ++j) v[j] = (vm >> j) & 1u ? v[j] : A::none();
         }
         if (MODE == kModeGroupMax) {
           // column j of every 32-row block belongs to group j (tiles start at multiples of 32)
           if constexpr (I8) {
-            const int blk = (tile_row0 >> 5) + b;
+            const int lb = (it % kWinTiles) * kTileBlocks + half * kBlocksPerWarp + b;
+            if (vm == 0xffffffffu) {
 #pragma unroll
-            for (int j = 0; j < 32; ++j) {
-              if (v[j] > gmax[j]) { gmax[j] = v[j]; gblk[j] = blk; }
+              for (int j = 0; j < 32; ++j) gmax[j] = max(gmax[j], v[j] * 256 + lb);
+            } else {
+#pragma unroll
+              for (int j = 0; j < 32; ++j) gmax[j] = max(gmax[j], (vm >> j) & 1u ? v[j] * 256 + lb : A::none());
             }
           } else {
 #pragma unroll
@@ -640,7 +666,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
           // The block maximum is built from four 8-column group maxima, and a thread that holds a candidate walks
           // only the group(s) that contain one: ~35 instructions instead of ~110 for all 32 columns.  A warp takes
           // this path whenever one of its 32 queries has a candidate among the 32 rows (about a quarter of all
-          // blocks), and the slowest epilogue warp decides when the accumulator buffer goes back to the MMA warp.
+          // blocks), and (bf16) the slowest epilogue warp decides when the accumulator buffer goes back to the MMA warp.
           // Measured against the 32-column walk (profiles/r02_ab_grouped.txt, same box, sustained clocks): -3.6 /
           // -4.8 / -7 % of the step at F = 256 / 512 / 1024, neutral at F <= 128 (HBM-bound, the epilogue has slack).
           AccT g0 = v[0], g1 = v[8], g2 = v[16], g3 = v[24];
@@ -667,25 +693,52 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
         }
       };
       __syncwarp();
-      tmem_ld32(taddr, va);
+      if constexpr (I8 && MODE == kModeFilter) {
+        // Early release: the int8 MMA takes as long as the TMEM reads of its tile (~2048 clk per pair tile at dim
+        // 512), so a buffer held through the rare paths stalls the tensor pipe.  All of the warp's blocks go to
+        // registers first; the buffer goes back to the MMA warp before any of them is processed.
+        AccT vs[kBlocksPerWarp][32];
 #pragma unroll
-      for (int b = 0; b < kBlocksPerWarp; b += 2) {
-        tmem_ld_wait();                    // va (block b) has landed
-        __syncwarp();                      // tcgen05.ld is .sync.aligned: reconverge after a slow path
-        tmem_ld32(taddr + (b + 1) * 32, vb);
-        process(va, b);
-        tmem_ld_wait();                    // vb (block b + 1)
+        for (int b = 0; b < kBlocksPerWarp; ++b) tmem_ld32(taddr + b * 32, vs[b]);
+        tmem_ld_wait();
+        tc_fence_before();
         __syncwarp();
-        if (b + 2 < kBlocksPerWarp) tmem_ld32(taddr + (b + 2) * 32, va);
-        process(vb, b + 1);
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) {
-        if (PAIR) mbar_arrive_remote(bar_tempty(buf), 0);      // the leader's MMA thread waits on it
-        else mbar_arrive(bar_tempty(buf));
+        if (lane == 0) {
+          if (PAIR) mbar_arrive_remote(bar_tempty(buf), 0);
+          else mbar_arrive(bar_tempty(buf));
+        }
+#pragma unroll
+        for (int b = 0; b < kBlocksPerWarp; ++b) process(vs[b], b);
+      } else {
+        tmem_ld32(taddr, va);
+#pragma unroll
+        for (int b = 0; b < kBlocksPerWarp; b += 2) {
+          tmem_ld_wait();                    // va (block b) has landed
+          __syncwarp();                      // tcgen05.ld is .sync.aligned: reconverge after a slow path
+          tmem_ld32(taddr + (b + 1) * 32, vb);
+          process(va, b);
+          tmem_ld_wait();                    // vb (block b + 1)
+          __syncwarp();
+          if (b + 2 < kBlocksPerWarp) tmem_ld32(taddr + (b + 2) * 32, va);
+          process(vb, b + 1);
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) {
+          if (PAIR) mbar_arrive_remote(bar_tempty(buf), 0);      // the leader's MMA thread waits on it
+          else mbar_arrive(bar_tempty(buf));
+        }
       }
       if (++buf == 2) { buf = 0; tphase ^= 1; }
+      if constexpr (MODE == kModeGroupMax && I8) {
+        // a window's blocks fill the 8 bits of lb: publish this warp's keys and start the next window
+        if ((it + 1) % kWinTiles == 0 && it + 1 < n_iter) {
+          if (q_real) publish_i8(win0);
+#pragma unroll
+          for (int j = 0; j < kGroups; ++j) gmax[j] = A::none();
+          win0 = it + 1;
+        }
+      }
 
       if constexpr (MODE == kModeFused && !I8) {
         const int since = it - (n_probe - 1);           // 0 at the last probe tile
@@ -714,20 +767,26 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
         }
       }
     }
-    if (q_real && !idle) {
+    if constexpr (MODE == kModeGroupMax && I8) {
+      // fold the two warps of the quarter through shared memory (the ring: the last tile's MMAs have retired),
+      // then ONE 64-bit atomicMax per (query, group) and CTA
+      int* fold = reinterpret_cast<int*>(sm + q_bytes);
+      if (half == 1) {
+#pragma unroll
+        for (int j = 0; j < kGroups; ++j) fold[j * kTileQ + q_local] = gmax[j];
+      }
+      asm volatile("bar.sync %0, 64;" ::"r"(2 + quarter) : "memory");
+      if (half == 0) {
+#pragma unroll
+        for (int j = 0; j < kGroups; ++j) gmax[j] = max(gmax[j], fold[j * kTileQ + q_local]);
+        if (q_real) publish_i8(win0);
+      }
+    } else if (q_real && !idle) {
       if (MODE == kModeGroupMax) {
-        if constexpr (I8) {
-          unsigned long long* o = p.group_key64 + size_t(q) * kGroups;
+        uint32_t* o = p.group_key + size_t(q) * kGroups;
 #pragma unroll
-          for (int j = 0; j < kGroups; ++j)
-            if (gmax[j] != A::none())
-              atomicMax(o + j, (uint64_t(uint32_t(gmax[j]) ^ 0x80000000u) << 32) | uint32_t(gblk[j] * 32 + j));
-        } else {
-          uint32_t* o = p.group_key + size_t(q) * kGroups;
-#pragma unroll
-          for (int j = 0; j < kGroups; ++j)
-            if (gmax[j] > p.none_score) atomicMax(o + j, float_key(gmax[j]));
-        }
+        for (int j = 0; j < kGroups; ++j)
+          if (gmax[j] > p.none_score) atomicMax(o + j, float_key(gmax[j]));
       } else {
         // pack this thread's few candidates into the query's dense list: one atomicAdd per (query, CTA),
         // outside the scan loop.  A private-segment overflow poisons the total so that select flags it
