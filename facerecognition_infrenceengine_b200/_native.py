@@ -74,6 +74,8 @@ SIGNATURES = {
     "frg_store_fill_synthetic": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_uint64, C.c_int32, _P]),
     "frg_match": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
     "frg_match_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
+    "frg_match_tenants": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P, _P]),
+    "frg_match_tenants_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
     "frg_first_match": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
     "frg_first_match_host": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), _P, _P]),
     "frg_match_range": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),

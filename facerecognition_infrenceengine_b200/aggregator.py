@@ -22,7 +22,9 @@ class BatchAggregator:
     """submit(embeddings [f, dim], company_id) -> Future of (rows [f,k], scores [f,k], accept [f]).
 
     A batch is flushed when `max_batch` faces are waiting or the oldest request is `max_delay_ms` old.
-    Requests with different company_id are batched separately (the tenant filter is per call).
+    Requests with different company_id are batched separately (the tenant filter is per call) - unless
+    `match_many_fn(Q, company_ids)` is given, a matcher with one company filter per face (``Matcher.match_tenants``):
+    then one batch takes the pending requests of every company in arrival order, up to `max_batch` faces.
     Rows are positions in the gallery: if the store may be compacted while requests are in flight, let `match_fn`
     translate rows to ids itself (``Matcher.match(..., with_ids=True)`` does so inside the store's read section) or
     carry ``MatchResult.layout_version`` along (``store.ids_of(rows, layout_version=...)``).
@@ -31,8 +33,11 @@ class BatchAggregator:
     other (bench `e2e.concurrent`: +10 % at 1024 queries per batch, +30 % at 64)."""
 
     def __init__(self, match_fn: Callable[[np.ndarray, Optional[str]], Tuple[np.ndarray, np.ndarray, np.ndarray]],
-                 max_batch: int = 256, max_delay_ms: float = 5.0, workers: int = 1):
+                 max_batch: int = 256, max_delay_ms: float = 5.0, workers: int = 1,
+                 match_many_fn: Optional[Callable[[np.ndarray, List[Optional[str]]],
+                                                  Tuple[np.ndarray, np.ndarray, np.ndarray]]] = None):
         self.match_fn = match_fn
+        self.match_many_fn = match_many_fn
         self.max_batch = max_batch
         self.max_delay = max_delay_ms / 1e3
         self._cv = threading.Condition()
@@ -62,11 +67,12 @@ class BatchAggregator:
             t.join(timeout=5)
 
     def _take(self):
-        """Called with the lock held: the requests of the oldest request's tenant, up to max_batch faces."""
+        """Called with the lock held: the requests of the oldest request's tenant (of every tenant with
+        match_many_fn), up to max_batch faces."""
         tenant = self._pending[0][1]
         take, rest, n = [], [], 0
         for item in self._pending:
-            if item[1] == tenant and (n == 0 or n + len(item[0]) <= self.max_batch):
+            if (self.match_many_fn is not None or item[1] == tenant) and (n == 0 or n + len(item[0]) <= self.max_batch):
                 take.append(item)
                 n += len(item[0])
             else:
@@ -93,7 +99,10 @@ class BatchAggregator:
                 take, tenant = self._take()
             try:
                 Q = np.concatenate([t[0] for t in take], axis=0)
-                rows, scores, accept = self.match_fn(Q, tenant)
+                if self.match_many_fn is not None:
+                    rows, scores, accept = self.match_many_fn(Q, [t[1] for t in take for _ in range(len(t[0]))])
+                else:
+                    rows, scores, accept = self.match_fn(Q, tenant)
                 with self._cv:
                     self.batches += 1
                     self.faces += len(Q)

@@ -3,6 +3,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <new>
 
 #include "frg_internal.cuh"
@@ -921,6 +922,29 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
   return rc;
 }
 
+// the match itself, s->mu held and the read ordered (store_begin_read)
+static int match_locked(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                        int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st,
+                        const ExchangeTail& tail, int sm_count) {
+  struct SeqBump { ~SeqBump() { ++g_match_seq; } } bump;      // sampled profiling: every 4th match is bracketed
+  // a tenant-filtered call scans only the rows that tenant can sit in (the whole gallery otherwise)
+  const int variant = pick_variant(s, p, nq);
+  const GalleryWindow w = window_of(s, p->tenant, variant == FRG_VARIANT_TC_EXACT || variant == FRG_VARIANT_TC_BF16);
+  frg_match_params_t pw = *p;
+  pw.row_offset += w.row0;
+  switch (variant) {
+    case FRG_VARIANT_SCAN_F32:
+      return match_scan(&w, q, nq, k, &pw, sm_count, out_rows, out_scores, out_accept, st, tail);
+    case FRG_VARIANT_TC_EXACT:
+      return match_tc(&w, q, nq, k, &pw, true, sm_count, out_rows, out_scores, out_accept, st, tail);
+    case FRG_VARIANT_TC_BF16:
+      return match_tc(&w, q, nq, k, &pw, false, sm_count, out_rows, out_scores, out_accept, st, tail);
+    default:
+      set_error("match: unknown variant %d", p->variant);
+      return FRG_ERR_INVALID;
+  }
+}
+
 static int match_impl(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
                       int64_t* out_rows, float* out_scores, uint8_t* out_accept, void* stream,
                       const ExchangeTail& tail) {
@@ -938,28 +962,133 @@ static int match_impl(frg_store* s, const float* q, int32_t nq, int32_t k, const
   std::lock_guard<std::mutex> lk(s->mu);   // enqueue under the lock: the snapshot a match sees is the
                                            // store as of this call (peopleCount.py:816-819 semantics)
   FRG_CHECK(store_begin_read(s, st));
-  struct SeqBump { ~SeqBump() { ++g_match_seq; } } bump;      // sampled profiling: every 4th match is bracketed
-  // a tenant-filtered call scans only the rows that tenant can sit in (the whole gallery otherwise)
-  const int variant = pick_variant(s, p, nq);
-  const GalleryWindow w = window_of(s, p->tenant, variant == FRG_VARIANT_TC_EXACT || variant == FRG_VARIANT_TC_BF16);
-  frg_match_params_t pw = *p;
-  pw.row_offset += w.row0;
-  switch (variant) {
-    case FRG_VARIANT_SCAN_F32:
-      return match_scan(&w, q, nq, k, &pw, di.sm_count, out_rows, out_scores, out_accept, st, tail);
-    case FRG_VARIANT_TC_EXACT:
-      return match_tc(&w, q, nq, k, &pw, true, di.sm_count, out_rows, out_scores, out_accept, st, tail);
-    case FRG_VARIANT_TC_BF16:
-      return match_tc(&w, q, nq, k, &pw, false, di.sm_count, out_rows, out_scores, out_accept, st, tail);
-    default:
-      set_error("match: unknown variant %d", p->variant);
-      return FRG_ERR_INVALID;
-  }
+  return match_locked(s, q, nq, k, p, out_rows, out_scores, out_accept, st, tail, di.sm_count);
 }
 
 int frg_match(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
               int64_t* out_rows, float* out_scores, uint8_t* out_accept, void* stream) {
   return match_impl(s, q, nq, k, p, out_rows, out_scores, out_accept, stream, ExchangeTail());
+}
+
+// ---- per-query tenants (frg_match_tenants)
+}  // extern "C"
+
+int frg::stage_upload(void* dev, const void* host, size_t bytes, cudaStream_t st) {
+  if (bytes == 0) return FRG_OK;
+  int slot = -1;
+  unsigned char* h = bytes <= PinnedRing::kMaxBytes ? g_upload_ring.acquire(bytes, &slot) : nullptr;
+  if (!h) {
+    (void)cudaGetLastError();
+    FRG_CUDA(cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, st));   // pageable: staged before it returns
+    return FRG_OK;
+  }
+  memcpy(h, host, bytes);
+  cudaError_t e = cudaMemcpyAsync(dev, h, bytes, cudaMemcpyHostToDevice, st);
+  g_upload_ring.release(slot, st);
+  if (e != cudaSuccess) return cuda_fail(e, "stage_upload", __FILE__, __LINE__);
+  return FRG_OK;
+}
+
+extern "C" {
+
+// Tiles a tenant's rows can sit in, in kTcTileRows-row tiles: its cached tile list when that is shorter than its
+// extent's tile range, else that range (other tenants' rows in it are masked by the filter's tag check), else every
+// tile (tenant < 0, or extents not known).  A tag no row carries: no tiles.  s->mu held.
+static int tenant_tiles(frg_store* s, int32_t tenant, cudaStream_t st, TcTenantGroup* g) {
+  g->tile0 = 0; g->n_tiles = int((s->rows + kTcTileRows - 1) / kTcTileRows); g->list = nullptr;
+  if (tenant < 0 || !s->extents_known) return FRG_OK;
+  auto it = s->extents.find(tenant);
+  const int64_t lo = it != s->extents.end() ? it->second.lo : 0;
+  const int64_t hi = it != s->extents.end() ? (it->second.hi < s->rows ? it->second.hi : s->rows) : 0;
+  if (hi <= lo) { g->n_tiles = 0; return FRG_OK; }
+  g->tile0 = int(lo / kTcTileRows);
+  g->n_tiles = int((hi - 1) / kTcTileRows) - g->tile0 + 1;
+  const int32_t* list = nullptr;
+  int n = 0;
+  FRG_CHECK(store_tile_list(s, tenant, kTcTileRows, st, &list, &n));
+  if (list && n < g->n_tiles) { g->list = list; g->n_tiles = n; }
+  return FRG_OK;
+}
+
+static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                              const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept,
+                              cudaStream_t st) {
+  reset_launches();
+  if (!s || !p || nq < 0 || (nq > 0 && (!q || !out_rows || !out_scores || !tenants))) {
+    set_error("match_tenants: bad argument");
+    return FRG_ERR_INVALID;
+  }
+  if (k < 1 || k > FRG_MAX_K) { set_error("match: k=%d out of range 1..%d", k, FRG_MAX_K); return FRG_ERR_INVALID; }
+  if (p->metric != FRG_METRIC_COSINE && p->metric != FRG_METRIC_EUCLIDEAN) { set_error("match: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
+  if (nq == 0) return FRG_OK;
+  // stable sort by tenant (every negative tag means "all tenants")
+  auto norm = [&](int32_t i) { return tenants[i] < 0 ? int32_t(-1) : tenants[i]; };
+  std::vector<int32_t> perm(static_cast<size_t>(nq));
+  for (int32_t i = 0; i < nq; ++i) perm[size_t(i)] = i;
+  std::stable_sort(perm.begin(), perm.end(), [&](int32_t a, int32_t b) { return norm(a) < norm(b); });
+  frg_match_params_t pg = *p;
+  if (norm(perm.front()) == norm(perm.back())) {            // one tenant: exactly frg_match
+    pg.tenant = norm(perm.front());
+    return match_impl(s, q, nq, k, &pg, out_rows, out_scores, out_accept, st, ExchangeTail());
+  }
+  std::vector<TcTenantGroup> groups;
+  for (int32_t i = 0; i < nq;) {
+    int32_t j = i + 1;
+    while (j < nq && norm(perm[size_t(j)]) == norm(perm[size_t(i)])) ++j;
+    TcTenantGroup g{};
+    g.tenant = norm(perm[size_t(i)]); g.q0 = i; g.nq = j - i;
+    groups.push_back(g);
+    i = j;
+  }
+  DeviceGuard dg(s->device);
+  if (!dg.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
+  DeviceInfo di;
+  FRG_CHECK(device_info(s->device, &di));
+  std::lock_guard<std::mutex> lk(s->mu);    // one snapshot of the store for every tenant of the call
+  FRG_CHECK(store_begin_read(s, st));
+  const int variant = pick_variant(s, p, nq);
+  const char* why = "";
+  const bool grouped = (variant == FRG_VARIANT_TC_EXACT || variant == FRG_VARIANT_TC_BF16) && has_plane8(s) &&
+                       s->master && p->metric == FRG_METRIC_COSINE && !(p->flags & FRG_QUERY_PRENORMALISED) &&
+                       tc_supported(s->dim, p->metric, &why) && s->rows > 0 && s->rows <= 0x7fffffff;
+  if (grouped) {
+    struct SeqBump { ~SeqBump() { ++g_match_seq; } } bump;
+    for (TcTenantGroup& g : groups) FRG_CHECK(tenant_tiles(s, g.tenant, st, &g));
+    const GalleryWindow w = window_of(s, -1);
+    FRG_CHECK(launch_tc_match_grouped(&w, q, perm, groups, k, p->threshold, p->row_offset, di.sm_count, out_rows,
+                                      out_scores, out_accept, st));
+    g_variant = "tc_exact_grouped";
+    return FRG_OK;
+  }
+  // every other store / variant: frg_match's own path once per tenant, into tenant-sorted scratch, then scattered
+  const size_t qb = (size_t(nq) * s->dim * 4 + 255) & ~size_t(255), pb = (size_t(nq) * 4 + 255) & ~size_t(255);
+  const size_t rb = (size_t(nq) * k * 8 + 255) & ~size_t(255), sb = (size_t(nq) * k * 4 + 255) & ~size_t(255);
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qb + pb + rb + sb + size_t(nq), st));
+  float* qs = reinterpret_cast<float*>(ws);
+  int32_t* dperm = reinterpret_cast<int32_t*>(ws + qb);
+  int64_t* srows = reinterpret_cast<int64_t*>(ws + qb + pb);
+  float* sscores = reinterpret_cast<float*>(ws + qb + pb + rb);
+  uint8_t* sacc = ws + qb + pb + rb + sb;
+  int rc = stage_upload(dperm, perm.data(), size_t(nq) * 4, st);
+  if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, s->dim, qs, st);
+  for (size_t i = 0; rc == FRG_OK && i < groups.size(); ++i) {
+    pg.tenant = groups[i].tenant;
+    const int q0 = groups[i].q0;
+    rc = match_locked(s, qs + size_t(q0) * s->dim, groups[i].nq, k, &pg, srows + size_t(q0) * k,
+                      sscores + size_t(q0) * k, sacc + q0, st, ExchangeTail(), di.sm_count);
+  }
+  const char* ran = g_variant;               // the per-tenant path that ran (the scatter does not rename it)
+  if (rc == FRG_OK) rc = launch_scatter_results(srows, sscores, sacc, dperm, nq, k, out_rows, out_scores, out_accept, st);
+  g_variant = ran;
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
+int frg_match_tenants(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                      const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept, void* stream) {
+  return match_tenants_impl(s, q, nq, k, p, tenants, out_rows, out_scores, out_accept, static_cast<cudaStream_t>(stream));
 }
 
 static int check_exchange(const frg_exchange_t* x, int32_t nq, int32_t k, XPush* out) {
@@ -1029,9 +1158,9 @@ struct PinnedScratch {
 };
 static thread_local PinnedScratch g_result_bounce;
 
-int frg_match_host(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
-                   int64_t* out_rows, float* out_scores, uint8_t* out_accept) {
-  if (!s || nq < 0 || (nq > 0 && (!q || !out_rows || !out_scores))) { set_error("match_host: bad argument"); return FRG_ERR_INVALID; }
+// tenants == nullptr: frg_match, else frg_match_tenants
+static int match_host_impl(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                           const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept) {
   if (k < 1 || k > FRG_MAX_K) { set_error("match: k=%d out of range 1..%d", k, FRG_MAX_K); return FRG_ERR_INVALID; }
   if (nq == 0) return FRG_OK;
   DeviceGuard g(s->device);
@@ -1045,8 +1174,10 @@ int frg_match_host(frg_store* s, const float* q, int32_t nq, int32_t k, const fr
   cudaError_t e = cudaMemcpyAsync(d, q, qb, cudaMemcpyHostToDevice, st);
   if (e != cudaSuccess) rc = cuda_fail(e, "H2D queries", __FILE__, __LINE__);
   if (rc == FRG_OK)
-    rc = frg_match(s, reinterpret_cast<float*>(d), nq, k, p, reinterpret_cast<int64_t*>(d + o_r),
-                   reinterpret_cast<float*>(d + o_s), d + o_a, st);
+    rc = tenants ? match_tenants_impl(s, reinterpret_cast<float*>(d), nq, k, p, tenants, reinterpret_cast<int64_t*>(d + o_r),
+                                      reinterpret_cast<float*>(d + o_s), d + o_a, st)
+                 : frg_match(s, reinterpret_cast<float*>(d), nq, k, p, reinterpret_cast<int64_t*>(d + o_r),
+                             reinterpret_cast<float*>(d + o_s), d + o_a, st);
   if (rc == FRG_OK) {
     // rows | scores | accept sit in one device range [o_r, o_a + ab): one copy into the pinned bounce
     const size_t span = o_a + ab - o_r;
@@ -1071,6 +1202,21 @@ int frg_match_host(frg_store* s, const float* q, int32_t nq, int32_t k, const fr
   }
   cudaFreeAsync(d, st);
   return rc;
+}
+
+int frg_match_host(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                   int64_t* out_rows, float* out_scores, uint8_t* out_accept) {
+  if (!s || nq < 0 || (nq > 0 && (!q || !out_rows || !out_scores))) { set_error("match_host: bad argument"); return FRG_ERR_INVALID; }
+  return match_host_impl(s, q, nq, k, p, nullptr, out_rows, out_scores, out_accept);
+}
+
+int frg_match_tenants_host(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                           const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept) {
+  if (!s || !p || nq < 0 || (nq > 0 && (!q || !out_rows || !out_scores || !tenants))) {
+    set_error("match_tenants_host: bad argument");
+    return FRG_ERR_INVALID;
+  }
+  return match_host_impl(s, q, nq, k, p, tenants, out_rows, out_scores, out_accept);
 }
 
 int frg_first_match(frg_store* s, const float* q, int32_t nq, const frg_match_params_t* p,

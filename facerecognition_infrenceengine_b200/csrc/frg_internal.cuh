@@ -360,6 +360,27 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
                     const __nv_bfloat16* qb_prepass = nullptr, const float* coef = nullptr,
                     const int8_t* qi8 = nullptr, const float* qstep = nullptr);
 
+// tc_match.cu: per-query tenants (frg_match_tenants) on the int8 filter of a unit cosine store.  The batch is sorted by
+// tenant (perm[i] = caller position of sorted query i); group g holds sorted queries q0 .. q0 + nq - 1 of one tenant and
+// scans the absolute kTcTileRows-row tiles list[0 .. n_tiles) or tile0 .. tile0 + n_tiles - 1 (a masked range).  One
+// grid per stage serves every group; results go to the caller's order.  s: the whole store (row0 = 0).
+constexpr int kTcTileRows = 128;
+struct TcTenantGroup { int32_t tenant; int q0, nq; int tile0, n_tiles; const int32_t* list; };
+int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::vector<int32_t>& perm,
+                            const std::vector<TcTenantGroup>& groups, int k, float threshold, int64_t row_offset,
+                            int sm_count, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st);
+// tc_match.cu: out[i] = q[perm[i]] (rows of dim floats); out[perm[i]] = sorted result i (rows / scores [nq][k], accept)
+int launch_gather_queries(const float* q, const int32_t* perm, int nq, int dim, float* out, cudaStream_t st);
+int launch_scatter_results(const int64_t* rows, const float* scores, const uint8_t* accept, const int32_t* perm, int nq,
+                           int k, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st);
+// scan_f32.cu: the exact re-do of launch_scan_f32_flagged, each flagged query q with its own tenant q_tenant[q]
+// (device array; cosine, fp32 master, a.tenant ignored)
+int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, const int* flagged,
+                                    int* n_flagged_and_ticket, int64_t row_offset, float threshold, int64_t* out_rows,
+                                    float* out_scores, uint8_t* out_accept, cudaStream_t st);
+// api.cu: host -> device copy through the per-thread pinned staging ring (pageable copy when larger than a slot)
+int stage_upload(void* dev, const void* host, size_t bytes, cudaStream_t st);
+
 // tc_match.cu: range search over a unit cosine store (frg_match_range).  The filter keeps every row with
 // S >= threshold - eps[q] (no pre-pass); range_select_kernel rescores each candidate exactly, keeps those that pass
 // (score >= threshold, '>' when strict), writes the first max_hits in gallery order and the count.  Queries whose

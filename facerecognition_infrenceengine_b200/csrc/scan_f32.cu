@@ -370,6 +370,97 @@ scan_f32_flagged_kernel(const ROW* __restrict__ master, const int32_t* __restric
   }
 }
 
+// The exact re-do of scan_f32_flagged_kernel for a batch whose queries carry their own tenants (frg_match_tenants):
+// flagged query q is scanned alone with tenant q_tenant[q] - a tenant-filtered one reads the tags first and fetches
+// only its tenant's rows (SPARSE sweep), an unfiltered one streams every row.  Same partial lists, ticket and merge.
+template <int NJ, int KMAX>
+__global__ void __launch_bounds__(kScanWarps * 32, 2)
+scan_f32_flagged_tenants_kernel(const float* __restrict__ master, const int32_t* __restrict__ tags, int64_t rows,
+                                const float* __restrict__ qn, int nq_total, const int32_t* __restrict__ q_tenant,
+                                const int* __restrict__ flagged, int* __restrict__ ctl, int K, float threshold,
+                                int64_t row_offset, float* __restrict__ part_sc, int32_t* __restrict__ part_ix,
+                                int64_t* __restrict__ out_rows, float* __restrict__ out_scores,
+                                uint8_t* __restrict__ out_accept) {
+  extern __shared__ unsigned char smem_raw[];
+  float* l_sc = reinterpret_cast<float*>(smem_raw);
+  int32_t* l_ix = reinterpret_cast<int32_t*>(l_sc + kScanWarps * K);
+  __shared__ int is_last;
+  pdl_wait();             // the select kernel's list of flagged queries
+  pdl_trigger();
+  const int nf = ctl[0];
+  for (int slot = 0; slot < nf; ++slot) {
+    const int q_of[1] = {flagged[slot]};
+    const int32_t tenant = q_tenant[q_of[0]];
+    if (tenant >= 0)
+      scan_pass<NJ, 1, FRG_METRIC_COSINE, float, true>(master, tags, rows, qn, q_of, 1, nq_total, slot, K, tenant,
+                                                       part_sc, part_ix, l_sc, l_ix);
+    else
+      scan_pass<NJ, 1, FRG_METRIC_COSINE>(master, tags, rows, qn, q_of, 1, nq_total, slot, K, -1, part_sc, part_ix,
+                                          l_sc, l_ix);
+    __syncthreads();
+  }
+  if (nf == 0) return;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) is_last = atomicAdd(ctl + 1, 1) == int(gridDim.x) - 1;
+  __syncthreads();
+  if (!is_last) return;
+  __threadfence();
+  for (int slot = threadIdx.x >> 5; slot < nf; slot += kScanWarps)
+    merge_one<int32_t, KMAX>(part_sc, part_ix, int(gridDim.x), nq_total, K, K, FRG_METRIC_COSINE, threshold, row_offset,
+                             0, slot, flagged[slot], int64_t(nq_total) * K, int64_t(nq_total) * K, out_rows, out_scores,
+                             out_accept);
+}
+
+template <int NJ, int KMAX>
+static int launch_flagged_tenants_k(const ScanArgs& a, int grid, const int32_t* q_tenant, const int* flagged, int* ctl,
+                                    float threshold, int64_t row_offset, float* ps, int32_t* pi, int64_t* out_rows,
+                                    float* out_scores, uint8_t* out_accept, cudaStream_t st) {
+  const size_t smem = size_t(kScanWarps) * a.k * (sizeof(float) + sizeof(int32_t));
+  auto kern = scan_f32_flagged_tenants_kernel<NJ, KMAX>;
+  FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+  FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn, a.nq,
+                         q_tenant, flagged, ctl, a.k, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept));
+  note_launch(nullptr);
+  return FRG_OK;
+}
+
+template <int NJ>
+static int launch_flagged_tenants_t(const ScanArgs& a, int grid, const int32_t* q_tenant, const int* flagged, int* ctl,
+                                    float threshold, int64_t row_offset, float* ps, int32_t* pi, int64_t* out_rows,
+                                    float* out_scores, uint8_t* out_accept, cudaStream_t st) {
+#define FRG_FT(KM) return launch_flagged_tenants_k<NJ, KM>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, \
+                                                            pi, out_rows, out_scores, out_accept, st)
+  if (a.k == 1) FRG_FT(1);
+  if (a.k <= 4) FRG_FT(4);
+  if (a.k <= 8) FRG_FT(8);
+  FRG_FT(16);
+#undef FRG_FT
+}
+
+int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, const int* flagged, int* ctl,
+                                    int64_t row_offset, float threshold, int64_t* out_rows, float* out_scores,
+                                    uint8_t* out_accept, cudaStream_t st) {
+  if (a.rows <= 0 || a.nq <= 0) return FRG_OK;
+  if (!a.master || a.metric != FRG_METRIC_COSINE) { set_error("flagged scan: per-query tenants need a cosine master"); return FRG_ERR_UNSUPPORTED; }
+  const int grid = a.sm_count;
+  const size_t n_part = size_t(grid) * a.nq * a.k;
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_part * 8, st));
+  float* ps = reinterpret_cast<float*>(ws);
+  int32_t* pi = reinterpret_cast<int32_t*>(ps + n_part);
+  int rc;
+  switch (a.dim) {
+    case 128: rc = launch_flagged_tenants_t<1>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept, st); break;
+    case 256: rc = launch_flagged_tenants_t<2>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept, st); break;
+    case 512: rc = launch_flagged_tenants_t<4>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept, st); break;
+    default: set_error("flagged scan: dim %d not built", a.dim); rc = FRG_ERR_UNSUPPORTED; break;
+  }
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
 static int scan_grid(const ScanArgs& a) {
   const int r = a.dim >= 512 ? 2 : (a.dim == 256 ? 4 : 8);     // rows in flight per warp (scan_pass)
   int64_t want = (a.rows + kScanWarps * r - 1) / (kScanWarps * r);

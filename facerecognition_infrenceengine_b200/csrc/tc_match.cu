@@ -2,7 +2,9 @@
 // on tcgen05 with the threshold / top-k in the epilogue, so no score matrix reaches HBM.  Which store runs which filter:
 //   - a unit cosine store with an fp32 master: the int8 filter (I8; pre-pass, i8_floor_kernel, filter, select);
 //   - the Euclidean plane of a raw store and a bf16-only store: the bf16 filter described below;
-//   - a bf16-only store matched with nq <= 8 queries: the bf16 filter with the pre-pass folded in (MODE = FUSED).
+//   - a bf16-only store matched with nq <= 8 queries: the bf16 filter with the pre-pass folded in (MODE = FUSED);
+//   - per-query tenants on a unit cosine store (frg_match_tenants): the int8 pre-pass and filter in their GROUPED
+//     single-CTA form, every CTA one (query tile of one tenant, chunk of that tenant's tiles) of a host-built table.
 //
 //   S[q, r] = sum_k Qb[q, k] * Gb[r, k]        Qb, Gb = bf16 images of the unit fp32 vectors
 //
@@ -39,6 +41,7 @@
 #include <cuda.h>
 
 #include <cmath>
+#include <cstring>
 
 #include "frg_internal.cuh"
 
@@ -279,6 +282,16 @@ constexpr int kGroups = 32;
 // (float_key / key_float, frg_internal.cuh: the group maxima of all pre-pass CTAs are folded with one atomicMax per
 // (query, group) on order-preserving keys)
 
+// GROUPED launch (frg_match_tenants): what one CTA of a grid over many (query tile, tenant) pairs works on.  Queries
+// q0 .. q0 + nq - 1 of the tenant-sorted batch (one tenant), chunk `chunk` of `chunks` over its gallery tiles: the
+// absolute 128-row tiles list[0 .. n_tiles) or, without a list, tile0 .. tile0 + n_tiles - 1; every scale-th of them
+// (pre-pass sample).  Its candidate segments start at cand[cand0], seg entries each.
+struct TcGroupCta {
+  int q0, nq, tenant, chunk, chunks, tile0, n_tiles, scale, seg;
+  long long cand0;
+  const int32_t* list;
+};
+
 struct TcScanParams {
   int dim;                 // 512 etc. (multiple of 64; of 128 for the int8 filter)
   int n_rows;              // gallery rows
@@ -317,6 +330,8 @@ struct TcScanParams {
   // n_list listed tiles instead of every tile of the window; entry = absolute tile index (tile = kAccN rows)
   const int32_t* tile_list;
   int n_list;
+  // GROUPED: one descriptor per CTA (blockIdx.x), frg_match_tenants
+  const TcGroupCta* groups;
 };
 
 // MASKED: rows can be invalid for this call (tombstones, or a tenant filter): their tags are read
@@ -329,11 +344,14 @@ struct TcScanParams {
 // owns the full/tmem_empty barriers and issues the MMAs; commits are multicast to both CTAs.
 // I8: int8 operands (unit cosine store's int8 plane): tcgen05.mma kind::i8, K = 32 per MMA, 128 int8 per k-block,
 // exact s32 accumulators; half the MMA time and half the plane bytes of bf16 per score.  Not FUSED.
-template <int MODE, bool MASKED, bool PAIR, bool I8 = false>
+// GROUPED: blockIdx.x selects a TcGroupCta (single-CTA int8 form only); the query tile, tenant, tile source and chunk
+// come from it instead of the grid and the scalar parameters.
+template <int MODE, bool MASKED, bool PAIR, bool I8 = false, bool GROUPED = false>
 __global__ void __launch_bounds__(kTcThreads, 1)
 tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant__ CUtensorMap g_map,
                const __grid_constant__ CUtensorMap pad_map, const TcScanParams p) {
   static_assert(!(I8 && MODE == kModeFused), "the int8 filter takes its floor from i8_floor_kernel");
+  static_assert(!GROUPED || (I8 && MASKED && !PAIR), "the grouped form is the single-CTA int8 masked filter");
   using A = Acc<I8>;
   using AccT = typename A::T;
   constexpr int kAccN = PAIR ? 2 * kTileR : kTileR;        // accumulator columns = gallery rows per tile
@@ -368,13 +386,20 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int qtile = blockIdx.x;
-  const int chunk = blockIdx.y, chunks = gridDim.y;
+  TcGroupCta gd{};
+  if constexpr (GROUPED) gd = p.groups[blockIdx.x];     // written by the host copy that precedes the whole match
+  const int chunk = GROUPED ? gd.chunk : int(blockIdx.y), chunks = GROUPED ? gd.chunks : int(gridDim.y);
+  const int tile_scale = GROUPED ? gd.scale : p.tile_scale;
   // view tile v stands for gallery tile v * tile_scale (the pre-pass samples whole 128-row tiles:
   // contiguous 128 KB reads, spread evenly over the gallery)
-  const int tiles_all = p.tile_list ? p.n_list : (p.n_rows + kAccN - 1) / kAccN;
-  const int tiles_total = (tiles_all + p.tile_scale - 1) / p.tile_scale;
+  const int tiles_all = GROUPED ? gd.n_tiles : (p.tile_list ? p.n_list : (p.n_rows + kAccN - 1) / kAccN);
+  const int tiles_total = (tiles_all + tile_scale - 1) / tile_scale;
   // gallery tile behind view tile v
-  auto gtile = [&](int v) { const int i = v * p.tile_scale; return p.tile_list ? __ldg(p.tile_list + i) : i; };
+  auto gtile = [&](int v) {
+    const int i = v * tile_scale;
+    if constexpr (GROUPED) return gd.list ? __ldg(gd.list + i) : gd.tile0 + i;
+    else return p.tile_list ? __ldg(p.tile_list + i) : i;
+  };
   const int tile_begin = int((int64_t(tiles_total) * chunk) / chunks);
   const int tile_end = int((int64_t(tiles_total) * (chunk + 1)) / chunks);
   // FUSED: the CTA's first n_probe tiles (1/64 of its chunk, at least one) are visited twice - first as
@@ -423,10 +448,10 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
             // the query tile's k-block kb, issued just ahead of the first gallery block that meets it
             if (PAIR) {
               if (leader) mbar_expect_tx(bar_q(kb), 2 * kQBlockBytes);
-              tma_load_2d_pair(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlk, qtile * kTileQ, kEvictLast);
+              tma_load_2d_pair(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlk, GROUPED ? gd.q0 : qtile * kTileQ, kEvictLast);
             } else {
               mbar_expect_tx(bar_q(kb), kQBlockBytes);
-              tma_load_2d(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlk, qtile * kTileQ, kEvictLast);
+              tma_load_2d(q_smem + kb * kQBlockBytes, &q_map, bar_q(kb), kb * kBlk, GROUPED ? gd.q0 : qtile * kTileQ, kEvictLast);
             }
           }
           mbar_wait(bar_empty(stage), phase ^ 1, abort_flag);
@@ -517,8 +542,9 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     const bool idle = !kSplitCols && warp >= 6;
     constexpr int kBlocksPerWarp = (kAccN / 32) / kSplit;
     const int q_local = quarter * 32 + lane;
-    const int q = qtile * kTileQ + q_local;
-    const bool q_real = q < p.nq;
+    const int q = (GROUPED ? gd.q0 : qtile * kTileQ) + q_local;
+    const bool q_real = GROUPED ? q_local < gd.nq : q < p.nq;
+    const int32_t tenant = GROUPED ? gd.tenant : p.tenant;
 
     // GROUPMAX / FUSED probe: running maximum per row group.  I8 GROUPMAX keeps ONE packed key per group instead,
     // acc * 256 + lb (|acc| <= 127^2 * 512 < 2^23, so the key is exact and orders by (acc, lb)), lb = the CTA-local
@@ -601,7 +627,8 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
     if (MODE != kModeGroupMax && q_real) {
       if constexpr (I8) thr = derive_thr_i8();
       else if (MODE == kModeFilter) thr = derive_thr();
-      my_seg = p.cand + ((size_t(q) * chunks + chunk) * (kEpiWarps / 4) + half) * p.seg;
+      if constexpr (GROUPED) my_seg = p.cand + gd.cand0 + ((size_t(q_local) * chunks + chunk) * (kEpiWarps / 4) + half) * gd.seg;
+      else my_seg = p.cand + ((size_t(q) * chunks + chunk) * (kEpiWarps / 4) + half) * p.seg;
     }
 
     int buf = 0; uint32_t tphase = 0;
@@ -627,7 +654,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
         bool ok = row < p.n_rows;
         if (MASKED && ok) {
           const int32_t tag = __ldg(p.tags + row);
-          ok = tag >= 0 && (p.tenant < 0 || tag == p.tenant);
+          ok = tag >= 0 && (tenant < 0 || tag == tenant);
         }
         vmask[b] = __ballot_sync(0xffffffffu, ok);
       }
@@ -683,7 +710,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
 #pragma unroll
                 for (int j = 8 * g; j < 8 * g + 8; ++j) {
                   if (v[j] >= thr) {
-                    if (emitted < p.seg) my_seg[emitted] = make_int2(row0 + j, A::bits(v[j]));
+                    if (emitted < (GROUPED ? gd.seg : p.seg)) my_seg[emitted] = make_int2(row0 + j, A::bits(v[j]));
                     ++emitted;
                   }
                 }
@@ -791,8 +818,9 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap q_map, const __grid_constant_
         // pack this thread's few candidates into the query's dense list: one atomicAdd per (query, CTA),
         // outside the scan loop.  A private-segment overflow poisons the total so that select flags it
         // (2^20 > any dense_cap; a query has at most 2 * 148 segments, so the sum of poisons cannot wrap).
-        const int base = atomicAdd(p.cand_total + q, emitted > p.seg ? (1 << 20) : emitted);
-        const int mine_n = emitted < p.seg ? emitted : p.seg;
+        const int seg = GROUPED ? gd.seg : p.seg;
+        const int base = atomicAdd(p.cand_total + q, emitted > seg ? (1 << 20) : emitted);
+        const int mine_n = emitted < seg ? emitted : seg;
         for (int i = 0; i < mine_n; ++i)
           if (unsigned(base + i) < unsigned(p.dense_cap)) p.dense[size_t(q) * p.dense_cap + base + i] = my_seg[i];
       }
@@ -1285,11 +1313,11 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   pl->total = off;
 }
 
-template <int MODE, bool MASKED, bool PAIR, bool I8>
+template <int MODE, bool MASKED, bool PAIR, bool I8, bool GROUPED = false>
 static int launch_tc_scan(const CUtensorMap& qm, const CUtensorMap& gm, const CUtensorMap& pm, const TcScanParams& p,
                           int qtiles, int chunks, cudaStream_t st) {
   const size_t smem = tc_smem_bytes(I8 ? p.dim : 2 * p.dim);
-  auto kern = tc_scan_kernel<MODE, MASKED, PAIR, I8>;
+  auto kern = tc_scan_kernel<MODE, MASKED, PAIR, I8, GROUPED>;
   FRG_CUDA(func_attr_once(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kSmemLimit)));
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(qtiles, chunks);
@@ -1609,6 +1637,231 @@ int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, 
   FRG_CUDA(cudaGetLastError());
   profile_end(st, 1);
   return FRG_OK;
+}
+
+// ------------------------------------------------------------------------------------------ per-query tenants
+static_assert(kTileR == kTcTileRows, "the host plans tile sources in kTcTileRows-row tiles");
+
+// rows -> original query position: sorted[i] = q[perm[i]]
+__global__ void __launch_bounds__(128)
+gather_queries_kernel(const float* __restrict__ q, const int32_t* __restrict__ perm, int nq, int dim,
+                      float* __restrict__ out) {
+  pdl_wait();
+  pdl_trigger();
+  const int lane = threadIdx.x & 31;
+  const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (w >= nq) return;
+  const float4* src = reinterpret_cast<const float4*>(q + size_t(__ldg(perm + w)) * dim);
+  float4* dst = reinterpret_cast<float4*>(out + size_t(w) * dim);
+  for (int v = lane; v < (dim >> 2); v += 32) dst[v] = __ldg(src + v);
+}
+
+// results of sorted query i -> the caller's slot perm[i]
+__global__ void __launch_bounds__(256)
+scatter_results_kernel(const int64_t* __restrict__ rows, const float* __restrict__ scores,
+                       const uint8_t* __restrict__ accept, const int32_t* __restrict__ perm, int nq, int k,
+                       int64_t* __restrict__ out_rows, float* __restrict__ out_scores, uint8_t* __restrict__ out_accept) {
+  pdl_wait();
+  pdl_trigger();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nq * k) return;
+  const int q = i / k, j = i - q * k;
+  const size_t o = size_t(__ldg(perm + q)) * k + j;
+  out_rows[o] = rows[i];
+  out_scores[o] = scores[i];
+  if (out_accept && j == 0) out_accept[o / k] = accept[q];
+}
+
+int launch_gather_queries(const float* q, const int32_t* perm, int nq, int dim, float* out, cudaStream_t st) {
+  if (nq <= 0) return FRG_OK;
+  FRG_CUDA(launch_kernel(gather_queries_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, q, perm, nq, dim, out));
+  note_launch(nullptr);
+  return FRG_OK;
+}
+
+int launch_scatter_results(const int64_t* rows, const float* scores, const uint8_t* accept, const int32_t* perm, int nq,
+                           int k, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st) {
+  if (nq <= 0) return FRG_OK;
+  FRG_CUDA(launch_kernel(scatter_results_kernel, dim3((nq * k + 255) / 256), dim3(256), 0, st, rows, scores, accept,
+                         perm, nq, k, out_rows, out_scores, out_accept));
+  note_launch(nullptr);
+  return FRG_OK;
+}
+
+// Chunks of each unit in proportion to its tiles, so that the whole grid stays near one wave of sm_count CTAs
+// (at least one chunk per unit, at most one per tile).
+static std::vector<int> proportional_chunks(const std::vector<int>& tiles, int sm_count) {
+  int64_t total = 0;
+  for (int t : tiles) total += t;
+  std::vector<int> c(tiles.size(), 0);
+  for (size_t i = 0; i < tiles.size(); ++i) {
+    if (tiles[i] <= 0) continue;
+    int64_t x = total > 0 ? int64_t(sm_count) * tiles[i] / total : 1;
+    if (x < 1) x = 1;
+    if (x > tiles[i]) x = tiles[i];
+    c[i] = int(x);
+  }
+  return c;
+}
+
+int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::vector<int32_t>& perm,
+                            const std::vector<TcTenantGroup>& groups, int k, float threshold, int64_t row_offset,
+                            int sm_count, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st) {
+  const int nq = int(perm.size());
+  const int dim = s->dim;
+  if (!s->plane8 || !s->master || s->rows <= 0 || s->rows > 0x7fffffff) {
+    set_error("tc_match_grouped: needs a non-empty unit store with an int8 plane and an fp32 master");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  // ---- plan: query tiles of at most kTileQ queries, never across tenants
+  struct Unit { int q0, nq, g; };
+  std::vector<Unit> units;
+  for (int g = 0; g < int(groups.size()); ++g)
+    for (int a = 0; a < groups[g].nq; a += kTileQ)
+      units.push_back(Unit{groups[g].q0 + a, groups[g].nq - a < kTileQ ? groups[g].nq - a : kTileQ, g});
+  std::vector<int> tiles_main(units.size()), tiles_pre(units.size()), stride(units.size()), entries(units.size());
+  int dense_cap = 0;
+  for (size_t u = 0; u < units.size(); ++u) {
+    const int n = groups[units[u].g].n_tiles;
+    // the plan of a single-tenant match over the same tiles (tc_plan): pre-pass stride and candidate budget
+    TcPlan pl;
+    tc_plan(int64_t(n) * kTileR, dim, 1, k, sm_count, &pl, false, true);
+    stride[u] = pl.stride;
+    entries[u] = pl.stage_entries;
+    tiles_main[u] = n;
+    tiles_pre[u] = (n + pl.stride - 1) / pl.stride;
+    if (pl.stage_entries > dense_cap) dense_cap = pl.stage_entries;
+  }
+  const std::vector<int> ch_main = proportional_chunks(tiles_main, sm_count);
+  const std::vector<int> ch_pre = proportional_chunks(tiles_pre, sm_count);
+  std::vector<TcGroupCta> pre, main;
+  int64_t cand_entries = 0;
+  for (size_t u = 0; u < units.size(); ++u) {
+    const TcTenantGroup& G = groups[units[u].g];
+    if (tiles_main[u] == 0) continue;                  // an unknown tag: no rows, nothing to scan
+    // private segments of this tile's queries: one per (query, chunk, column half), x2 headroom (as tc_plan)
+    const int nseg = ch_main[u] * (kEpiWarps / 4);
+    int seg = (2 * entries[u] + nseg - 1) / nseg;
+    if (seg < 12) seg = 12;
+    TcGroupCta d{};
+    d.q0 = units[u].q0; d.nq = units[u].nq; d.tenant = G.tenant; d.tile0 = G.tile0; d.n_tiles = G.n_tiles;
+    d.list = G.list; d.seg = seg; d.cand0 = cand_entries;
+    for (int c = 0; c < ch_main[u]; ++c) { d.chunk = c; d.chunks = ch_main[u]; d.scale = 1; main.push_back(d); }
+    for (int c = 0; c < ch_pre[u]; ++c) { d.chunk = c; d.chunks = ch_pre[u]; d.scale = stride[u]; pre.push_back(d); }
+    cand_entries += int64_t(kTileQ) * nseg * seg;
+  }
+  if (dense_cap < 256) dense_cap = 256;
+  // ---- workspace (one stream-ordered allocation)
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
+  const size_t o_qs = take(size_t(nq) * dim * 4), o_qn = take(size_t(nq) * dim * 4), o_qi8 = take(size_t(nq) * dim);
+  const size_t o_eps = take(size_t(nq) * 4), o_step = take(size_t(nq) * 4), o_keys = take(size_t(nq) * kGroups * 8);
+  const size_t o_cnt = take(size_t(nq) * 4), o_flag = take(size_t(nq) * 4 + 12), o_floor = take(size_t(nq) * 4);
+  const size_t o_cand = take(size_t(cand_entries > 0 ? cand_entries : 1) * 8);
+  const size_t o_dense = take(size_t(nq) * dense_cap * 8);
+  const size_t o_rows = take(size_t(nq) * k * 8), o_sc = take(size_t(nq) * k * 4), o_acc = take(size_t(nq));
+  // the only host -> device copy of the call: [perm][tenant of each sorted query][pre-pass CTAs][filter CTAs]
+  std::vector<unsigned char> table;
+  const size_t t_perm = 0, t_ten = size_t(nq) * 4, t_pre = (t_ten + size_t(nq) * 4 + 15) & ~size_t(15);
+  const size_t t_main = t_pre + pre.size() * sizeof(TcGroupCta);
+  table.resize(t_main + main.size() * sizeof(TcGroupCta));
+  memcpy(table.data() + t_perm, perm.data(), size_t(nq) * 4);
+  for (const TcTenantGroup& G : groups)
+    for (int i = 0; i < G.nq; ++i) memcpy(table.data() + t_ten + size_t(G.q0 + i) * 4, &G.tenant, 4);
+  if (!pre.empty()) memcpy(table.data() + t_pre, pre.data(), pre.size() * sizeof(TcGroupCta));
+  if (!main.empty()) memcpy(table.data() + t_main, main.data(), main.size() * sizeof(TcGroupCta));
+  const size_t o_table = take(table.size());
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), off, st));
+  float* qs = reinterpret_cast<float*>(ws + o_qs);
+  float* qn = reinterpret_cast<float*>(ws + o_qn);
+  int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
+  float* eps = reinterpret_cast<float*>(ws + o_eps);
+  float* qstep = reinterpret_cast<float*>(ws + o_step);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + o_keys);
+  int* cnt = reinterpret_cast<int*>(ws + o_cnt);
+  int* flagged = reinterpret_cast<int*>(ws + o_flag);
+  int* n_flagged = flagged + nq;
+  float* floor_v = reinterpret_cast<float*>(ws + o_floor);
+  int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
+  float* sscores = reinterpret_cast<float*>(ws + o_sc);
+  uint8_t* sacc = ws + o_acc;
+  const int32_t* dperm = reinterpret_cast<const int32_t*>(ws + o_table + t_perm);
+  const int32_t* dten = reinterpret_cast<const int32_t*>(ws + o_table + t_ten);
+  int rc = stage_upload(ws + o_table, table.data(), table.size(), st);
+  if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, dim, qs, st);
+  profile_begin(st, kStagePrep);
+  if (rc == FRG_OK)
+    rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, keys, cnt, n_flagged, st);
+  profile_end(st, 1);
+  CUtensorMap qm, gm;
+  if (rc == FRG_OK) rc = make_map(&qm, qi8, dim, nq, size_t(dim), kTileQ, kBlockK, true);
+  if (rc == FRG_OK) rc = make_map(&gm, s->plane8, dim, s->rows, size_t(dim), kTileR, kBlockK, true);
+  TcScanParams p{};
+  p.fault = s->fault; p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
+  p.dim = dim; p.nq = nq; p.tenant = -1; p.tags = s->tags; p.n_rows = int(s->rows); p.k = k; p.tile_scale = 1;
+  p.group_key64 = keys; p.floor = floor_v; p.qstep = qstep;
+  p.cand = reinterpret_cast<int2*>(ws + o_cand); p.cand_total = cnt;
+  p.dense = reinterpret_cast<int2*>(ws + o_dense); p.dense_cap = dense_cap;
+  // 1. int8 pre-pass, 2. exact floor, 3. filter: every (query tile, chunk) of every tenant in one grid each
+  profile_begin(st, kStagePrepass);
+  if (rc == FRG_OK && !pre.empty()) {
+    p.groups = reinterpret_cast<const TcGroupCta*>(ws + o_table + t_pre);
+    rc = launch_tc_scan<kModeGroupMax, true, false, true, true>(qm, gm, gm, p, int(pre.size()), 1, st);
+  }
+  profile_end(st, 1);
+  profile_begin(st, kStageFloor);
+  if (rc == FRG_OK) {
+    cudaError_t e = launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, keys, nq, k, dim, qn,
+                                  s->master, eps, floor_v);
+    if (e != cudaSuccess) rc = cuda_fail(e, "i8_floor_kernel", __FILE__, __LINE__);
+    else note_launch(nullptr);
+  }
+  profile_end(st, 1);
+  profile_begin(st, kStageDominant);
+  if (rc == FRG_OK && !main.empty()) {
+    p.groups = reinterpret_cast<const TcGroupCta*>(ws + o_table + t_main);
+    rc = launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, int(main.size()), 1, st);
+  }
+  profile_end(st, 1);
+  // 4. select + exact rescoring into the sorted scratch (the tenant filter was applied by the filter's tag check)
+  profile_begin(st, kStageSelect);
+  if (rc == FRG_OK) {
+    cudaError_t e = cudaSuccess;
+#define FRG_SELECT_G(KK)                                                                                          \
+  e = func_attr_once(select_rescore_kernel<KK, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);       \
+  if (e == cudaSuccess)                                                                                          \
+    e = launch_kernel(select_rescore_kernel<KK, false>, dim3(nq), dim3(kSelectWarps * 32), 0, st,               \
+                      const_cast<const int2*>(p.dense), const_cast<const int*>(cnt), dense_cap, nq, k, dim,       \
+                      const_cast<const float*>(qn), const_cast<const float*>(eps),                              \
+                      static_cast<const __nv_bfloat16*>(nullptr), dim, static_cast<const float*>(nullptr),        \
+                      const_cast<const float*>(qstep), s->master, 1, threshold, row_offset, srows, sscores, sacc,  \
+                      flagged, n_flagged, XPush())
+    switch (reg_k(k)) {
+      case 1: FRG_SELECT_G(1); break;
+      case 4: FRG_SELECT_G(4); break;
+      case 8: FRG_SELECT_G(8); break;
+      default: FRG_SELECT_G(16); break;
+    }
+#undef FRG_SELECT_G
+    if (e != cudaSuccess) rc = cuda_fail(e, "select_rescore_kernel", __FILE__, __LINE__);
+    else note_launch(nullptr);
+  }
+  profile_end(st, 1);
+  // 5. the queries whose candidates overflowed: exact scan of the whole store, each with its own tenant
+  profile_begin(st, kStageFallback);
+  if (rc == FRG_OK) {
+    ScanArgs a;
+    a.master = s->master; a.plane = nullptr; a.tags = s->tags; a.rows = s->rows; a.dim = dim;
+    a.qn = qn; a.nq = nq; a.k = k; a.metric = FRG_METRIC_COSINE; a.tenant = -1; a.sm_count = sm_count;
+    rc = launch_scan_f32_flagged_tenants(a, dten, flagged, n_flagged, row_offset, threshold, srows, sscores, sacc, st);
+  }
+  profile_end(st, 1);
+  if (rc == FRG_OK) rc = launch_scatter_results(srows, sscores, sacc, dperm, nq, k, out_rows, out_scores, out_accept, st);
+  if (rc == FRG_OK) { cudaError_t e = cudaGetLastError(); if (e != cudaSuccess) rc = cuda_fail(e, "grouped match", __FILE__, __LINE__); }
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
 }
 
 }  // namespace frg

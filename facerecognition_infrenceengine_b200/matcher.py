@@ -127,6 +127,60 @@ class Matcher:
                                 C.c_void_p(accept.data_ptr()), C.c_void_p(stream)))
         return rows, scores, accept
 
+    # ---- one call for a batch whose queries belong to different companies
+    def _tenant_codes(self, company_ids, F: int) -> np.ndarray:
+        company_ids = list(company_ids)
+        if len(company_ids) != F:
+            raise ValueError("%d company ids for %d queries" % (len(company_ids), F))
+        return np.array([-1 if c is None else self.store.tenant_code(c, create=False) for c in company_ids], np.int32)
+
+    def match_tenants(self, Q: np.ndarray, company_ids: Sequence[Optional[str]], k: int = 1,
+                      threshold: float = LIVE_THRESHOLD, variant: str = "auto", with_ids: bool = True) -> MatchResult:
+        """``match`` with a company filter PER QUERY: row f of the result equals ``match(Q[f:f+1], k, threshold,
+        company_ids[f])`` bit for bit, in the caller's order (None = all companies; an unknown company matches
+        nothing).  One frg_match_tenants_host call, one read section for the match and the id lookup."""
+        Q = np.asarray(Q)
+        if Q.ndim != 2 or Q.shape[1] != self.store.dim:
+            raise ValueError("Q must be [queries, %d], got shape %s" % (self.store.dim, Q.shape))
+        Q = np.ascontiguousarray(Q, dtype=np.float32)
+        F = len(Q)
+        tenants = self._tenant_codes(company_ids, F)
+        out = MatchResult(np.empty((F, k), np.int64), np.empty((F, k), np.float32), np.zeros(F, np.uint8))
+        p = _params(self.metric, variant, threshold, -1, 0)
+        with _reading(self.store):
+            out.layout_version = getattr(self.store, "layout_version", 0)
+            N.check(N.lib.frg_match_tenants_host(self.store.handle, Q.ctypes.data, F, int(k), C.byref(p),
+                                                 tenants.ctypes.data, out.rows.ctypes.data, out.scores.ctypes.data,
+                                                 out.accept.ctypes.data))
+            out.variant, out.launches = N.last_variant(), N.last_launch_count()
+            out.accept = out.accept.view(np.bool_)
+            if with_ids:
+                out.ids = self.store.ids_of(out.rows)
+        return out
+
+    def match_tenants_device(self, Q, tenants: Sequence[int], k: int = 1, threshold: float = LIVE_THRESHOLD,
+                             variant: str = "auto", out=None, stream: Optional[int] = None):
+        """Device tensors in / out on the caller's stream, like ``match_device``; tenants: one tag code per query as
+        host ints (-1 = all tenants)."""
+        import torch
+        assert Q.is_cuda and Q.dtype == torch.float32 and Q.is_contiguous() and Q.dim() == 2
+        F = Q.shape[0]
+        t = np.ascontiguousarray([int(x) for x in tenants], dtype=np.int32)
+        if len(t) != F:
+            raise ValueError("%d tenants for %d queries" % (len(t), F))
+        if out is None:
+            out = (torch.empty((F, k), dtype=torch.int64, device=Q.device),
+                   torch.empty((F, k), dtype=torch.float32, device=Q.device),
+                   torch.empty((F,), dtype=torch.uint8, device=Q.device))
+        rows, scores, accept = out
+        if stream is None:
+            stream = torch.cuda.current_stream(Q.device).cuda_stream
+        p = _params(self.metric, variant, threshold, -1, 0)
+        N.check(N.lib.frg_match_tenants(self.store.handle, C.c_void_p(Q.data_ptr()), F, int(k), C.byref(p),
+                                        t.ctypes.data, C.c_void_p(rows.data_ptr()), C.c_void_p(scores.data_ptr()),
+                                        C.c_void_p(accept.data_ptr()), C.c_void_p(stream)))
+        return rows, scores, accept
+
     # ---- every row whose score reaches the threshold (exact fp32)
     def range_host(self, Q: np.ndarray, threshold: float, tenant: int = -1, max_hits: int = 64, strict: bool = False,
                    variant: str = "auto", row_offset: int = 0):
@@ -213,6 +267,42 @@ class FaceRecognitionProcessor:
                 else:
                     out.append({"person_id": None, "person_info": {"name": "Unknown", "type": "unknown"},
                                 "recognition_score": 0})
+        return out
+
+    def recognize_frames(self, frames: Sequence) -> List[List[Dict]]:
+        """frames: (embeddings, company_id) per frame, each frame of its own company -> one list per frame, equal to
+        ``recognize(embeddings, company_id)`` frame by frame, from ONE match_tenants call."""
+        frames = list(frames)
+        match_tenants = getattr(self.matcher, "match_tenants", None)
+        if match_tenants is None:
+            raise NotImplementedError("%s has no match_tenants: per-query company filters need a single-GPU Matcher"
+                                      % type(self.matcher).__name__)
+        embs = []
+        for e, _ in frames:
+            e = np.asarray(e, dtype=np.float32)
+            if e.ndim != 2:
+                raise ValueError("embeddings of a frame must be [faces, dim]")
+            embs.append(e)
+        store = self.store
+        if sum(len(e) for e in embs) == 0 or len(store) == 0:
+            return [[] for _ in frames]
+        Q = np.concatenate([e for e in embs if len(e)], axis=0)
+        ids = [c for e, (_, c) in zip(embs, frames) for _ in range(len(e))]
+        out, o = [], 0
+        with _reading(store):
+            r = match_tenants(Q, ids, 1, self.recognition_threshold, with_ids=False)
+            for e in embs:
+                faces = []
+                for f in range(o, o + len(e)):
+                    if r.accept[f]:
+                        pid = store.id_of(r.rows[f, 0])
+                        info = store.metadata(pid) or {"name": pid, "type": "employee"}
+                        faces.append({"person_id": pid, "person_info": info, "recognition_score": r.scores[f, 0]})
+                    else:
+                        faces.append({"person_id": None, "person_info": {"name": "Unknown", "type": "unknown"},
+                                      "recognition_score": 0})
+                out.append(faces)
+                o += len(e)
         return out
 
 

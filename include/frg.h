@@ -158,6 +158,22 @@ FRG_API int frg_match(frg_store* s, const float* q, int32_t nq, int32_t k, const
 FRG_API int frg_match_host(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
                    int64_t* out_rows, float* out_scores, uint8_t* out_accept);
 
+/* ---- one match call in which every query carries its own tenant filter (a server for many companies' cameras).
+ * tenants: HOST array [nq]; tenants[i] < 0 = all tenants, else only rows tagged tenants[i] (a tag no row carries:
+ *   every slot of that query row -1 / reject).  p->tenant is not read; everything else of *p applies to all queries.
+ * Result of query i == frg_match(s, q_i, 1, k, p') with p' = *p, p'.tenant = tenants[i], bit for bit (rows,
+ *   scores, accept), in the caller's query order.
+ * A unit cosine store with an fp32 master and a scan plane (AUTO / TC_EXACT / TC_BF16 with dim 128 / 256 / 512)
+ *   runs every tenant in ONE pass of the int8 tensor-core filter (frg_last_variant() "tc_exact_grouped"; the launch
+ *   count does not grow with the number of tenants).  All queries on one tenant: exactly frg_match.  Every other
+ *   store or variant (SCAN_F32, raw / Euclidean, bf16-only, no plane) runs frg_match's path once per tenant inside
+ *   the same call - correct, but no faster than separate calls. */
+FRG_API int frg_match_tenants(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                              const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept,
+                              void* stream);
+FRG_API int frg_match_tenants_host(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
+                                   const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept);
+
 /* ---- first row, in gallery order, whose score reaches the threshold (exact fp32).  Replaces the two
  *      "first hit" scans next to the matching path:
  *        trainingServer.py:170-200  duplicate face at enrolment: first stored template with cos > 0.4
