@@ -18,6 +18,8 @@ VARIANT_AUTO, VARIANT_SCAN_F32, VARIANT_TC_EXACT, VARIANT_TC_BF16 = 0, 1, 2, 3
 STORE_BF16_PLANE, STORE_RAW, STORE_BF16_ONLY = 1, 2, 4
 ROWS_PRENORMALISED = 1
 FIRST_STRICT, QUERY_PRENORMALISED = 1, 2
+JOIN_SAME_TAG = 4
+JOIN_SLAB_ROWS = 1024
 XCHG_PUSH_ONLY, XCHG_MERGE_ONLY = 1, 2
 MAX_K = 16
 
@@ -80,6 +82,8 @@ SIGNATURES = {
     "frg_first_match_host": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), _P, _P]),
     "frg_match_range": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
     "frg_match_range_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
+    "frg_self_join": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
+    "frg_self_join_host": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
     "frg_merge_topk": (C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                  C.c_float, _P, _P, _P, _P]),
     "frg_merge_topk_strided": (C.c_int, [C.c_int32, _P, C.c_int64, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32,

@@ -1414,6 +1414,246 @@ int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32_t max_h
   return rc;
 }
 
+// --------------------------------------------------------------------------------------------- gallery self-join
+// The store's rows [row0, row0 + n) as queries against the rows after them (the upper triangle), in slabs of
+// FRG_JOIN_SLAB_ROWS query rows that reuse one workspace.  Query tile u of 128 rows [R, R + 128) scans the rows from
+// its own tile R / 128 to an end row: the store's last row; with p->tenant >= 0 that tenant's extent end; with
+// FRG_JOIN_SAME_TAG the largest extent end among the tags whose extent overlaps the tile.  When exactly one tag's extent
+// overlaps the tile, the filter masks with that tag.  A tile no live row of the rule can sit in scans nothing.
+// Tensor-core path (unit store with an int8 plane and a covered dim): per slab query prep straight from the master
+// rows -> floor threshold - eps[q] -> GROUPED filter -> join_select_kernel -> exact join scan of the overflowed
+// queries.  SCAN_F32 (and plane-less stores): per slab query prep -> exact join scan of every query.
+static_assert(FRG_JOIN_SLAB_ROWS % kTcTileRows == 0, "slabs are whole query tiles");
+
+struct JoinTile { int32_t tenant; int32_t end_row; };
+
+static void join_plan_tiles(const frg_store* s, int64_t row0, int64_t n, int32_t tenant, bool same_tag,
+                            std::vector<JoinTile>* out) {
+  const int64_t rows = s->rows;
+  const int64_t nt = (n + kTcTileRows - 1) / kTcTileRows;
+  out->assign(size_t(nt), JoinTile{tenant >= 0 ? tenant : -1, int32_t(rows)});
+  if (!s->extents_known || (tenant < 0 && !same_tag)) return;
+  if (tenant >= 0) {
+    auto it = s->extents.find(tenant);
+    const int64_t lo = it != s->extents.end() ? it->second.lo : 0;
+    const int64_t hi = it != s->extents.end() ? (it->second.hi < rows ? it->second.hi : rows) : 0;
+    for (int64_t u = 0; u < nt; ++u) {
+      const int64_t R = row0 + u * kTcTileRows, Re = R + kTcTileRows < row0 + n ? R + kTcTileRows : row0 + n;
+      (*out)[size_t(u)].end_row = int32_t(hi > lo && Re > lo && R < hi ? hi : R);
+    }
+    return;
+  }
+  // sweep over the query tiles (ascending) with the extents sorted by start and their ends sorted: the extents that
+  // overlap [R, Re) are those starting before Re minus those ending at or before R, and the largest end among the
+  // started ones, when it is past R, belongs to an overlapping extent
+  struct Ext { int64_t lo, hi; int32_t tag; };
+  std::vector<Ext> ext;
+  std::vector<int64_t> ends;
+  for (const auto& kv : s->extents) {
+    const int64_t hi = kv.second.hi < rows ? kv.second.hi : rows;
+    if (hi <= kv.second.lo) continue;
+    ext.push_back(Ext{kv.second.lo, hi, kv.first});
+    ends.push_back(hi);
+  }
+  std::sort(ext.begin(), ext.end(), [](const Ext& x, const Ext& y) { return x.lo < y.lo || (x.lo == y.lo && x.tag < y.tag); });
+  std::sort(ends.begin(), ends.end());
+  size_t i = 0, j = 0;
+  int64_t max_hi = 0;
+  int32_t max_tag = -1;
+  for (int64_t u = 0; u < nt; ++u) {
+    const int64_t R = row0 + u * kTcTileRows, Re = R + kTcTileRows < row0 + n ? R + kTcTileRows : row0 + n;
+    for (; i < ext.size() && ext[i].lo < Re; ++i)
+      if (ext[i].hi > max_hi) { max_hi = ext[i].hi; max_tag = ext[i].tag; }
+    while (j < ends.size() && ends[j] <= R) ++j;
+    const size_t overlap = i - j;
+    JoinTile& t = (*out)[size_t(u)];
+    t.end_row = int32_t(overlap > 0 ? max_hi : R);
+    t.tenant = overlap == 1 ? max_tag : -1;
+  }
+}
+
+static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hits, const frg_match_params_t* p,
+                          int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  reset_launches();
+  if (!s || !p || n < 0 || row0 < 0 || (n > 0 && (!out_counts || !out_rows || !out_scores))) {
+    set_error("self_join: bad argument");
+    return FRG_ERR_INVALID;
+  }
+  if (max_hits < 1) { set_error("self_join: max_hits=%d must be >= 1", max_hits); return FRG_ERR_INVALID; }
+  if (p->metric == FRG_METRIC_EUCLIDEAN) { set_error("self_join: cosine only (Euclidean stores are raw)"); return FRG_ERR_UNSUPPORTED; }
+  if (p->metric != FRG_METRIC_COSINE) { set_error("self_join: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
+  if (p->variant < FRG_VARIANT_AUTO || p->variant > FRG_VARIANT_TC_BF16) { set_error("self_join: unknown variant %d", p->variant); return FRG_ERR_INVALID; }
+  if (p->variant == FRG_VARIANT_TC_BF16) {
+    set_error("self_join: FRG_VARIANT_TC_BF16 has no exact scores to hold against the threshold (use AUTO, TC_EXACT or SCAN_F32)");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  if (p->flags & ~(FRG_FIRST_STRICT | FRG_QUERY_PRENORMALISED | FRG_JOIN_SAME_TAG)) {
+    set_error("self_join: unknown flags 0x%x", p->flags);
+    return FRG_ERR_INVALID;
+  }
+  if (p->flags & FRG_QUERY_PRENORMALISED) { set_error("self_join: the queries are the store's rows (FRG_QUERY_PRENORMALISED does not apply)"); return FRG_ERR_UNSUPPORTED; }
+  if (!s->master) { set_error("self_join: a bf16-only store has no fp32 master for the exact scores"); return FRG_ERR_UNSUPPORTED; }
+  if (s->flags & FRG_STORE_RAW) { set_error("self_join: scores on a raw store are not symmetric (unit cosine stores only)"); return FRG_ERR_UNSUPPORTED; }
+  const char* why = "";
+  if (!range_scan_supported(s->dim, &why)) { set_error("self_join: %s", why); return FRG_ERR_UNSUPPORTED; }
+  const bool tc_ok = s->plane8 != nullptr && tc_supported(s->dim, FRG_METRIC_COSINE, &why);
+  const bool use_tc = p->variant == FRG_VARIANT_TC_EXACT || (p->variant == FRG_VARIANT_AUTO && tc_ok);
+  if (use_tc && !tc_ok) {
+    set_error("self_join: FRG_VARIANT_TC_EXACT needs a unit-row store with a scan plane and dim 128 / 256 / 512");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  DeviceGuard g(s->device);
+  if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
+  DeviceInfo di;
+  FRG_CHECK(device_info(s->device, &di));
+  std::lock_guard<std::mutex> lk(s->mu);
+  if (row0 + n > s->rows) {
+    set_error("self_join: rows [%lld, %lld) beyond the %lld rows in use", (long long)row0, (long long)(row0 + n), (long long)s->rows);
+    return FRG_ERR_INVALID;
+  }
+  if (s->rows > 0x7fffffff) { set_error("self_join: more than 2^31-1 rows in one shard"); return FRG_ERR_UNSUPPORTED; }
+  g_variant = use_tc ? "join_tc" : "join_scan";
+  if (n == 0) return FRG_OK;
+  FRG_CHECK(store_begin_read(s, st));
+  const bool same_tag = (p->flags & FRG_JOIN_SAME_TAG) != 0, strict = (p->flags & FRG_FIRST_STRICT) != 0;
+  const int dim = s->dim;
+  std::vector<JoinTile> plan;
+  join_plan_tiles(s, row0, n, p->tenant, same_tag, &plan);
+  // per slab: the upload [end row of each query tile][filter descriptors] and the filter's candidate entries
+  const int64_t S = n < FRG_JOIN_SLAB_ROWS ? n : FRG_JOIN_SLAB_ROWS;
+  const size_t t_cta = (size_t(S / kTcTileRows + 1) * 4 + 15) & ~size_t(15);
+  std::vector<std::vector<unsigned char>> tables;
+  std::vector<int> ctas;
+  int64_t max_cand = 1;
+  size_t max_table = t_cta;
+  for (int64_t s0 = 0; s0 < n; s0 += S) {
+    const int64_t ns = n - s0 < S ? n - s0 : S;
+    const int64_t u0 = s0 / kTcTileRows, nu = (ns + kTcTileRows - 1) / kTcTileRows;
+    std::vector<TcTenantGroup> tiles;
+    std::vector<unsigned char> cta_bytes;
+    int n_ctas = 0;
+    int64_t cand = 0;
+    if (use_tc) {
+      for (int64_t u = 0; u < nu; ++u) {
+        const JoinTile& t = plan[size_t(u0 + u)];
+        const int64_t R = row0 + (u0 + u) * kTcTileRows;
+        TcTenantGroup G{};
+        G.tenant = t.tenant; G.q0 = int(u * kTcTileRows); G.nq = int(ns - u * kTcTileRows < kTcTileRows ? ns - u * kTcTileRows : kTcTileRows);
+        G.tile0 = int(R / kTcTileRows);
+        G.n_tiles = t.end_row > R + 1 ? int((t.end_row - 1) / kTcTileRows) - G.tile0 + 1 : 0;   // b > a >= R
+        G.list = nullptr;
+        tiles.push_back(G);
+      }
+      tc_join_plan(tiles, di.sm_count, &cta_bytes, &n_ctas, &cand);
+    }
+    std::vector<unsigned char> table(t_cta + cta_bytes.size(), 0);
+    for (int64_t u = 0; u < nu; ++u) memcpy(table.data() + u * 4, &plan[size_t(u0 + u)].end_row, 4);
+    if (!cta_bytes.empty()) memcpy(table.data() + t_cta, cta_bytes.data(), cta_bytes.size());
+    if (cand > max_cand) max_cand = cand;
+    if (table.size() > max_table) max_table = table.size();
+    tables.push_back(std::move(table));
+    ctas.push_back(n_ctas);
+  }
+  // ---- one workspace for every slab
+  ScanArgs a;
+  a.master = s->master; a.tags = s->tags; a.rows = s->rows; a.dim = dim;
+  a.qn = nullptr; a.nq = int(S); a.k = 1; a.metric = FRG_METRIC_COSINE; a.tenant = p->tenant; a.sm_count = di.sm_count;
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
+  const size_t o_qn = take(size_t(S) * dim * 4), o_table = take(max_table), o_scan = take(join_scan_workspace_bytes(a));
+  size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_keys = 0, o_cnt = 0, o_flag = 0, o_floor = 0, o_dense = 0, o_cand = 0;
+  if (use_tc) {
+    o_qi8 = take(size_t(S) * dim); o_eps = take(size_t(S) * 4); o_step = take(size_t(S) * 4);
+    o_keys = take(size_t(S) * 32 * 8); o_cnt = take(size_t(S) * 4); o_flag = take(size_t(S) * 4 + 12);
+    o_floor = take(size_t(S) * 4); o_dense = take(size_t(S) * kRangeBudget * 8); o_cand = take(size_t(max_cand) * 8);
+  }
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), off, st));
+  float* qn = reinterpret_cast<float*>(ws + o_qn);
+  const int32_t* tile_end = reinterpret_cast<const int32_t*>(ws + o_table);
+  a.qn = qn;
+  const GalleryWindow w = window_of(s, -1);
+  const int64_t row_offset = p->row_offset;
+  int rc = FRG_OK;
+  for (size_t i = 0; rc == FRG_OK && i < tables.size(); ++i) {
+    const int64_t s0 = int64_t(i) * S, ns = n - s0 < S ? n - s0 : S, qrow0 = row0 + s0;
+    int64_t* oc = out_counts + s0;
+    int64_t* orow = out_rows + s0 * max_hits;
+    float* osc = out_scores + s0 * max_hits;
+    a.nq = int(ns);
+    rc = stage_upload(ws + o_table, tables[i].data(), tables[i].size(), st);
+    if (rc != FRG_OK) break;
+    if (use_tc) {
+      int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
+      float* eps = reinterpret_cast<float*>(ws + o_eps);
+      float* qstep = reinterpret_cast<float*>(ws + o_step);
+      int* cnt = reinterpret_cast<int*>(ws + o_cnt);
+      int* flagged = reinterpret_cast<int*>(ws + o_flag);
+      int* n_flagged = flagged + S;
+      profile_begin(st, kStagePrep);
+      rc = launch_prepare_queries_i8(s->master + qrow0 * dim, int(ns), dim, qn, qi8, qstep, eps, s->gmax_bits,
+                                     reinterpret_cast<unsigned long long*>(ws + o_keys), cnt, n_flagged, st);
+      profile_end(st, 1);
+      if (rc == FRG_OK)
+        rc = launch_tc_join(&w, qn, qi8, qstep, eps, int(ns), ws + o_table + t_cta, ctas[i], qrow0, p->tenant, same_tag,
+                            p->threshold, strict, max_hits, row_offset, reinterpret_cast<int2*>(ws + o_cand), cnt,
+                            reinterpret_cast<int2*>(ws + o_dense), reinterpret_cast<float*>(ws + o_floor), flagged,
+                            n_flagged, oc, orow, osc, st);
+      if (rc == FRG_OK) {
+        profile_begin(st, kStageFallback);
+        rc = launch_join_scan(a, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, p->threshold, strict,
+                              row_offset, ws + o_scan, oc, orow, osc, st);
+        profile_end(st, 3);
+      }
+    } else {
+      profile_begin(st, kStagePrep);
+      rc = launch_normalise_queries(s->master + qrow0 * dim, int(ns), dim, true, qn, nullptr, nullptr, nullptr, nullptr, st);
+      profile_end(st, 1);
+      if (rc == FRG_OK) {
+        profile_begin(st, kStageDominant);
+        rc = launch_join_scan(a, qrow0, tile_end, same_tag, nullptr, nullptr, max_hits, p->threshold, strict,
+                              row_offset, ws + o_scan, oc, orow, osc, st);
+        profile_end(st, 3);
+      }
+    }
+  }
+  g_variant = use_tc ? "join_tc" : "join_scan";
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
+int frg_self_join(frg_store* s, int64_t row0, int64_t n, int32_t max_hits, const frg_match_params_t* p,
+                  int64_t* out_counts, int64_t* out_rows, float* out_scores, void* stream) {
+  return self_join_impl(s, row0, n, max_hits, p, out_counts, out_rows, out_scores, static_cast<cudaStream_t>(stream));
+}
+
+int frg_self_join_host(frg_store* s, int64_t row0, int64_t n, int32_t max_hits, const frg_match_params_t* p,
+                       int64_t* out_counts, int64_t* out_rows, float* out_scores) {
+  if (!s || !p || n <= 0 || row0 < 0 || !out_counts || !out_rows || !out_scores || max_hits < 1) {
+    // the device entry point names the argument (and takes n = 0)
+    return self_join_impl(s, row0, n, max_hits, p, out_counts, out_rows, out_scores, nullptr);
+  }
+  DeviceGuard g(s->device);
+  cudaStream_t st = cudaStreamPerThread;
+  const size_t slots = size_t(n) * size_t(max_hits), cb = size_t(n) * sizeof(int64_t);
+  const size_t o_r = (cb + 255) & ~size_t(255), o_s = (o_r + slots * sizeof(int64_t) + 255) & ~size_t(255);
+  unsigned char* d = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), o_s + slots * sizeof(float), st));
+  int rc = self_join_impl(s, row0, n, max_hits, p, reinterpret_cast<int64_t*>(d), reinterpret_cast<int64_t*>(d + o_r),
+                          reinterpret_cast<float*>(d + o_s), st);
+  if (rc == FRG_OK) {
+    cudaError_t e = cudaMemcpyAsync(out_counts, d, cb, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_rows, d + o_r, slots * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_scores, d + o_s, slots * sizeof(float), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) rc = cuda_fail(e, "D2H results", __FILE__, __LINE__);
+    else rc = store_fault(s);
+  }
+  cudaFreeAsync(d, st);
+  return rc;
+}
+
 int frg_merge_topk(int32_t device, const float* scores, const int64_t* rows, int32_t parts,
                    int32_t nq, int32_t k, int32_t metric, float threshold,
                    int64_t* out_rows, float* out_scores, uint8_t* out_accept, void* stream) {

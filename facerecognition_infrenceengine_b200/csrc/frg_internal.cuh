@@ -399,6 +399,35 @@ int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagge
                       bool strict, int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
                       cudaStream_t st);
 
+// Candidate entries per query of a range-mode filter (range search and self-join; DESIGN.md section 7.3)
+constexpr int kRangeBudget = 4096;
+
+// ---- gallery self-join (frg_self_join): the queries are the store's own rows qrow0 .. qrow0 + nq - 1 of one slab,
+// and a pair (a, b) counts only for b > a (plus the tag rule: tenant >= 0 -> both rows carry it; same_tag -> tag[b] ==
+// tag[a]).  Query tile u of the slab holds queries 128u .. 128u + 127.
+// tc_match.cu, host: descriptor table of the slab's GROUPED filter grid (tiles[u]: tenant the filter masks with, -1 =
+// none, and the absolute gallery tiles tile0 .. tile0 + n_tiles - 1 of query tile u; q0 / nq: its queries), the
+// number of CTAs and the candidate segment entries (int2) the grid writes.  The planner of launch_tc_match_grouped.
+void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::vector<unsigned char>* table,
+                  int* n_ctas, int64_t* cand_entries);
+// tc_match.cu: the int8 filter path of one slab: floor threshold - eps[q] (range_floor_kernel), the GROUPED filter
+// over the uploaded table (d_table, n_ctas; none when 0) with kRangeBudget dense entries per query, and
+// join_select_kernel (exact rescoring, b > a, tag rule, counts and the first max_hits hits in gallery order).  Queries
+// whose candidates overflowed are left in (flagged, n_flagged) for launch_join_scan.  s: the whole store.
+int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
+                   int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
+                   float threshold, bool strict, int max_hits, int64_t row_offset, int2* cand, int* cand_total,
+                   int2* dense, float* floor_v, int* flagged, int* n_flagged, int64_t* out_counts, int64_t* out_rows,
+                   float* out_scores, cudaStream_t st);
+// scan_f32.cu: exact, counting join scan (launch_range_scan's passes with the join rules).  a: the whole store, a.qn /
+// a.nq the slab's unit queries, a.tenant the tenant rule, cosine.  tile_end[u]: exclusive end row of query tile u's
+// plan (device).  A pass of queries reads only the rows from its lowest live query row + 1 to its largest end.
+// flagged == nullptr: every query of the slab; else only the n_flagged[0] listed ones.  ws: join_scan_workspace_bytes.
+size_t join_scan_workspace_bytes(const ScanArgs& a);
+int launch_join_scan(const ScanArgs& a, int64_t qrow0, const int32_t* tile_end, bool same_tag, const int* flagged,
+                     const int* n_flagged, int max_hits, float threshold, bool strict, int64_t row_offset, void* ws,
+                     int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st);
+
 // first_match.cu
 int launch_first_match(const float* master, const int32_t* tags, int64_t rows, int dim, const float* qn, int nq,
                        int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned long long* scratch,

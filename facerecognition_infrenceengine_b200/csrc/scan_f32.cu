@@ -825,4 +825,145 @@ int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagge
   return rc;
 }
 
+// ------------------------------------------------------------------------------------------ gallery self-join
+// range_scan_kernel with the join rules (cosine): query q of the slab is the stored row a = qrow0 + q, and row b counts
+// for it only when b > a and (same_tag) tag[b] == tag[a]; a dead query, or one outside the tenant, counts nothing.  A
+// pass of QB queries reads only the rows [lowest live a + 1, largest plan end of its queries), split into contiguous
+// strips in warp order as range_scan_kernel splits the whole gallery, so pass 2 finds the same strips and the
+// concatenation of the warps' hits is gallery order.  The scores come from row_dots + butterfly: bit-identical.
+template <int NJ, int QB, bool WRITE>
+__global__ void __launch_bounds__(kScanWarps * 32, 2)
+join_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ tags, const float* __restrict__ qn,
+                 int nq, int64_t qrow0, const int32_t* __restrict__ tile_end, const int* __restrict__ flagged,
+                 const int* __restrict__ n_flagged, int32_t tenant, int same_tag, float threshold, int strict,
+                 int max_hits, int64_t row_offset, int* __restrict__ cnt, const int* __restrict__ off,
+                 int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
+  constexpr int DIM = NJ * 128;
+  pdl_wait();
+  pdl_trigger();
+  const int n_slots = flagged ? *n_flagged : nq;
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = int64_t(gridDim.x) * kScanWarps;
+  const int64_t gw = int64_t(blockIdx.x) * kScanWarps + (threadIdx.x >> 5);
+  const int my_b = lane_query<QB>(lane);
+  const bool rep = lane_is_rep<QB>(lane);
+  for (int s0 = 0; s0 < n_slots; s0 += QB) {
+    const int nb = n_slots - s0 < QB ? n_slots - s0 : QB;
+    const int slot = s0 + (my_b < nb ? my_b : 0);
+    const int q = flagged ? flagged[slot] : slot;
+    const int a = int(qrow0 + q);                                     // rows < 2^31 (frg_self_join)
+    const int32_t ta = __ldg(tags + a);
+    const bool live = my_b < nb && ta >= 0 && (tenant < 0 || ta == tenant);
+    // rows of this pass: [lowest live a + 1, largest plan end); none when no query of the pass is live
+    const int lo = __reduce_min_sync(0xffffffffu, live ? a + 1 : 0x7fffffff);
+    const int hi = __reduce_max_sync(0xffffffffu, live ? __ldg(tile_end + q / 128) : 0);
+    const int64_t span = hi > lo ? int64_t(hi - lo) : 0;
+    const int64_t r0 = lo + span * gw / nw, r1 = lo + span * (gw + 1) / nw;
+    int pos = 0, room = 0;
+    if (WRITE) {
+      if (my_b < nb && cnt[size_t(slot) * nw + gw] > 0) {
+        pos = off[size_t(slot) * nw + gw];
+        room = max_hits;
+      }
+      if (!__any_sync(0xffffffffu, pos < room)) continue;
+    }
+    float4 qv[QB][NJ];
+#pragma unroll
+    for (int b = 0; b < QB; ++b) {
+      const int qb_ = flagged ? flagged[s0 + (b < nb ? b : 0)] : s0 + (b < nb ? b : 0);
+#pragma unroll
+      for (int j = 0; j < NJ; ++j) qv[b][j] = __ldg(reinterpret_cast<const float4*>(qn + size_t(qb_) * DIM) + j * 32 + lane);
+    }
+    int count = 0;
+    for (int64_t r = r0; r < r1; ++r) {
+      const int32_t tg = __ldg(tags + r);
+      float4 g[NJ];                                                     // issued together with the tag load
+      const float4* pr = reinterpret_cast<const float4*>(master + r * DIM) + lane;
+#pragma unroll
+      for (int j = 0; j < NJ; ++j) g[j] = ldg_stream(pr + j * 32);
+      if (tg < 0 || (tenant >= 0 && tg != tenant)) continue;           // warp-uniform
+      const bool mine = live && r > a && (!same_tag || tg == ta);
+      if (!__any_sync(0xffffffffu, mine)) continue;
+      float acc[QB];
+      row_dots<NJ, QB, FRG_METRIC_COSINE>(g, qv, acc);
+      const float sdot = butterfly<QB>(acc, lane);
+      const bool hit = mine && range_pass<FRG_METRIC_COSINE>(sdot, threshold, strict);
+      if (WRITE) {
+        if (hit && pos < room) {
+          if (rep) {
+            out_rows[size_t(q) * max_hits + pos] = r + row_offset;
+            out_scores[size_t(q) * max_hits + pos] = sdot;
+          }
+          ++pos;
+        }
+        if (!__any_sync(0xffffffffu, pos < room)) break;
+      } else {
+        count += hit ? 1 : 0;
+      }
+    }
+    if (!WRITE && rep && my_b < nb) cnt[size_t(slot) * nw + gw] = count;
+  }
+}
+
+size_t join_scan_workspace_bytes(const ScanArgs& a) {
+  return size_t(scan_grid(a)) * kScanWarps * size_t(a.nq > 0 ? a.nq : 1) * 2 * sizeof(int);
+}
+
+template <int NJ, int QB>
+static int launch_join_passes(const ScanArgs& a, int grid, int64_t qrow0, const int32_t* tile_end, bool same_tag,
+                              const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
+                              int64_t row_offset, int* cnt, int* off, int64_t* out_counts, int64_t* out_rows,
+                              float* out_scores, cudaStream_t st) {
+  const int nw = grid * kScanWarps;
+  const int s = strict ? 1 : 0, t = same_tag ? 1 : 0;
+  FRG_CUDA(launch_kernel(join_scan_kernel<NJ, QB, false>, dim3(grid), dim3(kScanWarps * 32), 0, st, a.master, a.tags,
+                         a.qn, a.nq, qrow0, tile_end, flagged, n_flagged, a.tenant, t, threshold, s, max_hits,
+                         row_offset, cnt, const_cast<const int*>(off), out_rows, out_scores));
+  note_launch(nullptr);
+  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(a.nq), dim3(256), 0, st, a.nq, flagged, n_flagged, nw,
+                         const_cast<const int*>(cnt), off, max_hits, kNoScore, out_counts, out_rows, out_scores));
+  note_launch(nullptr);
+  FRG_CUDA(launch_kernel(join_scan_kernel<NJ, QB, true>, dim3(grid), dim3(kScanWarps * 32), 0, st, a.master, a.tags,
+                         a.qn, a.nq, qrow0, tile_end, flagged, n_flagged, a.tenant, t, threshold, s, max_hits,
+                         row_offset, cnt, const_cast<const int*>(off), out_rows, out_scores));
+  note_launch(nullptr);
+  FRG_CUDA(cudaGetLastError());
+  return FRG_OK;
+}
+
+template <int NJ>
+static int launch_join_qb(const ScanArgs& a, int qb, int grid, int64_t qrow0, const int32_t* tile_end, bool same_tag,
+                          const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
+                          int64_t row_offset, int* cnt, int* off, int64_t* out_counts, int64_t* out_rows,
+                          float* out_scores, cudaStream_t st) {
+#define FRG_JOIN_QB(QB) return launch_join_passes<NJ, QB>(a, grid, qrow0, tile_end, same_tag, flagged, n_flagged,     \
+                                                         max_hits, threshold, strict, row_offset, cnt, off, out_counts, \
+                                                         out_rows, out_scores, st)
+  if (qb == 1) { FRG_JOIN_QB(1); }
+  if (qb == 2) { FRG_JOIN_QB(2); }
+  if constexpr (NJ <= 4) { if (qb == 4) { FRG_JOIN_QB(4); } }
+  if constexpr (NJ <= 2) { if (qb == 8) { FRG_JOIN_QB(8); } }
+#undef FRG_JOIN_QB
+  set_error("join scan: unsupported queries-per-pass %d for dim %d", qb, NJ * 128);
+  return FRG_ERR_UNSUPPORTED;
+}
+
+int launch_join_scan(const ScanArgs& a, int64_t qrow0, const int32_t* tile_end, bool same_tag, const int* flagged,
+                     const int* n_flagged, int max_hits, float threshold, bool strict, int64_t row_offset, void* ws,
+                     int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  const char* why = "";
+  if (!range_scan_supported(a.dim, &why)) { set_error("join scan: %s", why); return FRG_ERR_UNSUPPORTED; }
+  if (a.nq <= 0) return FRG_OK;
+  const int grid = scan_grid(a);
+  int* cnt = static_cast<int*>(ws);
+  int* off = cnt + size_t(grid) * kScanWarps * a.nq;
+  const int qb = scan_qb(a.dim, a.nq);
+  switch (a.dim) {
+    case 128: return launch_join_qb<1>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
+    case 256: return launch_join_qb<2>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
+    case 512: return launch_join_qb<4>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
+    default:  return launch_join_qb<8>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
+  }
+}
+
 }  // namespace frg

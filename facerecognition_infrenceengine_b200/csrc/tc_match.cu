@@ -1237,7 +1237,6 @@ static int reg_k(int k) { return k == 1 ? 1 : (k <= 4 ? 4 : (k <= 8 ? 8 : 16)); 
 // Range search (range = true): no pre-pass, and a fixed dense list of kRangeBudget entries per query instead of one
 // sized from k (DESIGN.md section 7.3).
 // i8: the int8 filter - pre-pass at most every 16th tile, floor from i8_floor_kernel, never fused.
-constexpr int kRangeBudget = 4096;
 static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range = false, bool i8 = false) {
   const bool euclid_plane = dim < 0;
   pl->qtiles = (nq + kTileQ - 1) / kTileQ;
@@ -1704,6 +1703,40 @@ static std::vector<int> proportional_chunks(const std::vector<int>& tiles, int s
   return c;
 }
 
+// One query tile of a GROUPED grid: queries q0 .. q0 + nq - 1 (nq <= kTileQ) of src's tenant, which scan src's tiles
+// with `entries` candidates per query and (pre-pass) every stride-th tile.
+struct GroupUnit { const TcTenantGroup* src; int q0, nq, entries, stride; };
+
+// The descriptors of a GROUPED filter grid (main) and, when pre != nullptr, of its pre-pass grid: each unit's tiles cut
+// into chunks in proportion to its share of all tiles, its candidate segments one per (query, chunk, column half) with
+// x2 headroom (as tc_plan).  Returns the candidate entries (int2) the filter grid writes.
+static int64_t plan_group_ctas(const std::vector<GroupUnit>& units, int sm_count, std::vector<TcGroupCta>* pre,
+                               std::vector<TcGroupCta>* main) {
+  std::vector<int> tiles_main(units.size()), tiles_pre(units.size());
+  for (size_t u = 0; u < units.size(); ++u) {
+    tiles_main[u] = units[u].src->n_tiles;
+    tiles_pre[u] = (tiles_main[u] + units[u].stride - 1) / units[u].stride;
+  }
+  const std::vector<int> ch_main = proportional_chunks(tiles_main, sm_count);
+  const std::vector<int> ch_pre = proportional_chunks(tiles_pre, sm_count);
+  int64_t cand_entries = 0;
+  for (size_t u = 0; u < units.size(); ++u) {
+    const TcTenantGroup& G = *units[u].src;
+    if (tiles_main[u] == 0) continue;                  // an unknown tag: no rows, nothing to scan
+    const int nseg = ch_main[u] * (kEpiWarps / 4);
+    int seg = (2 * units[u].entries + nseg - 1) / nseg;
+    if (seg < 12) seg = 12;
+    TcGroupCta d{};
+    d.q0 = units[u].q0; d.nq = units[u].nq; d.tenant = G.tenant; d.tile0 = G.tile0; d.n_tiles = G.n_tiles;
+    d.list = G.list; d.seg = seg; d.cand0 = cand_entries;
+    for (int c = 0; c < ch_main[u]; ++c) { d.chunk = c; d.chunks = ch_main[u]; d.scale = 1; main->push_back(d); }
+    if (pre)
+      for (int c = 0; c < ch_pre[u]; ++c) { d.chunk = c; d.chunks = ch_pre[u]; d.scale = units[u].stride; pre->push_back(d); }
+    cand_entries += int64_t(kTileQ) * nseg * seg;
+  }
+  return cand_entries;
+}
+
 int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::vector<int32_t>& perm,
                             const std::vector<TcTenantGroup>& groups, int k, float threshold, int64_t row_offset,
                             int sm_count, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st) {
@@ -1714,42 +1747,21 @@ int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::v
     return FRG_ERR_UNSUPPORTED;
   }
   // ---- plan: query tiles of at most kTileQ queries, never across tenants
-  struct Unit { int q0, nq, g; };
-  std::vector<Unit> units;
+  std::vector<GroupUnit> units;
   for (int g = 0; g < int(groups.size()); ++g)
     for (int a = 0; a < groups[g].nq; a += kTileQ)
-      units.push_back(Unit{groups[g].q0 + a, groups[g].nq - a < kTileQ ? groups[g].nq - a : kTileQ, g});
-  std::vector<int> tiles_main(units.size()), tiles_pre(units.size()), stride(units.size()), entries(units.size());
+      units.push_back(GroupUnit{&groups[g], groups[g].q0 + a, groups[g].nq - a < kTileQ ? groups[g].nq - a : kTileQ, 0, 0});
   int dense_cap = 0;
-  for (size_t u = 0; u < units.size(); ++u) {
-    const int n = groups[units[u].g].n_tiles;
+  for (GroupUnit& U : units) {
     // the plan of a single-tenant match over the same tiles (tc_plan): pre-pass stride and candidate budget
     TcPlan pl;
-    tc_plan(int64_t(n) * kTileR, dim, 1, k, sm_count, &pl, false, true);
-    stride[u] = pl.stride;
-    entries[u] = pl.stage_entries;
-    tiles_main[u] = n;
-    tiles_pre[u] = (n + pl.stride - 1) / pl.stride;
+    tc_plan(int64_t(U.src->n_tiles) * kTileR, dim, 1, k, sm_count, &pl, false, true);
+    U.stride = pl.stride;
+    U.entries = pl.stage_entries;
     if (pl.stage_entries > dense_cap) dense_cap = pl.stage_entries;
   }
-  const std::vector<int> ch_main = proportional_chunks(tiles_main, sm_count);
-  const std::vector<int> ch_pre = proportional_chunks(tiles_pre, sm_count);
   std::vector<TcGroupCta> pre, main;
-  int64_t cand_entries = 0;
-  for (size_t u = 0; u < units.size(); ++u) {
-    const TcTenantGroup& G = groups[units[u].g];
-    if (tiles_main[u] == 0) continue;                  // an unknown tag: no rows, nothing to scan
-    // private segments of this tile's queries: one per (query, chunk, column half), x2 headroom (as tc_plan)
-    const int nseg = ch_main[u] * (kEpiWarps / 4);
-    int seg = (2 * entries[u] + nseg - 1) / nseg;
-    if (seg < 12) seg = 12;
-    TcGroupCta d{};
-    d.q0 = units[u].q0; d.nq = units[u].nq; d.tenant = G.tenant; d.tile0 = G.tile0; d.n_tiles = G.n_tiles;
-    d.list = G.list; d.seg = seg; d.cand0 = cand_entries;
-    for (int c = 0; c < ch_main[u]; ++c) { d.chunk = c; d.chunks = ch_main[u]; d.scale = 1; main.push_back(d); }
-    for (int c = 0; c < ch_pre[u]; ++c) { d.chunk = c; d.chunks = ch_pre[u]; d.scale = stride[u]; pre.push_back(d); }
-    cand_entries += int64_t(kTileQ) * nseg * seg;
-  }
+  const int64_t cand_entries = plan_group_ctas(units, sm_count, &pre, &main);
   if (dense_cap < 256) dense_cap = 256;
   // ---- workspace (one stream-ordered allocation)
   size_t off = 0;
@@ -1862,6 +1874,130 @@ int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::v
   cudaError_t e = cudaFreeAsync(ws, st);
   if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
   return rc;
+}
+
+// ------------------------------------------------------------------------------------------ gallery self-join
+// range_select_kernel for a slab of the self-join: query q is the stored row a = qrow0 + q.  A dead query, or one
+// outside the tenant, has no pairs.  A candidate counts when b > a and, with same_tag, tag[b] == tag[a] (the filter
+// has masked dead rows, and other tenants' rows when its descriptor carried a tenant); it is rescored with the same
+// arithmetic as range_select_kernel, so the scores are bit-identical to a range search with row a as the query.
+__global__ void __launch_bounds__(kSelectWarps * 32)
+join_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand_total, int dense_cap, int dim,
+                   const float* __restrict__ qn, const float* __restrict__ master, const int32_t* __restrict__ tags,
+                   int64_t qrow0, int32_t tenant, int same_tag, float threshold, int strict, int max_hits,
+                   int64_t row_offset, int64_t* __restrict__ out_counts, int64_t* __restrict__ out_rows,
+                   float* __restrict__ out_scores, int* __restrict__ flagged, int* __restrict__ n_flagged) {
+  extern __shared__ unsigned long long hits[];        // [pow2 >= dense_cap]
+  __shared__ int s_m;
+  const int lane = threadIdx.x & 31;
+  const int w = threadIdx.x >> 5;
+  const int q = blockIdx.x;
+  const int64_t a = qrow0 + q;
+  pdl_wait();             // the filter kernel's candidate lists
+  pdl_trigger();
+  const int32_t ta = __ldg(tags + a);
+  const bool live = ta >= 0 && (tenant < 0 || ta == tenant);
+  const int total = live ? cand_total[q] : 0;
+  if (total > dense_cap) {                           // also set by a poisoned total (segment overflow)
+    if (threadIdx.x == 0) flagged[atomicAdd(n_flagged, 1)] = q;
+    return;
+  }
+  if (threadIdx.x == 0) s_m = 0;
+  __syncthreads();
+  const int2* mine = dense + size_t(q) * dense_cap;
+  const int nvec = dim >> 2;
+  const float4* qq = reinterpret_cast<const float4*>(qn + size_t(q) * dim);
+  for (int c = w; c < total; c += kSelectWarps) {
+    const int row = mine[c].x;
+    if (row <= a || (same_tag && __ldg(tags + row) != ta)) continue;     // warp-uniform
+    const float4* g = reinterpret_cast<const float4*>(master + size_t(row) * dim);
+    float acc = 0.f;
+#pragma unroll 4
+    for (int v = lane; v < nvec; v += 32) {
+      const float4 x = __ldg(g + v), y = __ldg(qq + v);
+      acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc); acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    const bool pass = strict ? (acc > threshold) : (acc >= threshold);      // false for NaN
+    if (lane == 0 && pass) hits[atomicAdd(&s_m, 1)] = (uint64_t(uint32_t(row)) << 32) | __float_as_uint(acc);
+  }
+  __syncthreads();
+  const int m = s_m;
+  int n2 = 1;
+  while (n2 < m) n2 <<= 1;
+  for (int i = m + threadIdx.x; i < n2; i += blockDim.x) hits[i] = ~0ull;
+  __syncthreads();
+  // rows are distinct: ascending keys = gallery order
+  for (int kk = 2; kk <= n2; kk <<= 1) {
+    for (int j = kk >> 1; j > 0; j >>= 1) {
+      for (int i = threadIdx.x; i < n2; i += blockDim.x) {
+        const int ij = i ^ j;
+        if (ij > i) {
+          const unsigned long long x = hits[i], y = hits[ij];
+          if ((x > y) == ((i & kk) == 0)) { hits[i] = y; hits[ij] = x; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  for (int i = threadIdx.x; i < max_hits; i += blockDim.x) {
+    const bool filled = i < m;
+    out_rows[size_t(q) * max_hits + i] = filled ? int64_t(hits[i] >> 32) + row_offset : int64_t(kNoRow);
+    out_scores[size_t(q) * max_hits + i] = filled ? __uint_as_float(uint32_t(hits[i])) : kNoScore;
+  }
+  if (threadIdx.x == 0) out_counts[q] = m;
+}
+
+void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::vector<unsigned char>* table,
+                  int* n_ctas, int64_t* cand_entries) {
+  std::vector<GroupUnit> units;
+  for (const TcTenantGroup& t : tiles) units.push_back(GroupUnit{&t, t.q0, t.nq, kRangeBudget, 1});
+  std::vector<TcGroupCta> main;
+  *cand_entries = plan_group_ctas(units, sm_count, nullptr, &main);
+  *n_ctas = int(main.size());
+  table->resize(main.size() * sizeof(TcGroupCta));
+  if (!main.empty()) memcpy(table->data(), main.data(), table->size());
+}
+
+int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
+                   int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
+                   float threshold, bool strict, int max_hits, int64_t row_offset, int2* cand, int* cand_total,
+                   int2* dense, float* floor_v, int* flagged, int* n_flagged, int64_t* out_counts, int64_t* out_rows,
+                   float* out_scores, cudaStream_t st) {
+  if (!s->plane8 || !s->master || s->row0 != 0 || s->rows > 0x7fffffff) {
+    set_error("tc_join: needs the whole unit store with an int8 plane and an fp32 master");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  CUtensorMap qm, gm;
+  FRG_CHECK(make_map(&qm, qi8, s->dim, nq, size_t(s->dim), kTileQ, kBlockK, true));
+  FRG_CHECK(make_map(&gm, s->plane8, s->dim, s->rows, size_t(s->dim), kTileR, kBlockK, true));
+  TcScanParams p{};
+  p.fault = s->fault; p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
+  p.dim = s->dim; p.nq = nq; p.tenant = -1; p.tags = s->tags; p.n_rows = int(s->rows); p.k = 1; p.tile_scale = 1;
+  p.floor = floor_v; p.qstep = qstep;
+  p.cand = cand; p.cand_total = cand_total; p.dense = dense; p.dense_cap = kRangeBudget;
+  p.groups = static_cast<const TcGroupCta*>(d_table);
+  profile_begin(st, kStageFloor);
+  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, eps, threshold, floor_v, nq));
+  note_launch(nullptr);
+  profile_end(st, 1);
+  profile_begin(st, kStageDominant);
+  if (n_ctas > 0) FRG_CHECK((launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, n_ctas, 1, st)));
+  profile_end(st, n_ctas > 0 ? 1 : 0);
+  profile_begin(st, kStageSelect);
+  int n2 = 1;
+  while (n2 < kRangeBudget) n2 <<= 1;
+  const size_t smem = size_t(n2) * sizeof(unsigned long long);
+  FRG_CUDA(func_attr_once(join_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  FRG_CUDA(launch_kernel(join_select_kernel, dim3(nq), dim3(kSelectWarps * 32), smem, st,
+                         const_cast<const int2*>(dense), const_cast<const int*>(cand_total), kRangeBudget, s->dim, qn,
+                         s->master, s->tags, qrow0, tenant, same_tag ? 1 : 0, threshold, strict ? 1 : 0, max_hits,
+                         row_offset, out_counts, out_rows, out_scores, flagged, n_flagged));
+  note_launch(nullptr);
+  FRG_CUDA(cudaGetLastError());
+  profile_end(st, 1);
+  return FRG_OK;
 }
 
 }  // namespace frg

@@ -23,6 +23,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
+from . import _native as N
 from .gallery import GalleryStore
 from .matcher import Matcher, _reading
 
@@ -125,29 +126,99 @@ class EnrolmentChecker:
         tenant = None if company_id is None and kind is None else enrolment_tenant(company_id, kind)
         return find_duplicate_pairs(self.store, self.duplicate_threshold, tenant, batch, self.matcher)
 
+    def audit_all_duplicates(self) -> Dict[str, List[Tuple[str, str, float]]]:
+        """Every company's duplicate audit in ONE pass over the gallery: {tenant key: pairs} for every tenant key the
+        gallery knows (an :class:`EnrolmentGallery`: ``enrolment_tenant(company, kind)``), each value equal to
+        ``audit_duplicates`` of that company and kind.  Pairs across companies are not duplicates under the
+        reference's rule (trainingServer.py:170-200 scans one company's collection) and are not reported."""
+        base = self.store.store if isinstance(self.store, EnrolmentGallery) else self.store
+        matcher = _self_join_matcher(base, self.matcher)
+        if matcher is None:
+            raise ValueError("audit_all_duplicates needs a unit GalleryStore / EnrolmentGallery on this process's "
+                             "matcher (raw stores and sharded galleries: audit_duplicates per company)")
+        keys = base.tenant_keys()
+        out: Dict[str, List[Tuple[str, str, float]]] = {key: [] for key in keys.values()}
+        with _reading(base):
+            tags = base.read_tags()
+            for a, ia, ib, sc in _self_join_pairs(base, matcher, self.duplicate_threshold, None, True):
+                key = keys.get(int(tags[a]))
+                if key is not None:
+                    out[key].append((ia, ib, sc))
+        return out
+
     @staticmethod
     def template_from_poses(pose_embeddings: Sequence[np.ndarray]) -> np.ndarray:
         """trainingServer.py:355."""
         return np.mean(pose_embeddings, axis=0)
 
 
-def find_duplicate_pairs(store, threshold: float = DUPLICATE_THRESHOLD, company_id: Optional[str] = None,
-                         batch: int = 1024, matcher=None) -> List[Tuple[str, str, float]]:
-    """Whole-gallery duplicate audit: every pair of live rows a < b (gallery order) with cos > threshold - the rule
-    of the enrol-time check (trainingServer.py:170-200), applied to what is already enrolled.  company_id: only
-    that tenant's rows (an :class:`EnrolmentGallery` takes the key of ``enrolment_tenant``).  Each pair is
-    reported once, from the lower row's query, as (id_a, id_b, score); pairs whose ids are equal are skipped (an
-    enrolment gallery holds several templates per person: the id is the template's `ref_id` when it has one).
-    Mechanism: the stored rows are read back in batches and sent as queries through ``Matcher.match_range``, so
-    the whole audit is one N x N contraction - on the tensor cores when the store keeps a scan plane."""
-    base = store.store if isinstance(store, EnrolmentGallery) else store
-    matcher = matcher if matcher is not None else Matcher(base)
-    code = None if company_id is None else base.tenant_code(company_id, create=False)
-
+def _identity(base):
     def ident(row: int) -> Optional[str]:
         pid = base.id_of(row)
         ref = (base.metadata(pid) or {}).get("ref_id") if pid is not None else None
         return ref if ref is not None else pid
+    return ident
+
+
+def _self_join_matcher(base, matcher) -> Optional[Matcher]:
+    """The matcher of the device self-join, or None when the store is not one it serves: a raw store, a bf16-only
+    store, or a foreign matcher (a ShardedMatcher over a ShardedGallery) whose pairs need the other ranks' rows."""
+    if not isinstance(base, GalleryStore) or base.bf16_only or (base.stats().flags & N.STORE_RAW):
+        return None
+    if matcher is None:
+        return Matcher(base)
+    if type(matcher) is Matcher and matcher.store is base and matcher.metric == "cosine":
+        return matcher
+    return None
+
+
+def _self_join_pairs(base, matcher: Matcher, threshold: float, company_id: Optional[str], same_company: bool):
+    """(row a, id a, id b, score) of every pair of the device self-join, strict, in the audit's order; pairs whose ids
+    are equal (several templates of one person) are skipped.  The caller holds the store's read section."""
+    ident = _identity(base)
+    A, B, S = matcher.self_join(threshold, company_id=company_id, same_company=same_company, strict=True, max_hits=16)
+    out = []
+    for a, b, sc in zip(A.tolist(), B.tolist(), S.tolist()):
+        ia, ib = ident(a), ident(b)
+        if ia != ib:
+            out.append((a, ia, ib, sc))
+    return out
+
+
+def find_duplicate_pairs(store, threshold: float = DUPLICATE_THRESHOLD, company_id: Optional[str] = None,
+                         batch: int = 1024, matcher=None, within_companies: bool = False) -> List[Tuple[str, str, float]]:
+    """Whole-gallery duplicate audit: every pair of live rows a < b (gallery order) with cos > threshold - the rule
+    of the enrol-time check (trainingServer.py:170-200), applied to what is already enrolled.  company_id: only
+    that tenant's rows (an :class:`EnrolmentGallery` takes the key of ``enrolment_tenant``).  within_companies: every
+    company at once, each within itself (only pairs whose two rows carry the same tenant tag).  Each pair is reported
+    once, from the lower row's query, as (id_a, id_b, score), ordered by row a, then score desc, then row b; pairs
+    whose ids are equal are skipped (an enrolment gallery holds several templates per person: the id is the
+    template's `ref_id` when it has one).
+    Mechanism: a unit ``GalleryStore`` (or :class:`EnrolmentGallery`) without a foreign `matcher` runs the device
+    self-join (``Matcher.self_join``: the upper triangle only, no row leaves the device).  Raw stores and sharded
+    galleries with a ``ShardedMatcher`` read the rows back in batches of `batch` and send them as queries through
+    ``match_range``; the scores are the same on both paths, bit for bit."""
+    base = store.store if isinstance(store, EnrolmentGallery) else store
+    join = _self_join_matcher(base, matcher)
+    if join is not None:
+        with _reading(base):
+            return [(ia, ib, sc) for _, ia, ib, sc in _self_join_pairs(base, join, threshold, company_id,
+                                                                         within_companies)]
+    if within_companies:
+        raise ValueError("within_companies runs on the device self-join only (a unit GalleryStore / "
+                         "EnrolmentGallery without a foreign matcher)")
+    return _find_duplicate_pairs_readback(store, threshold, company_id, batch, matcher)
+
+
+def _find_duplicate_pairs_readback(store, threshold: float = DUPLICATE_THRESHOLD, company_id: Optional[str] = None,
+                                   batch: int = 1024, matcher=None) -> List[Tuple[str, str, float]]:
+    """The audit by readback: the stored rows are read back in batches and sent as queries through
+    ``Matcher.match_range``, the pairs with rows <= a dropped on the host (every pair is computed twice).  The path
+    of the stores the self-join does not serve, and the yardstick it is tested against."""
+    base = store.store if isinstance(store, EnrolmentGallery) else store
+    matcher = matcher if matcher is not None else Matcher(base)
+    code = None if company_id is None else base.tenant_code(company_id, create=False)
+    ident = _identity(base)
 
     pairs: List[Tuple[str, str, float]] = []
     with _reading(base):

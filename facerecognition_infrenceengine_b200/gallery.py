@@ -142,6 +142,11 @@ class GalleryStore:
                 self._tenants[key] = len(self._tenants) + 1
             return self._tenants[key]
 
+    def tenant_keys(self) -> Dict[int, str]:
+        """tag code -> company key, for every company this store has given a code."""
+        with self._lock:
+            return {code: key for key, code in self._tenants.items()}
+
     # ------------------------------------------------------------------ raw row API
     def stats(self) -> N.StoreStats:
         st = N.StoreStats()
@@ -183,6 +188,14 @@ class GalleryStore:
             tags = np.empty(n, np.int32)
             N.check(N.lib.frg_store_read_host(self.handle, int(row0), int(n), _ptr(vecs), _ptr(tags)))
             return vecs, tags
+
+    def read_tags(self, row0: int = 0, n: Optional[int] = None) -> np.ndarray:
+        """Tags of rows [row0, row0 + n) (company code, -1 = removed), without their vectors."""
+        with self._lock:
+            n = self._rows - row0 if n is None else n
+            tags = np.empty(n, np.int32)
+            N.check(N.lib.frg_store_read_host(self.handle, int(row0), int(n), None, _ptr(tags)))
+            return tags
 
     def fill_synthetic(self, n: int, global_row0: int = 0, seed: int = 1234, tag: int = 0, stream=None):
         """Append n rows of the frg-synth-v1 gallery (bench / scale tests; oracle.synth is the CPU twin).

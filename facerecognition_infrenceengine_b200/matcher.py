@@ -219,6 +219,57 @@ class Matcher:
                 out.ids = [self.store.ids_of(r[None, :])[0] if len(r) else [] for r in lists_r]
         return out
 
+    # ---- the gallery against itself: every pair of stored rows a < b at or above the threshold
+    def self_join(self, threshold: float, company_id: Optional[str] = None, same_company: bool = False,
+                  strict: bool = False, max_hits: int = 16, variant: str = "auto"):
+        """Every pair of stored rows a < b with score(a, b) >= threshold ('>' when strict), where score(a, b) is what
+        ``match_range`` returns for row b when row a's stored vector is the query.  company_id: only that company's
+        rows; same_company: only pairs whose two rows carry the same company tag (every company at once, each within
+        itself).  Returns (a int64, b int64, score fp32) arrays ordered by a, then score desc, then b.
+        One frg_self_join over the whole store on the device; only the rows that have pairs are copied back, and a row
+        with more than max_hits pairs is redone once on its own, with room for its count."""
+        import torch
+        tenant = -1 if company_id is None else self.store.tenant_code(company_id, create=False)
+        p = _params(self.metric, variant, threshold, tenant, 0)
+        p.flags = (N.FIRST_STRICT if strict else 0) | (N.JOIN_SAME_TAG if same_company else 0)
+        dev = torch.device("cuda", self.store.device)
+        none = (np.zeros(0, np.int64), np.zeros(0, np.int64), np.zeros(0, np.float32))
+
+        def run(row0, n, hits):
+            counts = torch.empty(n, dtype=torch.int64, device=dev)
+            rows = torch.empty((n, hits), dtype=torch.int64, device=dev)
+            scores = torch.empty((n, hits), dtype=torch.float32, device=dev)
+            N.check(N.lib.frg_self_join(self.store.handle, int(row0), int(n), int(hits), C.byref(p),
+                                        C.c_void_p(counts.data_ptr()), C.c_void_p(rows.data_ptr()),
+                                        C.c_void_p(scores.data_ptr()), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+            return counts, rows, scores
+
+        with _reading(self.store), torch.cuda.device(dev):
+            n = self.store.rows
+            if n == 0:
+                return none
+            counts, rows, scores = run(0, n, max_hits)
+            hit = torch.nonzero(counts).squeeze(1)          # compacted on the device: only these rows come back
+            a = hit.cpu().numpy()
+            c = counts[hit].cpu().numpy()
+            r = rows[hit].cpu().numpy()
+            s = scores[hit].cpu().numpy()
+            if not len(a):
+                return none
+            over = c > max_hits
+            fit = np.where(over, 0, c)
+            keep = np.arange(max_hits)[None, :] < fit[:, None]
+            A, B, S = [np.repeat(a, fit)], [r[keep]], [s[keep]]
+            for i in np.nonzero(over)[0].tolist():
+                c2, r2, s2 = run(int(a[i]), 1, int(c[i]))
+                m = min(int(c2.cpu()[0]), int(c[i]))
+                A.append(np.full(m, a[i], np.int64))
+                B.append(r2[0, :m].cpu().numpy())
+                S.append(s2[0, :m].cpu().numpy())
+        A, B, S = np.concatenate(A), np.concatenate(B), np.concatenate(S)
+        order = np.lexsort((B, -S, A))
+        return A[order], B[order], S[order]
+
     # ---- first row, in gallery order, whose score reaches the threshold (exact fp32)
     def first_above(self, Q: np.ndarray, threshold: float, strict: bool = False, company_id: Optional[str] = None,
                     query_prenormalised: bool = False):

@@ -208,6 +208,33 @@ FRG_API int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32
                                  const frg_match_params_t* p, int64_t* out_counts, int64_t* out_rows,
                                  float* out_scores);
 
+/* ---- gallery self-join: every pair of stored rows a < b whose score reaches the threshold, in one pass over the
+ *      upper triangle on the device (NOT in the reference: the duplicate rule of trainingServer.py:170-200 applied to
+ *      what is already enrolled - after a bulk import or a snapshot load).  The queries are the store's own rows; no
+ *      row travels to the host.  For each row a in [row0, row0 + n):
+ * out_counts[a - row0] int64: the exact number of rows b with a < b < stats.rows such that
+ *   score rule:  score(a, b) >= p->threshold ('>' with FRG_FIRST_STRICT);
+ *   tag rule:    row b is live; with p->tenant >= 0 both a and b carry that tag; with FRG_JOIN_SAME_TAG
+ *                tag[b] == tag[a] (every tenant at once, each within itself).
+ *   A dead row a, or one outside p->tenant, has count 0.
+ * score(a, b) equals, bit for bit, what frg_match_range returns for row b given the stored fp32 row a as a query.
+ * out_rows [n*max_hits] int64, out_scores [n*max_hits] fp32: the FIRST min(count, max_hits) such rows IN GALLERY ORDER
+ *   (+ p->row_offset) with their scores; unused slots row -1 / score -1.0f (the range-search layout).
+ * Supported: unit cosine stores with an fp32 master.  p->variant: AUTO (the int8 tensor-core filter when the store
+ *   keeps a scan plane and dim is 128 / 256 / 512, else the exact scan), TC_EXACT (needs that plane and dim) or
+ *   SCAN_F32.  Raw (FRG_STORE_RAW), Euclidean and bf16-only stores, TC_BF16 and FRG_QUERY_PRENORMALISED:
+ *   FRG_ERR_UNSUPPORTED (scores on a raw store are not symmetric).  row0 < 0, row0 + n > stats.rows or max_hits < 1:
+ *   FRG_ERR_INVALID.  frg_last_variant(): "join_tc" or "join_scan".
+ * The call works through [row0, row0 + n) in slabs of FRG_JOIN_SLAB_ROWS query rows with ONE device workspace, whatever
+ *   n is: below 2^27 bytes (128 MB) for dim 512 on a 148-SM device, about FRG_JOIN_SLAB_ROWS * (5 * dim + 120 KB).
+ *   The launch count is fixed per slab (it does not grow with the number of tenants). */
+#define FRG_JOIN_SAME_TAG   4u   /* p->flags: only pairs whose two rows carry the same tag */
+#define FRG_JOIN_SLAB_ROWS  1024
+FRG_API int frg_self_join(frg_store* s, int64_t row0, int64_t n, int32_t max_hits, const frg_match_params_t* p,
+                          int64_t* out_counts, int64_t* out_rows, float* out_scores, void* stream);
+FRG_API int frg_self_join_host(frg_store* s, int64_t row0, int64_t n, int32_t max_hits,
+                               const frg_match_params_t* p, int64_t* out_counts, int64_t* out_rows, float* out_scores);
+
 /* ---- k-way merge of per-shard results (multi-GPU tail, SURVEY.md section 8e).
  * scores/rows: [parts][nq][k] (each list best-first, unfilled slots row -1), e.g. the output of an
  * all-gather of every rank's frg_match result.  Order: score desc (euclidean: asc), then row asc. */
