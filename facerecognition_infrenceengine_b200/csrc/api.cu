@@ -814,14 +814,15 @@ static int match_scan(const GalleryWindow* s, const float* q, int nq, int k, con
   a.nq = nq; a.k = k; a.metric = p->metric; a.tenant = p->tenant; a.sm_count = sm_count;
   size_t part_bytes = 0;
   FRG_CHECK(scan_f32_workspace_bytes(a, &part_bytes));
-  const size_t qn_bytes = (size_t(nq) * s->dim * sizeof(float) + 255) & ~size_t(255);
+  Carve c;
+  const size_t o_qn = c.take(size_t(nq) * s->dim * sizeof(float)), o_part = c.take(part_bytes);
   unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + part_bytes, st));
-  float* qn = reinterpret_cast<float*>(ws);
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  float* qn = reinterpret_cast<float*>(ws + o_qn);
   a.qn = qn;
   int rc = launch_normalise_queries(q, nq, s->dim, p->metric == FRG_METRIC_COSINE && !(p->flags & FRG_QUERY_PRENORMALISED), qn, nullptr, nullptr, nullptr, nullptr, st);
   if (rc == FRG_OK)
-    rc = launch_scan_f32(a, ws + qn_bytes, p->row_offset, p->threshold, out_rows, out_scores, out_accept, st);
+    rc = launch_scan_f32(a, ws + o_part, p->row_offset, p->threshold, out_rows, out_scores, out_accept, st);
   if (rc == FRG_OK && tail.active)       // no select stage here: a push kernel sends every query (and the hello)
     rc = launch_exchange_push(tail.x, out_rows, out_scores, nq, k, sm_count, st);
   if (rc == FRG_OK && tail.active && tail.merge)
@@ -864,29 +865,30 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
   // with exact scores, which meet its tolerance a fortiori
   const bool i8 = !euclid && s->plane8 != nullptr;
   if (i8) rescore = true;
-  const size_t qn_bytes = (size_t(nq) * s->dim * sizeof(float) + 255) & ~size_t(255);
-  const size_t qb_bytes = (size_t(nq) * (s->dim + (euclid ? kEuclidQPad : 0)) * (i8 ? 1 : sizeof(__nv_bfloat16)) + 255) & ~size_t(255);
-  const size_t eps_bytes = (size_t(nq) * sizeof(float) + 255) & ~size_t(255);     // per-query filter error bound
-  const size_t qb2_bytes = euclid ? qb_bytes : 0;                                 // the pre-pass (lower-bound) image
-  // Euclidean: the bound coefficients [nq][4]; int8: the per-query step of the integer scores [nq]
-  const size_t coef_bytes = euclid ? ((size_t(nq) * 4 * sizeof(float) + 255) & ~size_t(255)) : i8 ? eps_bytes : 0;
   const int32_t* tile_list = nullptr;
   int n_list = 0;
   const int64_t plan_rows = tc_effective_rows(s, nq, st, &tile_list, &n_list);
   if (plan_rows < 0) return FRG_ERR_CUDA;
   const int plan_dim = euclid ? -s->dim : s->dim;          // (negative: Euclidean plane, tc_plan)
-  const size_t tc_bytes = tc_workspace_bytes(plan_rows, plan_dim, nq, k, sm_count, false, i8);
+  const size_t qb_bytes = size_t(nq) * (s->dim + (euclid ? kEuclidQPad : 0)) * (i8 ? 1 : sizeof(__nv_bfloat16));
+  Carve c;
+  const size_t o_qn = c.take(size_t(nq) * s->dim * sizeof(float)), o_qb = c.take(qb_bytes);
+  const size_t o_eps = c.take(size_t(nq) * sizeof(float));                        // per-query filter error bound
+  const size_t o_qb2 = euclid ? c.take(qb_bytes) : 0;                            // the pre-pass (lower-bound) image
+  // Euclidean: the bound coefficients [nq][4]; int8: the per-query step of the integer scores [nq]
+  const size_t o_coef = euclid ? c.take(size_t(nq) * 4 * sizeof(float)) : i8 ? c.take(size_t(nq) * sizeof(float)) : 0;
+  const size_t o_tc = c.take(tc_workspace_bytes(plan_rows, plan_dim, nq, k, sm_count, i8));
   unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + qb_bytes + eps_bytes + qb2_bytes + coef_bytes + tc_bytes, st));
-  float* qn = reinterpret_cast<float*>(ws);
-  __nv_bfloat16* qb = reinterpret_cast<__nv_bfloat16*>(ws + qn_bytes);
-  float* eps = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes);
-  __nv_bfloat16* qb2 = euclid ? reinterpret_cast<__nv_bfloat16*>(ws + qn_bytes + qb_bytes + eps_bytes) : nullptr;
-  float* coef = (euclid || i8) ? reinterpret_cast<float*>(ws + qn_bytes + qb_bytes + eps_bytes + qb2_bytes) : nullptr;
-  unsigned char* tc_ws = ws + qn_bytes + qb_bytes + eps_bytes + qb2_bytes + coef_bytes;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  float* qn = reinterpret_cast<float*>(ws + o_qn);
+  __nv_bfloat16* qb = reinterpret_cast<__nv_bfloat16*>(ws + o_qb);
+  float* eps = reinterpret_cast<float*>(ws + o_eps);
+  __nv_bfloat16* qb2 = euclid ? reinterpret_cast<__nv_bfloat16*>(ws + o_qb2) : nullptr;
+  float* coef = (euclid || i8) ? reinterpret_cast<float*>(ws + o_coef) : nullptr;
+  unsigned char* tc_ws = ws + o_tc;
   int* flagged = nullptr; int* n_flagged = nullptr;
   void* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
-  tc_workspace_init_targets(plan_rows, plan_dim, nq, k, sm_count, tc_ws, &keys, &ct0, &nf0, false, i8);
+  tc_workspace_init_targets(plan_rows, plan_dim, nq, k, sm_count, tc_ws, &keys, &ct0, &nf0, i8);
   int8_t* qi8 = i8 ? reinterpret_cast<int8_t*>(qb) : nullptr;
   profile_begin(st, kStagePrep);
   int rc = euclid ? launch_prepare_queries_euclid(q, nq, s->dim, s->gmax_bits, qn, qb, qb2, coef, eps,
@@ -1061,15 +1063,16 @@ static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     return FRG_OK;
   }
   // every other store / variant: frg_match's own path once per tenant, into tenant-sorted scratch, then scattered
-  const size_t qb = (size_t(nq) * s->dim * 4 + 255) & ~size_t(255), pb = (size_t(nq) * 4 + 255) & ~size_t(255);
-  const size_t rb = (size_t(nq) * k * 8 + 255) & ~size_t(255), sb = (size_t(nq) * k * 4 + 255) & ~size_t(255);
+  Carve c;
+  const size_t o_qs = c.take(size_t(nq) * s->dim * 4), o_perm = c.take(size_t(nq) * 4);
+  const size_t o_rows = c.take(size_t(nq) * k * 8), o_sc = c.take(size_t(nq) * k * 4), o_acc = c.take(size_t(nq));
   unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qb + pb + rb + sb + size_t(nq), st));
-  float* qs = reinterpret_cast<float*>(ws);
-  int32_t* dperm = reinterpret_cast<int32_t*>(ws + qb);
-  int64_t* srows = reinterpret_cast<int64_t*>(ws + qb + pb);
-  float* sscores = reinterpret_cast<float*>(ws + qb + pb + rb);
-  uint8_t* sacc = ws + qb + pb + rb + sb;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  float* qs = reinterpret_cast<float*>(ws + o_qs);
+  int32_t* dperm = reinterpret_cast<int32_t*>(ws + o_perm);
+  int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
+  float* sscores = reinterpret_cast<float*>(ws + o_sc);
+  uint8_t* sacc = ws + o_acc;
   int rc = stage_upload(dperm, perm.data(), size_t(nq) * 4, st);
   if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, s->dim, qs, st);
   for (size_t i = 0; rc == FRG_OK && i < groups.size(); ++i) {
@@ -1167,9 +1170,11 @@ static int match_host_impl(frg_store* s, const float* q, int32_t nq, int32_t k, 
   cudaStream_t st = cudaStreamPerThread;
   const size_t qb = size_t(nq) * s->dim * sizeof(float);
   const size_t rb = size_t(nq) * k * sizeof(int64_t), sb = size_t(nq) * k * sizeof(float), ab = size_t(nq);
-  const size_t o_r = (qb + 255) & ~size_t(255), o_s = (o_r + rb + 255) & ~size_t(255), o_a = (o_s + sb + 255) & ~size_t(255);
+  Carve c;
+  c.take(qb);
+  const size_t o_r = c.take(rb), o_s = c.take(sb), o_a = c.take(ab);
   unsigned char* d = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), o_a + ab, st));
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), c.off, st));
   int rc = FRG_OK;
   cudaError_t e = cudaMemcpyAsync(d, q, qb, cudaMemcpyHostToDevice, st);
   if (e != cudaSuccess) rc = cuda_fail(e, "H2D queries", __FILE__, __LINE__);
@@ -1233,17 +1238,18 @@ int frg_first_match(frg_store* s, const float* q, int32_t nq, const frg_match_pa
   FRG_CHECK(device_info(s->device, &di));
   std::lock_guard<std::mutex> lk(s->mu);
   FRG_CHECK(store_begin_read(s, st));
-  const size_t qn_bytes = (size_t(nq) * s->dim * sizeof(float) + 255) & ~size_t(255);
+  Carve c;
+  const size_t o_qn = c.take(size_t(nq) * s->dim * sizeof(float)), o_scratch = c.take(size_t(nq) * 8);
   unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + size_t(nq) * 8, st));
-  float* qn = reinterpret_cast<float*>(ws);
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  float* qn = reinterpret_cast<float*>(ws + o_qn);
   int rc = launch_normalise_queries(q, nq, s->dim, !(p->flags & FRG_QUERY_PRENORMALISED), qn, nullptr, nullptr,
                                     nullptr, nullptr, st);
   const GalleryWindow w = window_of(s, p->tenant);
   if (rc == FRG_OK)
     rc = launch_first_match(w.master, w.tags, w.rows, s->dim, qn, nq, p->tenant, p->threshold,
                             (p->flags & FRG_FIRST_STRICT) != 0, p->row_offset + w.row0,
-                            reinterpret_cast<unsigned long long*>(ws + qn_bytes), di.sm_count, out_rows, out_scores, st);
+                            reinterpret_cast<unsigned long long*>(ws + o_scratch), di.sm_count, out_rows, out_scores, st);
   cudaError_t e = cudaFreeAsync(ws, st);
   if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
   return rc;
@@ -1256,9 +1262,11 @@ int frg_first_match_host(frg_store* s, const float* q, int32_t nq, const frg_mat
   DeviceGuard g(s->device);
   cudaStream_t st = cudaStreamPerThread;
   const size_t qb = size_t(nq) * s->dim * sizeof(float);
-  const size_t o_r = (qb + 255) & ~size_t(255), o_s = o_r + ((size_t(nq) * 8 + 255) & ~size_t(255));
+  Carve c;
+  c.take(qb);
+  const size_t o_r = c.take(size_t(nq) * 8), o_s = c.take(size_t(nq) * 4);
   unsigned char* d = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), o_s + size_t(nq) * 4, st));
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), c.off, st));
   int rc = FRG_OK;
   cudaError_t e = cudaMemcpyAsync(d, q, qb, cudaMemcpyHostToDevice, st);
   if (e != cudaSuccess) rc = cuda_fail(e, "H2D queries", __FILE__, __LINE__);
@@ -1279,6 +1287,54 @@ int frg_first_match_host(frg_store* s, const float* q, int32_t nq, const frg_mat
 // Tensor-core path (unit cosine stores with a plane and a covered dim): query prep (fp32 unit queries, int8 image,
 // eps[q]) -> filter with the fixed floor threshold - eps[q] -> range_select_kernel -> exact range scan of the
 // queries whose candidates overflowed.  Everything else: the exact range scan over all queries.
+// The checks range search and the self-join share, after each call's own: max_hits, the variant, an fp32 master for
+// the exact scores, a dim the exact range scan is built for.  *use_tc: AUTO takes the tensor-core path when tc_ok;
+// TC_EXACT insists on it (tc_needs names what it needs).  `what` prefixes every message.
+static int check_range_call(const frg_store* s, const frg_match_params_t* p, int32_t max_hits, bool tc_ok,
+                            const char* tc_needs, const char* what, bool* use_tc) {
+  if (max_hits < 1) { set_error("%s: max_hits=%d must be >= 1", what, max_hits); return FRG_ERR_INVALID; }
+  if (p->variant < FRG_VARIANT_AUTO || p->variant > FRG_VARIANT_TC_BF16) { set_error("%s: unknown variant %d", what, p->variant); return FRG_ERR_INVALID; }
+  if (p->variant == FRG_VARIANT_TC_BF16) {
+    set_error("%s: FRG_VARIANT_TC_BF16 has no exact scores to hold against the threshold (use AUTO, TC_EXACT or SCAN_F32)", what);
+    return FRG_ERR_UNSUPPORTED;
+  }
+  if (!s->master) { set_error("%s: a bf16-only store has no fp32 master for the exact scores", what); return FRG_ERR_UNSUPPORTED; }
+  const char* why = "";
+  if (!range_scan_supported(s->dim, &why)) { set_error("%s: %s", what, why); return FRG_ERR_UNSUPPORTED; }
+  *use_tc = p->variant == FRG_VARIANT_TC_EXACT || (p->variant == FRG_VARIANT_AUTO && tc_ok);
+  if (*use_tc && !tc_ok) { set_error("%s: FRG_VARIANT_TC_EXACT needs %s", what, tc_needs); return FRG_ERR_UNSUPPORTED; }
+  return FRG_OK;
+}
+
+// [counts | rows | scores] of n query rows in one device block behind in_bytes for the call's inputs:
+// run(inputs, counts, rows, scores, stream), then three copies into the caller's arrays, the sync and the fault word.
+extern "C++" {
+template <typename Run>
+static int range_results_host(frg_store* s, int64_t n, int32_t max_hits, size_t in_bytes, int64_t* out_counts,
+                              int64_t* out_rows, float* out_scores, Run run) {
+  DeviceGuard g(s->device);
+  cudaStream_t st = cudaStreamPerThread;
+  const size_t slots = size_t(n) * size_t(max_hits), cb = size_t(n) * sizeof(int64_t);
+  Carve c;
+  const size_t o_in = c.take(in_bytes), o_c = c.take(cb);
+  const size_t o_r = c.take(slots * sizeof(int64_t)), o_s = c.take(slots * sizeof(float));
+  unsigned char* d = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), c.off, st));
+  int rc = run(d + o_in, reinterpret_cast<int64_t*>(d + o_c), reinterpret_cast<int64_t*>(d + o_r),
+               reinterpret_cast<float*>(d + o_s), st);
+  if (rc == FRG_OK) {
+    cudaError_t e = cudaMemcpyAsync(out_counts, d + o_c, cb, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_rows, d + o_r, slots * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out_scores, d + o_s, slots * sizeof(float), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) rc = cuda_fail(e, "D2H results", __FILE__, __LINE__);
+    else rc = store_fault(s);
+  }
+  cudaFreeAsync(d, st);
+  return rc;
+}
+}  // extern "C++"
+
 static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
                       int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
   reset_launches();
@@ -1286,28 +1342,18 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
     set_error("match_range: bad argument");
     return FRG_ERR_INVALID;
   }
-  if (max_hits < 1) { set_error("match_range: max_hits=%d must be >= 1", max_hits); return FRG_ERR_INVALID; }
   if (p->metric != FRG_METRIC_COSINE && p->metric != FRG_METRIC_EUCLIDEAN) { set_error("match_range: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
-  if (p->variant < FRG_VARIANT_AUTO || p->variant > FRG_VARIANT_TC_BF16) { set_error("match_range: unknown variant %d", p->variant); return FRG_ERR_INVALID; }
-  if (p->variant == FRG_VARIANT_TC_BF16) {
-    set_error("match_range: FRG_VARIANT_TC_BF16 has no exact scores to hold against the threshold (use AUTO, TC_EXACT or SCAN_F32)");
-    return FRG_ERR_UNSUPPORTED;
-  }
-  if (!s->master) { set_error("match_range: a bf16-only store has no fp32 master for the exact scores"); return FRG_ERR_UNSUPPORTED; }
   if (p->variant == FRG_VARIANT_TC_EXACT && p->metric == FRG_METRIC_EUCLIDEAN) {
     set_error("match_range: the Euclidean range search runs on the exact scan only (FRG_VARIANT_SCAN_F32 / AUTO)");
     return FRG_ERR_UNSUPPORTED;
   }
   const char* why = "";
-  if (!range_scan_supported(s->dim, &why)) { set_error("match_range: %s", why); return FRG_ERR_UNSUPPORTED; }
   const bool unit = !(s->flags & FRG_STORE_RAW) && !(p->flags & FRG_QUERY_PRENORMALISED);
   const bool tc_ok = s->plane8 != nullptr && unit && p->metric == FRG_METRIC_COSINE && tc_supported(s->dim, p->metric, &why);
-  const bool use_tc = p->variant == FRG_VARIANT_TC_EXACT || (p->variant == FRG_VARIANT_AUTO && tc_ok);
-  if (use_tc && !tc_ok) {
-    set_error("match_range: FRG_VARIANT_TC_EXACT needs a unit-row store with a scan plane, normalised queries and "
-              "dim 128 / 256 / 512");
-    return FRG_ERR_UNSUPPORTED;
-  }
+  bool use_tc = false;
+  FRG_CHECK(check_range_call(s, p, max_hits, tc_ok,
+                             "a unit-row store with a scan plane, normalised queries and dim 128 / 256 / 512",
+                             "match_range", &use_tc));
   if (nq == 0) return FRG_OK;
   DeviceGuard g(s->device);
   if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
@@ -1322,45 +1368,43 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
   ScanArgs a;
   a.master = w.master; a.plane = w.plane; a.tags = w.tags; a.rows = w.rows; a.dim = w.dim;
   a.nq = nq; a.k = 1; a.metric = p->metric; a.tenant = p->tenant; a.sm_count = di.sm_count;
-  const size_t qn_bytes = (size_t(nq) * w.dim * sizeof(float) + 255) & ~size_t(255);
+  Carve c;
+  const size_t o_qn = c.take(size_t(nq) * w.dim * sizeof(float));
   unsigned char* ws = nullptr;
   int rc = FRG_OK;
   if (use_tc && w.rows > 0) {
-    const size_t qb_bytes = (size_t(nq) * w.dim + 255) & ~size_t(255);              // int8 image
-    const size_t eps_bytes = (size_t(nq) * sizeof(float) + 255) & ~size_t(255);
     const int32_t* tile_list = nullptr;
     int n_list = 0;
     const int64_t plan_rows = tc_effective_rows(&w, nq, st, &tile_list, &n_list);
     if (plan_rows < 0) return FRG_ERR_CUDA;
-    const size_t tc_bytes = tc_workspace_bytes(plan_rows, w.dim, nq, 1, di.sm_count, true, true);
-    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes + qb_bytes + 2 * eps_bytes + tc_bytes, st));
-    float* qn = reinterpret_cast<float*>(ws);
-    int8_t* qi8 = reinterpret_cast<int8_t*>(ws + qn_bytes);
-    float* eps = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes);
-    float* qstep = reinterpret_cast<float*>(ws + qn_bytes + qb_bytes + eps_bytes);
-    unsigned char* tc_ws = ws + qn_bytes + qb_bytes + 2 * eps_bytes;
-    void* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
-    tc_workspace_init_targets(plan_rows, w.dim, nq, 1, di.sm_count, tc_ws, &keys, &ct0, &nf0, true, true);
-    int* flagged = nullptr; int* n_flagged = nullptr;
+    const int64_t cand = tc_range_cand_entries(plan_rows, w.dim, nq, di.sm_count);
+    const size_t o_qi8 = c.take(size_t(nq) * w.dim), o_eps = c.take(size_t(nq) * sizeof(float));
+    const size_t o_step = c.take(size_t(nq) * sizeof(float)), o_tc = c.take(tc_range_workspace(nq, cand, nullptr, nullptr));
+    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+    float* qn = reinterpret_cast<float*>(ws + o_qn);
+    int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
+    float* eps = reinterpret_cast<float*>(ws + o_eps);
+    float* qstep = reinterpret_cast<float*>(ws + o_step);
+    TcRangeWs tw;
+    tc_range_workspace(nq, cand, ws + o_tc, &tw);
     profile_begin(st, kStagePrep);
-    rc = launch_prepare_queries_i8(q, nq, w.dim, qn, qi8, qstep, eps, s->gmax_bits,
-                                   static_cast<unsigned long long*>(keys), ct0, nf0, st);
+    rc = launch_prepare_queries_i8(q, nq, w.dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
+                                   tw.n_flagged, st);
     profile_end(st, 1);
     if (rc == FRG_OK)
-      rc = launch_tc_range(&w, qn, qi8, qstep, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, tc_ws,
-                           di.sm_count, out_counts, out_rows, out_scores, &flagged, &n_flagged, st, plan_rows,
-                           tile_list, n_list);
+      rc = launch_tc_range(&w, qn, qi8, qstep, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, tw,
+                           di.sm_count, out_counts, out_rows, out_scores, st, plan_rows, tile_list, n_list);
     if (rc == FRG_OK) {
       a.qn = qn;
       profile_begin(st, kStageFallback);
-      rc = launch_range_scan(a, flagged, n_flagged, max_hits, p->threshold, strict, row_offset, out_counts,
+      rc = launch_range_scan(a, tw.flagged, tw.n_flagged, max_hits, p->threshold, strict, row_offset, out_counts,
                              out_rows, out_scores, st);
       profile_end(st, 1);
     }
     g_variant = "range_tc";
   } else {
-    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), qn_bytes, st));
-    float* qn = reinterpret_cast<float*>(ws);
+    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+    float* qn = reinterpret_cast<float*>(ws + o_qn);
     a.qn = qn;
     rc = launch_normalise_queries(q, nq, w.dim, p->metric == FRG_METRIC_COSINE && !(p->flags & FRG_QUERY_PRENORMALISED),
                                   qn, nullptr, nullptr, nullptr, nullptr, st);
@@ -1388,30 +1432,13 @@ int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32_t max_h
     return range_impl(s, q, nq, max_hits, p, out_counts, out_rows, out_scores, nullptr);
   }
   if (nq == 0) return range_impl(s, q, nq, max_hits, p, out_counts, out_rows, out_scores, nullptr);
-  DeviceGuard g(s->device);
-  cudaStream_t st = cudaStreamPerThread;
-  const size_t slots = size_t(nq) * size_t(max_hits);
-  const size_t qb = size_t(nq) * s->dim * sizeof(float), cb = size_t(nq) * sizeof(int64_t);
-  const size_t o_c = (qb + 255) & ~size_t(255), o_r = (o_c + cb + 255) & ~size_t(255),
-               o_s = (o_r + slots * sizeof(int64_t) + 255) & ~size_t(255);
-  unsigned char* d = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), o_s + slots * sizeof(float), st));
-  int rc = FRG_OK;
-  cudaError_t e = cudaMemcpyAsync(d, q, qb, cudaMemcpyHostToDevice, st);
-  if (e != cudaSuccess) rc = cuda_fail(e, "H2D queries", __FILE__, __LINE__);
-  if (rc == FRG_OK)
-    rc = range_impl(s, reinterpret_cast<float*>(d), nq, max_hits, p, reinterpret_cast<int64_t*>(d + o_c),
-                    reinterpret_cast<int64_t*>(d + o_r), reinterpret_cast<float*>(d + o_s), st);
-  if (rc == FRG_OK) {
-    e = cudaMemcpyAsync(out_counts, d + o_c, cb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out_rows, d + o_r, slots * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out_scores, d + o_s, slots * sizeof(float), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) rc = cuda_fail(e, "D2H results", __FILE__, __LINE__);
-    else rc = store_fault(s);
-  }
-  cudaFreeAsync(d, st);
-  return rc;
+  const size_t qb = size_t(nq) * s->dim * sizeof(float);
+  return range_results_host(s, nq, max_hits, qb, out_counts, out_rows, out_scores,
+                            [&](unsigned char* dq, int64_t* dc, int64_t* dr, float* ds, cudaStream_t st) {
+    const cudaError_t e = cudaMemcpyAsync(dq, q, qb, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return cuda_fail(e, "H2D queries", __FILE__, __LINE__);
+    return range_impl(s, reinterpret_cast<float*>(dq), nq, max_hits, p, dc, dr, ds, st);
+  });
 }
 
 // --------------------------------------------------------------------------------------------- gallery self-join
@@ -1479,29 +1506,19 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
     set_error("self_join: bad argument");
     return FRG_ERR_INVALID;
   }
-  if (max_hits < 1) { set_error("self_join: max_hits=%d must be >= 1", max_hits); return FRG_ERR_INVALID; }
   if (p->metric == FRG_METRIC_EUCLIDEAN) { set_error("self_join: cosine only (Euclidean stores are raw)"); return FRG_ERR_UNSUPPORTED; }
   if (p->metric != FRG_METRIC_COSINE) { set_error("self_join: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
-  if (p->variant < FRG_VARIANT_AUTO || p->variant > FRG_VARIANT_TC_BF16) { set_error("self_join: unknown variant %d", p->variant); return FRG_ERR_INVALID; }
-  if (p->variant == FRG_VARIANT_TC_BF16) {
-    set_error("self_join: FRG_VARIANT_TC_BF16 has no exact scores to hold against the threshold (use AUTO, TC_EXACT or SCAN_F32)");
-    return FRG_ERR_UNSUPPORTED;
-  }
   if (p->flags & ~(FRG_FIRST_STRICT | FRG_QUERY_PRENORMALISED | FRG_JOIN_SAME_TAG)) {
     set_error("self_join: unknown flags 0x%x", p->flags);
     return FRG_ERR_INVALID;
   }
   if (p->flags & FRG_QUERY_PRENORMALISED) { set_error("self_join: the queries are the store's rows (FRG_QUERY_PRENORMALISED does not apply)"); return FRG_ERR_UNSUPPORTED; }
-  if (!s->master) { set_error("self_join: a bf16-only store has no fp32 master for the exact scores"); return FRG_ERR_UNSUPPORTED; }
   if (s->flags & FRG_STORE_RAW) { set_error("self_join: scores on a raw store are not symmetric (unit cosine stores only)"); return FRG_ERR_UNSUPPORTED; }
   const char* why = "";
-  if (!range_scan_supported(s->dim, &why)) { set_error("self_join: %s", why); return FRG_ERR_UNSUPPORTED; }
   const bool tc_ok = s->plane8 != nullptr && tc_supported(s->dim, FRG_METRIC_COSINE, &why);
-  const bool use_tc = p->variant == FRG_VARIANT_TC_EXACT || (p->variant == FRG_VARIANT_AUTO && tc_ok);
-  if (use_tc && !tc_ok) {
-    set_error("self_join: FRG_VARIANT_TC_EXACT needs a unit-row store with a scan plane and dim 128 / 256 / 512");
-    return FRG_ERR_UNSUPPORTED;
-  }
+  bool use_tc = false;
+  FRG_CHECK(check_range_call(s, p, max_hits, tc_ok, "a unit-row store with a scan plane and dim 128 / 256 / 512",
+                             "self_join", &use_tc));
   DeviceGuard g(s->device);
   if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
   DeviceInfo di;
@@ -1558,17 +1575,18 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
   ScanArgs a;
   a.master = s->master; a.tags = s->tags; a.rows = s->rows; a.dim = dim;
   a.qn = nullptr; a.nq = int(S); a.k = 1; a.metric = FRG_METRIC_COSINE; a.tenant = p->tenant; a.sm_count = di.sm_count;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-  const size_t o_qn = take(size_t(S) * dim * 4), o_table = take(max_table), o_scan = take(join_scan_workspace_bytes(a));
-  size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_keys = 0, o_cnt = 0, o_flag = 0, o_floor = 0, o_dense = 0, o_cand = 0;
+  Carve c;
+  const size_t o_qn = c.take(size_t(S) * dim * 4), o_table = c.take(max_table);
+  const size_t o_scan = c.take(join_scan_workspace_bytes(a));
+  size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_tc = 0;
   if (use_tc) {
-    o_qi8 = take(size_t(S) * dim); o_eps = take(size_t(S) * 4); o_step = take(size_t(S) * 4);
-    o_keys = take(size_t(S) * 32 * 8); o_cnt = take(size_t(S) * 4); o_flag = take(size_t(S) * 4 + 12);
-    o_floor = take(size_t(S) * 4); o_dense = take(size_t(S) * kRangeBudget * 8); o_cand = take(size_t(max_cand) * 8);
+    o_qi8 = c.take(size_t(S) * dim); o_eps = c.take(size_t(S) * 4); o_step = c.take(size_t(S) * 4);
+    o_tc = c.take(tc_range_workspace(int(S), max_cand, nullptr, nullptr));
   }
   unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), off, st));
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  TcRangeWs tw{};
+  if (use_tc) tc_range_workspace(int(S), max_cand, ws + o_tc, &tw);
   float* qn = reinterpret_cast<float*>(ws + o_qn);
   const int32_t* tile_end = reinterpret_cast<const int32_t*>(ws + o_table);
   a.qn = qn;
@@ -1587,21 +1605,16 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
       int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
       float* eps = reinterpret_cast<float*>(ws + o_eps);
       float* qstep = reinterpret_cast<float*>(ws + o_step);
-      int* cnt = reinterpret_cast<int*>(ws + o_cnt);
-      int* flagged = reinterpret_cast<int*>(ws + o_flag);
-      int* n_flagged = flagged + S;
       profile_begin(st, kStagePrep);
-      rc = launch_prepare_queries_i8(s->master + qrow0 * dim, int(ns), dim, qn, qi8, qstep, eps, s->gmax_bits,
-                                     reinterpret_cast<unsigned long long*>(ws + o_keys), cnt, n_flagged, st);
+      rc = launch_prepare_queries_i8(s->master + qrow0 * dim, int(ns), dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys,
+                                     tw.cand_total, tw.n_flagged, st);
       profile_end(st, 1);
       if (rc == FRG_OK)
         rc = launch_tc_join(&w, qn, qi8, qstep, eps, int(ns), ws + o_table + t_cta, ctas[i], qrow0, p->tenant, same_tag,
-                            p->threshold, strict, max_hits, row_offset, reinterpret_cast<int2*>(ws + o_cand), cnt,
-                            reinterpret_cast<int2*>(ws + o_dense), reinterpret_cast<float*>(ws + o_floor), flagged,
-                            n_flagged, oc, orow, osc, st);
+                            p->threshold, strict, max_hits, row_offset, tw, oc, orow, osc, st);
       if (rc == FRG_OK) {
         profile_begin(st, kStageFallback);
-        rc = launch_join_scan(a, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, p->threshold, strict,
+        rc = launch_join_scan(a, qrow0, tile_end, same_tag, tw.flagged, tw.n_flagged, max_hits, p->threshold, strict,
                               row_offset, ws + o_scan, oc, orow, osc, st);
         profile_end(st, 3);
       }
@@ -1617,7 +1630,6 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
       }
     }
   }
-  g_variant = use_tc ? "join_tc" : "join_scan";
   cudaError_t e = cudaFreeAsync(ws, st);
   if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
   return rc;
@@ -1634,24 +1646,10 @@ int frg_self_join_host(frg_store* s, int64_t row0, int64_t n, int32_t max_hits, 
     // the device entry point names the argument (and takes n = 0)
     return self_join_impl(s, row0, n, max_hits, p, out_counts, out_rows, out_scores, nullptr);
   }
-  DeviceGuard g(s->device);
-  cudaStream_t st = cudaStreamPerThread;
-  const size_t slots = size_t(n) * size_t(max_hits), cb = size_t(n) * sizeof(int64_t);
-  const size_t o_r = (cb + 255) & ~size_t(255), o_s = (o_r + slots * sizeof(int64_t) + 255) & ~size_t(255);
-  unsigned char* d = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), o_s + slots * sizeof(float), st));
-  int rc = self_join_impl(s, row0, n, max_hits, p, reinterpret_cast<int64_t*>(d), reinterpret_cast<int64_t*>(d + o_r),
-                          reinterpret_cast<float*>(d + o_s), st);
-  if (rc == FRG_OK) {
-    cudaError_t e = cudaMemcpyAsync(out_counts, d, cb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out_rows, d + o_r, slots * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out_scores, d + o_s, slots * sizeof(float), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) rc = cuda_fail(e, "D2H results", __FILE__, __LINE__);
-    else rc = store_fault(s);
-  }
-  cudaFreeAsync(d, st);
-  return rc;
+  return range_results_host(s, n, max_hits, 0, out_counts, out_rows, out_scores,
+                            [&](unsigned char*, int64_t* dc, int64_t* dr, float* ds, cudaStream_t st) {
+    return self_join_impl(s, row0, n, max_hits, p, dc, dr, ds, st);
+  });
 }
 
 int frg_merge_topk(int32_t device, const float* scores, const int64_t* rows, int32_t parts,

@@ -119,6 +119,13 @@ inline cudaError_t func_attr_once(F* kern, cudaFuncAttribute attr, int value) {
   return e;
 }
 
+// Pieces of one workspace allocation: take(bytes) returns the 256-byte aligned offset of the next piece; `off` is the
+// end of the last piece, the bytes to allocate.
+struct Carve {
+  size_t off = 0;
+  size_t take(size_t bytes) { const size_t o = (off + 255) & ~size_t(255); off = o + bytes; return o; }
+};
+
 struct DeviceInfo {
   int sm_count = 0;
   int cc_major = 0, cc_minor = 0;
@@ -342,12 +349,11 @@ constexpr int kEuclidPad = 16;      // plane: one more 32-byte group of k (one U
 constexpr int kEuclidQPad = 64;     // query image: padded to a whole 128-byte swizzle row (the tile's k-block)
 constexpr float kEuclidNone = -3.0e38f;   // "no score yet" of the Euclidean filter (scores are unbounded below)
 int tc_supported(int dim, int metric, const char** why);
-// range: the plan of launch_tc_range (k is ignored there)
 // i8: the int8 filter of a unit store (64-bit group keys, per-query floor)
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range = false, bool i8 = false);
+size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool i8 = false);
 // keys: [nq][32] group keys, uint32 (bf16 filter) or uint64 (int8 filter)
 void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               void** keys, int** cand_total, int** n_flagged, bool range = false, bool i8 = false);
+                               void** keys, int** cand_total, int** n_flagged, bool i8 = false);
 // metric cosine, int8 plane (s->plane8): qi8 / qstep / eps from launch_prepare_queries_i8, qb unused.
 // metric cosine, bf16 plane (bf16-only store): qb = [nq][dim] bf16 unit queries, eps[nq] per-query bounds.
 // metric euclidean: qb = [nq][dim + kEuclidQPad] augmented image, eps[nq] per-query bounds.
@@ -381,14 +387,32 @@ int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, 
 // api.cu: host -> device copy through the per-thread pinned staging ring (pageable copy when larger than a slot)
 int stage_upload(void* dev, const void* host, size_t bytes, cudaStream_t st);
 
+// Candidate entries per query of a range-mode filter (range search and self-join; DESIGN.md section 7.3)
+constexpr int kRangeBudget = 4096;
+
+// tc_match.cu: the workspace of a range-mode int8 filter call (range search, or one self-join slab) of nq queries
+struct TcRangeWs {
+  unsigned long long* keys;   // [nq][32] group keys (the query prep resets them)
+  int* cand_total;            // [nq] candidates per query
+  int* flagged;               // [nq] queries whose candidates overflowed, then their count and the fallback's ticket
+  int* n_flagged;             // flagged + nq
+  float* floor;               // [nq] threshold - eps[q]
+  int2* dense;                // [nq][kRangeBudget] packed candidates
+  int2* cand;                 // the filter's candidate segments
+};
+// Bytes of that workspace when the filter writes cand_entries segment entries (int2); with ws, its pieces in *out.
+size_t tc_range_workspace(int nq, int64_t cand_entries, unsigned char* ws, TcRangeWs* out);
+// the candidate segment entries of range search's filter over plan_rows rows (the self-join's: tc_join_plan)
+int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count);
+
 // tc_match.cu: range search over a unit cosine store (frg_match_range).  The filter keeps every row with
 // S >= threshold - eps[q] (no pre-pass); range_select_kernel rescores each candidate exactly, keeps those that pass
 // (score >= threshold, '>' when strict), writes the first max_hits in gallery order and the count.  Queries whose
-// candidates overflowed the plan are left in (flagged, n_flagged) for launch_range_scan's flagged mode.
-int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps, int nq,
-                    int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned char* ws,
-                    int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores, int** flagged_out,
-                    int** n_flagged_out, cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list);
+// candidates overflowed the plan are left in (w.flagged, w.n_flagged) for launch_range_scan's flagged mode.
+int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
+                    int nq, int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset,
+                    const TcRangeWs& w, int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                    cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list);
 
 // scan_f32.cu: exact, counting range scan.  Pass 1: every warp owns a contiguous row range and counts its hits per
 // query; a per-query exclusive scan over the warp counts gives the total and each warp's output offset; pass 2: the
@@ -399,9 +423,6 @@ int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagge
                       bool strict, int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
                       cudaStream_t st);
 
-// Candidate entries per query of a range-mode filter (range search and self-join; DESIGN.md section 7.3)
-constexpr int kRangeBudget = 4096;
-
 // ---- gallery self-join (frg_self_join): the queries are the store's own rows qrow0 .. qrow0 + nq - 1 of one slab,
 // and a pair (a, b) counts only for b > a (plus the tag rule: tenant >= 0 -> both rows carry it; same_tag -> tag[b] ==
 // tag[a]).  Query tile u of the slab holds queries 128u .. 128u + 127.
@@ -410,15 +431,14 @@ constexpr int kRangeBudget = 4096;
 // number of CTAs and the candidate segment entries (int2) the grid writes.  The planner of launch_tc_match_grouped.
 void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::vector<unsigned char>* table,
                   int* n_ctas, int64_t* cand_entries);
-// tc_match.cu: the int8 filter path of one slab: floor threshold - eps[q] (range_floor_kernel), the GROUPED filter
-// over the uploaded table (d_table, n_ctas; none when 0) with kRangeBudget dense entries per query, and
-// join_select_kernel (exact rescoring, b > a, tag rule, counts and the first max_hits hits in gallery order).  Queries
-// whose candidates overflowed are left in (flagged, n_flagged) for launch_join_scan.  s: the whole store.
+// tc_match.cu: the int8 filter path of one slab, launch_tc_range's with the GROUPED filter over the uploaded table
+// (d_table, n_ctas; none when 0) and join_select_kernel (exact rescoring, b > a, tag rule, counts and the first
+// max_hits hits in gallery order).  Queries whose candidates overflowed are left in (w.flagged, w.n_flagged) for
+// launch_join_scan.  s: the whole store.
 int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
                    int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
-                   float threshold, bool strict, int max_hits, int64_t row_offset, int2* cand, int* cand_total,
-                   int2* dense, float* floor_v, int* flagged, int* n_flagged, int64_t* out_counts, int64_t* out_rows,
-                   float* out_scores, cudaStream_t st);
+                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcRangeWs& w,
+                   int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st);
 // scan_f32.cu: exact, counting join scan (launch_range_scan's passes with the join rules).  a: the whole store, a.qn /
 // a.nq the slab's unit queries, a.tenant the tenant rule, cosine.  tile_end[u]: exclusive end row of query tile u's
 // plan (device).  A pass of queries reads only the rows from its lowest live query row + 1 to its largest end.

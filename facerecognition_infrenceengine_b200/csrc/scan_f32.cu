@@ -11,6 +11,8 @@
 // matrix ever reaches HBM.
 //
 // Algorithmic bytes per launch = rows * dim * 4 (DESIGN.md); grid = 2 CTAs x SM count.
+#include <type_traits>
+
 #include "merge_device.cuh"
 
 namespace frg {
@@ -496,20 +498,26 @@ static int launch_one(const ScanArgs& a, int grid, int q0, int nq_pass, float* p
   return FRG_OK;
 }
 
-template <int NJ, int QB>
-static int launch_metric(const ScanArgs& a, int grid, int q0, int nq_pass, float* ps, int32_t* pi, cudaStream_t st) {
-  if (a.metric == FRG_METRIC_COSINE) return launch_one<NJ, QB, FRG_METRIC_COSINE>(a, grid, q0, nq_pass, ps, pi, st);
-  return launch_one<NJ, QB, FRG_METRIC_EUCLIDEAN>(a, grid, q0, nq_pass, ps, pi, st);
-}
-
-template <int NJ>
-static int launch_qb(const ScanArgs& a, int qb, int grid, int q0, int nq_pass, float* ps, int32_t* pi, cudaStream_t st) {
-  if (qb == 1) return launch_metric<NJ, 1>(a, grid, q0, nq_pass, ps, pi, st);
-  if (qb == 2) return launch_metric<NJ, 2>(a, grid, q0, nq_pass, ps, pi, st);
-  if constexpr (NJ <= 4) { if (qb == 4) return launch_metric<NJ, 4>(a, grid, q0, nq_pass, ps, pi, st); }
-  if constexpr (NJ <= 2) { if (qb == 8) return launch_metric<NJ, 8>(a, grid, q0, nq_pass, ps, pi, st); }
-  set_error("scan_f32: unsupported queries-per-pass %d for dim %d", qb, NJ * 128);
-  return FRG_ERR_UNSUPPORTED;
+// Calls f(NJ, QB), both std::integral_constant<int, ...>, for dim = NJ * 128 (NJ 1, 2, 4 or 8; the caller has checked
+// dim) and qb queries per pass: 1 and 2 at every dim, 4 for NJ <= 4 and 8 for NJ <= 2 (the QB x NJ float4 of queries
+// live in registers, scan_qb).  `what` prefixes the error of any other qb.
+template <typename F>
+static int dispatch_nj_qb(int dim, int qb, const char* what, F&& f) {
+  auto by_qb = [&](auto nj) -> int {
+    constexpr int NJ = decltype(nj)::value;
+    if (qb == 1) return f(nj, std::integral_constant<int, 1>());
+    if (qb == 2) return f(nj, std::integral_constant<int, 2>());
+    if constexpr (NJ <= 4) { if (qb == 4) return f(nj, std::integral_constant<int, 4>()); }
+    if constexpr (NJ <= 2) { if (qb == 8) return f(nj, std::integral_constant<int, 8>()); }
+    set_error("%s: unsupported queries-per-pass %d for dim %d", what, qb, NJ * 128);
+    return FRG_ERR_UNSUPPORTED;
+  };
+  switch (dim) {
+    case 128: return by_qb(std::integral_constant<int, 1>());
+    case 256: return by_qb(std::integral_constant<int, 2>());
+    case 512: return by_qb(std::integral_constant<int, 4>());
+    default:  return by_qb(std::integral_constant<int, 8>());
+  }
 }
 
 int launch_scan_f32(const ScanArgs& a, void* workspace, int64_t row_offset, float threshold,
@@ -530,14 +538,12 @@ int launch_scan_f32(const ScanArgs& a, void* workspace, int64_t row_offset, floa
     for (int q0 = 0; q0 < a.nq; q0 += qb) {
       ++passes;
       const int nq_pass = a.nq - q0 < qb ? a.nq - q0 : qb;
-      int rc;
-      switch (a.dim) {
-        case 128: rc = launch_qb<1>(a, qb, grid, q0, nq_pass, part_sc, part_ix, st); break;
-        case 256: rc = launch_qb<2>(a, qb, grid, q0, nq_pass, part_sc, part_ix, st); break;
-        case 512: rc = launch_qb<4>(a, qb, grid, q0, nq_pass, part_sc, part_ix, st); break;
-        default:  rc = launch_qb<8>(a, qb, grid, q0, nq_pass, part_sc, part_ix, st); break;
-      }
-      FRG_CHECK(rc);
+      FRG_CHECK(dispatch_nj_qb(a.dim, qb, "scan_f32", [&](auto nj, auto qbc) {
+        constexpr int NJ = decltype(nj)::value, QB = decltype(qbc)::value;
+        if (a.metric == FRG_METRIC_COSINE)
+          return launch_one<NJ, QB, FRG_METRIC_COSINE>(a, grid, q0, nq_pass, part_sc, part_ix, st);
+        return launch_one<NJ, QB, FRG_METRIC_EUCLIDEAN>(a, grid, q0, nq_pass, part_sc, part_ix, st);
+      }));
     }
     profile_end(st, passes);
   }
@@ -639,6 +645,64 @@ __device__ __forceinline__ bool range_pass(float sdot, float threshold, int stri
   return strict ? (d < threshold) : (d <= threshold);
 }
 
+// One counting pass of the nb queries in slots s0 .. over warp gw's row strip [r0, r1): pass 1 (WRITE = false) stores
+// each query's hit count, pass 2 writes the hits from the warp's offset on.  The lane's query (my_b of the pass) is slot
+// `slot`, output row q.  Dead rows and other tenants' rows are skipped; for every other row, rule(r, tag, mine) sets
+// whether row r counts for the lane's query and returns false when the whole warp can skip the row.
+template <int NJ, int QB, int METRIC, bool WRITE, typename Rule>
+__device__ __forceinline__ void range_strip(const float* master, const int32_t* tags, const float* qn,
+                                            const int* flagged, int s0, int nb, int slot, int q, int64_t r0,
+                                            int64_t r1, int64_t nw, int64_t gw, int lane, int my_b, bool rep,
+                                            int32_t tenant, float threshold, int strict, int max_hits,
+                                            int64_t row_offset, int* cnt, const int* off, int64_t* out_rows,
+                                            float* out_scores, Rule rule) {
+  constexpr int DIM = NJ * 128;
+  // pass 2: this lane's query needs this warp iff the warp has hits that land below max_hits
+  int pos = 0, room = 0;
+  if (WRITE) {
+    if (my_b < nb && cnt[size_t(slot) * nw + gw] > 0) {
+      pos = off[size_t(slot) * nw + gw];
+      room = max_hits;
+    }
+    if (!__any_sync(0xffffffffu, pos < room)) return;
+  }
+  float4 qv[QB][NJ];
+#pragma unroll
+  for (int b = 0; b < QB; ++b) {
+    const int qb_ = flagged ? flagged[s0 + (b < nb ? b : 0)] : s0 + (b < nb ? b : 0);
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) qv[b][j] = __ldg(reinterpret_cast<const float4*>(qn + size_t(qb_) * DIM) + j * 32 + lane);
+  }
+  int count = 0;
+  for (int64_t r = r0; r < r1; ++r) {
+    const int32_t tg = __ldg(tags + r);
+    float4 g[NJ];                                                     // issued together with the tag load
+    const float4* pr = reinterpret_cast<const float4*>(master + r * DIM) + lane;
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) g[j] = ldg_stream(pr + j * 32);
+    if (tg < 0 || (tenant >= 0 && tg != tenant)) continue;           // warp-uniform
+    bool mine;
+    if (!rule(r, tg, mine)) continue;
+    float a[QB];
+    row_dots<NJ, QB, METRIC>(g, qv, a);
+    const float sdot = butterfly<QB>(a, lane);
+    const bool hit = mine && range_pass<METRIC>(sdot, threshold, strict);
+    if (WRITE) {
+      if (hit && pos < room) {
+        if (rep) {
+          out_rows[size_t(q) * max_hits + pos] = r + row_offset;
+          out_scores[size_t(q) * max_hits + pos] = METRIC == FRG_METRIC_COSINE ? sdot : __fsqrt_rn(sdot);
+        }
+        ++pos;
+      }
+      if (!__any_sync(0xffffffffu, pos < room)) break;
+    } else {
+      count += hit ? 1 : 0;
+    }
+  }
+  if (!WRITE && rep && my_b < nb) cnt[size_t(slot) * nw + gw] = count;
+}
+
 template <int NJ, int QB, int METRIC, bool WRITE>
 __global__ void __launch_bounds__(kScanWarps * 32, 2)
 range_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ tags, int64_t rows,
@@ -646,7 +710,6 @@ range_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ 
                   const int* __restrict__ n_flagged, int32_t tenant, float threshold, int strict, int max_hits,
                   int64_t row_offset, int* __restrict__ cnt, const int* __restrict__ off,
                   int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
-  constexpr int DIM = NJ * 128;
   pdl_wait();
   pdl_trigger();
   const int n_slots = flagged ? *n_flagged : nq;
@@ -660,48 +723,11 @@ range_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ 
     const int nb = n_slots - s0 < QB ? n_slots - s0 : QB;
     const int slot = s0 + (my_b < nb ? my_b : 0);
     const int q = flagged ? flagged[slot] : slot;
-    // pass 2: this lane's query needs this warp iff the warp has hits that land below max_hits
-    int pos = 0, room = 0;
-    if (WRITE) {
-      if (my_b < nb && cnt[size_t(slot) * nw + gw] > 0) {
-        pos = off[size_t(slot) * nw + gw];
-        room = max_hits;
-      }
-      if (!__any_sync(0xffffffffu, pos < room)) continue;
-    }
-    float4 qv[QB][NJ];
-#pragma unroll
-    for (int b = 0; b < QB; ++b) {
-      const int qb_ = flagged ? flagged[s0 + (b < nb ? b : 0)] : s0 + (b < nb ? b : 0);
-#pragma unroll
-      for (int j = 0; j < NJ; ++j) qv[b][j] = __ldg(reinterpret_cast<const float4*>(qn + size_t(qb_) * DIM) + j * 32 + lane);
-    }
-    int count = 0;
-    for (int64_t r = r0; r < r1; ++r) {
-      const int32_t tg = __ldg(tags + r);
-      float4 g[NJ];                                                     // issued together with the tag load
-      const float4* pr = reinterpret_cast<const float4*>(master + r * DIM) + lane;
-#pragma unroll
-      for (int j = 0; j < NJ; ++j) g[j] = ldg_stream(pr + j * 32);
-      if (tg < 0 || (tenant >= 0 && tg != tenant)) continue;           // warp-uniform
-      float a[QB];
-      row_dots<NJ, QB, METRIC>(g, qv, a);
-      const float sdot = butterfly<QB>(a, lane);
-      const bool hit = my_b < nb && range_pass<METRIC>(sdot, threshold, strict);
-      if (WRITE) {
-        if (hit && pos < room) {
-          if (rep) {
-            out_rows[size_t(q) * max_hits + pos] = r + row_offset;
-            out_scores[size_t(q) * max_hits + pos] = METRIC == FRG_METRIC_COSINE ? sdot : __fsqrt_rn(sdot);
-          }
-          ++pos;
-        }
-        if (!__any_sync(0xffffffffu, pos < room)) break;
-      } else {
-        count += hit ? 1 : 0;
-      }
-    }
-    if (!WRITE && rep && my_b < nb) cnt[size_t(slot) * nw + gw] = count;
+    // every live row of the tenant counts for every query of the pass
+    auto rule = [&](int64_t, int32_t, bool& mine) { mine = my_b < nb; return true; };
+    range_strip<NJ, QB, METRIC, WRITE>(master, tags, qn, flagged, s0, nb, slot, q, r0, r1, nw, gw, lane, my_b, rep,
+                                       tenant, threshold, strict, max_hits, row_offset, cnt, off, out_rows,
+                                       out_scores, rule);
   }
 }
 
@@ -750,52 +776,21 @@ int range_scan_supported(int dim, const char** why) {
   return 1;
 }
 
-template <int NJ, int QB, int METRIC>
-static int launch_range_passes(const ScanArgs& a, int grid, const int* flagged, const int* n_flagged, int max_hits,
-                               float threshold, bool strict, int64_t row_offset, int* cnt, int* off,
-                               int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
-  const int nw = grid * kScanWarps;
-  const int s = strict ? 1 : 0;
-  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, false>, dim3(grid), dim3(kScanWarps * 32), 0, st,
-                         a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged, a.tenant, threshold, s, max_hits,
-                         row_offset, cnt, off, out_rows, out_scores));
+// Pass 1, the per-query offsets and pass 2 of a counting scan of nq query slots: scan(std::bool_constant<WRITE>())
+// launches the caller's scan kernel for one pass.  none_score fills the unused output slots.
+template <typename Scan>
+static int launch_counting_passes(Scan scan, int grid, int nq, const int* flagged, const int* n_flagged, int max_hits,
+                                  float none_score, int* cnt, int* off, int64_t* out_counts, int64_t* out_rows,
+                                  float* out_scores, cudaStream_t st) {
+  FRG_CUDA(scan(std::false_type()));
   note_launch(nullptr);
-  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(a.nq), dim3(256), 0, st, a.nq, flagged, n_flagged, nw, cnt,
-                         off, max_hits, METRIC == FRG_METRIC_COSINE ? kNoScore : INFINITY, out_counts, out_rows,
-                         out_scores));
+  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(nq), dim3(256), 0, st, nq, flagged, n_flagged, grid * kScanWarps,
+                         cnt, off, max_hits, none_score, out_counts, out_rows, out_scores));
   note_launch(nullptr);
-  FRG_CUDA(launch_kernel(range_scan_kernel<NJ, QB, METRIC, true>, dim3(grid), dim3(kScanWarps * 32), 0, st,
-                         a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged, a.tenant, threshold, s, max_hits,
-                         row_offset, cnt, off, out_rows, out_scores));
+  FRG_CUDA(scan(std::true_type()));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   return FRG_OK;
-}
-
-template <int NJ, int QB>
-static int launch_range_m(const ScanArgs& a, int grid, const int* flagged, const int* n_flagged, int max_hits,
-                          float threshold, bool strict, int64_t row_offset, int* cnt, int* off, int64_t* out_counts,
-                          int64_t* out_rows, float* out_scores, cudaStream_t st) {
-  if (a.metric == FRG_METRIC_COSINE)
-    return launch_range_passes<NJ, QB, FRG_METRIC_COSINE>(a, grid, flagged, n_flagged, max_hits, threshold, strict,
-                                                          row_offset, cnt, off, out_counts, out_rows, out_scores, st);
-  return launch_range_passes<NJ, QB, FRG_METRIC_EUCLIDEAN>(a, grid, flagged, n_flagged, max_hits, threshold, strict,
-                                                           row_offset, cnt, off, out_counts, out_rows, out_scores, st);
-}
-
-template <int NJ>
-static int launch_range_qb(const ScanArgs& a, int qb, int grid, const int* flagged, const int* n_flagged,
-                           int max_hits, float threshold, bool strict, int64_t row_offset, int* cnt, int* off,
-                           int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
-#define FRG_RANGE_QB(QB) return launch_range_m<NJ, QB>(a, grid, flagged, n_flagged, max_hits, threshold, strict, \
-                                                      row_offset, cnt, off, out_counts, out_rows, out_scores, st)
-  if (qb == 1) { FRG_RANGE_QB(1); }
-  if (qb == 2) { FRG_RANGE_QB(2); }
-  if constexpr (NJ <= 4) { if (qb == 4) { FRG_RANGE_QB(4); } }
-  if constexpr (NJ <= 2) { if (qb == 8) { FRG_RANGE_QB(8); } }
-#undef FRG_RANGE_QB
-  set_error("range scan: unsupported queries-per-pass %d for dim %d", qb, NJ * 128);
-  return FRG_ERR_UNSUPPORTED;
 }
 
 int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagged, int max_hits, float threshold,
@@ -812,16 +807,25 @@ int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagge
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_cnt * 2 * sizeof(int), st));
   int* cnt = reinterpret_cast<int*>(ws);
   int* off = cnt + n_cnt;
-  const int qb = scan_qb(a.dim, a.nq);
-  int rc;
-  switch (a.dim) {
-    case 128: rc = launch_range_qb<1>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
-    case 256: rc = launch_range_qb<2>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
-    case 512: rc = launch_range_qb<4>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
-    default:  rc = launch_range_qb<8>(a, qb, grid, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st); break;
-  }
+  const int s = strict ? 1 : 0;
+  const int rc = dispatch_nj_qb(a.dim, scan_qb(a.dim, a.nq), "range scan", [&](auto nj, auto qbc) {
+    constexpr int NJ = decltype(nj)::value, QB = decltype(qbc)::value;
+    auto passes = [&](auto metric) {
+      constexpr int METRIC = decltype(metric)::value;
+      auto scan = [&](auto write) {
+        return launch_kernel(range_scan_kernel<NJ, QB, METRIC, decltype(write)::value>, dim3(grid),
+                             dim3(kScanWarps * 32), 0, st, a.master, a.tags, a.rows, a.qn, a.nq, flagged, n_flagged,
+                             a.tenant, threshold, s, max_hits, row_offset, cnt, off, out_rows, out_scores);
+      };
+      return launch_counting_passes(scan, grid, a.nq, flagged, n_flagged, max_hits,
+                                    METRIC == FRG_METRIC_COSINE ? kNoScore : INFINITY, cnt, off, out_counts, out_rows,
+                                    out_scores, st);
+    };
+    if (a.metric == FRG_METRIC_COSINE) return passes(std::integral_constant<int, FRG_METRIC_COSINE>());
+    return passes(std::integral_constant<int, FRG_METRIC_EUCLIDEAN>());
+  });
   cudaError_t e = cudaFreeAsync(ws, st);
-  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  if (rc == FRG_OK && e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
   return rc;
 }
 
@@ -838,7 +842,6 @@ join_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ t
                  const int* __restrict__ n_flagged, int32_t tenant, int same_tag, float threshold, int strict,
                  int max_hits, int64_t row_offset, int* __restrict__ cnt, const int* __restrict__ off,
                  int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
-  constexpr int DIM = NJ * 128;
   pdl_wait();
   pdl_trigger();
   const int n_slots = flagged ? *n_flagged : nq;
@@ -859,93 +862,19 @@ join_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ t
     const int hi = __reduce_max_sync(0xffffffffu, live ? __ldg(tile_end + q / 128) : 0);
     const int64_t span = hi > lo ? int64_t(hi - lo) : 0;
     const int64_t r0 = lo + span * gw / nw, r1 = lo + span * (gw + 1) / nw;
-    int pos = 0, room = 0;
-    if (WRITE) {
-      if (my_b < nb && cnt[size_t(slot) * nw + gw] > 0) {
-        pos = off[size_t(slot) * nw + gw];
-        room = max_hits;
-      }
-      if (!__any_sync(0xffffffffu, pos < room)) continue;
-    }
-    float4 qv[QB][NJ];
-#pragma unroll
-    for (int b = 0; b < QB; ++b) {
-      const int qb_ = flagged ? flagged[s0 + (b < nb ? b : 0)] : s0 + (b < nb ? b : 0);
-#pragma unroll
-      for (int j = 0; j < NJ; ++j) qv[b][j] = __ldg(reinterpret_cast<const float4*>(qn + size_t(qb_) * DIM) + j * 32 + lane);
-    }
-    int count = 0;
-    for (int64_t r = r0; r < r1; ++r) {
-      const int32_t tg = __ldg(tags + r);
-      float4 g[NJ];                                                     // issued together with the tag load
-      const float4* pr = reinterpret_cast<const float4*>(master + r * DIM) + lane;
-#pragma unroll
-      for (int j = 0; j < NJ; ++j) g[j] = ldg_stream(pr + j * 32);
-      if (tg < 0 || (tenant >= 0 && tg != tenant)) continue;           // warp-uniform
-      const bool mine = live && r > a && (!same_tag || tg == ta);
-      if (!__any_sync(0xffffffffu, mine)) continue;
-      float acc[QB];
-      row_dots<NJ, QB, FRG_METRIC_COSINE>(g, qv, acc);
-      const float sdot = butterfly<QB>(acc, lane);
-      const bool hit = mine && range_pass<FRG_METRIC_COSINE>(sdot, threshold, strict);
-      if (WRITE) {
-        if (hit && pos < room) {
-          if (rep) {
-            out_rows[size_t(q) * max_hits + pos] = r + row_offset;
-            out_scores[size_t(q) * max_hits + pos] = sdot;
-          }
-          ++pos;
-        }
-        if (!__any_sync(0xffffffffu, pos < room)) break;
-      } else {
-        count += hit ? 1 : 0;
-      }
-    }
-    if (!WRITE && rep && my_b < nb) cnt[size_t(slot) * nw + gw] = count;
+    // row b counts for a live a when b > a and, with same_tag, tag[b] == tag[a]; a row no lane wants is skipped
+    auto rule = [&](int64_t r, int32_t tg, bool& mine) {
+      mine = live && r > a && (!same_tag || tg == ta);
+      return __any_sync(0xffffffffu, mine);
+    };
+    range_strip<NJ, QB, FRG_METRIC_COSINE, WRITE>(master, tags, qn, flagged, s0, nb, slot, q, r0, r1, nw, gw, lane,
+                                                  my_b, rep, tenant, threshold, strict, max_hits, row_offset, cnt, off,
+                                                  out_rows, out_scores, rule);
   }
 }
 
 size_t join_scan_workspace_bytes(const ScanArgs& a) {
   return size_t(scan_grid(a)) * kScanWarps * size_t(a.nq > 0 ? a.nq : 1) * 2 * sizeof(int);
-}
-
-template <int NJ, int QB>
-static int launch_join_passes(const ScanArgs& a, int grid, int64_t qrow0, const int32_t* tile_end, bool same_tag,
-                              const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
-                              int64_t row_offset, int* cnt, int* off, int64_t* out_counts, int64_t* out_rows,
-                              float* out_scores, cudaStream_t st) {
-  const int nw = grid * kScanWarps;
-  const int s = strict ? 1 : 0, t = same_tag ? 1 : 0;
-  FRG_CUDA(launch_kernel(join_scan_kernel<NJ, QB, false>, dim3(grid), dim3(kScanWarps * 32), 0, st, a.master, a.tags,
-                         a.qn, a.nq, qrow0, tile_end, flagged, n_flagged, a.tenant, t, threshold, s, max_hits,
-                         row_offset, cnt, const_cast<const int*>(off), out_rows, out_scores));
-  note_launch(nullptr);
-  FRG_CUDA(launch_kernel(range_offsets_kernel, dim3(a.nq), dim3(256), 0, st, a.nq, flagged, n_flagged, nw,
-                         const_cast<const int*>(cnt), off, max_hits, kNoScore, out_counts, out_rows, out_scores));
-  note_launch(nullptr);
-  FRG_CUDA(launch_kernel(join_scan_kernel<NJ, QB, true>, dim3(grid), dim3(kScanWarps * 32), 0, st, a.master, a.tags,
-                         a.qn, a.nq, qrow0, tile_end, flagged, n_flagged, a.tenant, t, threshold, s, max_hits,
-                         row_offset, cnt, const_cast<const int*>(off), out_rows, out_scores));
-  note_launch(nullptr);
-  FRG_CUDA(cudaGetLastError());
-  return FRG_OK;
-}
-
-template <int NJ>
-static int launch_join_qb(const ScanArgs& a, int qb, int grid, int64_t qrow0, const int32_t* tile_end, bool same_tag,
-                          const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
-                          int64_t row_offset, int* cnt, int* off, int64_t* out_counts, int64_t* out_rows,
-                          float* out_scores, cudaStream_t st) {
-#define FRG_JOIN_QB(QB) return launch_join_passes<NJ, QB>(a, grid, qrow0, tile_end, same_tag, flagged, n_flagged,     \
-                                                         max_hits, threshold, strict, row_offset, cnt, off, out_counts, \
-                                                         out_rows, out_scores, st)
-  if (qb == 1) { FRG_JOIN_QB(1); }
-  if (qb == 2) { FRG_JOIN_QB(2); }
-  if constexpr (NJ <= 4) { if (qb == 4) { FRG_JOIN_QB(4); } }
-  if constexpr (NJ <= 2) { if (qb == 8) { FRG_JOIN_QB(8); } }
-#undef FRG_JOIN_QB
-  set_error("join scan: unsupported queries-per-pass %d for dim %d", qb, NJ * 128);
-  return FRG_ERR_UNSUPPORTED;
 }
 
 int launch_join_scan(const ScanArgs& a, int64_t qrow0, const int32_t* tile_end, bool same_tag, const int* flagged,
@@ -957,13 +886,17 @@ int launch_join_scan(const ScanArgs& a, int64_t qrow0, const int32_t* tile_end, 
   const int grid = scan_grid(a);
   int* cnt = static_cast<int*>(ws);
   int* off = cnt + size_t(grid) * kScanWarps * a.nq;
-  const int qb = scan_qb(a.dim, a.nq);
-  switch (a.dim) {
-    case 128: return launch_join_qb<1>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
-    case 256: return launch_join_qb<2>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
-    case 512: return launch_join_qb<4>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
-    default:  return launch_join_qb<8>(a, qb, grid, qrow0, tile_end, same_tag, flagged, n_flagged, max_hits, threshold, strict, row_offset, cnt, off, out_counts, out_rows, out_scores, st);
-  }
+  const int s = strict ? 1 : 0, t = same_tag ? 1 : 0;
+  return dispatch_nj_qb(a.dim, scan_qb(a.dim, a.nq), "join scan", [&](auto nj, auto qbc) {
+    constexpr int NJ = decltype(nj)::value, QB = decltype(qbc)::value;
+    auto scan = [&](auto write) {
+      return launch_kernel(join_scan_kernel<NJ, QB, decltype(write)::value>, dim3(grid), dim3(kScanWarps * 32), 0, st,
+                           a.master, a.tags, a.qn, a.nq, qrow0, tile_end, flagged, n_flagged, a.tenant, t, threshold,
+                           s, max_hits, row_offset, cnt, off, out_rows, out_scores);
+    };
+    return launch_counting_passes(scan, grid, a.nq, flagged, n_flagged, max_hits, kNoScore, cnt, off, out_counts,
+                                  out_rows, out_scores, st);
+  });
 }
 
 }  // namespace frg

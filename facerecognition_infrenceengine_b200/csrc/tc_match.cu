@@ -42,6 +42,8 @@
 
 #include <cmath>
 #include <cstring>
+#include <type_traits>
+#include <utility>
 
 #include "frg_internal.cuh"
 
@@ -1301,15 +1303,14 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   int seg = (2 * stage_entries + nseg - 1) / nseg;
   if (seg < 12) seg = 12;
   pl->seg = seg;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-  pl->off_keys = take(size_t(nq) * kGroups * (i8 ? 8 : 4));
-  pl->off_cnt = take(size_t(nq) * 4);
-  pl->off_cand = take(size_t(nq) * nseg * seg * 8);
-  pl->off_dense = take(size_t(nq) * stage_entries * 8);
-  pl->off_flag = take(size_t(nq) * 4 + 12);    // flagged[nq], count, ticket, probe-arrival counter
-  pl->off_floor = take(i8 ? size_t(nq) * 4 : 0);
-  pl->total = off;
+  Carve c;
+  pl->off_keys = c.take(size_t(nq) * kGroups * (i8 ? 8 : 4));
+  pl->off_cnt = c.take(size_t(nq) * 4);
+  pl->off_cand = c.take(size_t(nq) * nseg * seg * 8);
+  pl->off_dense = c.take(size_t(nq) * stage_entries * 8);
+  pl->off_flag = c.take(size_t(nq) * 4 + 12);    // flagged[nq], count, ticket, probe-arrival counter
+  pl->off_floor = c.take(i8 ? size_t(nq) * 4 : 0);
+  pl->total = c.off;
 }
 
 template <int MODE, bool MASKED, bool PAIR, bool I8, bool GROUPED = false>
@@ -1361,20 +1362,89 @@ int64_t tc_effective_rows(const GalleryWindow* s, int nq, cudaStream_t st, const
   return int64_t(n) * gran;
 }
 
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool range, bool i8) {
+size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool i8) {
   TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl, range, i8);
+  tc_plan(rows, dim, nq, k, sm_count, &pl, false, i8);
   return pl.total;
 }
 
 // the pieces of the workspace the query-prep kernel initialises (group keys := "nothing seen", counters := 0)
 void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               void** keys, int** cand_total, int** n_flagged, bool range, bool i8) {
+                               void** keys, int** cand_total, int** n_flagged, bool i8) {
   TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl, range, i8);
+  tc_plan(rows, dim, nq, k, sm_count, &pl, false, i8);
   *keys = ws + pl.off_keys;
   *cand_total = reinterpret_cast<int*>(ws + pl.off_cnt);
   *n_flagged = reinterpret_cast<int*>(ws + pl.off_flag) + nq;
+}
+
+int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count) {
+  TcPlan pl;
+  tc_plan(plan_rows, dim, nq, 1, sm_count, &pl, true, true);
+  return int64_t(nq) * pl.chunks_main * (kEpiWarps / 4) * pl.seg;
+}
+
+size_t tc_range_workspace(int nq, int64_t cand_entries, unsigned char* ws, TcRangeWs* out) {
+  Carve c;
+  const size_t o_keys = c.take(size_t(nq) * kGroups * 8), o_cnt = c.take(size_t(nq) * 4);
+  const size_t o_flag = c.take(size_t(nq) * 4 + 12);     // flagged[nq], count, ticket, probe-arrival counter
+  const size_t o_floor = c.take(size_t(nq) * 4), o_dense = c.take(size_t(nq) * kRangeBudget * 8);
+  const size_t o_cand = c.take(size_t(cand_entries) * 8);
+  if (ws) {
+    out->keys = reinterpret_cast<unsigned long long*>(ws + o_keys);
+    out->cand_total = reinterpret_cast<int*>(ws + o_cnt);
+    out->flagged = reinterpret_cast<int*>(ws + o_flag);
+    out->n_flagged = out->flagged + nq;
+    out->floor = reinterpret_cast<float*>(ws + o_floor);
+    out->dense = reinterpret_cast<int2*>(ws + o_dense);
+    out->cand = reinterpret_cast<int2*>(ws + o_cand);
+  }
+  return c.off;
+}
+
+// The two TMA maps of an int8 filter call: the int8 query image [nq][dim] and the store's int8 plane.
+static int make_i8_maps(const GalleryWindow* s, const int8_t* qi8, int nq, CUtensorMap* qm, CUtensorMap* gm) {
+  FRG_CHECK(make_map(qm, qi8, s->dim, nq, size_t(s->dim), kTileQ, kBlockK, true));
+  return make_map(gm, s->plane8, s->dim, s->rows, size_t(s->dim), kTileR, kBlockK, true);
+}
+
+// The filter parameters every call over the window s sets alike (cosine: no pad block; query tile of dim columns).
+// The caller adds its tenant, k, tile source, group keys and tile_scale.
+static TcScanParams filter_params(const GalleryWindow* s, int dim, int nq, const float* eps, const float* qstep,
+                                  float* floor_v, int2* cand, int* cand_total, int2* dense, int dense_cap) {
+  TcScanParams p{};
+  p.fault = s->fault;
+  p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
+  p.dim = dim; p.nq = nq; p.tags = s->tags; p.n_rows = int(s->rows);
+  p.qstep = qstep; p.floor = floor_v;
+  p.cand = cand; p.cand_total = cand_total; p.dense = dense; p.dense_cap = dense_cap;
+  return p;
+}
+
+// select + exact rescoring (select_rescore_kernel<kreg, euclid>): one CTA per query
+static cudaError_t launch_select_rescore(int kreg, bool euclid, int nq, cudaStream_t st, const int2* dense,
+                                         const int* cand_total, int dense_cap, int k, int dim, const float* qn,
+                                         const float* eps, const __nv_bfloat16* plane, int plane_dim,
+                                         const float* coef, const float* qstep, const float* master, int rescore,
+                                         float threshold, int64_t row_offset, int64_t* out_rows, float* out_scores,
+                                         uint8_t* out_accept, int* flagged, int* n_flagged, const XPush& push) {
+  auto launch = [&](auto kern) {
+    cudaError_t e = func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(kern, dim3(nq), dim3(kSelectWarps * 32), 0, st, dense, cand_total, dense_cap, nq, k, dim, qn,
+                         eps, plane, plane_dim, coef, qstep, master, rescore, threshold, row_offset, out_rows,
+                         out_scores, out_accept, flagged, n_flagged, push);
+  };
+  auto by_k = [&](auto eu) {
+    constexpr bool EU = decltype(eu)::value;
+    switch (kreg) {
+      case 1: return launch(select_rescore_kernel<1, EU>);
+      case 4: return launch(select_rescore_kernel<4, EU>);
+      case 8: return launch(select_rescore_kernel<8, EU>);
+      default: return launch(select_rescore_kernel<16, EU>);
+    }
+  };
+  return euclid ? by_k(std::true_type()) : by_k(std::false_type());
 }
 
 // qn / qb: normalised fp32 queries and their bf16 image [nq][dim]; ws: tc_workspace_bytes() of scratch.
@@ -1410,29 +1480,27 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   const bool masked = tenant >= 0 || s->maybe_dead;
 
   CUtensorMap qm, qm_pre, gm_full, pm;
-  if (i8) FRG_CHECK(make_map(&qm, qi8, kdim, nq, size_t(kdim), kTileQ, kBlockK, true));
-  else FRG_CHECK(make_map(&qm, qb, kdim, nq, size_t(kdim) * 2, kTileQ));
+  if (i8) {
+    FRG_CHECK(make_i8_maps(s, qi8, nq, &qm, &gm_full));
+  } else {
+    FRG_CHECK(make_map(&qm, qb, kdim, nq, size_t(kdim) * 2, kTileQ));
+    FRG_CHECK(make_map(&gm_full, s->plane, s->dim, s->rows, pitch, kTileR));   // box = one CTA's half
+  }
   if (euclid) FRG_CHECK(make_map(&qm_pre, qb_prepass, kdim, nq, size_t(kdim) * 2, kTileQ));   // lower-bound image
   else qm_pre = qm;
-  if (i8) FRG_CHECK(make_map(&gm_full, s->plane8, s->dim, s->rows, pitch, kTileR, kBlockK, true));
-  else FRG_CHECK(make_map(&gm_full, s->plane, s->dim, s->rows, pitch, kTileR));   // box = one CTA's half
   if (euclid) FRG_CHECK(make_map(&pm, s->plane + s->dim, kEuclidPad, s->rows, pitch, kTileR, kEuclidPad));
   else pm = gm_full;                                                          // never dereferenced (p.pad == 0)
 
-  TcScanParams p{};
-  p.fault = s->fault;
+  TcScanParams p = filter_params(s, kdim, nq, eps, i8 ? qstep : nullptr,
+                                 i8 ? reinterpret_cast<float*>(ws + pl.off_floor) : nullptr, cand, cnt, dense,
+                                 pl.stage_entries);
+  if (euclid) { p.none_score = kEuclidNone; p.pad = 1; }
   p.tile_list = tile_list; p.n_list = n_list;
-  p.eps = eps; p.none_score = euclid ? kEuclidNone : kNoScore; p.pad = euclid ? 1 : 0;
-  p.stages = kStages;
-  p.dim = kdim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
-  p.n_rows = int(s->rows); p.group_key = keys; p.k = k;
-  p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
+  p.tenant = tenant; p.group_key = keys; p.k = k; p.seg = pl.seg;
   int rc;
   if (i8) {
     // 1. int8 pre-pass over the sampled tiles: (s32 product, row) of every row group's best sampled row
     p.group_key64 = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
-    p.floor = reinterpret_cast<float*>(ws + pl.off_floor);
-    p.qstep = qstep;
     p.tile_scale = pl.stride;
     profile_begin(st, kStagePrepass);
     FRG_CHECK((launch_tc_scan_m<kModeGroupMax, true>(masked, pl.pair, qm, gm_full, gm_full, p, pl.qtiles, pl.chunks_pre, st)));
@@ -1479,25 +1547,9 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   }
   // 3. select + exact rescoring
   profile_begin(st, kStageSelect);
-  const int grid = nq;                                   // one CTA per query
-  const int rs = rescore ? 1 : 0;
-#define FRG_SELECT_M(KK, EU)                                                                                    \
-  FRG_CUDA(func_attr_once(select_rescore_kernel<KK, EU>, cudaFuncAttributePreferredSharedMemoryCarveout, 100)); \
-  FRG_CUDA(launch_kernel(select_rescore_kernel<KK, EU>, dim3(grid), dim3(kSelectWarps * 32), 0, st, dense, \
-      cnt, pl.stage_entries, nq, k, s->dim, qn, eps, s->plane, s->plane_dim, coef, i8 ? qstep : nullptr,         \
-      s->master, rs, threshold,                                                                                    \
-      row_offset, out_rows, out_scores,                                                                             \
-      out_accept, flagged, n_flagged, push))
-#define FRG_SELECT(KK)                                                                                          \
-  if (euclid) { FRG_SELECT_M(KK, true); } else { FRG_SELECT_M(KK, false); }
-  switch (pl.kreg) {
-    case 1: FRG_SELECT(1); break;
-    case 4: FRG_SELECT(4); break;
-    case 8: FRG_SELECT(8); break;
-    default: FRG_SELECT(16); break;
-  }
-#undef FRG_SELECT
-#undef FRG_SELECT_M
+  FRG_CUDA(launch_select_rescore(pl.kreg, euclid, nq, st, dense, cnt, pl.stage_entries, k, s->dim, qn, eps, s->plane,
+                                 s->plane_dim, coef, i8 ? qstep : nullptr, s->master, rescore ? 1 : 0, threshold,
+                                 row_offset, out_rows, out_scores, out_accept, flagged, n_flagged, push));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   profile_end(st, 1);
@@ -1515,6 +1567,51 @@ range_floor_kernel(const float* __restrict__ eps, float threshold, float* __rest
   pdl_trigger();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < nq) floor_out[i] = threshold - __ldg(eps + i);
+}
+
+// The exact fp32 score of one candidate row for a range-mode select: float4 dot with the same element -> lane mapping
+// and xor 16..1 reduction as the streaming scan, so the scores are bit-identical to launch_range_scan's.  Every lane
+// returns the full dot.
+__device__ __forceinline__ float rescore_dot(const float* row, const float4* qq, int nvec, int lane) {
+  const float4* g = reinterpret_cast<const float4*>(row);
+  float a = 0.f;
+#pragma unroll 4
+  for (int v = lane; v < nvec; v += 32) {
+    const float4 x = __ldg(g + v), y = __ldg(qq + v);
+    a = fmaf(x.x, y.x, a); a = fmaf(x.y, y.y, a); a = fmaf(x.z, y.z, a); a = fmaf(x.w, y.w, a);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+  return a;
+}
+
+// The m hits of query q, packed (row << 32 | score bits) in shared memory, in gallery order: padded to a power of two,
+// sorted (bitonic; rows are distinct, so ascending keys = gallery order), the first max_hits written, the rest of the
+// slots marked "none", and the count m.  The whole CTA calls it.
+__device__ __forceinline__ void write_hits(unsigned long long* hits, int m, int max_hits, int q, int64_t row_offset,
+                                           int64_t* out_counts, int64_t* out_rows, float* out_scores) {
+  int n2 = 1;
+  while (n2 < m) n2 <<= 1;
+  for (int i = m + threadIdx.x; i < n2; i += blockDim.x) hits[i] = ~0ull;
+  __syncthreads();
+  for (int kk = 2; kk <= n2; kk <<= 1) {
+    for (int j = kk >> 1; j > 0; j >>= 1) {
+      for (int i = threadIdx.x; i < n2; i += blockDim.x) {
+        const int ij = i ^ j;
+        if (ij > i) {
+          const unsigned long long x = hits[i], y = hits[ij];
+          if ((x > y) == ((i & kk) == 0)) { hits[i] = y; hits[ij] = x; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  for (int i = threadIdx.x; i < max_hits; i += blockDim.x) {
+    const bool filled = i < m;
+    out_rows[size_t(q) * max_hits + i] = filled ? int64_t(hits[i] >> 32) + row_offset : int64_t(kNoRow);
+    out_scores[size_t(q) * max_hits + i] = filled ? __uint_as_float(uint32_t(hits[i])) : kNoScore;
+  }
+  if (threadIdx.x == 0) out_counts[q] = m;
 }
 
 // ONE CTA (4 warps) per query over the dense candidate list of a range-mode filter: every candidate is rescored
@@ -1546,96 +1643,63 @@ range_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand
   const float4* qq = reinterpret_cast<const float4*>(qn + size_t(q) * dim);
   for (int c = w; c < total; c += kSelectWarps) {
     const int row = mine[c].x;
-    const float4* g = reinterpret_cast<const float4*>(master + size_t(row) * dim);
-    float a = 0.f;
-#pragma unroll 4
-    for (int v = lane; v < nvec; v += 32) {
-      const float4 x = __ldg(g + v), y = __ldg(qq + v);
-      a = fmaf(x.x, y.x, a); a = fmaf(x.y, y.y, a); a = fmaf(x.z, y.z, a); a = fmaf(x.w, y.w, a);
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    const float a = rescore_dot(master + size_t(row) * dim, qq, nvec, lane);
     const bool pass = strict ? (a > threshold) : (a >= threshold);      // false for NaN
     if (lane == 0 && pass) hits[atomicAdd(&s_m, 1)] = (uint64_t(uint32_t(row)) << 32) | __float_as_uint(a);
   }
   __syncthreads();
-  const int m = s_m;
-  int n2 = 1;
-  while (n2 < m) n2 <<= 1;
-  for (int i = m + threadIdx.x; i < n2; i += blockDim.x) hits[i] = ~0ull;
-  __syncthreads();
-  // rows are distinct: ascending keys = gallery order
-  for (int kk = 2; kk <= n2; kk <<= 1) {
-    for (int j = kk >> 1; j > 0; j >>= 1) {
-      for (int i = threadIdx.x; i < n2; i += blockDim.x) {
-        const int ij = i ^ j;
-        if (ij > i) {
-          const unsigned long long x = hits[i], y = hits[ij];
-          if ((x > y) == ((i & kk) == 0)) { hits[i] = y; hits[ij] = x; }
-        }
-      }
-      __syncthreads();
-    }
-  }
-  for (int i = threadIdx.x; i < max_hits; i += blockDim.x) {
-    const bool filled = i < m;
-    out_rows[size_t(q) * max_hits + i] = filled ? int64_t(hits[i] >> 32) + row_offset : int64_t(kNoRow);
-    out_scores[size_t(q) * max_hits + i] = filled ? __uint_as_float(uint32_t(hits[i])) : kNoScore;
-  }
-  if (threadIdx.x == 0) out_counts[q] = m;
+  write_hits(hits, s_m, max_hits, q, row_offset, out_counts, out_rows, out_scores);
 }
 
-int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
-                    int nq, int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset,
-                    unsigned char* ws, int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores,
-                    int** flagged_out, int** n_flagged_out, cudaStream_t st, int64_t plan_rows,
-                    const int32_t* tile_list, int n_list) {
-  if (!s->plane8) { set_error("tc_range: the store has no int8 scan plane"); return FRG_ERR_UNSUPPORTED; }
-  TcPlan pl;
-  tc_plan(plan_rows, s->dim, nq, 1, sm_count, &pl, true, true);
-  int* cnt = reinterpret_cast<int*>(ws + pl.off_cnt);
-  int2* cand = reinterpret_cast<int2*>(ws + pl.off_cand);
-  int2* dense = reinterpret_cast<int2*>(ws + pl.off_dense);
-  int* flagged = reinterpret_cast<int*>(ws + pl.off_flag);
-  int* n_flagged = flagged + nq;
-  *flagged_out = flagged;
-  *n_flagged_out = n_flagged;
-  const bool masked = tenant >= 0 || s->maybe_dead;
-
+// The range-mode int8 filter path of range search and of one self-join slab: floor threshold - eps[q]
+// (range_floor_kernel), filter(qm, gm, p) - the caller's filter grid over the common parameters with kRangeBudget dense
+// entries per query - and the caller's select kernel with its arguments (one CTA per query; the dense list's sort
+// buffer in shared memory).
+template <typename Filter, typename... KArgs, typename... Args>
+static int launch_range_family(const GalleryWindow* s, const int8_t* qi8, const float* qstep, const float* eps, int nq,
+                               float threshold, const TcRangeWs& w, cudaStream_t st, Filter filter,
+                               void (*select)(KArgs...), Args&&... select_args) {
   CUtensorMap qm, gm;
-  FRG_CHECK(make_map(&qm, qi8, s->dim, nq, size_t(s->dim), kTileQ, kBlockK, true));
-  FRG_CHECK(make_map(&gm, s->plane8, s->dim, s->rows, size_t(s->dim), kTileR, kBlockK, true));
-
-  TcScanParams p{};
-  p.fault = s->fault;
-  p.tile_list = tile_list; p.n_list = n_list;
-  p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
-  p.dim = s->dim; p.nq = nq; p.tenant = tenant; p.tags = s->tags;
-  p.n_rows = int(s->rows); p.k = 1;
-  p.floor = reinterpret_cast<float*>(ws + pl.off_floor); p.qstep = qstep;
-  p.seg = pl.seg; p.cand = cand; p.cand_total = cnt; p.dense = dense; p.dense_cap = pl.stage_entries;
-  p.tile_scale = 1;
+  FRG_CHECK(make_i8_maps(s, qi8, nq, &qm, &gm));
+  TcScanParams p = filter_params(s, s->dim, nq, eps, qstep, w.floor, w.cand, w.cand_total, w.dense, kRangeBudget);
+  p.k = 1; p.tile_scale = 1;
   profile_begin(st, kStageFloor);
-  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, eps, threshold,
-                         const_cast<float*>(p.floor), nq));
+  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, eps, threshold, w.floor, nq));
   note_launch(nullptr);
   profile_end(st, 1);
-  profile_begin(st, kStageDominant);
-  FRG_CHECK((launch_tc_scan_m<kModeFilter, true>(masked, pl.pair, qm, gm, gm, p, pl.qtiles, pl.chunks_main, st)));
-  profile_end(st, 1);
+  FRG_CHECK(filter(qm, gm, p));
 
   profile_begin(st, kStageSelect);
   int n2 = 1;
-  while (n2 < pl.stage_entries) n2 <<= 1;
+  while (n2 < kRangeBudget) n2 <<= 1;
   const size_t smem = size_t(n2) * sizeof(unsigned long long);
-  FRG_CUDA(func_attr_once(range_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  FRG_CUDA(launch_kernel(range_select_kernel, dim3(nq), dim3(kSelectWarps * 32), smem, st, dense, cnt,
-                         pl.stage_entries, s->dim, qn, s->master, threshold, strict ? 1 : 0, max_hits, row_offset,
-                         out_counts, out_rows, out_scores, flagged, n_flagged));
+  FRG_CUDA(func_attr_once(select, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  FRG_CUDA(launch_kernel(select, dim3(nq), dim3(kSelectWarps * 32), smem, st, std::forward<Args>(select_args)...));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   profile_end(st, 1);
   return FRG_OK;
+}
+
+int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
+                    int nq, int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset,
+                    const TcRangeWs& w, int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                    cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list) {
+  if (!s->plane8) { set_error("tc_range: the store has no int8 scan plane"); return FRG_ERR_UNSUPPORTED; }
+  TcPlan pl;
+  tc_plan(plan_rows, s->dim, nq, 1, sm_count, &pl, true, true);
+  const bool masked = tenant >= 0 || s->maybe_dead;
+  // the ungrouped grid, in the pair form from two query tiles on
+  auto filter = [&](const CUtensorMap& qm, const CUtensorMap& gm, TcScanParams& p) {
+    p.tenant = tenant; p.tile_list = tile_list; p.n_list = n_list; p.seg = pl.seg;
+    profile_begin(st, kStageDominant);
+    FRG_CHECK((launch_tc_scan_m<kModeFilter, true>(masked, pl.pair, qm, gm, gm, p, pl.qtiles, pl.chunks_main, st)));
+    profile_end(st, 1);
+    return FRG_OK;
+  };
+  return launch_range_family(s, qi8, qstep, eps, nq, threshold, w, st, filter, range_select_kernel, w.dense,
+                             w.cand_total, kRangeBudget, s->dim, qn, s->master, threshold, strict ? 1 : 0, max_hits,
+                             row_offset, out_counts, out_rows, out_scores, w.flagged, w.n_flagged);
 }
 
 // ------------------------------------------------------------------------------------------ per-query tenants
@@ -1764,14 +1828,13 @@ int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::v
   const int64_t cand_entries = plan_group_ctas(units, sm_count, &pre, &main);
   if (dense_cap < 256) dense_cap = 256;
   // ---- workspace (one stream-ordered allocation)
-  size_t off = 0;
-  auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~size_t(255); return o; };
-  const size_t o_qs = take(size_t(nq) * dim * 4), o_qn = take(size_t(nq) * dim * 4), o_qi8 = take(size_t(nq) * dim);
-  const size_t o_eps = take(size_t(nq) * 4), o_step = take(size_t(nq) * 4), o_keys = take(size_t(nq) * kGroups * 8);
-  const size_t o_cnt = take(size_t(nq) * 4), o_flag = take(size_t(nq) * 4 + 12), o_floor = take(size_t(nq) * 4);
-  const size_t o_cand = take(size_t(cand_entries > 0 ? cand_entries : 1) * 8);
-  const size_t o_dense = take(size_t(nq) * dense_cap * 8);
-  const size_t o_rows = take(size_t(nq) * k * 8), o_sc = take(size_t(nq) * k * 4), o_acc = take(size_t(nq));
+  Carve c;
+  const size_t o_qs = c.take(size_t(nq) * dim * 4), o_qn = c.take(size_t(nq) * dim * 4), o_qi8 = c.take(size_t(nq) * dim);
+  const size_t o_eps = c.take(size_t(nq) * 4), o_step = c.take(size_t(nq) * 4), o_keys = c.take(size_t(nq) * kGroups * 8);
+  const size_t o_cnt = c.take(size_t(nq) * 4), o_flag = c.take(size_t(nq) * 4 + 12), o_floor = c.take(size_t(nq) * 4);
+  const size_t o_cand = c.take(size_t(cand_entries > 0 ? cand_entries : 1) * 8);
+  const size_t o_dense = c.take(size_t(nq) * dense_cap * 8);
+  const size_t o_rows = c.take(size_t(nq) * k * 8), o_sc = c.take(size_t(nq) * k * 4), o_acc = c.take(size_t(nq));
   // the only host -> device copy of the call: [perm][tenant of each sorted query][pre-pass CTAs][filter CTAs]
   std::vector<unsigned char> table;
   const size_t t_perm = 0, t_ten = size_t(nq) * 4, t_pre = (t_ten + size_t(nq) * 4 + 15) & ~size_t(15);
@@ -1782,9 +1845,9 @@ int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::v
     for (int i = 0; i < G.nq; ++i) memcpy(table.data() + t_ten + size_t(G.q0 + i) * 4, &G.tenant, 4);
   if (!pre.empty()) memcpy(table.data() + t_pre, pre.data(), pre.size() * sizeof(TcGroupCta));
   if (!main.empty()) memcpy(table.data() + t_main, main.data(), main.size() * sizeof(TcGroupCta));
-  const size_t o_table = take(table.size());
+  const size_t o_table = c.take(table.size());
   unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), off, st));
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
   float* qs = reinterpret_cast<float*>(ws + o_qs);
   float* qn = reinterpret_cast<float*>(ws + o_qn);
   int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
@@ -1807,14 +1870,10 @@ int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::v
     rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, keys, cnt, n_flagged, st);
   profile_end(st, 1);
   CUtensorMap qm, gm;
-  if (rc == FRG_OK) rc = make_map(&qm, qi8, dim, nq, size_t(dim), kTileQ, kBlockK, true);
-  if (rc == FRG_OK) rc = make_map(&gm, s->plane8, dim, s->rows, size_t(dim), kTileR, kBlockK, true);
-  TcScanParams p{};
-  p.fault = s->fault; p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
-  p.dim = dim; p.nq = nq; p.tenant = -1; p.tags = s->tags; p.n_rows = int(s->rows); p.k = k; p.tile_scale = 1;
-  p.group_key64 = keys; p.floor = floor_v; p.qstep = qstep;
-  p.cand = reinterpret_cast<int2*>(ws + o_cand); p.cand_total = cnt;
-  p.dense = reinterpret_cast<int2*>(ws + o_dense); p.dense_cap = dense_cap;
+  if (rc == FRG_OK) rc = make_i8_maps(s, qi8, nq, &qm, &gm);
+  TcScanParams p = filter_params(s, dim, nq, eps, qstep, floor_v, reinterpret_cast<int2*>(ws + o_cand), cnt,
+                                 reinterpret_cast<int2*>(ws + o_dense), dense_cap);
+  p.tenant = -1; p.k = k; p.tile_scale = 1; p.group_key64 = keys;
   // 1. int8 pre-pass, 2. exact floor, 3. filter: every (query tile, chunk) of every tenant in one grid each
   profile_begin(st, kStagePrepass);
   if (rc == FRG_OK && !pre.empty()) {
@@ -1839,23 +1898,9 @@ int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::v
   // 4. select + exact rescoring into the sorted scratch (the tenant filter was applied by the filter's tag check)
   profile_begin(st, kStageSelect);
   if (rc == FRG_OK) {
-    cudaError_t e = cudaSuccess;
-#define FRG_SELECT_G(KK)                                                                                          \
-  e = func_attr_once(select_rescore_kernel<KK, false>, cudaFuncAttributePreferredSharedMemoryCarveout, 100);       \
-  if (e == cudaSuccess)                                                                                          \
-    e = launch_kernel(select_rescore_kernel<KK, false>, dim3(nq), dim3(kSelectWarps * 32), 0, st,               \
-                      const_cast<const int2*>(p.dense), const_cast<const int*>(cnt), dense_cap, nq, k, dim,       \
-                      const_cast<const float*>(qn), const_cast<const float*>(eps),                              \
-                      static_cast<const __nv_bfloat16*>(nullptr), dim, static_cast<const float*>(nullptr),        \
-                      const_cast<const float*>(qstep), s->master, 1, threshold, row_offset, srows, sscores, sacc,  \
-                      flagged, n_flagged, XPush())
-    switch (reg_k(k)) {
-      case 1: FRG_SELECT_G(1); break;
-      case 4: FRG_SELECT_G(4); break;
-      case 8: FRG_SELECT_G(8); break;
-      default: FRG_SELECT_G(16); break;
-    }
-#undef FRG_SELECT_G
+    const cudaError_t e = launch_select_rescore(reg_k(k), false, nq, st, p.dense, cnt, dense_cap, k, dim, qn, eps,
+                                                nullptr, dim, nullptr, qstep, s->master, 1, threshold, row_offset,
+                                                srows, sscores, sacc, flagged, n_flagged, XPush());
     if (e != cudaSuccess) rc = cuda_fail(e, "select_rescore_kernel", __FILE__, __LINE__);
     else note_launch(nullptr);
   }
@@ -1910,43 +1955,12 @@ join_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand_
   for (int c = w; c < total; c += kSelectWarps) {
     const int row = mine[c].x;
     if (row <= a || (same_tag && __ldg(tags + row) != ta)) continue;     // warp-uniform
-    const float4* g = reinterpret_cast<const float4*>(master + size_t(row) * dim);
-    float acc = 0.f;
-#pragma unroll 4
-    for (int v = lane; v < nvec; v += 32) {
-      const float4 x = __ldg(g + v), y = __ldg(qq + v);
-      acc = fmaf(x.x, y.x, acc); acc = fmaf(x.y, y.y, acc); acc = fmaf(x.z, y.z, acc); acc = fmaf(x.w, y.w, acc);
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    const float acc = rescore_dot(master + size_t(row) * dim, qq, nvec, lane);
     const bool pass = strict ? (acc > threshold) : (acc >= threshold);      // false for NaN
     if (lane == 0 && pass) hits[atomicAdd(&s_m, 1)] = (uint64_t(uint32_t(row)) << 32) | __float_as_uint(acc);
   }
   __syncthreads();
-  const int m = s_m;
-  int n2 = 1;
-  while (n2 < m) n2 <<= 1;
-  for (int i = m + threadIdx.x; i < n2; i += blockDim.x) hits[i] = ~0ull;
-  __syncthreads();
-  // rows are distinct: ascending keys = gallery order
-  for (int kk = 2; kk <= n2; kk <<= 1) {
-    for (int j = kk >> 1; j > 0; j >>= 1) {
-      for (int i = threadIdx.x; i < n2; i += blockDim.x) {
-        const int ij = i ^ j;
-        if (ij > i) {
-          const unsigned long long x = hits[i], y = hits[ij];
-          if ((x > y) == ((i & kk) == 0)) { hits[i] = y; hits[ij] = x; }
-        }
-      }
-      __syncthreads();
-    }
-  }
-  for (int i = threadIdx.x; i < max_hits; i += blockDim.x) {
-    const bool filled = i < m;
-    out_rows[size_t(q) * max_hits + i] = filled ? int64_t(hits[i] >> 32) + row_offset : int64_t(kNoRow);
-    out_scores[size_t(q) * max_hits + i] = filled ? __uint_as_float(uint32_t(hits[i])) : kNoScore;
-  }
-  if (threadIdx.x == 0) out_counts[q] = m;
+  write_hits(hits, s_m, max_hits, q, row_offset, out_counts, out_rows, out_scores);
 }
 
 void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::vector<unsigned char>* table,
@@ -1962,42 +1976,24 @@ void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::ve
 
 int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
                    int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
-                   float threshold, bool strict, int max_hits, int64_t row_offset, int2* cand, int* cand_total,
-                   int2* dense, float* floor_v, int* flagged, int* n_flagged, int64_t* out_counts, int64_t* out_rows,
-                   float* out_scores, cudaStream_t st) {
+                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcRangeWs& w,
+                   int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
   if (!s->plane8 || !s->master || s->row0 != 0 || s->rows > 0x7fffffff) {
     set_error("tc_join: needs the whole unit store with an int8 plane and an fp32 master");
     return FRG_ERR_UNSUPPORTED;
   }
-  CUtensorMap qm, gm;
-  FRG_CHECK(make_map(&qm, qi8, s->dim, nq, size_t(s->dim), kTileQ, kBlockK, true));
-  FRG_CHECK(make_map(&gm, s->plane8, s->dim, s->rows, size_t(s->dim), kTileR, kBlockK, true));
-  TcScanParams p{};
-  p.fault = s->fault; p.eps = eps; p.none_score = kNoScore; p.pad = 0; p.stages = kStages;
-  p.dim = s->dim; p.nq = nq; p.tenant = -1; p.tags = s->tags; p.n_rows = int(s->rows); p.k = 1; p.tile_scale = 1;
-  p.floor = floor_v; p.qstep = qstep;
-  p.cand = cand; p.cand_total = cand_total; p.dense = dense; p.dense_cap = kRangeBudget;
-  p.groups = static_cast<const TcGroupCta*>(d_table);
-  profile_begin(st, kStageFloor);
-  FRG_CUDA(launch_kernel(range_floor_kernel, dim3((nq + 255) / 256), dim3(256), 0, st, eps, threshold, floor_v, nq));
-  note_launch(nullptr);
-  profile_end(st, 1);
-  profile_begin(st, kStageDominant);
-  if (n_ctas > 0) FRG_CHECK((launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, n_ctas, 1, st)));
-  profile_end(st, n_ctas > 0 ? 1 : 0);
-  profile_begin(st, kStageSelect);
-  int n2 = 1;
-  while (n2 < kRangeBudget) n2 <<= 1;
-  const size_t smem = size_t(n2) * sizeof(unsigned long long);
-  FRG_CUDA(func_attr_once(join_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  FRG_CUDA(launch_kernel(join_select_kernel, dim3(nq), dim3(kSelectWarps * 32), smem, st,
-                         const_cast<const int2*>(dense), const_cast<const int*>(cand_total), kRangeBudget, s->dim, qn,
-                         s->master, s->tags, qrow0, tenant, same_tag ? 1 : 0, threshold, strict ? 1 : 0, max_hits,
-                         row_offset, out_counts, out_rows, out_scores, flagged, n_flagged));
-  note_launch(nullptr);
-  FRG_CUDA(cudaGetLastError());
-  profile_end(st, 1);
-  return FRG_OK;
+  // the GROUPED single-CTA grid over the uploaded descriptors
+  auto filter = [&](const CUtensorMap& qm, const CUtensorMap& gm, TcScanParams& p) {
+    p.tenant = -1; p.groups = static_cast<const TcGroupCta*>(d_table);
+    profile_begin(st, kStageDominant);
+    if (n_ctas > 0) FRG_CHECK((launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, n_ctas, 1, st)));
+    profile_end(st, n_ctas > 0 ? 1 : 0);
+    return FRG_OK;
+  };
+  return launch_range_family(s, qi8, qstep, eps, nq, threshold, w, st, filter, join_select_kernel, w.dense,
+                             w.cand_total, kRangeBudget, s->dim, qn, s->master, s->tags, qrow0, tenant,
+                             same_tag ? 1 : 0, threshold, strict ? 1 : 0, max_hits, row_offset, out_counts, out_rows,
+                             out_scores, w.flagged, w.n_flagged);
 }
 
 }  // namespace frg
