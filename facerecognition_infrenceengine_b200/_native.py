@@ -82,6 +82,9 @@ SIGNATURES = {
     "frg_first_match_host": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), _P, _P]),
     "frg_match_range": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
     "frg_match_range_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
+    "frg_match_range_tenants": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P, _P]),
+    "frg_match_range_tenants_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.POINTER(MatchParams), _P, _P, _P,
+                                               _P]),
     "frg_self_join": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
     "frg_self_join_host": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
     "frg_merge_topk": (C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,

@@ -1335,6 +1335,23 @@ static int range_results_host(frg_store* s, int64_t n, int32_t max_hits, size_t 
 }
 }  // extern "C++"
 
+// The checks of a range search after its argument check (frg_match_range, frg_match_range_tenants): the metric, TC_EXACT
+// with Euclidean, and check_range_call.  *use_tc: the tensor-core path (a unit cosine store with an int8 plane, a
+// covered dim and queries to normalise).
+static int check_range_search(const frg_store* s, const frg_match_params_t* p, int32_t max_hits, const char* what,
+                              bool* use_tc) {
+  if (p->metric != FRG_METRIC_COSINE && p->metric != FRG_METRIC_EUCLIDEAN) { set_error("%s: unknown metric %d", what, p->metric); return FRG_ERR_INVALID; }
+  if (p->variant == FRG_VARIANT_TC_EXACT && p->metric == FRG_METRIC_EUCLIDEAN) {
+    set_error("%s: the Euclidean range search runs on the exact scan only (FRG_VARIANT_SCAN_F32 / AUTO)", what);
+    return FRG_ERR_UNSUPPORTED;
+  }
+  const char* why = "";
+  const bool unit = !(s->flags & FRG_STORE_RAW) && !(p->flags & FRG_QUERY_PRENORMALISED);
+  const bool tc_ok = s->plane8 != nullptr && unit && p->metric == FRG_METRIC_COSINE && tc_supported(s->dim, p->metric, &why);
+  return check_range_call(s, p, max_hits, tc_ok,
+                          "a unit-row store with a scan plane, normalised queries and dim 128 / 256 / 512", what, use_tc);
+}
+
 static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
                       int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
   reset_launches();
@@ -1342,18 +1359,8 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
     set_error("match_range: bad argument");
     return FRG_ERR_INVALID;
   }
-  if (p->metric != FRG_METRIC_COSINE && p->metric != FRG_METRIC_EUCLIDEAN) { set_error("match_range: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
-  if (p->variant == FRG_VARIANT_TC_EXACT && p->metric == FRG_METRIC_EUCLIDEAN) {
-    set_error("match_range: the Euclidean range search runs on the exact scan only (FRG_VARIANT_SCAN_F32 / AUTO)");
-    return FRG_ERR_UNSUPPORTED;
-  }
-  const char* why = "";
-  const bool unit = !(s->flags & FRG_STORE_RAW) && !(p->flags & FRG_QUERY_PRENORMALISED);
-  const bool tc_ok = s->plane8 != nullptr && unit && p->metric == FRG_METRIC_COSINE && tc_supported(s->dim, p->metric, &why);
   bool use_tc = false;
-  FRG_CHECK(check_range_call(s, p, max_hits, tc_ok,
-                             "a unit-row store with a scan plane, normalised queries and dim 128 / 256 / 512",
-                             "match_range", &use_tc));
+  FRG_CHECK(check_range_search(s, p, max_hits, "match_range", &use_tc));
   if (nq == 0) return FRG_OK;
   DeviceGuard g(s->device);
   if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
@@ -1438,6 +1445,172 @@ int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32_t max_h
     const cudaError_t e = cudaMemcpyAsync(dq, q, qb, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) return cuda_fail(e, "H2D queries", __FILE__, __LINE__);
     return range_impl(s, reinterpret_cast<float*>(dq), nq, max_hits, p, dc, dr, ds, st);
+  });
+}
+
+// --------------------------------------------------------------------------------------------- range search, per-query tenants
+// The batch is sorted stably by tenant (perm[i] = caller position of sorted query i), and every tenant runs in one set
+// of launches: gather the queries in tenant order, then
+//   tensor-core path (where range_impl takes it): int8 query prep -> floor -> GROUPED filter over query tiles of at
+//     most 128 queries of one tenant, each scanning its tenant's tiles (tenant_tiles) -> range_select_kernel -> the
+//     per-query-tenant exact scan of the queries whose candidates overflowed;
+//   exact path: normalise -> that exact scan over every query, each reading its tenant's row window;
+// and scatter the sorted results into the caller's order.
+static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
+                              const int32_t* tenants, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                              cudaStream_t st) {
+  reset_launches();
+  if (!s || !p || nq < 0 || (nq > 0 && (!q || !out_counts || !out_rows || !out_scores || !tenants))) {
+    set_error("match_range_tenants: bad argument");
+    return FRG_ERR_INVALID;
+  }
+  auto norm = [&](int32_t i) { return tenants[i] < 0 ? int32_t(-1) : tenants[i]; };
+  std::vector<int32_t> perm(static_cast<size_t>(nq));
+  for (int32_t i = 0; i < nq; ++i) perm[size_t(i)] = i;
+  std::stable_sort(perm.begin(), perm.end(), [&](int32_t a, int32_t b) { return norm(a) < norm(b); });
+  if (nq > 0 && norm(perm.front()) == norm(perm.back())) {           // one tenant: exactly frg_match_range
+    frg_match_params_t pg = *p;
+    pg.tenant = norm(perm.front());
+    return range_impl(s, q, nq, max_hits, &pg, out_counts, out_rows, out_scores, st);
+  }
+  bool use_tc = false;
+  FRG_CHECK(check_range_search(s, p, max_hits, "match_range_tenants", &use_tc));
+  if (nq == 0) return FRG_OK;
+  if (s->rows > 0x7fffffff) { set_error("match_range_tenants: more than 2^31-1 rows in one shard"); return FRG_ERR_UNSUPPORTED; }
+  DeviceGuard g(s->device);
+  if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
+  DeviceInfo di;
+  FRG_CHECK(device_info(s->device, &di));
+  std::lock_guard<std::mutex> lk(s->mu);    // one snapshot of the store for every tenant of the call
+  FRG_CHECK(store_begin_read(s, st));
+  const int dim = s->dim;
+  const bool tc = use_tc && s->rows > 0;
+  // the one upload: [perm][tenant of each sorted query][window lo][window hi][filter descriptors]
+  const size_t t_ten = size_t(nq) * 4, t_lo = t_ten + size_t(nq) * 4, t_hi = t_lo + size_t(nq) * 4;
+  const size_t t_cta = (t_hi + size_t(nq) * 4 + 15) & ~size_t(15);
+  std::vector<unsigned char> table(t_cta);
+  memcpy(table.data(), perm.data(), size_t(nq) * 4);
+  std::vector<TcTenantGroup> units;          // the filter's query tiles
+  for (int32_t i = 0; i < nq;) {
+    const int32_t t = norm(perm[size_t(i)]);
+    int32_t j = i + 1;
+    while (j < nq && norm(perm[size_t(j)]) == t) ++j;
+    // the rows tenant t can sit in: window_of's bounding window (every row for t < 0 or unknown extents)
+    int64_t lo = 0, hi = s->rows;
+    if (t >= 0 && s->extents_known) {
+      auto it = s->extents.find(t);
+      lo = hi = 0;
+      if (it != s->extents.end()) { lo = it->second.lo; hi = it->second.hi < s->rows ? it->second.hi : s->rows; }
+      if (hi < lo) hi = lo;
+    }
+    const int32_t lo32 = int32_t(lo), hi32 = int32_t(hi);
+    for (int32_t x = i; x < j; ++x) {
+      memcpy(table.data() + t_ten + size_t(x) * 4, &t, 4);
+      memcpy(table.data() + t_lo + size_t(x) * 4, &lo32, 4);
+      memcpy(table.data() + t_hi + size_t(x) * 4, &hi32, 4);
+    }
+    if (tc) {
+      TcTenantGroup G{};
+      G.tenant = t;
+      FRG_CHECK(tenant_tiles(s, t, st, &G));
+      for (int32_t a = i; a < j; a += kTcTileRows) {
+        G.q0 = a; G.nq = j - a < kTcTileRows ? j - a : kTcTileRows;
+        units.push_back(G);
+      }
+    }
+    i = j;
+  }
+  int n_ctas = 0;
+  int64_t cand = 1;
+  if (tc) {
+    std::vector<unsigned char> cta_bytes;
+    tc_join_plan(units, di.sm_count, &cta_bytes, &n_ctas, &cand);
+    table.insert(table.end(), cta_bytes.begin(), cta_bytes.end());
+  }
+  // ---- workspace: sorted queries, the table, the sorted results and the tensor-core path's pieces
+  const size_t slots = size_t(nq) * size_t(max_hits);
+  Carve c;
+  const size_t o_qs = c.take(size_t(nq) * dim * 4), o_qn = c.take(size_t(nq) * dim * 4), o_table = c.take(table.size());
+  const size_t o_cnt = c.take(size_t(nq) * 8), o_rows = c.take(slots * 8), o_sc = c.take(slots * 4);
+  size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_tc = 0;
+  if (tc) {
+    o_qi8 = c.take(size_t(nq) * dim); o_eps = c.take(size_t(nq) * 4); o_step = c.take(size_t(nq) * 4);
+    o_tc = c.take(tc_range_workspace(nq, cand, nullptr, nullptr));
+  }
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  float* qs = reinterpret_cast<float*>(ws + o_qs);
+  float* qn = reinterpret_cast<float*>(ws + o_qn);
+  const int32_t* dperm = reinterpret_cast<const int32_t*>(ws + o_table);
+  const int32_t* dten = reinterpret_cast<const int32_t*>(ws + o_table + t_ten);
+  const int32_t* dlo = reinterpret_cast<const int32_t*>(ws + o_table + t_lo);
+  const int32_t* dhi = reinterpret_cast<const int32_t*>(ws + o_table + t_hi);
+  int64_t* scnt = reinterpret_cast<int64_t*>(ws + o_cnt);
+  int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
+  float* sscores = reinterpret_cast<float*>(ws + o_sc);
+  ScanArgs a;
+  a.master = s->master; a.tags = s->tags; a.rows = s->rows; a.dim = dim;
+  a.qn = qn; a.nq = nq; a.k = 1; a.metric = p->metric; a.tenant = -1; a.sm_count = di.sm_count;
+  const bool strict = (p->flags & FRG_FIRST_STRICT) != 0;
+  int rc = stage_upload(ws + o_table, table.data(), table.size(), st);
+  if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, dim, qs, st);
+  if (tc) {
+    int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
+    float* eps = reinterpret_cast<float*>(ws + o_eps);
+    float* qstep = reinterpret_cast<float*>(ws + o_step);
+    TcRangeWs tw;
+    tc_range_workspace(nq, cand, ws + o_tc, &tw);
+    profile_begin(st, kStagePrep);
+    if (rc == FRG_OK)
+      rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
+                                     tw.n_flagged, st);
+    profile_end(st, 1);
+    const GalleryWindow w = window_of(s, -1);
+    if (rc == FRG_OK)
+      rc = launch_tc_range_grouped(&w, qn, qi8, qstep, eps, nq, ws + o_table + t_cta, n_ctas, max_hits, p->threshold,
+                                   strict, p->row_offset, tw, scnt, srows, sscores, st);
+    profile_begin(st, kStageFallback);
+    if (rc == FRG_OK)
+      rc = launch_range_tenants_scan(a, dten, dlo, dhi, tw.flagged, tw.n_flagged, max_hits, p->threshold, strict,
+                                     p->row_offset, scnt, srows, sscores, st);
+    profile_end(st, 1);
+  } else {
+    if (rc == FRG_OK)
+      rc = launch_normalise_queries(qs, nq, dim, p->metric == FRG_METRIC_COSINE && !(p->flags & FRG_QUERY_PRENORMALISED),
+                                    qn, nullptr, nullptr, nullptr, nullptr, st);
+    profile_begin(st, kStageDominant);
+    if (rc == FRG_OK)
+      rc = launch_range_tenants_scan(a, dten, dlo, dhi, nullptr, nullptr, max_hits, p->threshold, strict,
+                                     p->row_offset, scnt, srows, sscores, st);
+    profile_end(st, 3);
+  }
+  if (rc == FRG_OK) rc = launch_scatter_range(scnt, srows, sscores, dperm, nq, max_hits, out_counts, out_rows, out_scores, st);
+  g_variant = tc ? "range_tc_grouped" : "range_scan_tenants";
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
+int frg_match_range_tenants(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
+                            const int32_t* tenants, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                            void* stream) {
+  return range_tenants_impl(s, q, nq, max_hits, p, tenants, out_counts, out_rows, out_scores,
+                            static_cast<cudaStream_t>(stream));
+}
+
+int frg_match_range_tenants_host(frg_store* s, const float* q, int32_t nq, int32_t max_hits,
+                                 const frg_match_params_t* p, const int32_t* tenants, int64_t* out_counts,
+                                 int64_t* out_rows, float* out_scores) {
+  if (!s || !p || nq <= 0 || !q || !out_counts || !out_rows || !out_scores || !tenants || max_hits < 1) {
+    // the device entry point names the argument (and takes nq = 0)
+    return range_tenants_impl(s, q, nq, max_hits, p, tenants, out_counts, out_rows, out_scores, nullptr);
+  }
+  const size_t qb = size_t(nq) * s->dim * sizeof(float);
+  return range_results_host(s, nq, max_hits, qb, out_counts, out_rows, out_scores,
+                            [&](unsigned char* dq, int64_t* dc, int64_t* dr, float* ds, cudaStream_t st) {
+    const cudaError_t e = cudaMemcpyAsync(dq, q, qb, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return cuda_fail(e, "H2D queries", __FILE__, __LINE__);
+    return range_tenants_impl(s, reinterpret_cast<float*>(dq), nq, max_hits, p, tenants, dc, dr, ds, st);
   });
 }
 

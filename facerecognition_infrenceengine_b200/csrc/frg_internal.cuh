@@ -423,6 +423,25 @@ int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagge
                       bool strict, int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
                       cudaStream_t st);
 
+// ---- range search with a tenant per query (frg_match_range_tenants): the batch is sorted by tenant; sorted query q
+// has its tenant q_tenant[q] (-1 = all) and its row window [q_lo[q], q_hi[q]) (device arrays; rows < 2^31).
+// scan_f32.cu: launch_range_scan's passes with that tenant and window per query.  a: the whole store, a.qn / a.nq the
+// sorted queries (unit for cosine), a.tenant ignored.  flagged == nullptr: every query; else the n_flagged[0] listed ones.
+int launch_range_tenants_scan(const ScanArgs& a, const int32_t* q_tenant, const int32_t* q_lo, const int32_t* q_hi,
+                              const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
+                              int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                              cudaStream_t st);
+// tc_match.cu: launch_tc_range's path with the GROUPED filter over the uploaded table (d_table, n_ctas from tc_join_plan
+// over the query tiles; none when 0): each descriptor's tenant masks the other tenants' rows.  Queries whose candidates
+// overflowed are left in (w.flagged, w.n_flagged) for launch_range_tenants_scan.  s: the whole store.
+int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
+                            const float* eps, int nq, const void* d_table, int n_ctas, int max_hits, float threshold,
+                            bool strict, int64_t row_offset, const TcRangeWs& w, int64_t* out_counts,
+                            int64_t* out_rows, float* out_scores, cudaStream_t st);
+// tc_match.cu: out[perm[i]] = sorted range result i ([nq] counts, [nq][max_hits] rows and scores)
+int launch_scatter_range(const int64_t* counts, const int64_t* rows, const float* scores, const int32_t* perm, int nq,
+                         int max_hits, int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st);
+
 // ---- gallery self-join (frg_self_join): the queries are the store's own rows qrow0 .. qrow0 + nq - 1 of one slab,
 // and a pair (a, b) counts only for b > a (plus the tag rule: tenant >= 0 -> both rows carry it; same_tag -> tag[b] ==
 // tag[a]).  Query tile u of the slab holds queries 128u .. 128u + 127.

@@ -829,6 +829,90 @@ int launch_range_scan(const ScanArgs& a, const int* flagged, const int* n_flagge
   return rc;
 }
 
+// ------------------------------------------------------------------------------------------ per-query tenants
+// range_scan_kernel with a tenant per query (frg_match_range_tenants): query q keeps the live rows of its row window
+// [q_lo[q], q_hi[q]) that carry q_tenant[q] (every live row of the window when negative).  The window holds every row
+// of that tenant; it is empty for a tag no row carries.  A pass of QB queries reads only [lowest lo, largest hi) of its
+// queries, split into contiguous strips in warp order as range_scan_kernel splits the whole gallery, so pass 2 finds the
+// same strips and the concatenation of the warps' hits is gallery order.  The queries are sorted by tenant, so most
+// passes read one company's rows.  The scores come from row_dots + butterfly: bit-identical to launch_range_scan's.
+template <int NJ, int QB, int METRIC, bool WRITE>
+__global__ void __launch_bounds__(kScanWarps * 32, 2)
+range_tenants_scan_kernel(const float* __restrict__ master, const int32_t* __restrict__ tags,
+                          const float* __restrict__ qn, int nq, const int32_t* __restrict__ q_tenant,
+                          const int32_t* __restrict__ q_lo, const int32_t* __restrict__ q_hi,
+                          const int* __restrict__ flagged, const int* __restrict__ n_flagged, float threshold,
+                          int strict, int max_hits, int64_t row_offset, int* __restrict__ cnt,
+                          const int* __restrict__ off, int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
+  pdl_wait();
+  pdl_trigger();
+  const int n_slots = flagged ? *n_flagged : nq;
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = int64_t(gridDim.x) * kScanWarps;
+  const int64_t gw = int64_t(blockIdx.x) * kScanWarps + (threadIdx.x >> 5);
+  const int my_b = lane_query<QB>(lane);
+  const bool rep = lane_is_rep<QB>(lane);
+  for (int s0 = 0; s0 < n_slots; s0 += QB) {
+    const int nb = n_slots - s0 < QB ? n_slots - s0 : QB;
+    const int slot = s0 + (my_b < nb ? my_b : 0);
+    const int q = flagged ? flagged[slot] : slot;
+    const int32_t tq = __ldg(q_tenant + q);
+    const int qlo = __ldg(q_lo + q), qhi = __ldg(q_hi + q);              // rows < 2^31 (frg_match_range_tenants)
+    const bool live = my_b < nb && qhi > qlo;
+    // rows of this pass: the union of its live queries' windows; none when every window is empty
+    const int lo = __reduce_min_sync(0xffffffffu, live ? qlo : 0x7fffffff);
+    const int hi = __reduce_max_sync(0xffffffffu, live ? qhi : 0);
+    const int64_t span = hi > lo ? int64_t(hi - lo) : 0;
+    const int64_t r0 = lo + span * gw / nw, r1 = lo + span * (gw + 1) / nw;
+    // row r counts for the lane's query when it lies in the query's window and carries its tenant; a row no lane
+    // wants is skipped
+    auto rule = [&](int64_t r, int32_t tg, bool& mine) {
+      mine = live && r >= qlo && r < qhi && (tq < 0 || tg == tq);
+      return __any_sync(0xffffffffu, mine);
+    };
+    range_strip<NJ, QB, METRIC, WRITE>(master, tags, qn, flagged, s0, nb, slot, q, r0, r1, nw, gw, lane, my_b, rep,
+                                       -1, threshold, strict, max_hits, row_offset, cnt, off, out_rows, out_scores,
+                                       rule);
+  }
+}
+
+int launch_range_tenants_scan(const ScanArgs& a, const int32_t* q_tenant, const int32_t* q_lo, const int32_t* q_hi,
+                              const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
+                              int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                              cudaStream_t st) {
+  const char* why = "";
+  if (!range_scan_supported(a.dim, &why)) { set_error("range tenants scan: %s", why); return FRG_ERR_UNSUPPORTED; }
+  if (a.nq <= 0) return FRG_OK;
+  if (flagged && a.rows <= 0) return FRG_OK;
+  // the grid of launch_range_scan over the whole store: a pass of unfiltered queries reads every row
+  const int grid = scan_grid(a);
+  const size_t n_cnt = size_t(grid) * kScanWarps * a.nq;
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_cnt * 2 * sizeof(int), st));
+  int* cnt = reinterpret_cast<int*>(ws);
+  int* off = cnt + n_cnt;
+  const int s = strict ? 1 : 0;
+  const int rc = dispatch_nj_qb(a.dim, scan_qb(a.dim, a.nq), "range tenants scan", [&](auto nj, auto qbc) {
+    constexpr int NJ = decltype(nj)::value, QB = decltype(qbc)::value;
+    auto passes = [&](auto metric) {
+      constexpr int METRIC = decltype(metric)::value;
+      auto scan = [&](auto write) {
+        return launch_kernel(range_tenants_scan_kernel<NJ, QB, METRIC, decltype(write)::value>, dim3(grid),
+                             dim3(kScanWarps * 32), 0, st, a.master, a.tags, a.qn, a.nq, q_tenant, q_lo, q_hi, flagged,
+                             n_flagged, threshold, s, max_hits, row_offset, cnt, off, out_rows, out_scores);
+      };
+      return launch_counting_passes(scan, grid, a.nq, flagged, n_flagged, max_hits,
+                                    METRIC == FRG_METRIC_COSINE ? kNoScore : INFINITY, cnt, off, out_counts, out_rows,
+                                    out_scores, st);
+    };
+    if (a.metric == FRG_METRIC_COSINE) return passes(std::integral_constant<int, FRG_METRIC_COSINE>());
+    return passes(std::integral_constant<int, FRG_METRIC_EUCLIDEAN>());
+  });
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) return cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
 // ------------------------------------------------------------------------------------------ gallery self-join
 // range_scan_kernel with the join rules (cosine): query q of the slab is the stored row a = qrow0 + q, and row b counts
 // for it only when b > a and (same_tag) tag[b] == tag[a]; a dead query, or one outside the tenant, counts nothing.  A

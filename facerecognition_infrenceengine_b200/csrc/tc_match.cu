@@ -1974,26 +1974,75 @@ void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::ve
   if (!main.empty()) memcpy(table->data(), main.data(), table->size());
 }
 
-int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
-                   int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
-                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcRangeWs& w,
-                   int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
-  if (!s->plane8 || !s->master || s->row0 != 0 || s->rows > 0x7fffffff) {
-    set_error("tc_join: needs the whole unit store with an int8 plane and an fp32 master");
-    return FRG_ERR_UNSUPPORTED;
-  }
-  // the GROUPED single-CTA grid over the uploaded descriptors
-  auto filter = [&](const CUtensorMap& qm, const CUtensorMap& gm, TcScanParams& p) {
+// The filter grid of launch_range_family for a GROUPED table: the single-CTA grid over n_ctas uploaded descriptors
+// (none when 0).  The self-join and per-query-tenant range search.
+static auto grouped_filter(const void* d_table, int n_ctas, cudaStream_t st) {
+  return [=](const CUtensorMap& qm, const CUtensorMap& gm, TcScanParams& p) {
     p.tenant = -1; p.groups = static_cast<const TcGroupCta*>(d_table);
     profile_begin(st, kStageDominant);
     if (n_ctas > 0) FRG_CHECK((launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, n_ctas, 1, st)));
     profile_end(st, n_ctas > 0 ? 1 : 0);
     return FRG_OK;
   };
-  return launch_range_family(s, qi8, qstep, eps, nq, threshold, w, st, filter, join_select_kernel, w.dense,
-                             w.cand_total, kRangeBudget, s->dim, qn, s->master, s->tags, qrow0, tenant,
-                             same_tag ? 1 : 0, threshold, strict ? 1 : 0, max_hits, row_offset, out_counts, out_rows,
-                             out_scores, w.flagged, w.n_flagged);
+}
+
+static bool whole_unit_store(const GalleryWindow* s) {
+  return s->plane8 && s->master && s->row0 == 0 && s->rows <= 0x7fffffff;
+}
+
+int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
+                   int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
+                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcRangeWs& w,
+                   int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  if (!whole_unit_store(s)) {
+    set_error("tc_join: needs the whole unit store with an int8 plane and an fp32 master");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  return launch_range_family(s, qi8, qstep, eps, nq, threshold, w, st, grouped_filter(d_table, n_ctas, st),
+                             join_select_kernel, w.dense, w.cand_total, kRangeBudget, s->dim, qn, s->master, s->tags,
+                             qrow0, tenant, same_tag ? 1 : 0, threshold, strict ? 1 : 0, max_hits, row_offset,
+                             out_counts, out_rows, out_scores, w.flagged, w.n_flagged);
+}
+
+// ------------------------------------------------------------------------------------------ per-query-tenant range search
+int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
+                            const float* eps, int nq, const void* d_table, int n_ctas, int max_hits, float threshold,
+                            bool strict, int64_t row_offset, const TcRangeWs& w, int64_t* out_counts,
+                            int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  if (!whole_unit_store(s)) {
+    set_error("tc_range_grouped: needs the whole unit store with an int8 plane and an fp32 master");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  return launch_range_family(s, qi8, qstep, eps, nq, threshold, w, st, grouped_filter(d_table, n_ctas, st),
+                             range_select_kernel, w.dense, w.cand_total, kRangeBudget, s->dim, qn, s->master,
+                             threshold, strict ? 1 : 0, max_hits, row_offset, out_counts, out_rows, out_scores,
+                             w.flagged, w.n_flagged);
+}
+
+// range results of sorted query i -> the caller's slot perm[i]
+__global__ void __launch_bounds__(256)
+scatter_range_kernel(const int64_t* __restrict__ counts, const int64_t* __restrict__ rows,
+                     const float* __restrict__ scores, const int32_t* __restrict__ perm, int nq, int max_hits,
+                     int64_t* __restrict__ out_counts, int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
+  pdl_wait();
+  pdl_trigger();
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= int64_t(nq) * max_hits) return;
+  const int q = int(i / max_hits), j = int(i - int64_t(q) * max_hits);
+  const int dst = __ldg(perm + q);
+  out_rows[size_t(dst) * max_hits + j] = rows[i];
+  out_scores[size_t(dst) * max_hits + j] = scores[i];
+  if (j == 0) out_counts[dst] = counts[q];
+}
+
+int launch_scatter_range(const int64_t* counts, const int64_t* rows, const float* scores, const int32_t* perm, int nq,
+                         int max_hits, int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
+  if (nq <= 0) return FRG_OK;
+  const int64_t n = int64_t(nq) * max_hits;
+  FRG_CUDA(launch_kernel(scatter_range_kernel, dim3(unsigned((n + 255) / 256)), dim3(256), 0, st, counts, rows, scores,
+                         perm, nq, max_hits, out_counts, out_rows, out_scores));
+  note_launch(nullptr);
+  return FRG_OK;
 }
 
 }  // namespace frg

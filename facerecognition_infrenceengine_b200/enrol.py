@@ -89,6 +89,33 @@ class EnrolmentChecker:
         ref = (meta or {}).get("ref_id")
         return True, (ref if ref is not None else pid)
 
+    def check_duplicate_faces(self, embeddings: Sequence[np.ndarray], company_ids: Sequence[Optional[str]],
+                              kinds: Optional[Sequence[Optional[str]]] = None) -> List[Tuple[bool, Optional[str]]]:
+        """``check_duplicate_face`` for a batch of faces from any mix of companies: entry i equals
+        ``check_duplicate_face(embeddings[i], company_ids[i], kinds[i])``.  One range search in which every face
+        carries its own (company, kind) filter, strict, first hit only - the first-match rule - so a bulk import or a
+        queue of enrolment jobs pays one call instead of one per face."""
+        range_tenants_host = getattr(self.matcher, "range_tenants_host", None)
+        if range_tenants_host is None:
+            raise NotImplementedError("%s has no range_tenants_host: per-face company filters need a single-GPU Matcher"
+                                      % type(self.matcher).__name__)
+        E = np.asarray(embeddings, np.float32)
+        if E.ndim != 2:
+            raise ValueError("embeddings must be [faces, dim]")
+        if kinds is None:
+            kinds = [None] * len(E)
+        if len(company_ids) != len(E) or len(kinds) != len(E):
+            raise ValueError("%d faces, %d company ids, %d kinds" % (len(E), len(company_ids), len(kinds)))
+        if not len(E):
+            return []
+        store = self.store.store if isinstance(self.store, EnrolmentGallery) else self.store
+        ident = _identity(store)
+        with _reading(store):            # scan + row -> id translation are one read section (compact() renumbers)
+            tenants = self.matcher._tenant_codes([enrolment_tenant(c, k) for c, k in zip(company_ids, kinds)], len(E))
+            counts, rows, _ = range_tenants_host(E, tenants, self.duplicate_threshold, max_hits=1, strict=True)
+            return [(True, ident(r)) if c > 0 else (False, None)
+                    for c, r in zip(counts.tolist(), rows[:, 0].tolist())]
+
     def check_image_similarity(self, embeddings: Sequence[np.ndarray]) -> Tuple[bool, Optional[Tuple[int, int]]]:
         """(all poses show the same person, first offending pair) - trainingServer.py:202-214.  The pose
         embeddings go through the same device path: a scratch gallery of the poses, every pose matched

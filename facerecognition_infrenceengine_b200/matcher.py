@@ -204,20 +204,62 @@ class Matcher:
         Q = np.ascontiguousarray(Q, dtype=np.float32).reshape(-1, self.store.dim)
         tenant = -1 if company_id is None else self.store.tenant_code(company_id, create=False)
         with _reading(self.store):
-            layout = getattr(self.store, "layout_version", 0)
-            counts, rows, scores = self.range_host(Q, threshold, tenant, max_hits, strict, variant)
-            variant_ran = N.last_variant()
-            over = np.nonzero(counts > max_hits)[0]
-            if len(over):
-                c2, r2, s2 = self.range_host(Q[over], threshold, tenant, int(counts[over].max()), strict, variant)
-                counts[over] = c2
-            lists_r, lists_s = range_lists(np.minimum(counts, max_hits), rows, scores, self.metric)
-            for j, f in enumerate(over.tolist()):
-                lists_r[f], lists_s[f] = best_first(r2[j, :c2[j]], s2[j, :c2[j]], self.metric)
-            out = RangeResult(counts, lists_r, lists_s, variant=variant_ran, layout_version=layout)
-            if with_ids:
-                out.ids = [self.store.ids_of(r[None, :])[0] if len(r) else [] for r in lists_r]
+            return self._complete_range(lambda sel, hits: self.range_host(Q if sel is None else Q[sel], threshold,
+                                                                          tenant, hits, strict, variant),
+                                        max_hits, with_ids)
+
+    def _complete_range(self, run, max_hits: int, with_ids: bool) -> RangeResult:
+        """COMPLETE best-first lists from raw range blocks: run(sel, hits) returns (counts, rows, scores) of the queries
+        sel (None = all) with room for hits.  max_hits only sizes the first call: the queries whose count exceeded it
+        are re-run once, those queries only, with room for their largest count.  The caller holds the read section."""
+        layout = getattr(self.store, "layout_version", 0)
+        counts, rows, scores = run(None, max_hits)
+        variant_ran = N.last_variant()
+        over = np.nonzero(counts > max_hits)[0]
+        if len(over):
+            c2, r2, s2 = run(over, int(counts[over].max()))
+            counts[over] = c2
+        lists_r, lists_s = range_lists(np.minimum(counts, max_hits), rows, scores, self.metric)
+        for j, f in enumerate(over.tolist()):
+            lists_r[f], lists_s[f] = best_first(r2[j, :c2[j]], s2[j, :c2[j]], self.metric)
+        out = RangeResult(counts, lists_r, lists_s, variant=variant_ran, layout_version=layout)
+        if with_ids:
+            out.ids = [self.store.ids_of(r[None, :])[0] if len(r) else [] for r in lists_r]
         return out
+
+    def range_tenants_host(self, Q: np.ndarray, tenants, threshold: float, max_hits: int = 64, strict: bool = False,
+                           variant: str = "auto"):
+        """``range_host`` with a tenant tag PER QUERY (-1 = all tenants): one frg_match_range_tenants_host call, the
+        same raw blocks; row f equals ``range_host(Q[f:f+1], threshold, tenants[f], ...)`` bit for bit."""
+        Q = np.ascontiguousarray(Q, dtype=np.float32).reshape(-1, self.store.dim)
+        F = len(Q)
+        t = np.ascontiguousarray(tenants, dtype=np.int32).reshape(-1)
+        if len(t) != F:
+            raise ValueError("%d tenants for %d queries" % (len(t), F))
+        counts = np.zeros(F, np.int64)
+        rows, scores = np.empty((F, max_hits), np.int64), np.empty((F, max_hits), np.float32)
+        p = _params(self.metric, variant, threshold, -1, 0)
+        p.flags = N.FIRST_STRICT if strict else 0
+        N.check(N.lib.frg_match_range_tenants_host(self.store.handle, Q.ctypes.data, F, int(max_hits), C.byref(p),
+                                                   t.ctypes.data, counts.ctypes.data, rows.ctypes.data,
+                                                   scores.ctypes.data))
+        return counts, rows, scores
+
+    def match_range_tenants(self, Q: np.ndarray, company_ids: Sequence[Optional[str]], threshold: float,
+                            max_hits: int = 64, strict: bool = False, variant: str = "auto",
+                            with_ids: bool = True) -> RangeResult:
+        """``match_range`` with a company filter PER QUERY: entry f equals ``match_range(Q[f:f+1], threshold,
+        company_ids[f], ...)`` (None = all companies; an unknown company matches nothing).  One
+        frg_match_range_tenants_host call; the queries whose count exceeded max_hits are re-run once, each with its own
+        company, in one more call.  The calls and the id lookup are one read section."""
+        Q = np.ascontiguousarray(Q, dtype=np.float32).reshape(-1, self.store.dim)
+        tenants = self._tenant_codes(company_ids, len(Q))
+        with _reading(self.store):
+            return self._complete_range(
+                lambda sel, hits: self.range_tenants_host(Q if sel is None else Q[sel],
+                                                          tenants if sel is None else tenants[sel], threshold, hits,
+                                                          strict, variant),
+                max_hits, with_ids)
 
     # ---- the gallery against itself: every pair of stored rows a < b at or above the threshold
     def self_join(self, threshold: float, company_id: Optional[str] = None, same_company: bool = False,

@@ -208,6 +208,25 @@ FRG_API int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32
                                  const frg_match_params_t* p, int64_t* out_counts, int64_t* out_rows,
                                  float* out_scores);
 
+/* ---- range search in which every query carries its own tenant filter (watchlists per company on a server that mixes
+ *      companies in one batch; a batch of enrolment duplicate checks: max_hits = 1 with FRG_FIRST_STRICT).
+ * tenants: HOST array [nq]; tenants[i] < 0 = all tenants, else only rows tagged tenants[i] (a tag no row carries:
+ *   count 0 and "none" slots).  p->tenant is not read; everything else of *p applies to all queries.
+ * Result of query i (out_counts[i], out_rows[i*max_hits ..], out_scores[i*max_hits ..]) == frg_match_range(s, q_i, 1,
+ *   max_hits, p') with p' = *p, p'.tenant = tenants[i], bit for bit, in the caller's query order, for every metric,
+ *   variant, flag and store frg_match_range accepts.  Its refusals apply unchanged; tenants == NULL with nq > 0:
+ *   FRG_ERR_INVALID.  A store of more than 2^31 - 1 rows: FRG_ERR_UNSUPPORTED (unless all queries share one tenant).
+ * All queries on one tenant: exactly frg_match_range.  Otherwise every tenant runs in ONE set of launches (the launch
+ *   count does not grow with the number of tenants): the int8 tensor-core filter where frg_match_range takes it
+ *   (frg_last_variant() "range_tc_grouped"), else one exact counting scan in which each query reads only its
+ *   tenant's row window ("range_scan_tenants"). */
+FRG_API int frg_match_range_tenants(frg_store* s, const float* q, int32_t nq, int32_t max_hits,
+                                    const frg_match_params_t* p, const int32_t* tenants, int64_t* out_counts,
+                                    int64_t* out_rows, float* out_scores, void* stream);
+FRG_API int frg_match_range_tenants_host(frg_store* s, const float* q, int32_t nq, int32_t max_hits,
+                                         const frg_match_params_t* p, const int32_t* tenants, int64_t* out_counts,
+                                         int64_t* out_rows, float* out_scores);
+
 /* ---- gallery self-join: every pair of stored rows a < b whose score reaches the threshold, in one pass over the
  *      upper triangle on the device (NOT in the reference: the duplicate rule of trainingServer.py:170-200 applied to
  *      what is already enrolled - after a bulk import or a snapshot load).  The queries are the store's own rows; no
