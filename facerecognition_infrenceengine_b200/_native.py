@@ -20,6 +20,7 @@ ROWS_PRENORMALISED = 1
 FIRST_STRICT, QUERY_PRENORMALISED = 1, 2
 JOIN_SAME_TAG = 4
 JOIN_SLAB_ROWS = 1024
+CLUSTER_MAX_WINDOW = 16
 XCHG_PUSH_ONLY, XCHG_MERGE_ONLY = 1, 2
 MAX_K = 16
 
@@ -57,6 +58,11 @@ class ExchangeStatus(C.Structure):    # frg_exchange_status_t
                 ("slot", C.c_int32), ("reserved", C.c_int32)]
 
 
+class ClusterRing(C.Structure):       # frg_cluster_ring_t
+    _fields_ = [("members", C.c_void_p), ("len", C.c_void_p), ("head", C.c_void_p), ("capacity", C.c_int64),
+                ("window", C.c_int32)]
+
+
 # every symbol include/frg.h declares: (restype, argtypes)
 _P = C.c_void_p
 SIGNATURES = {
@@ -87,6 +93,8 @@ SIGNATURES = {
                                                _P]),
     "frg_self_join": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(MatchParams), _P, _P, _P, _P]),
     "frg_self_join_host": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int32, C.POINTER(MatchParams), _P, _P, _P]),
+    "frg_cluster_observe_host": (C.c_int, [_P, _P, C.c_int32, C.POINTER(MatchParams), C.POINTER(ClusterRing), _P,
+                                           _P]),
     "frg_merge_topk": (C.c_int, [C.c_int32, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                  C.c_float, _P, _P, _P, _P]),
     "frg_merge_topk_strided": (C.c_int, [C.c_int32, _P, C.c_int64, _P, C.c_int64, C.c_int32, C.c_int32, C.c_int32,

@@ -472,6 +472,18 @@ int frg_store_stats(frg_store* s, frg_store_stats_t* out) {
   return FRG_OK;
 }
 
+// The host bookkeeping of an upsert of n rows (appended at s->rows, or overwritten in place) whose device writes are
+// enqueued on st after store_begin_write: tenant extents, row and live counts, version and write ordering.  s->mu held.
+static int end_upsert(frg_store* s, bool append, int64_t n, bool may_tombstone, bool host_known, const int64_t* hrows,
+                      const int32_t* htags, cudaStream_t st) {
+  if (host_known) extents_note_upsert(s, hrows, htags, n, s->rows);
+  else s->extents_known = false;             // positions / tags live in device memory only
+  if (append) s->rows += n;
+  s->live = -1;
+  if (may_tombstone) s->maybe_dead = true;
+  return store_end_write(s, st);
+}
+
 // hrows / htags: HOST copies of rows / tags when the caller has them (host_known), for the tenant extents
 static int upsert_impl(frg_store* s, const int64_t* rows, const float* vecs, const int32_t* tags,
                        int64_t n, uint32_t flags, void* stream, bool tags_may_be_negative,
@@ -486,12 +498,7 @@ static int upsert_impl(frg_store* s, const int64_t* rows, const float* vecs, con
   const bool normalise = !(flags & FRG_ROWS_PRENORMALISED) && !(s->flags & FRG_STORE_RAW);
   FRG_CHECK(launch_ingest(vecs, rows, tags, n, s->rows, s->dim, normalise, s->master, s->plane, s->plane8,
                           s->plane_dim, s->gmax_bits, s->tags, st));
-  if (host_known) extents_note_upsert(s, hrows, htags, n, s->rows);
-  else s->extents_known = false;             // positions / tags live in device memory only
-  if (!rows) s->rows += n;
-  s->live = -1;
-  if (tags && tags_may_be_negative) s->maybe_dead = true;
-  return store_end_write(s, st);
+  return end_upsert(s, !rows, n, tags && tags_may_be_negative, host_known, hrows, htags, st);
 }
 
 int frg_store_upsert(frg_store* s, const int64_t* rows, const float* vecs, const int32_t* tags,
@@ -1281,6 +1288,89 @@ int frg_first_match_host(frg_store* s, const float* q, int32_t nq, const frg_mat
   }
   cudaFreeAsync(d, st);
   return rc;
+}
+
+// --------------------------------------------------------------------------------------------- unknown-face clustering
+// The faces go up, the pre-pass and the resolve kernel run (launch_cluster_observe), and the decisions come back in one
+// copy.  Only then is the number of new rows known: the bookkeeping of an append of that many rows follows.
+int frg_cluster_observe_host(frg_store* s, const float* q, int32_t nq, const frg_match_params_t* p,
+                             const frg_cluster_ring_t* ring, int64_t* out_cluster, uint8_t* out_created) {
+  reset_launches();
+  if (!s || !p || !ring || nq < 0 ||
+      (nq > 0 && (!q || !out_cluster || !out_created || !ring->members || !ring->len || !ring->head))) {
+    set_error("cluster_observe_host: bad argument");
+    return FRG_ERR_INVALID;
+  }
+  if (!(s->flags & FRG_STORE_RAW) || has_plane(s)) {
+    set_error("cluster_observe_host: needs a FRG_STORE_RAW store without a scan plane (the means are written in place)");
+    return FRG_ERR_UNSUPPORTED;
+  }
+  if (p->metric != FRG_METRIC_COSINE) { set_error("cluster_observe_host: cosine / dot only"); return FRG_ERR_UNSUPPORTED; }
+  const char* why = "";
+  if (!range_scan_supported(s->dim, &why)) { set_error("cluster_observe_host: %s", why); return FRG_ERR_UNSUPPORTED; }
+  if (ring->window < 1 || ring->window > FRG_CLUSTER_MAX_WINDOW) {
+    set_error("cluster_observe_host: window %d out of range 1..%d", ring->window, FRG_CLUSTER_MAX_WINDOW);
+    return FRG_ERR_INVALID;
+  }
+  DeviceGuard g(s->device);
+  if (!g.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
+  DeviceInfo di;
+  FRG_CHECK(device_info(s->device, &di));
+  std::lock_guard<std::mutex> lk(s->mu);
+  if (ring->capacity < s->rows + nq) {
+    set_error("cluster_observe_host: ring capacity %lld < rows %lld + faces %d", (long long)ring->capacity,
+              (long long)s->rows, nq);
+    return FRG_ERR_INVALID;
+  }
+  if (s->rows + nq > 0x7fffffff) { set_error("cluster_observe_host: more than 2^31-1 clusters"); return FRG_ERR_UNSUPPORTED; }
+  if (nq == 0) return FRG_OK;
+  if (s->rows + nq > s->capacity) FRG_CHECK(grow_locked(s, next_capacity(s->capacity, s->rows + nq)));
+  cudaStream_t st = cudaStreamPerThread;
+  FRG_CHECK(store_begin_write(s, st));
+  const int32_t new_tag = p->tenant < 0 ? 0 : p->tenant;
+  Carve c;
+  const size_t qb = size_t(nq) * s->dim * sizeof(float);
+  const size_t o_q = c.take(qb), o_cl = c.take(size_t(nq) * sizeof(int64_t)), o_cr = c.take(size_t(nq));
+  unsigned char* d = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d), c.off, st));
+  int rc = FRG_OK;
+  cudaError_t e = cudaMemcpyAsync(d + o_q, q, qb, cudaMemcpyHostToDevice, st);
+  if (e != cudaSuccess) rc = cuda_fail(e, "H2D faces", __FILE__, __LINE__);
+  if (rc == FRG_OK) {
+    ScanArgs a;
+    a.master = s->master; a.tags = s->tags; a.rows = s->rows; a.dim = s->dim;
+    a.qn = reinterpret_cast<float*>(d + o_q); a.nq = nq; a.k = 1; a.metric = FRG_METRIC_COSINE; a.tenant = p->tenant;
+    a.sm_count = di.sm_count;
+    rc = launch_cluster_observe(a, s->master, s->tags, p->threshold, (p->flags & FRG_FIRST_STRICT) != 0, new_tag, *ring,
+                                reinterpret_cast<int64_t*>(d + o_cl), d + o_cr, st);
+  }
+  if (rc == FRG_OK) {
+    // clusters | created flags sit in one device range: one copy into the pinned bounce
+    const size_t span = o_cr + size_t(nq) - o_cl;
+    unsigned char* h = g_result_bounce.get(span);
+    if (h) {
+      e = cudaMemcpyAsync(h, d + o_cl, span, cudaMemcpyDeviceToHost, st);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+      if (e == cudaSuccess) {
+        memcpy(out_cluster, h, size_t(nq) * sizeof(int64_t));
+        memcpy(out_created, h + (o_cr - o_cl), size_t(nq));
+      }
+    } else {
+      (void)cudaGetLastError();
+      e = cudaMemcpyAsync(out_cluster, d + o_cl, size_t(nq) * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
+      if (e == cudaSuccess) e = cudaMemcpyAsync(out_created, d + o_cr, size_t(nq), cudaMemcpyDeviceToHost, st);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    }
+    if (e != cudaSuccess) rc = cuda_fail(e, "D2H results", __FILE__, __LINE__);
+    else rc = store_fault(s);
+  }
+  cudaFreeAsync(d, st);
+  int64_t created = 0;
+  if (rc == FRG_OK)
+    for (int32_t i = 0; i < nq; ++i) created += out_created[i] != 0;
+  const std::vector<int32_t> new_tags(size_t(created), new_tag);
+  const int rc_end = end_upsert(s, true, created, false, true, nullptr, new_tags.data(), st);
+  return rc != FRG_OK ? rc : rc_end;
 }
 
 // --------------------------------------------------------------------------------------------- range search

@@ -467,6 +467,16 @@ int launch_join_scan(const ScanArgs& a, int64_t qrow0, const int32_t* tile_end, 
                      const int* n_flagged, int max_hits, float threshold, bool strict, int64_t row_offset, void* ws,
                      int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st);
 
+// scan_f32.cu: frg_cluster_observe_host's device work.  a: the store's first a.rows rows (the clusters before the call),
+// a.qn / a.nq the faces as given, a.tenant the call's filter.  Pre-pass: launch_range_scan of every face against those
+// rows (hit budget kClusterHits); then ONE CTA resolves the faces in order, writing the means to master, the tags of the
+// new rows (new_tag) and the ring, and out_cluster / out_created (device).  master / tags: the store's, with room for
+// a.rows + a.nq rows.
+constexpr int kClusterHits = 16;
+int launch_cluster_observe(const ScanArgs& a, float* master, int32_t* tags, float threshold, bool strict,
+                           int32_t new_tag, const frg_cluster_ring_t& ring, int64_t* out_cluster, uint8_t* out_created,
+                           cudaStream_t st);
+
 // first_match.cu
 int launch_first_match(const float* master, const int32_t* tags, int64_t rows, int dim, const float* qn, int nq,
                        int32_t tenant, float threshold, bool strict, int64_t row_offset, unsigned long long* scratch,

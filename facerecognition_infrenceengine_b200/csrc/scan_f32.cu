@@ -983,4 +983,180 @@ int launch_join_scan(const ScanArgs& a, int64_t qrow0, const int32_t* tile_end, 
   });
 }
 
+// ------------------------------------------------------------------------------------------ unknown-face clustering
+// frg_cluster_observe_host: face i joins the first live row with dot(mean, q_i) >= threshold, the means as faces
+// 0 .. i-1 left them, else founds a row.  The pre-pass (launch_range_scan over the c0 rows that existed before the call)
+// gives every face its hit count and its first kClusterHits hits in row order, scored with the arithmetic used here.
+// A row an earlier face of the batch joined or founded is "touched": its mean changed, so its pre-pass score is void,
+// while every untouched row still has the mean the pre-pass saw.  Hence, for face i:
+//   c_u = the first untouched hit (its listed hits are the first hits in row order; when all of them are touched and
+//         the list is truncated, the rows after the last listed one are rescanned, untouched ones only);
+//   c_t = the lowest touched row below c_u whose CURRENT mean qualifies (recomputed here);
+// and min(c_t, c_u) is exactly the first qualifying row of the sequential rule: every row below it is either untouched
+// and not a hit, or touched and recomputed.  One CTA works through the faces in order; its 32 warps share the dots.
+constexpr int kClusterWarps = 32;
+
+template <int NJ>
+__device__ __forceinline__ float cluster_dot(const float* row, const float4 (&qv)[1][NJ], int lane) {
+  float4 g[NJ];
+  const float4* pr = reinterpret_cast<const float4*>(row) + lane;     // plain loads: this kernel writes the means
+#pragma unroll
+  for (int j = 0; j < NJ; ++j) g[j] = pr[j * 32];
+  float a[1];
+  row_dots<NJ, 1, FRG_METRIC_COSINE>(g, qv, a);
+  return butterfly<1>(a, lane);
+}
+
+template <int NJ>
+__global__ void __launch_bounds__(kClusterWarps * 32, 1)
+cluster_resolve_kernel(float* master, int32_t* tags, int c0, const float* __restrict__ q, int nq,
+                       const int64_t* __restrict__ hit_count, const int64_t* __restrict__ hit_rows, float* members,
+                       int32_t* ring_len, int32_t* ring_head, int window, int32_t tenant, int32_t new_tag,
+                       float threshold, int strict, uint8_t* touched, int32_t* touched_list,
+                       int64_t* __restrict__ out_cluster, uint8_t* __restrict__ out_created) {
+  constexpr int DIM = NJ * 128;
+  constexpr int kNone = 0x7fffffff;
+  __shared__ int s_cu, s_best, s_from, s_nt, s_row, s_slot, s_len, s_head, s_created;
+  pdl_wait();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  auto pass = [&](float s) { return strict ? (s > threshold) : (s >= threshold); };     // false for NaN
+  if (threadIdx.x == 0) s_nt = 0;
+  int n_created = 0;                                                  // thread 0's
+  for (int i = 0; i < nq; ++i) {
+    float4 qv[1][NJ];
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) qv[0][j] = __ldg(reinterpret_cast<const float4*>(q + size_t(i) * DIM) + j * 32 + lane);
+    // (a) the first untouched listed hit; a truncated list whose listed hits are all touched needs the rescan
+    if (warp == 0) {
+      const int64_t cnt = hit_count[i];
+      const int listed = cnt < kClusterHits ? int(cnt) : kClusterHits;
+      const int r = lane < listed ? int(hit_rows[size_t(i) * kClusterHits + lane]) : -1;
+      const unsigned m = __ballot_sync(0xffffffffu, lane < listed && !touched[r]);
+      const int first = __shfl_sync(0xffffffffu, r, m ? __ffs(m) - 1 : 0);
+      const int last = __shfl_sync(0xffffffffu, r, kClusterHits - 1);
+      if (lane == 0) {
+        s_cu = m ? first : kNone;
+        s_from = (!m && cnt > kClusterHits) ? last + 1 : c0;
+        s_best = kNone;
+      }
+    }
+    __syncthreads();
+    for (int base = s_from; base < c0; base += kClusterWarps) {      // rare: all listed hits touched, list truncated
+      const int r = base + warp;
+      if (r < c0) {
+        const int32_t tg = tags[r];
+        if (tg >= 0 && (tenant < 0 || tg == tenant) && !touched[r]) {
+          const float s = cluster_dot<NJ>(master + size_t(r) * DIM, qv, lane);
+          if (lane == 0 && pass(s)) atomicMin(&s_cu, r);
+        }
+      }
+      __syncthreads();
+      const bool found = s_cu != kNone;
+      __syncthreads();
+      if (found) break;
+    }
+    // (b) the touched rows below c_u, with their current means; the lowest qualifying one wins
+    const int cu = s_cu, nt = s_nt;
+    for (int t = warp; t < nt; t += kClusterWarps) {
+      const int r = touched_list[t];
+      const int best = __shfl_sync(0xffffffffu, *reinterpret_cast<volatile int*>(&s_best), 0);
+      if (r >= cu || r >= best) continue;
+      const float s = cluster_dot<NJ>(master + size_t(r) * DIM, qv, lane);
+      if (lane == 0 && pass(s)) atomicMin(&s_best, r);
+    }
+    __syncthreads();
+    // (c) the decision, the ring's bookkeeping and the touched set
+    if (threadIdx.x == 0) {
+      int r = s_best < cu ? s_best : cu;
+      const bool created = r == kNone;
+      int len, head, slot;
+      if (created) {
+        r = c0 + n_created++;
+        len = 1; head = 0; slot = 0;
+        tags[r] = new_tag;
+        touched_list[s_nt++] = r;
+      } else {
+        len = ring_len[r]; head = ring_head[r];
+        if (len < window) { slot = (head + len) % window; ++len; }
+        else { slot = head; head = (head + 1) % window; }
+        if (r < c0 && !touched[r]) { touched[r] = 1; touched_list[s_nt++] = r; }
+      }
+      ring_len[r] = len; ring_head[r] = head;
+      s_row = r; s_slot = slot; s_len = len; s_head = head; s_created = created;
+      out_cluster[i] = r;
+      out_created[i] = created ? 1 : 0;
+    }
+    __syncthreads();
+    // (d) thread e owns element e of every window and mean: append q_i, then the mean of the window, oldest first, as
+    // np.mean computes it in fp32 (sum from +0.0f, one division); a new row's mean is q_i itself
+    {
+      const int r = s_row, slot = s_slot, len = s_len, head = s_head;
+      float* win = members + size_t(r) * window * DIM;
+      for (int e = threadIdx.x; e < DIM; e += blockDim.x) {
+        const float v = q[size_t(i) * DIM + e];
+        win[size_t(slot) * DIM + e] = v;
+        float m = v;
+        if (!s_created) {
+          float sum = 0.f;
+          for (int k = 0; k < len; ++k) {
+            int sl = head + k;
+            if (sl >= window) sl -= window;
+            sum = __fadd_rn(sum, sl == slot ? v : win[size_t(sl) * DIM + e]);
+          }
+          m = __fdiv_rn(sum, float(len));
+        }
+        master[size_t(r) * DIM + e] = m;
+      }
+    }
+    __syncthreads();
+  }
+}
+
+int launch_cluster_observe(const ScanArgs& a, float* master, int32_t* tags, float threshold, bool strict,
+                           int32_t new_tag, const frg_cluster_ring_t& ring, int64_t* out_cluster, uint8_t* out_created,
+                           cudaStream_t st) {
+  const char* why = "";
+  if (!range_scan_supported(a.dim, &why)) { set_error("cluster observe: %s", why); return FRG_ERR_UNSUPPORTED; }
+  if (a.nq <= 0) return FRG_OK;
+  const size_t slots = size_t(a.nq) * kClusterHits;
+  Carve c;
+  const size_t o_cnt = c.take(size_t(a.nq) * sizeof(int64_t)), o_rows = c.take(slots * sizeof(int64_t));
+  const size_t o_sc = c.take(slots * sizeof(float)), o_list = c.take(size_t(a.nq) * sizeof(int32_t));
+  const size_t o_touch = c.take(size_t(a.rows > 0 ? a.rows : 1));
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+  int64_t* cnt = reinterpret_cast<int64_t*>(ws + o_cnt);
+  int64_t* rows = reinterpret_cast<int64_t*>(ws + o_rows);
+  int rc = FRG_OK;
+  cudaError_t e = cudaMemsetAsync(ws + o_touch, 0, size_t(a.rows > 0 ? a.rows : 1), st);
+  if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemsetAsync", __FILE__, __LINE__);
+  if (rc == FRG_OK) {
+    profile_begin(st, kStagePrepass);
+    rc = launch_range_scan(a, nullptr, nullptr, kClusterHits, threshold, strict, 0, cnt, rows,
+                           reinterpret_cast<float*>(ws + o_sc), st);
+    profile_end(st, 3);
+  }
+  if (rc == FRG_OK) {
+    auto launch = [&](auto kern) {
+      return launch_kernel(kern, dim3(1), dim3(kClusterWarps * 32), 0, st, master, tags, int(a.rows), a.qn, a.nq, cnt,
+                           rows, ring.members, ring.len, ring.head, ring.window, a.tenant, new_tag, threshold,
+                           strict ? 1 : 0, ws + o_touch, reinterpret_cast<int32_t*>(ws + o_list), out_cluster,
+                           out_created);
+    };
+    profile_begin(st, kStageDominant);
+    switch (a.dim) {
+      case 128: e = launch(cluster_resolve_kernel<1>); break;
+      case 256: e = launch(cluster_resolve_kernel<2>); break;
+      case 512: e = launch(cluster_resolve_kernel<4>); break;
+      default:  e = launch(cluster_resolve_kernel<8>); break;
+    }
+    profile_end(st, 1);
+    note_launch("cluster_observe");
+    if (e != cudaSuccess) rc = cuda_fail(e, "cluster_resolve_kernel", __FILE__, __LINE__);
+  }
+  e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
+}
+
 }  // namespace frg

@@ -254,6 +254,32 @@ FRG_API int frg_self_join(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
 FRG_API int frg_self_join_host(frg_store* s, int64_t row0, int64_t n, int32_t max_hits,
                                const frg_match_params_t* p, int64_t* out_counts, int64_t* out_rows, float* out_scores);
 
+/* ---- online clustering of unknown faces, a whole batch in one call (peopleCount.py:432-500, the rule of
+ *      frg_first_match's clustering use applied face after face).  The store holds the cluster means: row r is the
+ *      mean of cluster r's last `window` faces, which the caller-owned ring keeps on the device.
+ * Result == observing q_0, q_1, ... one at a time: face i (used as given) joins the FIRST live row, in row order, with
+ *   dot(mean, q_i) >= p->threshold ('>' with FRG_FIRST_STRICT; p->tenant filters as in frg_first_match) - every mean
+ *   as the earlier faces of the batch left it - else founds a new row (mean = q_i, tag p->tenant, or 0 when
+ *   p->tenant < 0).  On a join q_i is appended to the row's window (the oldest member evicted when it is full) and the
+ *   mean becomes the fp32 sum of the members from +0.0f, oldest first, divided by their number (NumPy's
+ *   np.mean(window, axis=0), bit for bit).  The dot is frg_first_match's arithmetic, bit for bit.
+ * out_cluster [nq] int64: the row face i joined or founded; out_created [nq] uint8: 1 when it founded it.  New rows are
+ *   appended at stats.rows, stats.rows + 1, ... in face order.
+ * Only FRG_STORE_RAW stores without a scan plane (FRG_ERR_UNSUPPORTED otherwise); the store grows itself.  Refused
+ *   with FRG_ERR_INVALID and the store unchanged: ring->capacity < stats.rows + nq, a window outside 1..16, NULL
+ *   pointers with nq > 0.  The call synchronises (the number of new rows is known only on the device).
+ *   frg_last_variant(): "cluster_observe". */
+#define FRG_CLUSTER_MAX_WINDOW 16
+typedef struct frg_cluster_ring_t {
+  float*   members;   /* DEVICE [capacity][window][dim] fp32: the last `window` faces of cluster row r */
+  int32_t* len;       /* DEVICE [capacity] members held, 1..window */
+  int32_t* head;      /* DEVICE [capacity] slot of the oldest member */
+  int64_t  capacity;  /* cluster rows the ring has room for */
+  int32_t  window;    /* 1..FRG_CLUSTER_MAX_WINDOW */
+} frg_cluster_ring_t;
+FRG_API int frg_cluster_observe_host(frg_store* s, const float* q, int32_t nq, const frg_match_params_t* p,
+                                     const frg_cluster_ring_t* ring, int64_t* out_cluster, uint8_t* out_created);
+
 /* ---- k-way merge of per-shard results (multi-GPU tail, SURVEY.md section 8e).
  * scores/rows: [parts][nq][k] (each list best-first, unfilled slots row -1), e.g. the output of an
  * all-gather of every rank's frg_match result.  Order: score desc (euclidean: asc), then row asc. */
