@@ -250,6 +250,16 @@ static void extents_note_upsert(frg_store* s, const int64_t* hrows, const int32_
   }
 }
 
+// The rows [lo, hi) tenant's rows can sit in, hi >= lo: its extent clipped to the rows in use (empty for a tag no row
+// carries), or every row for tenant < 0 or while the extents are not known.  s->mu held.
+static frg_store::Extent tenant_rows(const frg_store* s, int32_t tenant) {
+  if (tenant < 0 || !s->extents_known) return frg_store::Extent{0, s->rows};
+  auto it = s->extents.find(tenant);
+  if (it == s->extents.end()) return frg_store::Extent{0, 0};
+  const int64_t lo = it->second.lo, hi = it->second.hi < s->rows ? it->second.hi : s->rows;
+  return frg_store::Extent{lo, hi > lo ? hi : lo};
+}
+
 // the whole gallery, or - for a tenant-filtered call whose tag extents are known - only the row window that
 // tenant's rows can sit in
 static GalleryWindow window_of(const frg_store* s, int32_t tenant, bool for_tc = false) {
@@ -258,10 +268,8 @@ static GalleryWindow window_of(const frg_store* s, int32_t tenant, bool for_tc =
   w.rows = s->rows; w.row0 = 0; w.dim = s->dim; w.plane_dim = s->plane_dim; w.flags = s->flags;
   w.maybe_dead = s->maybe_dead;
   if (tenant >= 0 && s->extents_known) {
-    int64_t lo = 0, hi = 0;
-    auto it = s->extents.find(tenant);
-    if (it != s->extents.end()) { lo = it->second.lo; hi = it->second.hi < s->rows ? it->second.hi : s->rows; }
-    if (hi < lo) hi = lo;
+    const frg_store::Extent x = tenant_rows(s, tenant);
+    const int64_t lo = x.lo, hi = x.hi;
     // A window that is mostly other tenants' rows (a company's block + one person re-enrolled at the far end):
     // keep the WHOLE store as the window and let the tensor-core kernels walk only the tiles of the tenant's
     // intervals.  (The exact scan and first_match still take the bounding window.)
@@ -1000,24 +1008,75 @@ int frg::stage_upload(void* dev, const void* host, size_t bytes, cudaStream_t st
 
 extern "C" {
 
-// Tiles a tenant's rows can sit in, in kTcTileRows-row tiles: its cached tile list when that is shorter than its
-// extent's tile range, else that range (other tenants' rows in it are masked by the filter's tag check), else every
-// tile (tenant < 0, or extents not known).  A tag no row carries: no tiles.  s->mu held.
-static int tenant_tiles(frg_store* s, int32_t tenant, cudaStream_t st, TcTenantGroup* g) {
-  g->tile0 = 0; g->n_tiles = int((s->rows + kTcTileRows - 1) / kTcTileRows); g->list = nullptr;
-  if (tenant < 0 || !s->extents_known) return FRG_OK;
-  auto it = s->extents.find(tenant);
-  const int64_t lo = it != s->extents.end() ? it->second.lo : 0;
-  const int64_t hi = it != s->extents.end() ? (it->second.hi < s->rows ? it->second.hi : s->rows) : 0;
-  if (hi <= lo) { g->n_tiles = 0; return FRG_OK; }
-  g->tile0 = int(lo / kTcTileRows);
-  g->n_tiles = int((hi - 1) / kTcTileRows) - g->tile0 + 1;
-  const int32_t* list = nullptr;
-  int n = 0;
-  FRG_CHECK(store_tile_list(s, tenant, kTcTileRows, st, &list, &n));
-  if (list && n < g->n_tiles) { g->list = list; g->n_tiles = n; }
-  return FRG_OK;
-}
+// A batch with a tenant per query, sorted stably by tenant with every negative tag read as -1 ("all tenants"):
+// perm[i] is the caller's position of sorted query i, and each run holds the sorted queries q0 .. q0 + nq - 1 of one
+// tenant and, once find_windows has run, the rows [lo, hi) that tenant's rows can sit in (tenant_rows).
+struct TenantBatch {
+  struct Run { int32_t tenant; int32_t q0, nq; int64_t lo, hi; };
+  std::vector<int32_t> perm;
+  std::vector<Run> runs;
+
+  TenantBatch(const int32_t* tenants, int32_t nq) : perm(static_cast<size_t>(nq)) {
+    auto norm = [&](int32_t i) { return tenants[i] < 0 ? int32_t(-1) : tenants[i]; };
+    for (int32_t i = 0; i < nq; ++i) perm[size_t(i)] = i;
+    std::stable_sort(perm.begin(), perm.end(), [&](int32_t a, int32_t b) { return norm(a) < norm(b); });
+    for (int32_t i = 0; i < nq;) {
+      int32_t j = i + 1;
+      while (j < nq && norm(perm[size_t(j)]) == norm(perm[size_t(i)])) ++j;
+      runs.push_back(Run{norm(perm[size_t(i)]), i, j - i, 0, 0});
+      i = j;
+    }
+  }
+  bool one_tenant() const { return runs.size() == 1; }
+  void find_windows(const frg_store* s) {               // s->mu held
+    for (Run& r : runs) {
+      const frg_store::Extent x = tenant_rows(s, r.tenant);
+      r.lo = x.lo; r.hi = x.hi;
+    }
+  }
+
+  // The GROUPED filter's query tiles: each run cut into tiles of at most kTcTileRows queries, which scan the tenant's
+  // cached tile list when that is shorter than its window's tile range, else that range (other tenants' rows in it are
+  // masked by the filter's tag check).  A tag no row carries: no tiles.  s->mu held; the tile lists may be built and
+  // uploaded on st.
+  int query_tiles(frg_store* s, cudaStream_t st, std::vector<TcTenantGroup>* out) const {
+    for (const Run& r : runs) {
+      TcTenantGroup g{};
+      g.tenant = r.tenant;
+      g.tile0 = int(r.lo / kTcTileRows);
+      g.n_tiles = r.hi > r.lo ? int((r.hi - 1) / kTcTileRows) - g.tile0 + 1 : 0;
+      if (r.tenant >= 0 && s->extents_known && g.n_tiles > 0) {
+        const int32_t* list = nullptr;
+        int n = 0;
+        FRG_CHECK(store_tile_list(s, r.tenant, kTcTileRows, st, &list, &n));
+        if (list && n < g.n_tiles) { g.list = list; g.n_tiles = n; }
+      }
+      for (int32_t a = 0; a < r.nq; a += kTcTileRows) {
+        g.q0 = r.q0 + a; g.nq = r.nq - a < kTcTileRows ? r.nq - a : kTcTileRows;
+        out->push_back(g);
+      }
+    }
+    return FRG_OK;
+  }
+
+  // The one upload of a grouped call: [perm][tenant][lo][hi] (int32 [nq] each) of the sorted queries, then the filter's
+  // CTA descriptors at cta_offset() (16 bytes per query: aligned for them).
+  size_t cta_offset() const { return perm.size() * 16; }
+  std::vector<unsigned char> table(const std::vector<unsigned char>& ctas) const {
+    const size_t nq = perm.size();
+    std::vector<unsigned char> t(cta_offset() + ctas.size());
+    int32_t* h = reinterpret_cast<int32_t*>(t.data());
+    std::copy(perm.begin(), perm.end(), h);
+    for (const Run& r : runs)
+      for (int32_t i = r.q0; i < r.q0 + r.nq; ++i) {
+        h[nq + size_t(i)] = r.tenant;
+        h[2 * nq + size_t(i)] = int32_t(r.lo);
+        h[3 * nq + size_t(i)] = int32_t(r.hi);
+      }
+    if (!ctas.empty()) memcpy(t.data() + cta_offset(), ctas.data(), ctas.size());
+    return t;
+  }
+};
 
 static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t k, const frg_match_params_t* p,
                               const int32_t* tenants, int64_t* out_rows, float* out_scores, uint8_t* out_accept,
@@ -1030,24 +1089,11 @@ static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
   if (k < 1 || k > FRG_MAX_K) { set_error("match: k=%d out of range 1..%d", k, FRG_MAX_K); return FRG_ERR_INVALID; }
   if (p->metric != FRG_METRIC_COSINE && p->metric != FRG_METRIC_EUCLIDEAN) { set_error("match: unknown metric %d", p->metric); return FRG_ERR_INVALID; }
   if (nq == 0) return FRG_OK;
-  // stable sort by tenant (every negative tag means "all tenants")
-  auto norm = [&](int32_t i) { return tenants[i] < 0 ? int32_t(-1) : tenants[i]; };
-  std::vector<int32_t> perm(static_cast<size_t>(nq));
-  for (int32_t i = 0; i < nq; ++i) perm[size_t(i)] = i;
-  std::stable_sort(perm.begin(), perm.end(), [&](int32_t a, int32_t b) { return norm(a) < norm(b); });
+  TenantBatch b(tenants, nq);
   frg_match_params_t pg = *p;
-  if (norm(perm.front()) == norm(perm.back())) {            // one tenant: exactly frg_match
-    pg.tenant = norm(perm.front());
+  if (b.one_tenant()) {                                     // one tenant: exactly frg_match
+    pg.tenant = b.runs[0].tenant;
     return match_impl(s, q, nq, k, &pg, out_rows, out_scores, out_accept, st, ExchangeTail());
-  }
-  std::vector<TcTenantGroup> groups;
-  for (int32_t i = 0; i < nq;) {
-    int32_t j = i + 1;
-    while (j < nq && norm(perm[size_t(j)]) == norm(perm[size_t(i)])) ++j;
-    TcTenantGroup g{};
-    g.tenant = norm(perm[size_t(i)]); g.q0 = i; g.nq = j - i;
-    groups.push_back(g);
-    i = j;
   }
   DeviceGuard dg(s->device);
   if (!dg.ok) { set_error("cannot select device %d", s->device); return FRG_ERR_CUDA; }
@@ -1055,23 +1101,71 @@ static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
   FRG_CHECK(device_info(s->device, &di));
   std::lock_guard<std::mutex> lk(s->mu);    // one snapshot of the store for every tenant of the call
   FRG_CHECK(store_begin_read(s, st));
+  b.find_windows(s);
+  const int dim = s->dim;
   const int variant = pick_variant(s, p, nq);
   const char* why = "";
   const bool grouped = (variant == FRG_VARIANT_TC_EXACT || variant == FRG_VARIANT_TC_BF16) && has_plane8(s) &&
                        s->master && p->metric == FRG_METRIC_COSINE && !(p->flags & FRG_QUERY_PRENORMALISED) &&
-                       tc_supported(s->dim, p->metric, &why) && s->rows > 0 && s->rows <= 0x7fffffff;
+                       tc_supported(dim, p->metric, &why) && s->rows > 0 && s->rows <= 0x7fffffff;
   if (grouped) {
+    // gather -> int8 prep -> pre-pass, floor, filter, select (launch_tc_match_grouped) -> per-query-tenant exact
+    // re-do of the overflowed queries -> scatter, one set of launches for every tenant
     struct SeqBump { ~SeqBump() { ++g_match_seq; } } bump;
-    for (TcTenantGroup& g : groups) FRG_CHECK(tenant_tiles(s, g.tenant, st, &g));
+    std::vector<TcTenantGroup> tiles;
+    FRG_CHECK(b.query_tiles(s, st, &tiles));
+    TcGroupPlan plan;
+    tc_group_plan(tiles, k, dim, di.sm_count, &plan);
+    const std::vector<unsigned char> table = b.table(plan.ctas);
+    Carve c;
+    const size_t o_qs = c.take(size_t(nq) * dim * 4), o_qn = c.take(size_t(nq) * dim * 4), o_table = c.take(table.size());
+    const size_t o_qi8 = c.take(size_t(nq) * dim), o_eps = c.take(size_t(nq) * 4), o_step = c.take(size_t(nq) * 4);
+    const size_t o_rows = c.take(size_t(nq) * k * 8), o_sc = c.take(size_t(nq) * k * 4), o_acc = c.take(size_t(nq));
+    const size_t o_tc = c.take(tc_range_workspace(nq, plan.cand_entries, plan.dense_cap, nullptr, nullptr));
+    unsigned char* ws = nullptr;
+    FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
+    float* qs = reinterpret_cast<float*>(ws + o_qs);
+    float* qn = reinterpret_cast<float*>(ws + o_qn);
+    const int32_t* dperm = reinterpret_cast<const int32_t*>(ws + o_table);
+    const int32_t* dten = dperm + nq;
+    int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
+    float* eps = reinterpret_cast<float*>(ws + o_eps);
+    float* qstep = reinterpret_cast<float*>(ws + o_step);
+    int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
+    float* sscores = reinterpret_cast<float*>(ws + o_sc);
+    uint8_t* sacc = ws + o_acc;
+    TcRangeWs tw;
+    tc_range_workspace(nq, plan.cand_entries, plan.dense_cap, ws + o_tc, &tw);
+    int rc = stage_upload(ws + o_table, table.data(), table.size(), st);
+    if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, dim, qs, st);
+    profile_begin(st, kStagePrep);
+    if (rc == FRG_OK)
+      rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
+                                     tw.n_flagged, st);
+    profile_end(st, 1);
     const GalleryWindow w = window_of(s, -1);
-    FRG_CHECK(launch_tc_match_grouped(&w, q, perm, groups, k, p->threshold, p->row_offset, di.sm_count, out_rows,
-                                      out_scores, out_accept, st));
-    g_variant = "tc_exact_grouped";
-    return FRG_OK;
+    if (rc == FRG_OK)
+      rc = launch_tc_match_grouped(&w, qn, qi8, qstep, eps, nq, ws + o_table + b.cta_offset(), plan.n_pre, plan.n_main,
+                                   k, p->threshold, p->row_offset, tw, srows, sscores, sacc, st);
+    profile_begin(st, kStageFallback);
+    if (rc == FRG_OK) {
+      ScanArgs a;
+      a.master = s->master; a.plane = nullptr; a.tags = s->tags; a.rows = s->rows; a.dim = dim;
+      a.qn = qn; a.nq = nq; a.k = k; a.metric = FRG_METRIC_COSINE; a.tenant = -1; a.sm_count = di.sm_count;
+      rc = launch_scan_f32_flagged_tenants(a, dten, tw.flagged, tw.n_flagged, p->row_offset, p->threshold, srows,
+                                           sscores, sacc, st);
+    }
+    profile_end(st, 1);
+    if (rc == FRG_OK) rc = launch_scatter_sorted(srows, sscores, sacc, dperm, nq, k, out_rows, out_scores, out_accept, st);
+    if (rc == FRG_OK) { cudaError_t e = cudaGetLastError(); if (e != cudaSuccess) rc = cuda_fail(e, "grouped match", __FILE__, __LINE__); }
+    cudaError_t e = cudaFreeAsync(ws, st);
+    if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+    if (rc == FRG_OK) g_variant = "tc_exact_grouped";
+    return rc;
   }
   // every other store / variant: frg_match's own path once per tenant, into tenant-sorted scratch, then scattered
   Carve c;
-  const size_t o_qs = c.take(size_t(nq) * s->dim * 4), o_perm = c.take(size_t(nq) * 4);
+  const size_t o_qs = c.take(size_t(nq) * dim * 4), o_perm = c.take(size_t(nq) * 4);
   const size_t o_rows = c.take(size_t(nq) * k * 8), o_sc = c.take(size_t(nq) * k * 4), o_acc = c.take(size_t(nq));
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
@@ -1080,16 +1174,16 @@ static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
   int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
   float* sscores = reinterpret_cast<float*>(ws + o_sc);
   uint8_t* sacc = ws + o_acc;
-  int rc = stage_upload(dperm, perm.data(), size_t(nq) * 4, st);
-  if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, s->dim, qs, st);
-  for (size_t i = 0; rc == FRG_OK && i < groups.size(); ++i) {
-    pg.tenant = groups[i].tenant;
-    const int q0 = groups[i].q0;
-    rc = match_locked(s, qs + size_t(q0) * s->dim, groups[i].nq, k, &pg, srows + size_t(q0) * k,
-                      sscores + size_t(q0) * k, sacc + q0, st, ExchangeTail(), di.sm_count);
+  int rc = stage_upload(dperm, b.perm.data(), size_t(nq) * 4, st);
+  if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, dim, qs, st);
+  for (size_t i = 0; rc == FRG_OK && i < b.runs.size(); ++i) {
+    const TenantBatch::Run& r = b.runs[i];
+    pg.tenant = r.tenant;
+    rc = match_locked(s, qs + size_t(r.q0) * dim, r.nq, k, &pg, srows + size_t(r.q0) * k, sscores + size_t(r.q0) * k,
+                      sacc + r.q0, st, ExchangeTail(), di.sm_count);
   }
   const char* ran = g_variant;               // the per-tenant path that ran (the scatter does not rename it)
-  if (rc == FRG_OK) rc = launch_scatter_results(srows, sscores, sacc, dperm, nq, k, out_rows, out_scores, out_accept, st);
+  if (rc == FRG_OK) rc = launch_scatter_sorted(srows, sscores, sacc, dperm, nq, k, out_rows, out_scores, out_accept, st);
   g_variant = ran;
   cudaError_t e = cudaFreeAsync(ws, st);
   if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
@@ -1476,14 +1570,14 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
     if (plan_rows < 0) return FRG_ERR_CUDA;
     const int64_t cand = tc_range_cand_entries(plan_rows, w.dim, nq, di.sm_count);
     const size_t o_qi8 = c.take(size_t(nq) * w.dim), o_eps = c.take(size_t(nq) * sizeof(float));
-    const size_t o_step = c.take(size_t(nq) * sizeof(float)), o_tc = c.take(tc_range_workspace(nq, cand, nullptr, nullptr));
+    const size_t o_step = c.take(size_t(nq) * sizeof(float)), o_tc = c.take(tc_range_workspace(nq, cand, kRangeBudget, nullptr, nullptr));
     FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
     float* qn = reinterpret_cast<float*>(ws + o_qn);
     int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
     float* eps = reinterpret_cast<float*>(ws + o_eps);
     float* qstep = reinterpret_cast<float*>(ws + o_step);
     TcRangeWs tw;
-    tc_range_workspace(nq, cand, ws + o_tc, &tw);
+    tc_range_workspace(nq, cand, kRangeBudget, ws + o_tc, &tw);
     profile_begin(st, kStagePrep);
     rc = launch_prepare_queries_i8(q, nq, w.dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
                                    tw.n_flagged, st);
@@ -1539,11 +1633,10 @@ int frg_match_range_host(frg_store* s, const float* q, int32_t nq, int32_t max_h
 }
 
 // --------------------------------------------------------------------------------------------- range search, per-query tenants
-// The batch is sorted stably by tenant (perm[i] = caller position of sorted query i), and every tenant runs in one set
-// of launches: gather the queries in tenant order, then
-//   tensor-core path (where range_impl takes it): int8 query prep -> floor -> GROUPED filter over query tiles of at
-//     most 128 queries of one tenant, each scanning its tenant's tiles (tenant_tiles) -> range_select_kernel -> the
-//     per-query-tenant exact scan of the queries whose candidates overflowed;
+// The batch is sorted stably by tenant (TenantBatch), and every tenant runs in one set of launches: gather the queries
+// in tenant order, then
+//   tensor-core path (where range_impl takes it): int8 query prep -> floor -> GROUPED filter over the batch's query
+//     tiles -> range_select_kernel -> the per-query-tenant exact scan of the queries whose candidates overflowed;
 //   exact path: normalise -> that exact scan over every query, each reading its tenant's row window;
 // and scatter the sorted results into the caller's order.
 static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits, const frg_match_params_t* p,
@@ -1554,13 +1647,10 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     set_error("match_range_tenants: bad argument");
     return FRG_ERR_INVALID;
   }
-  auto norm = [&](int32_t i) { return tenants[i] < 0 ? int32_t(-1) : tenants[i]; };
-  std::vector<int32_t> perm(static_cast<size_t>(nq));
-  for (int32_t i = 0; i < nq; ++i) perm[size_t(i)] = i;
-  std::stable_sort(perm.begin(), perm.end(), [&](int32_t a, int32_t b) { return norm(a) < norm(b); });
-  if (nq > 0 && norm(perm.front()) == norm(perm.back())) {           // one tenant: exactly frg_match_range
+  TenantBatch b(tenants, nq);
+  if (b.one_tenant()) {                                              // one tenant: exactly frg_match_range
     frg_match_params_t pg = *p;
-    pg.tenant = norm(perm.front());
+    pg.tenant = b.runs[0].tenant;
     return range_impl(s, q, nq, max_hits, &pg, out_counts, out_rows, out_scores, st);
   }
   bool use_tc = false;
@@ -1573,50 +1663,16 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
   FRG_CHECK(device_info(s->device, &di));
   std::lock_guard<std::mutex> lk(s->mu);    // one snapshot of the store for every tenant of the call
   FRG_CHECK(store_begin_read(s, st));
+  b.find_windows(s);
   const int dim = s->dim;
   const bool tc = use_tc && s->rows > 0;
-  // the one upload: [perm][tenant of each sorted query][window lo][window hi][filter descriptors]
-  const size_t t_ten = size_t(nq) * 4, t_lo = t_ten + size_t(nq) * 4, t_hi = t_lo + size_t(nq) * 4;
-  const size_t t_cta = (t_hi + size_t(nq) * 4 + 15) & ~size_t(15);
-  std::vector<unsigned char> table(t_cta);
-  memcpy(table.data(), perm.data(), size_t(nq) * 4);
-  std::vector<TcTenantGroup> units;          // the filter's query tiles
-  for (int32_t i = 0; i < nq;) {
-    const int32_t t = norm(perm[size_t(i)]);
-    int32_t j = i + 1;
-    while (j < nq && norm(perm[size_t(j)]) == t) ++j;
-    // the rows tenant t can sit in: window_of's bounding window (every row for t < 0 or unknown extents)
-    int64_t lo = 0, hi = s->rows;
-    if (t >= 0 && s->extents_known) {
-      auto it = s->extents.find(t);
-      lo = hi = 0;
-      if (it != s->extents.end()) { lo = it->second.lo; hi = it->second.hi < s->rows ? it->second.hi : s->rows; }
-      if (hi < lo) hi = lo;
-    }
-    const int32_t lo32 = int32_t(lo), hi32 = int32_t(hi);
-    for (int32_t x = i; x < j; ++x) {
-      memcpy(table.data() + t_ten + size_t(x) * 4, &t, 4);
-      memcpy(table.data() + t_lo + size_t(x) * 4, &lo32, 4);
-      memcpy(table.data() + t_hi + size_t(x) * 4, &hi32, 4);
-    }
-    if (tc) {
-      TcTenantGroup G{};
-      G.tenant = t;
-      FRG_CHECK(tenant_tiles(s, t, st, &G));
-      for (int32_t a = i; a < j; a += kTcTileRows) {
-        G.q0 = a; G.nq = j - a < kTcTileRows ? j - a : kTcTileRows;
-        units.push_back(G);
-      }
-    }
-    i = j;
-  }
-  int n_ctas = 0;
-  int64_t cand = 1;
+  TcGroupPlan plan;
   if (tc) {
-    std::vector<unsigned char> cta_bytes;
-    tc_join_plan(units, di.sm_count, &cta_bytes, &n_ctas, &cand);
-    table.insert(table.end(), cta_bytes.begin(), cta_bytes.end());
+    std::vector<TcTenantGroup> tiles;
+    FRG_CHECK(b.query_tiles(s, st, &tiles));
+    tc_group_plan(tiles, 0, dim, di.sm_count, &plan);
   }
+  const std::vector<unsigned char> table = b.table(plan.ctas);
   // ---- workspace: sorted queries, the table, the sorted results and the tensor-core path's pieces
   const size_t slots = size_t(nq) * size_t(max_hits);
   Carve c;
@@ -1625,16 +1681,16 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
   size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_tc = 0;
   if (tc) {
     o_qi8 = c.take(size_t(nq) * dim); o_eps = c.take(size_t(nq) * 4); o_step = c.take(size_t(nq) * 4);
-    o_tc = c.take(tc_range_workspace(nq, cand, nullptr, nullptr));
+    o_tc = c.take(tc_range_workspace(nq, plan.cand_entries, kRangeBudget, nullptr, nullptr));
   }
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
   float* qs = reinterpret_cast<float*>(ws + o_qs);
   float* qn = reinterpret_cast<float*>(ws + o_qn);
   const int32_t* dperm = reinterpret_cast<const int32_t*>(ws + o_table);
-  const int32_t* dten = reinterpret_cast<const int32_t*>(ws + o_table + t_ten);
-  const int32_t* dlo = reinterpret_cast<const int32_t*>(ws + o_table + t_lo);
-  const int32_t* dhi = reinterpret_cast<const int32_t*>(ws + o_table + t_hi);
+  const int32_t* dten = dperm + nq;
+  const int32_t* dlo = dperm + 2 * size_t(nq);
+  const int32_t* dhi = dperm + 3 * size_t(nq);
   int64_t* scnt = reinterpret_cast<int64_t*>(ws + o_cnt);
   int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
   float* sscores = reinterpret_cast<float*>(ws + o_sc);
@@ -1649,7 +1705,7 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     float* eps = reinterpret_cast<float*>(ws + o_eps);
     float* qstep = reinterpret_cast<float*>(ws + o_step);
     TcRangeWs tw;
-    tc_range_workspace(nq, cand, ws + o_tc, &tw);
+    tc_range_workspace(nq, plan.cand_entries, kRangeBudget, ws + o_tc, &tw);
     profile_begin(st, kStagePrep);
     if (rc == FRG_OK)
       rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
@@ -1657,8 +1713,8 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     profile_end(st, 1);
     const GalleryWindow w = window_of(s, -1);
     if (rc == FRG_OK)
-      rc = launch_tc_range_grouped(&w, qn, qi8, qstep, eps, nq, ws + o_table + t_cta, n_ctas, max_hits, p->threshold,
-                                   strict, p->row_offset, tw, scnt, srows, sscores, st);
+      rc = launch_tc_range_grouped(&w, qn, qi8, qstep, eps, nq, ws + o_table + b.cta_offset(), plan.n_main, max_hits,
+                                   p->threshold, strict, p->row_offset, tw, scnt, srows, sscores, st);
     profile_begin(st, kStageFallback);
     if (rc == FRG_OK)
       rc = launch_range_tenants_scan(a, dten, dlo, dhi, tw.flagged, tw.n_flagged, max_hits, p->threshold, strict,
@@ -1674,7 +1730,7 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
                                      p->row_offset, scnt, srows, sscores, st);
     profile_end(st, 3);
   }
-  if (rc == FRG_OK) rc = launch_scatter_range(scnt, srows, sscores, dperm, nq, max_hits, out_counts, out_rows, out_scores, st);
+  if (rc == FRG_OK) rc = launch_scatter_sorted(srows, sscores, scnt, dperm, nq, max_hits, out_rows, out_scores, out_counts, st);
   g_variant = tc ? "range_tc_grouped" : "range_scan_tenants";
   cudaError_t e = cudaFreeAsync(ws, st);
   if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
@@ -1724,9 +1780,8 @@ static void join_plan_tiles(const frg_store* s, int64_t row0, int64_t n, int32_t
   out->assign(size_t(nt), JoinTile{tenant >= 0 ? tenant : -1, int32_t(rows)});
   if (!s->extents_known || (tenant < 0 && !same_tag)) return;
   if (tenant >= 0) {
-    auto it = s->extents.find(tenant);
-    const int64_t lo = it != s->extents.end() ? it->second.lo : 0;
-    const int64_t hi = it != s->extents.end() ? (it->second.hi < rows ? it->second.hi : rows) : 0;
+    const frg_store::Extent x = tenant_rows(s, tenant);
+    const int64_t lo = x.lo, hi = x.hi;
     for (int64_t u = 0; u < nt; ++u) {
       const int64_t R = row0 + u * kTcTileRows, Re = R + kTcTileRows < row0 + n ? R + kTcTileRows : row0 + n;
       (*out)[size_t(u)].end_row = int32_t(hi > lo && Re > lo && R < hi ? hi : R);
@@ -1809,11 +1864,9 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
   for (int64_t s0 = 0; s0 < n; s0 += S) {
     const int64_t ns = n - s0 < S ? n - s0 : S;
     const int64_t u0 = s0 / kTcTileRows, nu = (ns + kTcTileRows - 1) / kTcTileRows;
-    std::vector<TcTenantGroup> tiles;
-    std::vector<unsigned char> cta_bytes;
-    int n_ctas = 0;
-    int64_t cand = 0;
+    TcGroupPlan gp;
     if (use_tc) {
+      std::vector<TcTenantGroup> tiles;
       for (int64_t u = 0; u < nu; ++u) {
         const JoinTile& t = plan[size_t(u0 + u)];
         const int64_t R = row0 + (u0 + u) * kTcTileRows;
@@ -1824,15 +1877,15 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
         G.list = nullptr;
         tiles.push_back(G);
       }
-      tc_join_plan(tiles, di.sm_count, &cta_bytes, &n_ctas, &cand);
+      tc_group_plan(tiles, 0, dim, di.sm_count, &gp);
     }
-    std::vector<unsigned char> table(t_cta + cta_bytes.size(), 0);
+    std::vector<unsigned char> table(t_cta + gp.ctas.size(), 0);
     for (int64_t u = 0; u < nu; ++u) memcpy(table.data() + u * 4, &plan[size_t(u0 + u)].end_row, 4);
-    if (!cta_bytes.empty()) memcpy(table.data() + t_cta, cta_bytes.data(), cta_bytes.size());
-    if (cand > max_cand) max_cand = cand;
+    if (!gp.ctas.empty()) memcpy(table.data() + t_cta, gp.ctas.data(), gp.ctas.size());
+    if (gp.cand_entries > max_cand) max_cand = gp.cand_entries;
     if (table.size() > max_table) max_table = table.size();
     tables.push_back(std::move(table));
-    ctas.push_back(n_ctas);
+    ctas.push_back(gp.n_main);
   }
   // ---- one workspace for every slab
   ScanArgs a;
@@ -1844,12 +1897,12 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
   size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_tc = 0;
   if (use_tc) {
     o_qi8 = c.take(size_t(S) * dim); o_eps = c.take(size_t(S) * 4); o_step = c.take(size_t(S) * 4);
-    o_tc = c.take(tc_range_workspace(int(S), max_cand, nullptr, nullptr));
+    o_tc = c.take(tc_range_workspace(int(S), max_cand, kRangeBudget, nullptr, nullptr));
   }
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
   TcRangeWs tw{};
-  if (use_tc) tc_range_workspace(int(S), max_cand, ws + o_tc, &tw);
+  if (use_tc) tc_range_workspace(int(S), max_cand, kRangeBudget, ws + o_tc, &tw);
   float* qn = reinterpret_cast<float*>(ws + o_qn);
   const int32_t* tile_end = reinterpret_cast<const int32_t*>(ws + o_table);
   a.qn = qn;

@@ -366,19 +366,28 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
                     const __nv_bfloat16* qb_prepass = nullptr, const float* coef = nullptr,
                     const int8_t* qi8 = nullptr, const float* qstep = nullptr);
 
-// tc_match.cu: per-query tenants (frg_match_tenants) on the int8 filter of a unit cosine store.  The batch is sorted by
-// tenant (perm[i] = caller position of sorted query i); group g holds sorted queries q0 .. q0 + nq - 1 of one tenant and
-// scans the absolute kTcTileRows-row tiles list[0 .. n_tiles) or tile0 .. tile0 + n_tiles - 1 (a masked range).  One
-// grid per stage serves every group; results go to the caller's order.  s: the whole store (row0 = 0).
+// ---- the GROUPED int8 filter grid (per-query tenants, self-join).  A query tile holds queries q0 .. q0 + nq - 1
+// (nq <= kTcTileRows) of one tenant (the filter masks with it; -1 = none), which scan the absolute kTcTileRows-row
+// tiles list[0 .. n_tiles) or tile0 .. tile0 + n_tiles - 1 (a masked range).
 constexpr int kTcTileRows = 128;
 struct TcTenantGroup { int32_t tenant; int q0, nq; int tile0, n_tiles; const int32_t* list; };
-int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::vector<int32_t>& perm,
-                            const std::vector<TcTenantGroup>& groups, int k, float threshold, int64_t row_offset,
-                            int sm_count, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st);
-// tc_match.cu: out[i] = q[perm[i]] (rows of dim floats); out[perm[i]] = sorted result i (rows / scores [nq][k], accept)
+// tc_match.cu, host: the grid's CTA descriptors over the query tiles.  k >= 1 (top-k): each tile takes the pre-pass
+// stride and candidate budget of a single-tenant tc_plan over its tiles, and the grid has a pre-pass; k = 0 (range
+// search, self-join): kRangeBudget candidates per query, no pre-pass.
+struct TcGroupPlan {
+  std::vector<unsigned char> ctas;    // [n_pre pre-pass descriptors][n_main filter descriptors]
+  int n_pre = 0, n_main = 0;
+  int64_t cand_entries = 0;           // candidate segment entries (int2) the filter grid writes
+  int dense_cap = 0;                  // dense list entries per query
+};
+void tc_group_plan(const std::vector<TcTenantGroup>& tiles, int k, int dim, int sm_count, TcGroupPlan* out);
+// tc_match.cu: out[i] = q[perm[i]] (rows of dim floats)
 int launch_gather_queries(const float* q, const int32_t* perm, int nq, int dim, float* out, cudaStream_t st);
-int launch_scatter_results(const int64_t* rows, const float* scores, const uint8_t* accept, const int32_t* perm, int nq,
-                           int k, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st);
+// tc_match.cu: out[perm[i]] = sorted result i: rows / scores [nq][width] and field[nq] (F = uint8_t: top-k's accept,
+// out_field may be null; F = int64_t: range search's counts)
+template <typename F>
+int launch_scatter_sorted(const int64_t* rows, const float* scores, const F* field, const int32_t* perm, int nq,
+                          int width, int64_t* out_rows, float* out_scores, F* out_field, cudaStream_t st);
 // scan_f32.cu: the exact re-do of launch_scan_f32_flagged, each flagged query q with its own tenant q_tenant[q]
 // (device array; cosine, fp32 master, a.tenant ignored)
 int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, const int* flagged,
@@ -390,20 +399,32 @@ int stage_upload(void* dev, const void* host, size_t bytes, cudaStream_t st);
 // Candidate entries per query of a range-mode filter (range search and self-join; DESIGN.md section 7.3)
 constexpr int kRangeBudget = 4096;
 
-// tc_match.cu: the workspace of a range-mode int8 filter call (range search, or one self-join slab) of nq queries
+// tc_match.cu: the workspace of an int8 filter call without a top-k plan of its own (range search, one self-join slab,
+// a per-query-tenant batch) of nq queries
 struct TcRangeWs {
   unsigned long long* keys;   // [nq][32] group keys (the query prep resets them)
   int* cand_total;            // [nq] candidates per query
   int* flagged;               // [nq] queries whose candidates overflowed, then their count and the fallback's ticket
   int* n_flagged;             // flagged + nq
   float* floor;               // [nq] threshold - eps[q]
-  int2* dense;                // [nq][kRangeBudget] packed candidates
+  int2* dense;                // [nq][dense_cap] packed candidates
   int2* cand;                 // the filter's candidate segments
+  int dense_cap;              // kRangeBudget in range mode
 };
 // Bytes of that workspace when the filter writes cand_entries segment entries (int2); with ws, its pieces in *out.
-size_t tc_range_workspace(int nq, int64_t cand_entries, unsigned char* ws, TcRangeWs* out);
-// the candidate segment entries of range search's filter over plan_rows rows (the self-join's: tc_join_plan)
+size_t tc_range_workspace(int nq, int64_t cand_entries, int dense_cap, unsigned char* ws, TcRangeWs* out);
+// the candidate segment entries of range search's filter over plan_rows rows (the grouped grid's: tc_group_plan)
 int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count);
+
+// tc_match.cu: top-k with a tenant per query (frg_match_tenants) on the int8 filter of a unit cosine store, over the
+// tenant-sorted batch: qn / qi8 / qstep / eps from launch_prepare_queries_i8 (which reset w's keys and counters),
+// d_ctas the uploaded descriptors of tc_group_plan (k >= 1; n_pre pre-pass, then n_main filter).  Pre-pass, floor,
+// filter and select-rescore into out_* (sorted order); queries whose candidates overflowed are left in (w.flagged,
+// w.n_flagged) for launch_scan_f32_flagged_tenants.  s: the whole store.
+int launch_tc_match_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
+                            const float* eps, int nq, const void* d_ctas, int n_pre, int n_main, int k, float threshold,
+                            int64_t row_offset, const TcRangeWs& w, int64_t* out_rows, float* out_scores,
+                            uint8_t* out_accept, cudaStream_t st);
 
 // tc_match.cu: range search over a unit cosine store (frg_match_range).  The filter keeps every row with
 // S >= threshold - eps[q] (no pre-pass); range_select_kernel rescores each candidate exactly, keeps those that pass
@@ -431,27 +452,19 @@ int launch_range_tenants_scan(const ScanArgs& a, const int32_t* q_tenant, const 
                               const int* flagged, const int* n_flagged, int max_hits, float threshold, bool strict,
                               int64_t row_offset, int64_t* out_counts, int64_t* out_rows, float* out_scores,
                               cudaStream_t st);
-// tc_match.cu: launch_tc_range's path with the GROUPED filter over the uploaded table (d_table, n_ctas from tc_join_plan
-// over the query tiles; none when 0): each descriptor's tenant masks the other tenants' rows.  Queries whose candidates
-// overflowed are left in (w.flagged, w.n_flagged) for launch_range_tenants_scan.  s: the whole store.
+// tc_match.cu: launch_tc_range's path with the GROUPED filter over the uploaded descriptors (d_table, n_ctas from
+// tc_group_plan in range mode; none when 0).  Queries whose candidates overflowed are left in (w.flagged, w.n_flagged)
+// for launch_range_tenants_scan.  s: the whole store.
 int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
                             const float* eps, int nq, const void* d_table, int n_ctas, int max_hits, float threshold,
                             bool strict, int64_t row_offset, const TcRangeWs& w, int64_t* out_counts,
                             int64_t* out_rows, float* out_scores, cudaStream_t st);
-// tc_match.cu: out[perm[i]] = sorted range result i ([nq] counts, [nq][max_hits] rows and scores)
-int launch_scatter_range(const int64_t* counts, const int64_t* rows, const float* scores, const int32_t* perm, int nq,
-                         int max_hits, int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st);
 
 // ---- gallery self-join (frg_self_join): the queries are the store's own rows qrow0 .. qrow0 + nq - 1 of one slab,
 // and a pair (a, b) counts only for b > a (plus the tag rule: tenant >= 0 -> both rows carry it; same_tag -> tag[b] ==
 // tag[a]).  Query tile u of the slab holds queries 128u .. 128u + 127.
-// tc_match.cu, host: descriptor table of the slab's GROUPED filter grid (tiles[u]: tenant the filter masks with, -1 =
-// none, and the absolute gallery tiles tile0 .. tile0 + n_tiles - 1 of query tile u; q0 / nq: its queries), the
-// number of CTAs and the candidate segment entries (int2) the grid writes.  The planner of launch_tc_match_grouped.
-void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::vector<unsigned char>* table,
-                  int* n_ctas, int64_t* cand_entries);
-// tc_match.cu: the int8 filter path of one slab, launch_tc_range's with the GROUPED filter over the uploaded table
-// (d_table, n_ctas; none when 0) and join_select_kernel (exact rescoring, b > a, tag rule, counts and the first
+// tc_match.cu: the int8 filter path of one slab, launch_tc_range's with the GROUPED filter over the uploaded
+// descriptors (d_table, n_ctas from tc_group_plan in range mode; none when 0) and join_select_kernel (exact rescoring, b > a, tag rule, counts and the first
 // max_hits hits in gallery order).  Queries whose candidates overflowed are left in (w.flagged, w.n_flagged) for
 // launch_join_scan.  s: the whole store.
 int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,

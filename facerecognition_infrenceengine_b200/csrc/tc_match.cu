@@ -1384,13 +1384,14 @@ int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count) 
   return int64_t(nq) * pl.chunks_main * (kEpiWarps / 4) * pl.seg;
 }
 
-size_t tc_range_workspace(int nq, int64_t cand_entries, unsigned char* ws, TcRangeWs* out) {
+size_t tc_range_workspace(int nq, int64_t cand_entries, int dense_cap, unsigned char* ws, TcRangeWs* out) {
   Carve c;
   const size_t o_keys = c.take(size_t(nq) * kGroups * 8), o_cnt = c.take(size_t(nq) * 4);
   const size_t o_flag = c.take(size_t(nq) * 4 + 12);     // flagged[nq], count, ticket, probe-arrival counter
-  const size_t o_floor = c.take(size_t(nq) * 4), o_dense = c.take(size_t(nq) * kRangeBudget * 8);
+  const size_t o_floor = c.take(size_t(nq) * 4), o_dense = c.take(size_t(nq) * dense_cap * 8);
   const size_t o_cand = c.take(size_t(cand_entries) * 8);
   if (ws) {
+    out->dense_cap = dense_cap;
     out->keys = reinterpret_cast<unsigned long long*>(ws + o_keys);
     out->cand_total = reinterpret_cast<int*>(ws + o_cnt);
     out->flagged = reinterpret_cast<int*>(ws + o_flag);
@@ -1719,20 +1720,22 @@ gather_queries_kernel(const float* __restrict__ q, const int32_t* __restrict__ p
   for (int v = lane; v < (dim >> 2); v += 32) dst[v] = __ldg(src + v);
 }
 
-// results of sorted query i -> the caller's slot perm[i]
+// results of sorted query i -> the caller's slot perm[i]: `width` rows and scores, and the per-query field (top-k's
+// accept byte, range search's count; out_field == nullptr: none)
+template <typename F>
 __global__ void __launch_bounds__(256)
-scatter_results_kernel(const int64_t* __restrict__ rows, const float* __restrict__ scores,
-                       const uint8_t* __restrict__ accept, const int32_t* __restrict__ perm, int nq, int k,
-                       int64_t* __restrict__ out_rows, float* __restrict__ out_scores, uint8_t* __restrict__ out_accept) {
+scatter_sorted_kernel(const int64_t* __restrict__ rows, const float* __restrict__ scores, const F* __restrict__ field,
+                      const int32_t* __restrict__ perm, int nq, int width, int64_t* __restrict__ out_rows,
+                      float* __restrict__ out_scores, F* __restrict__ out_field) {
   pdl_wait();
   pdl_trigger();
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= nq * k) return;
-  const int q = i / k, j = i - q * k;
-  const size_t o = size_t(__ldg(perm + q)) * k + j;
-  out_rows[o] = rows[i];
-  out_scores[o] = scores[i];
-  if (out_accept && j == 0) out_accept[o / k] = accept[q];
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= int64_t(nq) * width) return;
+  const int q = int(i / width), j = int(i - int64_t(q) * width);
+  const int dst = __ldg(perm + q);
+  out_rows[size_t(dst) * width + j] = rows[i];
+  out_scores[size_t(dst) * width + j] = scores[i];
+  if (out_field && j == 0) out_field[dst] = field[q];
 }
 
 int launch_gather_queries(const float* q, const int32_t* perm, int nq, int dim, float* out, cudaStream_t st) {
@@ -1742,17 +1745,23 @@ int launch_gather_queries(const float* q, const int32_t* perm, int nq, int dim, 
   return FRG_OK;
 }
 
-int launch_scatter_results(const int64_t* rows, const float* scores, const uint8_t* accept, const int32_t* perm, int nq,
-                           int k, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st) {
+template <typename F>
+int launch_scatter_sorted(const int64_t* rows, const float* scores, const F* field, const int32_t* perm, int nq,
+                          int width, int64_t* out_rows, float* out_scores, F* out_field, cudaStream_t st) {
   if (nq <= 0) return FRG_OK;
-  FRG_CUDA(launch_kernel(scatter_results_kernel, dim3((nq * k + 255) / 256), dim3(256), 0, st, rows, scores, accept,
-                         perm, nq, k, out_rows, out_scores, out_accept));
+  const int64_t n = int64_t(nq) * width;
+  FRG_CUDA(launch_kernel(scatter_sorted_kernel<F>, dim3(unsigned((n + 255) / 256)), dim3(256), 0, st, rows, scores,
+                         field, perm, nq, width, out_rows, out_scores, out_field));
   note_launch(nullptr);
   return FRG_OK;
 }
+template int launch_scatter_sorted(const int64_t*, const float*, const uint8_t*, const int32_t*, int, int, int64_t*,
+                                   float*, uint8_t*, cudaStream_t);
+template int launch_scatter_sorted(const int64_t*, const float*, const int64_t*, const int32_t*, int, int, int64_t*,
+                                   float*, int64_t*, cudaStream_t);
 
-// Chunks of each unit in proportion to its tiles, so that the whole grid stays near one wave of sm_count CTAs
-// (at least one chunk per unit, at most one per tile).
+// Chunks of each query tile in proportion to its tiles, so that the whole grid stays near one wave of sm_count CTAs
+// (at least one chunk per query tile, at most one per tile).
 static std::vector<int> proportional_chunks(const std::vector<int>& tiles, int sm_count) {
   int64_t total = 0;
   for (int t : tiles) total += t;
@@ -1767,158 +1776,95 @@ static std::vector<int> proportional_chunks(const std::vector<int>& tiles, int s
   return c;
 }
 
-// One query tile of a GROUPED grid: queries q0 .. q0 + nq - 1 (nq <= kTileQ) of src's tenant, which scan src's tiles
-// with `entries` candidates per query and (pre-pass) every stride-th tile.
-struct GroupUnit { const TcTenantGroup* src; int q0, nq, entries, stride; };
-
-// The descriptors of a GROUPED filter grid (main) and, when pre != nullptr, of its pre-pass grid: each unit's tiles cut
-// into chunks in proportion to its share of all tiles, its candidate segments one per (query, chunk, column half) with
-// x2 headroom (as tc_plan).  Returns the candidate entries (int2) the filter grid writes.
-static int64_t plan_group_ctas(const std::vector<GroupUnit>& units, int sm_count, std::vector<TcGroupCta>* pre,
-                               std::vector<TcGroupCta>* main) {
-  std::vector<int> tiles_main(units.size()), tiles_pre(units.size());
-  for (size_t u = 0; u < units.size(); ++u) {
-    tiles_main[u] = units[u].src->n_tiles;
-    tiles_pre[u] = (tiles_main[u] + units[u].stride - 1) / units[u].stride;
+// Each query tile's tiles cut into chunks in proportion to its share of all tiles, its candidate segments one per
+// (query, chunk, column half) with x2 headroom (as tc_plan).
+void tc_group_plan(const std::vector<TcTenantGroup>& tiles, int k, int dim, int sm_count, TcGroupPlan* out) {
+  const size_t n = tiles.size();
+  std::vector<int> entries(n, kRangeBudget), stride(n, 1), tiles_main(n), tiles_pre(n);
+  out->dense_cap = k > 0 ? 256 : kRangeBudget;
+  for (size_t u = 0; u < n; ++u) {
+    if (k > 0) {
+      // the plan of a single-tenant match over the same tiles (tc_plan): pre-pass stride and candidate budget
+      TcPlan pl;
+      tc_plan(int64_t(tiles[u].n_tiles) * kTileR, dim, 1, k, sm_count, &pl, false, true);
+      stride[u] = pl.stride;
+      entries[u] = pl.stage_entries;
+      if (pl.stage_entries > out->dense_cap) out->dense_cap = pl.stage_entries;
+    }
+    tiles_main[u] = tiles[u].n_tiles;
+    tiles_pre[u] = (tiles_main[u] + stride[u] - 1) / stride[u];
   }
   const std::vector<int> ch_main = proportional_chunks(tiles_main, sm_count);
   const std::vector<int> ch_pre = proportional_chunks(tiles_pre, sm_count);
-  int64_t cand_entries = 0;
-  for (size_t u = 0; u < units.size(); ++u) {
-    const TcTenantGroup& G = *units[u].src;
-    if (tiles_main[u] == 0) continue;                  // an unknown tag: no rows, nothing to scan
+  std::vector<TcGroupCta> pre, main;
+  out->cand_entries = 0;
+  for (size_t u = 0; u < n; ++u) {
+    const TcTenantGroup& G = tiles[u];
+    if (G.n_tiles == 0) continue;                      // an unknown tag: no rows, nothing to scan
     const int nseg = ch_main[u] * (kEpiWarps / 4);
-    int seg = (2 * units[u].entries + nseg - 1) / nseg;
+    int seg = (2 * entries[u] + nseg - 1) / nseg;
     if (seg < 12) seg = 12;
     TcGroupCta d{};
-    d.q0 = units[u].q0; d.nq = units[u].nq; d.tenant = G.tenant; d.tile0 = G.tile0; d.n_tiles = G.n_tiles;
-    d.list = G.list; d.seg = seg; d.cand0 = cand_entries;
-    for (int c = 0; c < ch_main[u]; ++c) { d.chunk = c; d.chunks = ch_main[u]; d.scale = 1; main->push_back(d); }
-    if (pre)
-      for (int c = 0; c < ch_pre[u]; ++c) { d.chunk = c; d.chunks = ch_pre[u]; d.scale = units[u].stride; pre->push_back(d); }
-    cand_entries += int64_t(kTileQ) * nseg * seg;
+    d.q0 = G.q0; d.nq = G.nq; d.tenant = G.tenant; d.tile0 = G.tile0; d.n_tiles = G.n_tiles;
+    d.list = G.list; d.seg = seg; d.cand0 = out->cand_entries;
+    for (int c = 0; c < ch_main[u]; ++c) { d.chunk = c; d.chunks = ch_main[u]; d.scale = 1; main.push_back(d); }
+    if (k > 0)
+      for (int c = 0; c < ch_pre[u]; ++c) { d.chunk = c; d.chunks = ch_pre[u]; d.scale = stride[u]; pre.push_back(d); }
+    out->cand_entries += int64_t(kTileQ) * nseg * seg;
   }
-  return cand_entries;
+  out->n_pre = int(pre.size());
+  out->n_main = int(main.size());
+  out->ctas.resize((pre.size() + main.size()) * sizeof(TcGroupCta));
+  if (!pre.empty()) memcpy(out->ctas.data(), pre.data(), pre.size() * sizeof(TcGroupCta));
+  if (!main.empty()) memcpy(out->ctas.data() + pre.size() * sizeof(TcGroupCta), main.data(), main.size() * sizeof(TcGroupCta));
 }
 
-int launch_tc_match_grouped(const GalleryWindow* s, const float* q, const std::vector<int32_t>& perm,
-                            const std::vector<TcTenantGroup>& groups, int k, float threshold, int64_t row_offset,
-                            int sm_count, int64_t* out_rows, float* out_scores, uint8_t* out_accept, cudaStream_t st) {
-  const int nq = int(perm.size());
-  const int dim = s->dim;
-  if (!s->plane8 || !s->master || s->rows <= 0 || s->rows > 0x7fffffff) {
-    set_error("tc_match_grouped: needs a non-empty unit store with an int8 plane and an fp32 master");
+static bool whole_unit_store(const GalleryWindow* s) {
+  return s->plane8 && s->master && s->row0 == 0 && s->rows <= 0x7fffffff;
+}
+
+int launch_tc_match_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
+                            const float* eps, int nq, const void* d_ctas, int n_pre, int n_main, int k, float threshold,
+                            int64_t row_offset, const TcRangeWs& w, int64_t* out_rows, float* out_scores,
+                            uint8_t* out_accept, cudaStream_t st) {
+  if (!whole_unit_store(s)) {
+    set_error("tc_match_grouped: needs the whole unit store with an int8 plane and an fp32 master");
     return FRG_ERR_UNSUPPORTED;
   }
-  // ---- plan: query tiles of at most kTileQ queries, never across tenants
-  std::vector<GroupUnit> units;
-  for (int g = 0; g < int(groups.size()); ++g)
-    for (int a = 0; a < groups[g].nq; a += kTileQ)
-      units.push_back(GroupUnit{&groups[g], groups[g].q0 + a, groups[g].nq - a < kTileQ ? groups[g].nq - a : kTileQ, 0, 0});
-  int dense_cap = 0;
-  for (GroupUnit& U : units) {
-    // the plan of a single-tenant match over the same tiles (tc_plan): pre-pass stride and candidate budget
-    TcPlan pl;
-    tc_plan(int64_t(U.src->n_tiles) * kTileR, dim, 1, k, sm_count, &pl, false, true);
-    U.stride = pl.stride;
-    U.entries = pl.stage_entries;
-    if (pl.stage_entries > dense_cap) dense_cap = pl.stage_entries;
-  }
-  std::vector<TcGroupCta> pre, main;
-  const int64_t cand_entries = plan_group_ctas(units, sm_count, &pre, &main);
-  if (dense_cap < 256) dense_cap = 256;
-  // ---- workspace (one stream-ordered allocation)
-  Carve c;
-  const size_t o_qs = c.take(size_t(nq) * dim * 4), o_qn = c.take(size_t(nq) * dim * 4), o_qi8 = c.take(size_t(nq) * dim);
-  const size_t o_eps = c.take(size_t(nq) * 4), o_step = c.take(size_t(nq) * 4), o_keys = c.take(size_t(nq) * kGroups * 8);
-  const size_t o_cnt = c.take(size_t(nq) * 4), o_flag = c.take(size_t(nq) * 4 + 12), o_floor = c.take(size_t(nq) * 4);
-  const size_t o_cand = c.take(size_t(cand_entries > 0 ? cand_entries : 1) * 8);
-  const size_t o_dense = c.take(size_t(nq) * dense_cap * 8);
-  const size_t o_rows = c.take(size_t(nq) * k * 8), o_sc = c.take(size_t(nq) * k * 4), o_acc = c.take(size_t(nq));
-  // the only host -> device copy of the call: [perm][tenant of each sorted query][pre-pass CTAs][filter CTAs]
-  std::vector<unsigned char> table;
-  const size_t t_perm = 0, t_ten = size_t(nq) * 4, t_pre = (t_ten + size_t(nq) * 4 + 15) & ~size_t(15);
-  const size_t t_main = t_pre + pre.size() * sizeof(TcGroupCta);
-  table.resize(t_main + main.size() * sizeof(TcGroupCta));
-  memcpy(table.data() + t_perm, perm.data(), size_t(nq) * 4);
-  for (const TcTenantGroup& G : groups)
-    for (int i = 0; i < G.nq; ++i) memcpy(table.data() + t_ten + size_t(G.q0 + i) * 4, &G.tenant, 4);
-  if (!pre.empty()) memcpy(table.data() + t_pre, pre.data(), pre.size() * sizeof(TcGroupCta));
-  if (!main.empty()) memcpy(table.data() + t_main, main.data(), main.size() * sizeof(TcGroupCta));
-  const size_t o_table = c.take(table.size());
-  unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
-  float* qs = reinterpret_cast<float*>(ws + o_qs);
-  float* qn = reinterpret_cast<float*>(ws + o_qn);
-  int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
-  float* eps = reinterpret_cast<float*>(ws + o_eps);
-  float* qstep = reinterpret_cast<float*>(ws + o_step);
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + o_keys);
-  int* cnt = reinterpret_cast<int*>(ws + o_cnt);
-  int* flagged = reinterpret_cast<int*>(ws + o_flag);
-  int* n_flagged = flagged + nq;
-  float* floor_v = reinterpret_cast<float*>(ws + o_floor);
-  int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
-  float* sscores = reinterpret_cast<float*>(ws + o_sc);
-  uint8_t* sacc = ws + o_acc;
-  const int32_t* dperm = reinterpret_cast<const int32_t*>(ws + o_table + t_perm);
-  const int32_t* dten = reinterpret_cast<const int32_t*>(ws + o_table + t_ten);
-  int rc = stage_upload(ws + o_table, table.data(), table.size(), st);
-  if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, dim, qs, st);
-  profile_begin(st, kStagePrep);
-  if (rc == FRG_OK)
-    rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, keys, cnt, n_flagged, st);
-  profile_end(st, 1);
+  const int dim = s->dim;
+  const TcGroupCta* ctas = static_cast<const TcGroupCta*>(d_ctas);
   CUtensorMap qm, gm;
-  if (rc == FRG_OK) rc = make_i8_maps(s, qi8, nq, &qm, &gm);
-  TcScanParams p = filter_params(s, dim, nq, eps, qstep, floor_v, reinterpret_cast<int2*>(ws + o_cand), cnt,
-                                 reinterpret_cast<int2*>(ws + o_dense), dense_cap);
-  p.tenant = -1; p.k = k; p.tile_scale = 1; p.group_key64 = keys;
+  FRG_CHECK(make_i8_maps(s, qi8, nq, &qm, &gm));
+  TcScanParams p = filter_params(s, dim, nq, eps, qstep, w.floor, w.cand, w.cand_total, w.dense, w.dense_cap);
+  p.tenant = -1; p.k = k; p.tile_scale = 1; p.group_key64 = w.keys;
   // 1. int8 pre-pass, 2. exact floor, 3. filter: every (query tile, chunk) of every tenant in one grid each
   profile_begin(st, kStagePrepass);
-  if (rc == FRG_OK && !pre.empty()) {
-    p.groups = reinterpret_cast<const TcGroupCta*>(ws + o_table + t_pre);
-    rc = launch_tc_scan<kModeGroupMax, true, false, true, true>(qm, gm, gm, p, int(pre.size()), 1, st);
+  if (n_pre > 0) {
+    p.groups = ctas;
+    FRG_CHECK((launch_tc_scan<kModeGroupMax, true, false, true, true>(qm, gm, gm, p, n_pre, 1, st)));
   }
   profile_end(st, 1);
   profile_begin(st, kStageFloor);
-  if (rc == FRG_OK) {
-    cudaError_t e = launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, keys, nq, k, dim, qn,
-                                  s->master, eps, floor_v);
-    if (e != cudaSuccess) rc = cuda_fail(e, "i8_floor_kernel", __FILE__, __LINE__);
-    else note_launch(nullptr);
-  }
+  cudaError_t e = launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, w.keys, nq, k, dim, qn,
+                                s->master, eps, w.floor);
+  if (e != cudaSuccess) return cuda_fail(e, "i8_floor_kernel", __FILE__, __LINE__);
+  note_launch(nullptr);
   profile_end(st, 1);
   profile_begin(st, kStageDominant);
-  if (rc == FRG_OK && !main.empty()) {
-    p.groups = reinterpret_cast<const TcGroupCta*>(ws + o_table + t_main);
-    rc = launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, int(main.size()), 1, st);
+  if (n_main > 0) {
+    p.groups = ctas + n_pre;
+    FRG_CHECK((launch_tc_scan<kModeFilter, true, false, true, true>(qm, gm, gm, p, n_main, 1, st)));
   }
   profile_end(st, 1);
   // 4. select + exact rescoring into the sorted scratch (the tenant filter was applied by the filter's tag check)
   profile_begin(st, kStageSelect);
-  if (rc == FRG_OK) {
-    const cudaError_t e = launch_select_rescore(reg_k(k), false, nq, st, p.dense, cnt, dense_cap, k, dim, qn, eps,
-                                                nullptr, dim, nullptr, qstep, s->master, 1, threshold, row_offset,
-                                                srows, sscores, sacc, flagged, n_flagged, XPush());
-    if (e != cudaSuccess) rc = cuda_fail(e, "select_rescore_kernel", __FILE__, __LINE__);
-    else note_launch(nullptr);
-  }
+  e = launch_select_rescore(reg_k(k), false, nq, st, w.dense, w.cand_total, w.dense_cap, k, dim, qn, eps, nullptr, dim,
+                            nullptr, qstep, s->master, 1, threshold, row_offset, out_rows, out_scores, out_accept,
+                            w.flagged, w.n_flagged, XPush());
+  if (e != cudaSuccess) return cuda_fail(e, "select_rescore_kernel", __FILE__, __LINE__);
+  note_launch(nullptr);
   profile_end(st, 1);
-  // 5. the queries whose candidates overflowed: exact scan of the whole store, each with its own tenant
-  profile_begin(st, kStageFallback);
-  if (rc == FRG_OK) {
-    ScanArgs a;
-    a.master = s->master; a.plane = nullptr; a.tags = s->tags; a.rows = s->rows; a.dim = dim;
-    a.qn = qn; a.nq = nq; a.k = k; a.metric = FRG_METRIC_COSINE; a.tenant = -1; a.sm_count = sm_count;
-    rc = launch_scan_f32_flagged_tenants(a, dten, flagged, n_flagged, row_offset, threshold, srows, sscores, sacc, st);
-  }
-  profile_end(st, 1);
-  if (rc == FRG_OK) rc = launch_scatter_results(srows, sscores, sacc, dperm, nq, k, out_rows, out_scores, out_accept, st);
-  if (rc == FRG_OK) { cudaError_t e = cudaGetLastError(); if (e != cudaSuccess) rc = cuda_fail(e, "grouped match", __FILE__, __LINE__); }
-  cudaError_t e = cudaFreeAsync(ws, st);
-  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
-  return rc;
+  return FRG_OK;
 }
 
 // ------------------------------------------------------------------------------------------ gallery self-join
@@ -1963,17 +1909,6 @@ join_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand_
   write_hits(hits, s_m, max_hits, q, row_offset, out_counts, out_rows, out_scores);
 }
 
-void tc_join_plan(const std::vector<TcTenantGroup>& tiles, int sm_count, std::vector<unsigned char>* table,
-                  int* n_ctas, int64_t* cand_entries) {
-  std::vector<GroupUnit> units;
-  for (const TcTenantGroup& t : tiles) units.push_back(GroupUnit{&t, t.q0, t.nq, kRangeBudget, 1});
-  std::vector<TcGroupCta> main;
-  *cand_entries = plan_group_ctas(units, sm_count, nullptr, &main);
-  *n_ctas = int(main.size());
-  table->resize(main.size() * sizeof(TcGroupCta));
-  if (!main.empty()) memcpy(table->data(), main.data(), table->size());
-}
-
 // The filter grid of launch_range_family for a GROUPED table: the single-CTA grid over n_ctas uploaded descriptors
 // (none when 0).  The self-join and per-query-tenant range search.
 static auto grouped_filter(const void* d_table, int n_ctas, cudaStream_t st) {
@@ -1984,10 +1919,6 @@ static auto grouped_filter(const void* d_table, int n_ctas, cudaStream_t st) {
     profile_end(st, n_ctas > 0 ? 1 : 0);
     return FRG_OK;
   };
-}
-
-static bool whole_unit_store(const GalleryWindow* s) {
-  return s->plane8 && s->master && s->row0 == 0 && s->rows <= 0x7fffffff;
 }
 
 int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
@@ -2017,32 +1948,6 @@ int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_
                              range_select_kernel, w.dense, w.cand_total, kRangeBudget, s->dim, qn, s->master,
                              threshold, strict ? 1 : 0, max_hits, row_offset, out_counts, out_rows, out_scores,
                              w.flagged, w.n_flagged);
-}
-
-// range results of sorted query i -> the caller's slot perm[i]
-__global__ void __launch_bounds__(256)
-scatter_range_kernel(const int64_t* __restrict__ counts, const int64_t* __restrict__ rows,
-                     const float* __restrict__ scores, const int32_t* __restrict__ perm, int nq, int max_hits,
-                     int64_t* __restrict__ out_counts, int64_t* __restrict__ out_rows, float* __restrict__ out_scores) {
-  pdl_wait();
-  pdl_trigger();
-  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i >= int64_t(nq) * max_hits) return;
-  const int q = int(i / max_hits), j = int(i - int64_t(q) * max_hits);
-  const int dst = __ldg(perm + q);
-  out_rows[size_t(dst) * max_hits + j] = rows[i];
-  out_scores[size_t(dst) * max_hits + j] = scores[i];
-  if (j == 0) out_counts[dst] = counts[q];
-}
-
-int launch_scatter_range(const int64_t* counts, const int64_t* rows, const float* scores, const int32_t* perm, int nq,
-                         int max_hits, int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
-  if (nq <= 0) return FRG_OK;
-  const int64_t n = int64_t(nq) * max_hits;
-  FRG_CUDA(launch_kernel(scatter_range_kernel, dim3(unsigned((n + 255) / 256)), dim3(256), 0, st, counts, rows, scores,
-                         perm, nq, max_hits, out_counts, out_rows, out_scores));
-  note_launch(nullptr);
-  return FRG_OK;
 }
 
 }  // namespace frg
