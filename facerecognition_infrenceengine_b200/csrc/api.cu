@@ -884,7 +884,8 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
   int n_list = 0;
   const int64_t plan_rows = tc_effective_rows(s, nq, st, &tile_list, &n_list);
   if (plan_rows < 0) return FRG_ERR_CUDA;
-  const int plan_dim = euclid ? -s->dim : s->dim;          // (negative: Euclidean plane, tc_plan)
+  TcPlan pl;
+  tc_plan(plan_rows, euclid ? -s->dim : s->dim, nq, k, sm_count, &pl, false, i8);
   const size_t qb_bytes = size_t(nq) * (s->dim + (euclid ? kEuclidQPad : 0)) * (i8 ? 1 : sizeof(__nv_bfloat16));
   Carve c;
   const size_t o_qn = c.take(size_t(nq) * s->dim * sizeof(float)), o_qb = c.take(qb_bytes);
@@ -892,7 +893,7 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
   const size_t o_qb2 = euclid ? c.take(qb_bytes) : 0;                            // the pre-pass (lower-bound) image
   // Euclidean: the bound coefficients [nq][4]; int8: the per-query step of the integer scores [nq]
   const size_t o_coef = euclid ? c.take(size_t(nq) * 4 * sizeof(float)) : i8 ? c.take(size_t(nq) * sizeof(float)) : 0;
-  const size_t o_tc = c.take(tc_workspace_bytes(plan_rows, plan_dim, nq, k, sm_count, i8));
+  const size_t o_tc = c.take(tc_workspace(nq, pl.cand_entries, pl.stage_entries, i8, nullptr, nullptr));
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
   float* qn = reinterpret_cast<float*>(ws + o_qn);
@@ -900,31 +901,29 @@ static int match_tc(const GalleryWindow* s, const float* q, int nq, int k, const
   float* eps = reinterpret_cast<float*>(ws + o_eps);
   __nv_bfloat16* qb2 = euclid ? reinterpret_cast<__nv_bfloat16*>(ws + o_qb2) : nullptr;
   float* coef = (euclid || i8) ? reinterpret_cast<float*>(ws + o_coef) : nullptr;
-  unsigned char* tc_ws = ws + o_tc;
-  int* flagged = nullptr; int* n_flagged = nullptr;
-  void* keys = nullptr; int* ct0 = nullptr; int* nf0 = nullptr;
-  tc_workspace_init_targets(plan_rows, plan_dim, nq, k, sm_count, tc_ws, &keys, &ct0, &nf0, i8);
+  TcWs tw;
+  tc_workspace(nq, pl.cand_entries, pl.stage_entries, i8, ws + o_tc, &tw);
+  uint32_t* keys32 = reinterpret_cast<uint32_t*>(tw.keys);      // the bf16 and Euclidean filters' 32-bit keys
   int8_t* qi8 = i8 ? reinterpret_cast<int8_t*>(qb) : nullptr;
   profile_begin(st, kStagePrep);
-  int rc = euclid ? launch_prepare_queries_euclid(q, nq, s->dim, s->gmax_bits, qn, qb, qb2, coef, eps,
-                                                  static_cast<uint32_t*>(keys), ct0, nf0, st)
-           : i8   ? launch_prepare_queries_i8(q, nq, s->dim, qn, qi8, coef, eps, s->gmax_bits,
-                                              static_cast<unsigned long long*>(keys), ct0, nf0, st)
-                  : launch_normalise_queries(q, nq, s->dim, !(p->flags & FRG_QUERY_PRENORMALISED), qn, qb,
-                                             static_cast<uint32_t*>(keys), ct0, nf0, st, eps, s->gmax_bits);
+  int rc = euclid ? launch_prepare_queries_euclid(q, nq, s->dim, s->gmax_bits, qn, qb, qb2, coef, eps, keys32,
+                                                  tw.cand_total, tw.n_flagged, st)
+           : i8   ? launch_prepare_queries_i8(q, nq, s->dim, qn, qi8, coef, eps, s->gmax_bits, tw.keys, tw.cand_total,
+                                              tw.n_flagged, st)
+                  : launch_normalise_queries(q, nq, s->dim, !(p->flags & FRG_QUERY_PRENORMALISED), qn, qb, keys32,
+                                             tw.cand_total, tw.n_flagged, st, eps, s->gmax_bits);
   profile_end(st, 1);
   if (rc == FRG_OK)
     rc = launch_tc_match(s, p->metric, qn, i8 ? nullptr : qb, eps, nq, k, p->tenant, rescore, p->threshold,
-                         p->row_offset, tc_ws, sm_count, tail.active ? tail.x : XPush(), out_rows, out_scores,
-                         out_accept, &flagged, &n_flagged, st, plan_rows, tile_list, n_list, qb2,
-                         euclid ? coef : nullptr, qi8, i8 ? coef : nullptr);
+                         p->row_offset, pl, tw, sm_count, tail.active ? tail.x : XPush(), out_rows, out_scores,
+                         out_accept, st, tile_list, n_list, qb2, euclid ? coef : nullptr, qi8, i8 ? coef : nullptr);
   if (rc == FRG_OK) {
     // queries whose candidate lists overflowed are redone exactly, inside the same enqueue
     ScanArgs a;
     a.master = s->master; a.plane = s->plane; a.tags = s->tags; a.rows = s->rows; a.dim = s->dim;
     a.qn = qn; a.nq = nq; a.k = k; a.metric = p->metric; a.tenant = p->tenant; a.sm_count = sm_count;
     profile_begin(st, kStageFallback);
-    rc = launch_scan_f32_flagged(a, flagged, n_flagged, p->row_offset, p->threshold,
+    rc = launch_scan_f32_flagged(a, tw.flagged, tw.n_flagged, p->row_offset, p->threshold,
                                  tail.active ? tail.x : XPush(), out_rows, out_scores, out_accept, st);
     profile_end(st, 1);
   }
@@ -1121,7 +1120,7 @@ static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     const size_t o_qs = c.take(size_t(nq) * dim * 4), o_qn = c.take(size_t(nq) * dim * 4), o_table = c.take(table.size());
     const size_t o_qi8 = c.take(size_t(nq) * dim), o_eps = c.take(size_t(nq) * 4), o_step = c.take(size_t(nq) * 4);
     const size_t o_rows = c.take(size_t(nq) * k * 8), o_sc = c.take(size_t(nq) * k * 4), o_acc = c.take(size_t(nq));
-    const size_t o_tc = c.take(tc_range_workspace(nq, plan.cand_entries, plan.dense_cap, nullptr, nullptr));
+    const size_t o_tc = c.take(tc_workspace(nq, plan.cand_entries, plan.dense_cap, true, nullptr, nullptr));
     unsigned char* ws = nullptr;
     FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
     float* qs = reinterpret_cast<float*>(ws + o_qs);
@@ -1134,8 +1133,8 @@ static int match_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     int64_t* srows = reinterpret_cast<int64_t*>(ws + o_rows);
     float* sscores = reinterpret_cast<float*>(ws + o_sc);
     uint8_t* sacc = ws + o_acc;
-    TcRangeWs tw;
-    tc_range_workspace(nq, plan.cand_entries, plan.dense_cap, ws + o_tc, &tw);
+    TcWs tw;
+    tc_workspace(nq, plan.cand_entries, plan.dense_cap, true, ws + o_tc, &tw);
     int rc = stage_upload(ws + o_table, table.data(), table.size(), st);
     if (rc == FRG_OK) rc = launch_gather_queries(q, dperm, nq, dim, qs, st);
     profile_begin(st, kStagePrep);
@@ -1568,23 +1567,25 @@ static int range_impl(frg_store* s, const float* q, int32_t nq, int32_t max_hits
     int n_list = 0;
     const int64_t plan_rows = tc_effective_rows(&w, nq, st, &tile_list, &n_list);
     if (plan_rows < 0) return FRG_ERR_CUDA;
-    const int64_t cand = tc_range_cand_entries(plan_rows, w.dim, nq, di.sm_count);
+    TcPlan pl;
+    tc_plan(plan_rows, w.dim, nq, 1, di.sm_count, &pl, true, true);
     const size_t o_qi8 = c.take(size_t(nq) * w.dim), o_eps = c.take(size_t(nq) * sizeof(float));
-    const size_t o_step = c.take(size_t(nq) * sizeof(float)), o_tc = c.take(tc_range_workspace(nq, cand, kRangeBudget, nullptr, nullptr));
+    const size_t o_step = c.take(size_t(nq) * sizeof(float));
+    const size_t o_tc = c.take(tc_workspace(nq, pl.cand_entries, pl.stage_entries, true, nullptr, nullptr));
     FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
     float* qn = reinterpret_cast<float*>(ws + o_qn);
     int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
     float* eps = reinterpret_cast<float*>(ws + o_eps);
     float* qstep = reinterpret_cast<float*>(ws + o_step);
-    TcRangeWs tw;
-    tc_range_workspace(nq, cand, kRangeBudget, ws + o_tc, &tw);
+    TcWs tw;
+    tc_workspace(nq, pl.cand_entries, pl.stage_entries, true, ws + o_tc, &tw);
     profile_begin(st, kStagePrep);
     rc = launch_prepare_queries_i8(q, nq, w.dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
                                    tw.n_flagged, st);
     profile_end(st, 1);
     if (rc == FRG_OK)
-      rc = launch_tc_range(&w, qn, qi8, qstep, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, tw,
-                           di.sm_count, out_counts, out_rows, out_scores, st, plan_rows, tile_list, n_list);
+      rc = launch_tc_range(&w, qn, qi8, qstep, eps, nq, max_hits, p->tenant, p->threshold, strict, row_offset, pl, tw,
+                           out_counts, out_rows, out_scores, st, tile_list, n_list);
     if (rc == FRG_OK) {
       a.qn = qn;
       profile_begin(st, kStageFallback);
@@ -1681,7 +1682,7 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
   size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_tc = 0;
   if (tc) {
     o_qi8 = c.take(size_t(nq) * dim); o_eps = c.take(size_t(nq) * 4); o_step = c.take(size_t(nq) * 4);
-    o_tc = c.take(tc_range_workspace(nq, plan.cand_entries, kRangeBudget, nullptr, nullptr));
+    o_tc = c.take(tc_workspace(nq, plan.cand_entries, kRangeBudget, true, nullptr, nullptr));
   }
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
@@ -1704,8 +1705,8 @@ static int range_tenants_impl(frg_store* s, const float* q, int32_t nq, int32_t 
     int8_t* qi8 = reinterpret_cast<int8_t*>(ws + o_qi8);
     float* eps = reinterpret_cast<float*>(ws + o_eps);
     float* qstep = reinterpret_cast<float*>(ws + o_step);
-    TcRangeWs tw;
-    tc_range_workspace(nq, plan.cand_entries, kRangeBudget, ws + o_tc, &tw);
+    TcWs tw;
+    tc_workspace(nq, plan.cand_entries, kRangeBudget, true, ws + o_tc, &tw);
     profile_begin(st, kStagePrep);
     if (rc == FRG_OK)
       rc = launch_prepare_queries_i8(qs, nq, dim, qn, qi8, qstep, eps, s->gmax_bits, tw.keys, tw.cand_total,
@@ -1897,12 +1898,12 @@ static int self_join_impl(frg_store* s, int64_t row0, int64_t n, int32_t max_hit
   size_t o_qi8 = 0, o_eps = 0, o_step = 0, o_tc = 0;
   if (use_tc) {
     o_qi8 = c.take(size_t(S) * dim); o_eps = c.take(size_t(S) * 4); o_step = c.take(size_t(S) * 4);
-    o_tc = c.take(tc_range_workspace(int(S), max_cand, kRangeBudget, nullptr, nullptr));
+    o_tc = c.take(tc_workspace(int(S), max_cand, kRangeBudget, true, nullptr, nullptr));
   }
   unsigned char* ws = nullptr;
   FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), c.off, st));
-  TcRangeWs tw{};
-  if (use_tc) tc_range_workspace(int(S), max_cand, kRangeBudget, ws + o_tc, &tw);
+  TcWs tw{};
+  if (use_tc) tc_workspace(int(S), max_cand, kRangeBudget, true, ws + o_tc, &tw);
   float* qn = reinterpret_cast<float*>(ws + o_qn);
   const int32_t* tile_end = reinterpret_cast<const int32_t*>(ws + o_table);
   a.qn = qn;

@@ -349,20 +349,50 @@ constexpr int kEuclidPad = 16;      // plane: one more 32-byte group of k (one U
 constexpr int kEuclidQPad = 64;     // query image: padded to a whole 128-byte swizzle row (the tile's k-block)
 constexpr float kEuclidNone = -3.0e38f;   // "no score yet" of the Euclidean filter (scores are unbounded below)
 int tc_supported(int dim, int metric, const char** why);
-// i8: the int8 filter of a unit store (64-bit group keys, per-query floor)
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool i8 = false);
-// keys: [nq][32] group keys, uint32 (bf16 filter) or uint64 (int8 filter)
-void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               void** keys, int** cand_total, int** n_flagged, bool i8 = false);
+
+// Candidate entries per query of a range-mode filter (range search and self-join; DESIGN.md section 7.3)
+constexpr int kRangeBudget = 4096;
+
+// The plan of one ungrouped tensor-core call over `rows` rows (the window's, or listed tiles x rows per tile): grid,
+// pre-pass sample and the sizes of its workspace.  dim < 0: Euclidean plane of |dim| columns.  range: no pre-pass and
+// kRangeBudget dense entries per query (range search); i8: the int8 filter of a unit store.
+struct TcPlan {
+  bool pair;              // CTA-pair kernels (F > 128)
+  bool fused;             // pre-pass folded into the filter kernel (probe tile + published group maxima)
+  int qtiles, stride, chunks_pre, chunks_main, kreg, seg;
+  int stage_entries;      // the dense width: dense list entries per query
+  int64_t cand_entries;   // candidate segment entries (int2): nq x chunks_main x (kEpiWarps / 4) x seg
+};
+void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range, bool i8);
+
+// The workspace of the filter behind every tensor-core call of nq queries (top-k, range search, one self-join slab, a
+// per-query-tenant batch).  The query prep resets keys, cand_total and n_flagged[0..2].
+struct TcWs {
+  unsigned long long* keys;   // [nq][32] group keys: uint64 (int8 filter), uint32 (bf16 and Euclidean filters)
+  int* cand_total;            // [nq] candidates per query
+  int* flagged;               // [nq] queries whose candidates overflowed, then their count, the fallback's ticket and
+                              // the fused kernel's probe-arrival counter
+  int* n_flagged;             // flagged + nq
+  float* floor;               // [nq] per-query float floor of the int8 filter (null otherwise)
+  int2* dense;                // [nq][dense_cap] packed candidates
+  int2* cand;                 // the filter's candidate segments
+  int dense_cap;
+};
+// Bytes of that workspace when the filter writes cand_entries segment entries (int2); with ws, its pieces in *out.
+// i8: 64-bit group keys and the floor.
+size_t tc_workspace(int nq, int64_t cand_entries, int dense_cap, bool i8, unsigned char* ws, TcWs* out);
+
 // metric cosine, int8 plane (s->plane8): qi8 / qstep / eps from launch_prepare_queries_i8, qb unused.
 // metric cosine, bf16 plane (bf16-only store): qb = [nq][dim] bf16 unit queries, eps[nq] per-query bounds.
 // metric euclidean: qb = [nq][dim + kEuclidQPad] augmented image, eps[nq] per-query bounds.
+// pl: tc_plan over the rows the call scans (tile_list: the listed tiles of a tenant-filtered call whose window is
+// mostly other tenants' rows, tc_effective_rows); w: tc_workspace of pl, its keys and counters reset by the query prep.
+// Queries whose candidates overflowed are left in (w.flagged, w.n_flagged) for launch_scan_f32_flagged.
 // push: the select stage sends every query's final top-k straight to all ranks (XPush::peer_bufs != null)
 int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const __nv_bfloat16* qb, const float* eps,
                     int nq, int k, int32_t tenant, bool rescore, float threshold, int64_t row_offset,
-                    unsigned char* ws, int sm_count, const XPush& push, int64_t* out_rows, float* out_scores,
-                    uint8_t* out_accept, int** flagged_out, int** n_flagged_out, cudaStream_t st,
-                    int64_t plan_rows, const int32_t* tile_list, int n_list,
+                    const TcPlan& pl, const TcWs& w, int sm_count, const XPush& push, int64_t* out_rows,
+                    float* out_scores, uint8_t* out_accept, cudaStream_t st, const int32_t* tile_list, int n_list,
                     const __nv_bfloat16* qb_prepass = nullptr, const float* coef = nullptr,
                     const int8_t* qi8 = nullptr, const float* qstep = nullptr);
 
@@ -396,26 +426,6 @@ int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, 
 // api.cu: host -> device copy through the per-thread pinned staging ring (pageable copy when larger than a slot)
 int stage_upload(void* dev, const void* host, size_t bytes, cudaStream_t st);
 
-// Candidate entries per query of a range-mode filter (range search and self-join; DESIGN.md section 7.3)
-constexpr int kRangeBudget = 4096;
-
-// tc_match.cu: the workspace of an int8 filter call without a top-k plan of its own (range search, one self-join slab,
-// a per-query-tenant batch) of nq queries
-struct TcRangeWs {
-  unsigned long long* keys;   // [nq][32] group keys (the query prep resets them)
-  int* cand_total;            // [nq] candidates per query
-  int* flagged;               // [nq] queries whose candidates overflowed, then their count and the fallback's ticket
-  int* n_flagged;             // flagged + nq
-  float* floor;               // [nq] threshold - eps[q]
-  int2* dense;                // [nq][dense_cap] packed candidates
-  int2* cand;                 // the filter's candidate segments
-  int dense_cap;              // kRangeBudget in range mode
-};
-// Bytes of that workspace when the filter writes cand_entries segment entries (int2); with ws, its pieces in *out.
-size_t tc_range_workspace(int nq, int64_t cand_entries, int dense_cap, unsigned char* ws, TcRangeWs* out);
-// the candidate segment entries of range search's filter over plan_rows rows (the grouped grid's: tc_group_plan)
-int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count);
-
 // tc_match.cu: top-k with a tenant per query (frg_match_tenants) on the int8 filter of a unit cosine store, over the
 // tenant-sorted batch: qn / qi8 / qstep / eps from launch_prepare_queries_i8 (which reset w's keys and counters),
 // d_ctas the uploaded descriptors of tc_group_plan (k >= 1; n_pre pre-pass, then n_main filter).  Pre-pass, floor,
@@ -423,17 +433,18 @@ int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count);
 // w.n_flagged) for launch_scan_f32_flagged_tenants.  s: the whole store.
 int launch_tc_match_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
                             const float* eps, int nq, const void* d_ctas, int n_pre, int n_main, int k, float threshold,
-                            int64_t row_offset, const TcRangeWs& w, int64_t* out_rows, float* out_scores,
+                            int64_t row_offset, const TcWs& w, int64_t* out_rows, float* out_scores,
                             uint8_t* out_accept, cudaStream_t st);
 
 // tc_match.cu: range search over a unit cosine store (frg_match_range).  The filter keeps every row with
 // S >= threshold - eps[q] (no pre-pass); range_select_kernel rescores each candidate exactly, keeps those that pass
-// (score >= threshold, '>' when strict), writes the first max_hits in gallery order and the count.  Queries whose
+// (score >= threshold, '>' when strict), writes the first max_hits in gallery order and the count.  pl: tc_plan in
+// range mode over the rows scanned (tile_list as in launch_tc_match); w: tc_workspace of pl.  Queries whose
 // candidates overflowed the plan are left in (w.flagged, w.n_flagged) for launch_range_scan's flagged mode.
 int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
                     int nq, int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset,
-                    const TcRangeWs& w, int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores,
-                    cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list);
+                    const TcPlan& pl, const TcWs& w, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                    cudaStream_t st, const int32_t* tile_list, int n_list);
 
 // scan_f32.cu: exact, counting range scan.  Pass 1: every warp owns a contiguous row range and counts its hits per
 // query; a per-query exclusive scan over the warp counts gives the total and each warp's output offset; pass 2: the
@@ -457,7 +468,7 @@ int launch_range_tenants_scan(const ScanArgs& a, const int32_t* q_tenant, const 
 // for launch_range_tenants_scan.  s: the whole store.
 int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
                             const float* eps, int nq, const void* d_table, int n_ctas, int max_hits, float threshold,
-                            bool strict, int64_t row_offset, const TcRangeWs& w, int64_t* out_counts,
+                            bool strict, int64_t row_offset, const TcWs& w, int64_t* out_counts,
                             int64_t* out_rows, float* out_scores, cudaStream_t st);
 
 // ---- gallery self-join (frg_self_join): the queries are the store's own rows qrow0 .. qrow0 + nq - 1 of one slab,
@@ -469,7 +480,7 @@ int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_
 // launch_join_scan.  s: the whole store.
 int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
                    int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
-                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcRangeWs& w,
+                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcWs& w,
                    int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st);
 // scan_f32.cu: exact, counting join scan (launch_range_scan's passes with the join rules).  a: the whole store, a.qn /
 // a.nq the slab's unit queries, a.tenant the tenant rule, cosine.  tile_end[u]: exclusive end row of query tile u's

@@ -315,6 +315,31 @@ __device__ __forceinline__ int sparse_row_list(const int32_t* __restrict__ tags,
   return n <= kSparseCap ? n : -1;
 }
 
+// The ticket-and-merge tail of both exact re-dos: the CTA that takes the last ticket (ctl[1]) folds every CTA's partial
+// lists of the nf flagged queries into their final top-k, one warp per query, and calls done(q) after each.
+template <int METRIC, int KMAX, typename Done>
+__device__ __forceinline__ void merge_flagged(int nf, const int* __restrict__ flagged, int* __restrict__ ctl,
+                                              int nq_total, int K, float threshold, int64_t row_offset,
+                                              const float* __restrict__ part_sc, const int32_t* __restrict__ part_ix,
+                                              int64_t* __restrict__ out_rows, float* __restrict__ out_scores,
+                                              uint8_t* __restrict__ out_accept, Done&& done) {
+  __shared__ int is_last;
+  if (nf == 0) return;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) is_last = atomicAdd(ctl + 1, 1) == int(gridDim.x) - 1;
+  __syncthreads();
+  if (!is_last) return;
+  __threadfence();
+  for (int slot = threadIdx.x >> 5; slot < nf; slot += kScanWarps) {
+    const int q = flagged[slot];
+    merge_one<int32_t, KMAX>(part_sc, part_ix, int(gridDim.x), nq_total, K, K, METRIC, threshold, row_offset,
+                             /*internal_euclid=*/METRIC == FRG_METRIC_EUCLIDEAN ? 1 : 0, slot, q, int64_t(nq_total) * K,
+                             int64_t(nq_total) * K, out_rows, out_scores, out_accept);
+    done(q);
+  }
+}
+
 // Exact re-do of the queries a tensor-core pass could not settle (candidate overflow).  The list
 // and its length live on the device; the kernel loops over it, so nothing waits for the host, and
 // the CTA that finishes last folds the per-CTA lists into the final results (ticket counter), so an
@@ -330,7 +355,6 @@ scan_f32_flagged_kernel(const ROW* __restrict__ master, const int32_t* __restric
   extern __shared__ unsigned char smem_raw[];
   float* l_sc = reinterpret_cast<float*>(smem_raw);
   int32_t* l_ix = reinterpret_cast<int32_t*>(l_sc + kScanWarps * QB * K);
-  __shared__ int is_last;
   __shared__ int32_t s_list[SPARSE ? kScanWarps : 1][SPARSE ? kSparseCap : 1];
   pdl_wait();             // the select kernel's list of flagged queries
   pdl_trigger();
@@ -347,18 +371,8 @@ scan_f32_flagged_kernel(const ROW* __restrict__ master, const int32_t* __restric
                                            part_ix, l_sc, l_ix, w_list, w_n);
     __syncthreads();
   }
-  if (nf == 0) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) is_last = atomicAdd(ctl + 1, 1) == int(gridDim.x) - 1;
-  __syncthreads();
-  if (!is_last) return;
-  __threadfence();
-  for (int slot = threadIdx.x >> 5; slot < nf; slot += kScanWarps) {
-    const int q = flagged[slot];
-    merge_one<int32_t, KMAX>(part_sc, part_ix, int(gridDim.x), nq_total, K, K, METRIC, threshold, row_offset,
-                             /*internal_euclid=*/METRIC == FRG_METRIC_EUCLIDEAN ? 1 : 0, slot, q, int64_t(nq_total) * K, int64_t(nq_total) * K, out_rows, out_scores,
-                             out_accept);
+  merge_flagged<METRIC, KMAX>(nf, flagged, ctl, nq_total, K, threshold, row_offset, part_sc, part_ix, out_rows,
+                              out_scores, out_accept, [&](int q) {
     if (x.peer_bufs) {
       // row-sharded gallery: the redone query's top-k is final now - send it to every rank (select skipped it)
       __syncwarp();                // lane 0's result stores are visible to the warp
@@ -369,7 +383,7 @@ scan_f32_flagged_kernel(const ROW* __restrict__ master, const int32_t* __restric
         xpush_slot(x, (x.rank + 1 + peer) % x.world, s_, out_rows[s_], out_scores[s_]);
       }
     }
-  }
+  });
 }
 
 // The exact re-do of scan_f32_flagged_kernel for a batch whose queries carry their own tenants (frg_match_tenants):
@@ -386,7 +400,6 @@ scan_f32_flagged_tenants_kernel(const float* __restrict__ master, const int32_t*
   extern __shared__ unsigned char smem_raw[];
   float* l_sc = reinterpret_cast<float*>(smem_raw);
   int32_t* l_ix = reinterpret_cast<int32_t*>(l_sc + kScanWarps * K);
-  __shared__ int is_last;
   pdl_wait();             // the select kernel's list of flagged queries
   pdl_trigger();
   const int nf = ctl[0];
@@ -401,66 +414,8 @@ scan_f32_flagged_tenants_kernel(const float* __restrict__ master, const int32_t*
                                           l_sc, l_ix);
     __syncthreads();
   }
-  if (nf == 0) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) is_last = atomicAdd(ctl + 1, 1) == int(gridDim.x) - 1;
-  __syncthreads();
-  if (!is_last) return;
-  __threadfence();
-  for (int slot = threadIdx.x >> 5; slot < nf; slot += kScanWarps)
-    merge_one<int32_t, KMAX>(part_sc, part_ix, int(gridDim.x), nq_total, K, K, FRG_METRIC_COSINE, threshold, row_offset,
-                             0, slot, flagged[slot], int64_t(nq_total) * K, int64_t(nq_total) * K, out_rows, out_scores,
-                             out_accept);
-}
-
-template <int NJ, int KMAX>
-static int launch_flagged_tenants_k(const ScanArgs& a, int grid, const int32_t* q_tenant, const int* flagged, int* ctl,
-                                    float threshold, int64_t row_offset, float* ps, int32_t* pi, int64_t* out_rows,
-                                    float* out_scores, uint8_t* out_accept, cudaStream_t st) {
-  const size_t smem = size_t(kScanWarps) * a.k * (sizeof(float) + sizeof(int32_t));
-  auto kern = scan_f32_flagged_tenants_kernel<NJ, KMAX>;
-  FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-  FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn, a.nq,
-                         q_tenant, flagged, ctl, a.k, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept));
-  note_launch(nullptr);
-  return FRG_OK;
-}
-
-template <int NJ>
-static int launch_flagged_tenants_t(const ScanArgs& a, int grid, const int32_t* q_tenant, const int* flagged, int* ctl,
-                                    float threshold, int64_t row_offset, float* ps, int32_t* pi, int64_t* out_rows,
-                                    float* out_scores, uint8_t* out_accept, cudaStream_t st) {
-#define FRG_FT(KM) return launch_flagged_tenants_k<NJ, KM>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, \
-                                                            pi, out_rows, out_scores, out_accept, st)
-  if (a.k == 1) FRG_FT(1);
-  if (a.k <= 4) FRG_FT(4);
-  if (a.k <= 8) FRG_FT(8);
-  FRG_FT(16);
-#undef FRG_FT
-}
-
-int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, const int* flagged, int* ctl,
-                                    int64_t row_offset, float threshold, int64_t* out_rows, float* out_scores,
-                                    uint8_t* out_accept, cudaStream_t st) {
-  if (a.rows <= 0 || a.nq <= 0) return FRG_OK;
-  if (!a.master || a.metric != FRG_METRIC_COSINE) { set_error("flagged scan: per-query tenants need a cosine master"); return FRG_ERR_UNSUPPORTED; }
-  const int grid = a.sm_count;
-  const size_t n_part = size_t(grid) * a.nq * a.k;
-  unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_part * 8, st));
-  float* ps = reinterpret_cast<float*>(ws);
-  int32_t* pi = reinterpret_cast<int32_t*>(ps + n_part);
-  int rc;
-  switch (a.dim) {
-    case 128: rc = launch_flagged_tenants_t<1>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept, st); break;
-    case 256: rc = launch_flagged_tenants_t<2>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept, st); break;
-    case 512: rc = launch_flagged_tenants_t<4>(a, grid, q_tenant, flagged, ctl, threshold, row_offset, ps, pi, out_rows, out_scores, out_accept, st); break;
-    default: set_error("flagged scan: dim %d not built", a.dim); rc = FRG_ERR_UNSUPPORTED; break;
-  }
-  cudaError_t e = cudaFreeAsync(ws, st);
-  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
-  return rc;
+  merge_flagged<FRG_METRIC_COSINE, KMAX>(nf, flagged, ctl, nq_total, K, threshold, row_offset, part_sc, part_ix,
+                                         out_rows, out_scores, out_accept, [](int) {});
 }
 
 static int scan_grid(const ScanArgs& a) {
@@ -552,52 +507,42 @@ int launch_scan_f32(const ScanArgs& a, void* workspace, int64_t row_offset, floa
                           out_accept, st);
 }
 
-template <int NJ, int QB, int KMAX>
-static int launch_flagged_k(const ScanArgs& a, int grid, const int* flagged, int* ctl, float threshold,
-                            int64_t row_offset, float* ps, int32_t* pi, const XPush& push, int64_t* out_rows,
-                            float* out_scores, uint8_t* out_accept, cudaStream_t st) {
+// The launch of an exact re-do (both entry points below): the partial lists of grid = sm_count CTAs, sized for the
+// worst case (every query flagged), allocated and freed on the stream; dim -> NJ; k -> KMAX; then
+// pick(NJ, KMAX, ps, pi, launch) names the kernel instance and calls launch(kernel, args...) once, which sets the
+// carveout and launches grid CTAs with QB queries' lists of k entries per warp in shared memory.
+template <int QB, typename Pick>
+static int launch_flagged_redo(const ScanArgs& a, cudaStream_t st, Pick&& pick) {
+  const int grid = a.sm_count;
+  const size_t n_part = size_t(grid) * a.nq * a.k;
+  unsigned char* ws = nullptr;
+  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_part * 8, st));
+  float* ps = reinterpret_cast<float*>(ws);
+  int32_t* pi = reinterpret_cast<int32_t*>(ps + n_part);
   const size_t smem = size_t(kScanWarps) * QB * a.k * (sizeof(float) + sizeof(int32_t));
-  // a tenant-filtered call whose queries overflowed: the tenant's rows are concentrated inside a wide window
-  // (DESIGN.md section 4.4) - read the tags first and fetch only that tenant's rows
-  if (a.master && a.metric == FRG_METRIC_COSINE && a.tenant >= 0) {
-    auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_COSINE, KMAX, float, true>;
+  auto launch = [&](auto kern, auto&&... args) -> int {
     FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn,
-                           a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
-                           out_accept, push));
-  } else if (a.master && a.metric == FRG_METRIC_EUCLIDEAN) {
-    auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_EUCLIDEAN, KMAX, float, false>;
-    FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn,
-                           a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
-                           out_accept, push));
-  } else if (a.master) {
-    auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_COSINE, KMAX, float, false>;
-    FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.master, a.tags, a.rows, a.qn,
-                           a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
-                           out_accept, push));
-  } else {
-    // bf16-only store: the exact re-do reads the scan plane (fp32 query x bf16 row, fp32 accumulation)
-    auto kern = scan_f32_flagged_kernel<NJ, QB, FRG_METRIC_COSINE, KMAX, __nv_bfloat16, false>;
-    FRG_CUDA(func_attr_once(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, a.plane, a.tags, a.rows, a.qn,
-                           a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi, out_rows, out_scores,
-                           out_accept, push));
+    FRG_CUDA(launch_kernel(kern, dim3(grid), dim3(kScanWarps * 32), smem, st, args...));
+    note_launch(nullptr);
+    FRG_CUDA(cudaGetLastError());
+    return FRG_OK;
+  };
+  auto by_k = [&](auto nj) -> int {
+    if (a.k == 1) return pick(nj, std::integral_constant<int, 1>(), ps, pi, launch);
+    if (a.k <= 4) return pick(nj, std::integral_constant<int, 4>(), ps, pi, launch);
+    if (a.k <= 8) return pick(nj, std::integral_constant<int, 8>(), ps, pi, launch);
+    return pick(nj, std::integral_constant<int, 16>(), ps, pi, launch);
+  };
+  int rc;
+  switch (a.dim) {
+    case 128: rc = by_k(std::integral_constant<int, 1>()); break;
+    case 256: rc = by_k(std::integral_constant<int, 2>()); break;
+    case 512: rc = by_k(std::integral_constant<int, 4>()); break;
+    default: set_error("flagged scan: dim %d not built", a.dim); rc = FRG_ERR_UNSUPPORTED; break;
   }
-  note_launch(nullptr);
-  FRG_CUDA(cudaGetLastError());
-  return FRG_OK;
-}
-
-template <int NJ, int QB>
-static int launch_flagged_t(const ScanArgs& a, int grid, const int* flagged, int* ctl, float threshold,
-                            int64_t row_offset, float* ps, int32_t* pi, const XPush& push, int64_t* out_rows,
-                            float* out_scores, uint8_t* out_accept, cudaStream_t st) {
-  if (a.k == 1) return launch_flagged_k<NJ, QB, 1>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st);
-  if (a.k <= 4) return launch_flagged_k<NJ, QB, 4>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st);
-  if (a.k <= 8) return launch_flagged_k<NJ, QB, 8>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st);
-  return launch_flagged_k<NJ, QB, 16>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st);
+  cudaError_t e = cudaFreeAsync(ws, st);
+  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
+  return rc;
 }
 
 // ctl: device int[2] = {number of flagged queries, ticket counter (0)}
@@ -605,22 +550,34 @@ int launch_scan_f32_flagged(const ScanArgs& a, const int* flagged, int* ctl, int
                             float threshold, const XPush& push, int64_t* out_rows, float* out_scores,
                             uint8_t* out_accept, cudaStream_t st) {
   if (a.rows <= 0 || a.nq <= 0) return FRG_OK;
-  const int grid = a.sm_count;       // partial lists are sized for the worst case (every query flagged)
-  const size_t n_part = size_t(grid) * a.nq * a.k;
-  unsigned char* ws = nullptr;
-  FRG_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), n_part * 8, st));
-  float* ps = reinterpret_cast<float*>(ws);
-  int32_t* pi = reinterpret_cast<int32_t*>(ps + n_part);
-  int rc;
-  switch (a.dim) {
-    case 128: rc = launch_flagged_t<1, 4>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st); break;
-    case 256: rc = launch_flagged_t<2, 4>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st); break;
-    case 512: rc = launch_flagged_t<4, 4>(a, grid, flagged, ctl, threshold, row_offset, ps, pi, push, out_rows, out_scores, out_accept, st); break;
-    default: set_error("flagged scan: dim %d not built", a.dim); rc = FRG_ERR_UNSUPPORTED; break;
-  }
-  cudaError_t e = cudaFreeAsync(ws, st);
-  if (rc == FRG_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync", __FILE__, __LINE__);
-  return rc;
+  return launch_flagged_redo<4>(a, st, [&](auto nj, auto kmax, float* ps, int32_t* pi, auto& launch) {
+    constexpr int NJ = decltype(nj)::value, KMAX = decltype(kmax)::value;
+    auto go = [&](auto kern, const auto* rows) {
+      return launch(kern, rows, a.tags, a.rows, a.qn, a.nq, flagged, ctl, a.k, a.tenant, threshold, row_offset, ps, pi,
+                    out_rows, out_scores, out_accept, push);
+    };
+    // a tenant-filtered call whose queries overflowed: the tenant's rows are concentrated inside a wide window
+    // (DESIGN.md section 4.4) - read the tags first and fetch only that tenant's rows
+    if (a.master && a.metric == FRG_METRIC_COSINE && a.tenant >= 0)
+      return go(scan_f32_flagged_kernel<NJ, 4, FRG_METRIC_COSINE, KMAX, float, true>, a.master);
+    if (a.master && a.metric == FRG_METRIC_EUCLIDEAN)
+      return go(scan_f32_flagged_kernel<NJ, 4, FRG_METRIC_EUCLIDEAN, KMAX, float, false>, a.master);
+    if (a.master) return go(scan_f32_flagged_kernel<NJ, 4, FRG_METRIC_COSINE, KMAX, float, false>, a.master);
+    // bf16-only store: the exact re-do reads the scan plane (fp32 query x bf16 row, fp32 accumulation)
+    return go(scan_f32_flagged_kernel<NJ, 4, FRG_METRIC_COSINE, KMAX, __nv_bfloat16, false>, a.plane);
+  });
+}
+
+int launch_scan_f32_flagged_tenants(const ScanArgs& a, const int32_t* q_tenant, const int* flagged, int* ctl,
+                                    int64_t row_offset, float threshold, int64_t* out_rows, float* out_scores,
+                                    uint8_t* out_accept, cudaStream_t st) {
+  if (a.rows <= 0 || a.nq <= 0) return FRG_OK;
+  if (!a.master || a.metric != FRG_METRIC_COSINE) { set_error("flagged scan: per-query tenants need a cosine master"); return FRG_ERR_UNSUPPORTED; }
+  return launch_flagged_redo<1>(a, st, [&](auto nj, auto kmax, float* ps, int32_t* pi, auto& launch) {
+    return launch(scan_f32_flagged_tenants_kernel<decltype(nj)::value, decltype(kmax)::value>, a.master, a.tags, a.rows,
+                  a.qn, a.nq, q_tenant, flagged, ctl, a.k, threshold, row_offset, ps, pi, out_rows, out_scores,
+                  out_accept);
+  });
 }
 
 

@@ -1219,13 +1219,6 @@ int tc_supported(int dim, int metric, const char** why) {
   return 1;
 }
 
-struct TcPlan {
-  bool pair;              // CTA-pair kernels (F > 128)
-  bool fused;             // pre-pass folded into the filter kernel (probe tile + published group maxima)
-  int qtiles, stride, chunks_pre, chunks_main, kreg, seg, stage_entries;
-  size_t off_keys, off_cnt, off_cand, off_dense, off_flag, off_floor, total;
-};
-
 // FUSED: share of every CTA's chunk probed before the floor is derived (1/64; larger probes, up to 1/8, measured no
 // faster, DESIGN.md section 4.2)
 constexpr int kProbeDiv = 64;
@@ -1239,7 +1232,7 @@ static int reg_k(int k) { return k == 1 ? 1 : (k <= 4 ? 4 : (k <= 8 ? 8 : 16)); 
 // Range search (range = true): no pre-pass, and a fixed dense list of kRangeBudget entries per query instead of one
 // sized from k (DESIGN.md section 7.3).
 // i8: the int8 filter - pre-pass at most every 16th tile, floor from i8_floor_kernel, never fused.
-static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range = false, bool i8 = false) {
+void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* pl, bool range, bool i8) {
   const bool euclid_plane = dim < 0;
   pl->qtiles = (nq + kTileQ - 1) / kTileQ;
   pl->pair = tc_uses_pairs(nq);
@@ -1303,14 +1296,7 @@ static void tc_plan(int64_t rows, int dim, int nq, int k, int sm_count, TcPlan* 
   int seg = (2 * stage_entries + nseg - 1) / nseg;
   if (seg < 12) seg = 12;
   pl->seg = seg;
-  Carve c;
-  pl->off_keys = c.take(size_t(nq) * kGroups * (i8 ? 8 : 4));
-  pl->off_cnt = c.take(size_t(nq) * 4);
-  pl->off_cand = c.take(size_t(nq) * nseg * seg * 8);
-  pl->off_dense = c.take(size_t(nq) * stage_entries * 8);
-  pl->off_flag = c.take(size_t(nq) * 4 + 12);    // flagged[nq], count, ticket, probe-arrival counter
-  pl->off_floor = c.take(i8 ? size_t(nq) * 4 : 0);
-  pl->total = c.off;
+  pl->cand_entries = int64_t(nq) * nseg * seg;
 }
 
 template <int MODE, bool MASKED, bool PAIR, bool I8, bool GROUPED = false>
@@ -1362,33 +1348,11 @@ int64_t tc_effective_rows(const GalleryWindow* s, int nq, cudaStream_t st, const
   return int64_t(n) * gran;
 }
 
-size_t tc_workspace_bytes(int64_t rows, int dim, int nq, int k, int sm_count, bool i8) {
-  TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl, false, i8);
-  return pl.total;
-}
-
-// the pieces of the workspace the query-prep kernel initialises (group keys := "nothing seen", counters := 0)
-void tc_workspace_init_targets(int64_t rows, int dim, int nq, int k, int sm_count, unsigned char* ws,
-                               void** keys, int** cand_total, int** n_flagged, bool i8) {
-  TcPlan pl;
-  tc_plan(rows, dim, nq, k, sm_count, &pl, false, i8);
-  *keys = ws + pl.off_keys;
-  *cand_total = reinterpret_cast<int*>(ws + pl.off_cnt);
-  *n_flagged = reinterpret_cast<int*>(ws + pl.off_flag) + nq;
-}
-
-int64_t tc_range_cand_entries(int64_t plan_rows, int dim, int nq, int sm_count) {
-  TcPlan pl;
-  tc_plan(plan_rows, dim, nq, 1, sm_count, &pl, true, true);
-  return int64_t(nq) * pl.chunks_main * (kEpiWarps / 4) * pl.seg;
-}
-
-size_t tc_range_workspace(int nq, int64_t cand_entries, int dense_cap, unsigned char* ws, TcRangeWs* out) {
+size_t tc_workspace(int nq, int64_t cand_entries, int dense_cap, bool i8, unsigned char* ws, TcWs* out) {
   Carve c;
-  const size_t o_keys = c.take(size_t(nq) * kGroups * 8), o_cnt = c.take(size_t(nq) * 4);
+  const size_t o_keys = c.take(size_t(nq) * kGroups * (i8 ? 8 : 4)), o_cnt = c.take(size_t(nq) * 4);
   const size_t o_flag = c.take(size_t(nq) * 4 + 12);     // flagged[nq], count, ticket, probe-arrival counter
-  const size_t o_floor = c.take(size_t(nq) * 4), o_dense = c.take(size_t(nq) * dense_cap * 8);
+  const size_t o_floor = i8 ? c.take(size_t(nq) * 4) : 0, o_dense = c.take(size_t(nq) * dense_cap * 8);
   const size_t o_cand = c.take(size_t(cand_entries) * 8);
   if (ws) {
     out->dense_cap = dense_cap;
@@ -1396,7 +1360,7 @@ size_t tc_range_workspace(int nq, int64_t cand_entries, int dense_cap, unsigned 
     out->cand_total = reinterpret_cast<int*>(ws + o_cnt);
     out->flagged = reinterpret_cast<int*>(ws + o_flag);
     out->n_flagged = out->flagged + nq;
-    out->floor = reinterpret_cast<float*>(ws + o_floor);
+    out->floor = i8 ? reinterpret_cast<float*>(ws + o_floor) : nullptr;
     out->dense = reinterpret_cast<int2*>(ws + o_dense);
     out->cand = reinterpret_cast<int2*>(ws + o_cand);
   }
@@ -1448,14 +1412,12 @@ static cudaError_t launch_select_rescore(int kreg, bool euclid, int nq, cudaStre
   return euclid ? by_k(std::true_type()) : by_k(std::false_type());
 }
 
-// qn / qb: normalised fp32 queries and their bf16 image [nq][dim]; ws: tc_workspace_bytes() of scratch.
-// Leaves the overflowed queries in (flagged, n_flagged) for the caller's exact fallback pass.
+// qn / qb: normalised fp32 queries and their bf16 image [nq][dim].
 int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const __nv_bfloat16* qb, const float* eps,
                     int nq, int k, int32_t tenant, bool rescore, float threshold, int64_t row_offset,
-                    unsigned char* ws, int sm_count, const XPush& push, int64_t* out_rows, float* out_scores,
-                    uint8_t* out_accept, int** flagged_out, int** n_flagged_out, cudaStream_t st,
-                    int64_t plan_rows, const int32_t* tile_list, int n_list, const __nv_bfloat16* qb_prepass,
-                    const float* coef, const int8_t* qi8, const float* qstep) {
+                    const TcPlan& pl, const TcWs& w, int sm_count, const XPush& push, int64_t* out_rows,
+                    float* out_scores, uint8_t* out_accept, cudaStream_t st, const int32_t* tile_list, int n_list,
+                    const __nv_bfloat16* qb_prepass, const float* coef, const int8_t* qi8, const float* qstep) {
   const bool euclid = metric == FRG_METRIC_EUCLIDEAN;
   const bool i8 = s->plane8 != nullptr;
   if (euclid && (!qb_prepass || !coef)) { set_error("tc_match: the Euclidean filter needs both query images"); return FRG_ERR_INVALID; }
@@ -1466,18 +1428,6 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   // columns of the query tile: dim, or dim + kEuclidQPad (its last k-block meets the plane's 16-column pad block)
   const int kdim = euclid ? s->dim + kEuclidQPad : s->dim;
   const size_t pitch = i8 ? size_t(s->dim) : size_t(s->plane_dim) * 2;
-  // (tile_list: a tenant-filtered call whose window is mostly other tenants' rows walks only the tiles that hold
-  // rows of the tenant; everything is planned for plan_rows = listed tiles x rows per tile)
-  TcPlan pl;
-  tc_plan(plan_rows, euclid ? -s->dim : s->dim, nq, k, sm_count, &pl, false, i8);
-  uint32_t* keys = reinterpret_cast<uint32_t*>(ws + pl.off_keys);
-  int* cnt = reinterpret_cast<int*>(ws + pl.off_cnt);
-  int2* cand = reinterpret_cast<int2*>(ws + pl.off_cand);
-  int2* dense = reinterpret_cast<int2*>(ws + pl.off_dense);
-  int* flagged = reinterpret_cast<int*>(ws + pl.off_flag);
-  int* n_flagged = flagged + nq;
-  *flagged_out = flagged;
-  *n_flagged_out = n_flagged;
   const bool masked = tenant >= 0 || s->maybe_dead;
 
   CUtensorMap qm, qm_pre, gm_full, pm;
@@ -1492,16 +1442,15 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   if (euclid) FRG_CHECK(make_map(&pm, s->plane + s->dim, kEuclidPad, s->rows, pitch, kTileR, kEuclidPad));
   else pm = gm_full;                                                          // never dereferenced (p.pad == 0)
 
-  TcScanParams p = filter_params(s, kdim, nq, eps, i8 ? qstep : nullptr,
-                                 i8 ? reinterpret_cast<float*>(ws + pl.off_floor) : nullptr, cand, cnt, dense,
-                                 pl.stage_entries);
+  TcScanParams p = filter_params(s, kdim, nq, eps, i8 ? qstep : nullptr, w.floor, w.cand, w.cand_total, w.dense,
+                                 w.dense_cap);
   if (euclid) { p.none_score = kEuclidNone; p.pad = 1; }
   p.tile_list = tile_list; p.n_list = n_list;
-  p.tenant = tenant; p.group_key = keys; p.k = k; p.seg = pl.seg;
+  p.tenant = tenant; p.group_key = reinterpret_cast<uint32_t*>(w.keys); p.k = k; p.seg = pl.seg;
   int rc;
   if (i8) {
     // 1. int8 pre-pass over the sampled tiles: (s32 product, row) of every row group's best sampled row
-    p.group_key64 = reinterpret_cast<unsigned long long*>(ws + pl.off_keys);
+    p.group_key64 = w.keys;
     p.tile_scale = pl.stride;
     profile_begin(st, kStagePrepass);
     FRG_CHECK((launch_tc_scan_m<kModeGroupMax, true>(masked, pl.pair, qm, gm_full, gm_full, p, pl.qtiles, pl.chunks_pre, st)));
@@ -1509,7 +1458,7 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
     // 2. exact floor e_k - eps from the k best group winners
     profile_begin(st, kStageFloor);
     FRG_CUDA(launch_kernel(i8_floor_kernel, dim3((nq + 3) / 4), dim3(128), 0, st, p.group_key64, nq, k, s->dim,
-                           qn, s->master, eps, const_cast<float*>(p.floor)));
+                           qn, s->master, eps, w.floor));
     note_launch(nullptr);
     profile_end(st, 1);
     // 3. filter over the whole plane against the integer floor
@@ -1523,7 +1472,7 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
     // what all CTAs published, filters the rest of its chunk and finally the probe tile itself
     p.tile_scale = 1;
     p.probe_div = kProbeDiv;
-    p.arrive = n_flagged + 2;
+    p.arrive = w.n_flagged + 2;
     {
       // the first wave holds min(all CTAs, one per SM): later waves find the counter already there
       const int ctas = pl.qtiles * pl.chunks_main;
@@ -1548,9 +1497,10 @@ int launch_tc_match(const GalleryWindow* s, int metric, const float* qn, const _
   }
   // 3. select + exact rescoring
   profile_begin(st, kStageSelect);
-  FRG_CUDA(launch_select_rescore(pl.kreg, euclid, nq, st, dense, cnt, pl.stage_entries, k, s->dim, qn, eps, s->plane,
-                                 s->plane_dim, coef, i8 ? qstep : nullptr, s->master, rescore ? 1 : 0, threshold,
-                                 row_offset, out_rows, out_scores, out_accept, flagged, n_flagged, push));
+  FRG_CUDA(launch_select_rescore(pl.kreg, euclid, nq, st, w.dense, w.cand_total, w.dense_cap, k, s->dim, qn, eps,
+                                 s->plane, s->plane_dim, coef, i8 ? qstep : nullptr, s->master, rescore ? 1 : 0,
+                                 threshold, row_offset, out_rows, out_scores, out_accept, w.flagged, w.n_flagged,
+                                 push));
   note_launch(nullptr);
   FRG_CUDA(cudaGetLastError());
   profile_end(st, 1);
@@ -1658,7 +1608,7 @@ range_select_kernel(const int2* __restrict__ dense, const int* __restrict__ cand
 // buffer in shared memory).
 template <typename Filter, typename... KArgs, typename... Args>
 static int launch_range_family(const GalleryWindow* s, const int8_t* qi8, const float* qstep, const float* eps, int nq,
-                               float threshold, const TcRangeWs& w, cudaStream_t st, Filter filter,
+                               float threshold, const TcWs& w, cudaStream_t st, Filter filter,
                                void (*select)(KArgs...), Args&&... select_args) {
   CUtensorMap qm, gm;
   FRG_CHECK(make_i8_maps(s, qi8, nq, &qm, &gm));
@@ -1684,11 +1634,9 @@ static int launch_range_family(const GalleryWindow* s, const int8_t* qi8, const 
 
 int launch_tc_range(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
                     int nq, int max_hits, int32_t tenant, float threshold, bool strict, int64_t row_offset,
-                    const TcRangeWs& w, int sm_count, int64_t* out_counts, int64_t* out_rows, float* out_scores,
-                    cudaStream_t st, int64_t plan_rows, const int32_t* tile_list, int n_list) {
+                    const TcPlan& pl, const TcWs& w, int64_t* out_counts, int64_t* out_rows, float* out_scores,
+                    cudaStream_t st, const int32_t* tile_list, int n_list) {
   if (!s->plane8) { set_error("tc_range: the store has no int8 scan plane"); return FRG_ERR_UNSUPPORTED; }
-  TcPlan pl;
-  tc_plan(plan_rows, s->dim, nq, 1, sm_count, &pl, true, true);
   const bool masked = tenant >= 0 || s->maybe_dead;
   // the ungrouped grid, in the pair form from two query tiles on
   auto filter = [&](const CUtensorMap& qm, const CUtensorMap& gm, TcScanParams& p) {
@@ -1825,7 +1773,7 @@ static bool whole_unit_store(const GalleryWindow* s) {
 
 int launch_tc_match_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
                             const float* eps, int nq, const void* d_ctas, int n_pre, int n_main, int k, float threshold,
-                            int64_t row_offset, const TcRangeWs& w, int64_t* out_rows, float* out_scores,
+                            int64_t row_offset, const TcWs& w, int64_t* out_rows, float* out_scores,
                             uint8_t* out_accept, cudaStream_t st) {
   if (!whole_unit_store(s)) {
     set_error("tc_match_grouped: needs the whole unit store with an int8 plane and an fp32 master");
@@ -1923,7 +1871,7 @@ static auto grouped_filter(const void* d_table, int n_ctas, cudaStream_t st) {
 
 int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep, const float* eps,
                    int nq, const void* d_table, int n_ctas, int64_t qrow0, int32_t tenant, bool same_tag,
-                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcRangeWs& w,
+                   float threshold, bool strict, int max_hits, int64_t row_offset, const TcWs& w,
                    int64_t* out_counts, int64_t* out_rows, float* out_scores, cudaStream_t st) {
   if (!whole_unit_store(s)) {
     set_error("tc_join: needs the whole unit store with an int8 plane and an fp32 master");
@@ -1938,7 +1886,7 @@ int launch_tc_join(const GalleryWindow* s, const float* qn, const int8_t* qi8, c
 // ------------------------------------------------------------------------------------------ per-query-tenant range search
 int launch_tc_range_grouped(const GalleryWindow* s, const float* qn, const int8_t* qi8, const float* qstep,
                             const float* eps, int nq, const void* d_table, int n_ctas, int max_hits, float threshold,
-                            bool strict, int64_t row_offset, const TcRangeWs& w, int64_t* out_counts,
+                            bool strict, int64_t row_offset, const TcWs& w, int64_t* out_counts,
                             int64_t* out_rows, float* out_scores, cudaStream_t st) {
   if (!whole_unit_store(s)) {
     set_error("tc_range_grouped: needs the whole unit store with an int8 plane and an fp32 master");
